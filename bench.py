@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native basetype core (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2|C3|C4|C5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2|C3|C4|C5] [--impl ours|reference] [--dump-outputs DIR]
 
 metric  : sample-sites/s of the BaseType core (likelihoods, EM, LRT, QUAL, strand-bias Fisher)
 workload: N = 1: BASELINE.json configs[1] = synthetic 1,000 samples x 1 Mb at 0.1x ("C2", SURVEY.md 8d).
@@ -21,6 +21,8 @@ roofline: algorithmic bytes S*(3N+128) per step / average step time (all kernels
 configs : N = 1 only: the other BASELINE.json shapes (C3, C4 shard shape, C5 in both EM abs modes), each with value, roofline,
           per-kernel times and the reference CPU baseline on a sub-range of >= 1e9 sample-sites of the same planes.
 cpu_baseline: the UNMODIFIED reference (oracle/_ref/libbvref.so: BaseType ctor + lrt() + strand_bias) on the host cores.
+dump    : --dump-outputs DIR writes the records of the last timed step (rank 0's) as DIR/<field>.npy, so that two builds can be
+          compared output for output on the same seeded inputs.
 Multi-GPU: sites are sharded by contiguous region, one process per GPU, no collective on the data path
           (weak scaling: every GPU gets its own S sites); torch.distributed only for the barrier / max-time.
 """
@@ -342,10 +344,27 @@ def cpu_baseline(res, ns, cores):
                       f"BaseType ctor+lrt()+strand_bias, {cores} threads, slowest thread's time in reference code"}
 
 
+DUMP_SITES = 1 << 18   # sites per dump: 156 bytes of .npy each, about 41 MB in all
+
+
+def dump_outputs(path, rec):
+    """One DIR/<field>.npy per field of struct bv_site_out: counts, codes and flags as float32 (exact, all are below 2^24), the
+    floating-point fields as float64, and site.npy with the site indices.  More than DUMP_SITES sites: the same seeded sample of
+    sites every run."""
+    os.makedirs(path, exist_ok=True)
+    S = rec.shape[0]
+    site = np.arange(S) if S <= DUMP_SITES else np.sort(np.random.default_rng(0).choice(S, DUMP_SITES, replace=False))
+    rec = rec[site]
+    np.save(os.path.join(path, "site.npy"), site.astype(np.float64))
+    for f in rec.dtype.names:
+        if not f.startswith("reserved"):
+            np.save(os.path.join(path, f + ".npy"), rec[f].astype(np.float64 if rec[f].dtype.kind == "f" else np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the kernel-only leg (the headline value)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default=None, choices=["C2", "C3", "C4", "C5"], help="main workload (default: C2 on one GPU, C4 shards on several)")
@@ -360,7 +379,14 @@ def main():
     ap.add_argument("--no-e2e-extra", action="store_true", help="skip the e2e_sparse_u32 / e2e_dense / fabric legs")
     ap.add_argument("--no-numa-bind", action="store_true", help="N > 1: do not bind the rank to the CPUs next to its GPU")
     ap.add_argument("--ref-min-sample-sites", type=int, default=1_000_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the records of the last timed step as DIR/<field>.npy (a fixed sample of %d sites when there are more); "
+                         "with several GPUs, rank 0's shard only" % DUMP_SITES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the records of the device path: not with --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -407,8 +433,8 @@ def main():
     total_ms, per_step_ms, launches = main_res.timed(args.steps, args.warmup, barrier)
     total_ms_max = shard.max_over_ranks(total_ms, dev)
     value = world * S * n_samples * args.steps / (total_ms_max * 1e-3)
-    kernel_ms = main_res.kernel_ms(args.steps)
     dev_rec = main_res.records()
+    kernel_ms = main_res.kernel_ms(args.steps)
 
     # ---- end to end through the C ABI with host buffers --------------------------------------------------------
     # sparse tiles: pinned host arrays of the covered cells -> bv_tile_submit_sparse (H2D of the cells, K0 expand, K1..K4, D2H of
@@ -647,6 +673,8 @@ def main():
             r.close()
         line["configs"] = configs
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dev_rec)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

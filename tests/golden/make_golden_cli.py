@@ -11,7 +11,8 @@ What it does (BASELINE.json configs[0]: `basevar basetype` on the repo's tests/d
   2. runs oracle/_ref/basevar basetype over the regions of tests/data/140k_thalassemia_brca_bam/work.log.sh:5-8 with
      the batchfiles kept (oracle/keep_batchfiles.c), once with and once without --pop-group;
   3. commits, under tests/golden/c1/: the batchfile rows the reference fed to `_basevar_caller` (gzip text), and the
-     VCF / CVG text it wrote for them -- the expected output of our host pipeline on the same rows.
+     VCF / CVG text it wrote for them -- the expected output of our host pipeline on the same rows;
+  4. keeps the chr17 batchfile under 1 MB: its called rows and a seeded sample of the others (sample_chr17).
 """
 import gzip
 import os
@@ -19,6 +20,8 @@ import shutil
 import struct
 import subprocess
 import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 REF = os.environ.get("BV_REFERENCE_DIR", "/root/reference")
@@ -162,6 +165,33 @@ def run(work, tag, extra):
     return vcf, cvg, os.path.join(work, "cache_" + tag)
 
 
+FULL_BF = "batch.chr17_41197764-41276135.1_1.bf.gz"
+SAMPLED_BF = "batch.chr17_41197764-41276135.sampled.bf.gz"
+
+
+def sample_chr17(out, frac=0.2, seed=17):
+    """The chr17 batchfile holds 78,372 rows (3.1 MB compressed); keep every row at a position either VCF calls plus a seeded
+    sample `frac` of the others (0.8 MB), and drop the CVG rows of the positions left out.  Every VCF / CVG row comes from its
+    own batchfile row, so the reference's text for the kept rows is its text for the whole region, filtered."""
+    bf = gzip.open(os.path.join(out, FULL_BF), "rb").read().split(b"\n")
+    hdr = [l for l in bf if l.startswith(b"#")]
+    rows = [l for l in bf if l and not l.startswith(b"#")]
+    called = {int(l.split("\t")[1]) for t in ("c1", "c1g") for l in gzip.open(os.path.join(out, t + ".vcf.gz"), "rt")
+              if l.startswith("chr17\t")}
+    u = np.random.default_rng(seed).random(len(rows))
+    keep = [r for r, x in zip(rows, u) if x < frac or int(r.split(b"\t", 2)[1]) in called]
+    kept = {int(r.split(b"\t", 2)[1]) for r in keep}
+    with gzip.GzipFile(os.path.join(out, SAMPLED_BF), "wb", mtime=0) as fo:
+        fo.write(b"\n".join(hdr + keep) + b"\n")
+    for t in ("c1", "c1g"):
+        lines = gzip.open(os.path.join(out, t + ".cvg.gz"), "rb").read().split(b"\n")[:-1]
+        lines = [l for l in lines if not l.startswith(b"chr17\t") or int(l.split(b"\t", 2)[1]) in kept]
+        with gzip.GzipFile(os.path.join(out, t + ".cvg.gz"), "wb", mtime=0) as fo:
+            fo.write(b"\n".join(lines) + b"\n")
+    os.remove(os.path.join(out, FULL_BF))
+    print(f"{SAMPLED_BF}: {len(keep)} of {len(rows)} rows, {len(called)} called positions")
+
+
 def main():
     work = os.environ.get("BV_GOLDEN_WORK", "/tmp/bv_golden_cli")
     os.makedirs(work, exist_ok=True)
@@ -187,6 +217,7 @@ def main():
                     fo.write(fi.read())
         print(tag, "done")
     shutil.copy(os.path.join(DATA, "sample_group.info"), os.path.join(OUT, "sample_group.info"))
+    sample_chr17(OUT)
 
 
 if __name__ == "__main__":

@@ -3,7 +3,7 @@
 CPU (no GPU needed): our BGZF/BAM/BAI/FASTA readers and the pileup, rendered back into the reference's batchfile text,
 against the rows the UNMODIFIED reference command wrote
   * for the committed synthetic BAM fixtures (tests/golden/bam, made by tests/golden/make_golden_bam.py), and
-  * for the reference's own bam100 fixture (BASELINE.json configs[0]) when /root/reference is present.
+  * for the reference's own bam100 fixture (BASELINE.json configs[0]) when BV_REFERENCE_DIR names its source tree.
 GPU: the whole command (BAM -> tiles -> GPU -> VCF / CVG files) against the files the reference command wrote.
 """
 import gzip
@@ -17,7 +17,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "tests", "cpp", "bin")
 FIX = os.path.join(ROOT, "tests", "golden", "bam")
 CLI = os.path.join(ROOT, "basevar_b200", "bin", "basevar")
-REF_DATA = "/root/reference/tests/data/140k_thalassemia_brca_bam"
+REF_DIR = os.environ.get("BV_REFERENCE_DIR")   # the original BaseVar source tree, for the test over its own bam100 fixture
+REF_DATA = os.path.join(REF_DIR, "tests", "data", "140k_thalassemia_brca_bam") if REF_DIR else ""
 N_SAMPLES = 12
 
 
@@ -102,23 +103,25 @@ def test_unknown_contig_fails_like_the_reference(host_built, syn):
     assert p.returncode != 0 and "Fail to fetch the alignment data" in p.stderr   # src/bam.cpp:93-98
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="needs the reference's bam100 fixture under /root/reference")
+@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="needs the reference's bam100 fixture: set BV_REFERENCE_DIR to its source tree")
 def test_packer_matches_reference_batchfiles_on_bam100(host_built, tmp_path_factory):
     """BASELINE.json configs[0]: the 100 BAM files of the reference's own test, over both regions of its work.log.sh;
-    every row (80,212 of them) equals the batchfile the unmodified reference wrote (tests/golden/c1/batch.*.bf.gz)."""
+    every row equals the batchfile the unmodified reference wrote (tests/golden/c1: of chr17 the rows it keeps)."""
     from tests.golden import make_golden_cli as G
-    work = os.environ.get("BV_GOLDEN_WORK", "/tmp/bv_golden_cli")
-    os.makedirs(work, exist_ok=True)
+    work = str(tmp_path_factory.mktemp("bam100"))
     bams = [os.path.join(REF_DATA, l.strip()) for l in open(os.path.join(REF_DATA, "bam100.list")) if l.strip()]
     fa = os.path.join(work, "standin.fa")
-    if not os.path.exists(fa):
-        G.build_fasta(bams, fa)
+    G.build_fasta(bams, fa)
     lst = os.path.join(work, "bam.list")
     with open(lst, "w") as f:
         f.write("\n".join(bams) + "\n")
-    for region in ("chr11:5246595-5248428", "chr17:41197764-41276135"):
-        want = gzip.open(os.path.join(ROOT, "tests", "golden", "c1", "batch.%s.1_1.bf.gz" % region.replace(":", "_")), "rb").read()
-        assert _dump(host_built, fa, lst, region) == want
+    for region, fn in (("chr11:5246595-5248428", "batch.chr11_5246595-5248428.1_1.bf.gz"), ("chr17:41197764-41276135", G.SAMPLED_BF)):
+        want = gzip.open(os.path.join(ROOT, "tests", "golden", "c1", fn), "rb").read().split(b"\n")
+        got = _dump(host_built, fa, lst, region).split(b"\n")
+        beg, end = map(int, region.split(":")[1].split("-"))
+        assert got[:3] == want[:3] and len(got) == 3 + end - beg + 1 + 1   # header, one row per position
+        kept = {l.split(b"\t", 2)[1] for l in want[3:] if l}
+        assert [l for l in got[3:] if l and l.split(b"\t", 2)[1] in kept] == [l for l in want[3:] if l]
 
 
 RANGE = os.path.join(ROOT, "tests", "golden", "range")
