@@ -10,8 +10,7 @@ import os
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# BASEVAR_B200_LIB points at another build of the same library (tuning builds with different -DBV_WARPS etc.)
-LIB_PATH = os.environ.get("BASEVAR_B200_LIB") or os.path.join(HERE, "libbasevar_b200.so")
+LIB_PATH = os.path.join(HERE, "libbasevar_b200.so")
 
 BV_OK = 0
 BV_LOC_HOST, BV_LOC_DEVICE = 0, 1

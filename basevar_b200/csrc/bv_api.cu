@@ -23,15 +23,8 @@
 #include "bv_expand_kernel.cuh"
 #include "bv_synth.cuh"
 
-#ifndef BV_SCALAR_CTAS_PER_SM
-#define BV_SCALAR_CTAS_PER_SM 8u
-#endif
-#ifndef BV_TASK_HI_CTAS
-#define BV_TASK_HI_CTAS 4
-#endif
-#ifndef BV_EM_POOL_BINS_PER_SITE
-#define BV_EM_POOL_BINS_PER_SITE 64u
-#endif
+constexpr uint32_t kScalarCtasPerSm = 8;      // grid cap of K2 and of bv_fisher_kernel, per SM
+constexpr uint32_t kEmPoolBinsPerSite = 64;   // EM bin pool per site of the tile (see scratch_reserve)
 
 // NVTX range over a scope (SURVEY.md section 5, "Tracing"): nsys / ncu timelines show the host side of every tile
 // (submit, wait) and the launch sequence K0, K1, K2, K3, K4a, K4b, K5, K6 under these names.
@@ -173,13 +166,11 @@ struct bv_ctx {
     double* d_logfact = nullptr;
     bv_synth_model* d_model = nullptr;
     bv_scratch dev_scratch;           // bv_tile_run_device
-    bool zero_copy_qual = true;       // BASEVAR_B200_ZERO_COPY_QUAL=0 uploads the whole qual plane instead
     uint64_t h2d_bytes_total = 0;
     bool profiling = false;
     cudaEvent_t ev[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    long long task_split_override = -1;   // BASEVAR_B200_TASK_SPLIT (tuning): tiles with more EM tasks than this run the high-occupancy build
-    int task_ctas_per_sm = 3;         // resident CTAs per SM of bv_em_task_kernel<BV_TASK_LO_CTAS> (asked of the runtime in bv_create) ...
-    int task_ctas_per_sm_hi = 4;      // ... and of bv_em_task_kernel<BV_TASK_HI_CTAS>, the build for tiles with many EM tasks
+    int task_ctas_per_sm = bv::kTaskLoCtas;      // resident CTAs per SM of bv_em_task_kernel<kTaskLoCtas> (asked of the runtime in bv_create) ...
+    int task_ctas_per_sm_hi = bv::kTaskHiCtas;   // ... and of bv_em_task_kernel<kTaskHiCtas>, the build for tiles with many EM tasks
     bool ev_valid = false;
     bool has_model = false;
     uint64_t pitch_cap = 0;
@@ -247,7 +238,7 @@ static int scratch_reserve(bv_ctx* ctx, bv_scratch& sc, uint32_t n_sites) {
         cudaFree(sc.d_em_hdr); cudaFree(sc.d_em_pool); cudaFree(sc.d_em_tasks); cudaFree(sc.d_em_res); cudaFree(sc.d_em_single);
         sc.d_em_hdr = nullptr; sc.d_em_pool = nullptr; sc.d_em_tasks = nullptr; sc.d_em_res = nullptr; sc.d_em_single = nullptr;
         cudaGetLastError();
-        const uint64_t pool = (uint64_t)n_sites * BV_EM_POOL_BINS_PER_SITE + 4096;
+        const uint64_t pool = (uint64_t)n_sites * kEmPoolBinsPerSite + 4096;
         sc.em_pool_cap = (uint32_t)(pool < 0x7ffffff0ull ? pool : 0x7ffffff0ull);
         // task slots for subsets of 2, 3 and 4 alleles: 2, 1 and 1/2 per site of the tile (header indices have 28 bits)
         sc.em_task_cap[0] = 2u * n_sites + 1024u; sc.em_task_cap[1] = n_sites + 512u; sc.em_task_cap[2] = n_sites / 2u + 256u;
@@ -294,8 +285,7 @@ static int fill_kernel_args(bv_ctx* ctx, const bv_tile* t, bv_site_out* d_out, b
     for (int k = 0; k < 3; ++k) a->em_task_cap[k] = sc.em_task_cap[k];
     a->brief = nullptr; a->full_out = nullptr;   // set by the submit paths of compact tiles
     a->em_resume = 0;
-    a->em_task_split = ctx->task_split_override >= 0 ? (uint32_t)ctx->task_split_override
-                     : (uint32_t)ctx->num_sms * (uint32_t)ctx->task_ctas_per_sm_hi * (uint32_t)bv::kTaskThreads;   // one round of resident threads
+    a->em_task_split = (uint32_t)ctx->num_sms * (uint32_t)ctx->task_ctas_per_sm_hi * (uint32_t)bv::kTaskThreads;   // one round of resident threads
     a->list_called = nullptr;   // set_call_args() turns the called-site kernels on
     a->mapq = nullptr; a->rpr = nullptr; a->aux_pitch = 0; a->rpr_pitch = 0;
     a->sample_group = nullptr; a->calls = nullptr; a->groups = nullptr; a->n_groups = 0; a->pad0 = 0;
@@ -346,20 +336,20 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
     // K1, persistent: one CTA per SM, each warp strides over the sites; kernel shape by row length
     uint32_t grid;
     if (a.n_samples > (uint32_t)bv::kLongRowSamples) {
-        grid = (a.n_sites + BV_COUNT_WARPS_LONG - 1) / BV_COUNT_WARPS_LONG;
+        grid = (a.n_sites + bv::kCountWarpsLong - 1) / bv::kCountWarpsLong;
         if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;
-        bv::bv_count_kernel<BV_COUNT_WARPS_LONG, BV_COUNT_STAGES_LONG><<<grid, BV_COUNT_WARPS_LONG * 32,
-            bv::count_smem_bytes<BV_COUNT_WARPS_LONG, BV_COUNT_STAGES_LONG>(), stream>>>(a);
+        bv::bv_count_kernel<bv::kCountWarpsLong, bv::kCountStagesLong><<<grid, bv::kCountWarpsLong * 32,
+            bv::count_smem_bytes<bv::kCountWarpsLong, bv::kCountStagesLong>(), stream>>>(a);
     } else {
-        grid = (a.n_sites + BV_COUNT_WARPS - 1) / BV_COUNT_WARPS;
+        grid = (a.n_sites + bv::kCountWarpsShort - 1) / bv::kCountWarpsShort;
         if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;
-        bv::bv_count_kernel<BV_COUNT_WARPS, BV_COUNT_STAGES><<<grid, BV_COUNT_WARPS * 32,
-            bv::count_smem_bytes<BV_COUNT_WARPS, BV_COUNT_STAGES>(), stream>>>(a);
+        bv::bv_count_kernel<bv::kCountWarpsShort, bv::kCountStagesShort><<<grid, bv::kCountWarpsShort * 32,
+            bv::count_smem_bytes<bv::kCountWarpsShort, bv::kCountStagesShort>(), stream>>>(a);
     }
     BV_CUDA(ctx, cudaGetLastError());
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[1], stream));
     grid = (a.n_sites + 255) / 256;   // grid-stride over K1's work list
-    if (grid > (uint32_t)ctx->num_sms * BV_SCALAR_CTAS_PER_SM) grid = (uint32_t)ctx->num_sms * BV_SCALAR_CTAS_PER_SM;
+    if (grid > (uint32_t)ctx->num_sms * kScalarCtasPerSm) grid = (uint32_t)ctx->num_sms * kScalarCtasPerSm;
     bv::bv_scalar_kernel<<<grid, 256, 0, stream>>>(a);
     BV_CUDA(ctx, cudaGetLastError());
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[2], stream));
@@ -396,15 +386,15 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
         b.em_resume = 1;
     }
     // two builds of the kernel (registers / occupancy); the tile's task count decides on the device which of them works
-    bv::bv_em_task_kernel<BV_TASK_LO_CTAS><<<grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(b);
+    bv::bv_em_task_kernel<bv::kTaskLoCtas><<<grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(b);
     BV_CUDA(ctx, cudaGetLastError());
-    bv::bv_em_task_kernel<BV_TASK_HI_CTAS><<<grid_hi, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(b);
+    bv::bv_em_task_kernel<bv::kTaskHiCtas><<<grid_hi, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(b);
     ctx->launches += 1;
     BV_CUDA(ctx, cudaGetLastError());
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[5], stream));
     // the Fisher tests K2 and K4 listed (as many as two per site; the counts are on the device): grid-stride
     grid = (4u * a.n_sites + bv::kFisherThreads - 1) / bv::kFisherThreads;   // (a pair of lanes per test)
-    if (grid > (uint32_t)ctx->num_sms * BV_SCALAR_CTAS_PER_SM) grid = (uint32_t)ctx->num_sms * BV_SCALAR_CTAS_PER_SM;
+    if (grid > (uint32_t)ctx->num_sms * kScalarCtasPerSm) grid = (uint32_t)ctx->num_sms * kScalarCtasPerSm;
     bv::bv_fisher_kernel<<<grid, bv::kFisherThreads, 0, stream>>>(a);
     BV_CUDA(ctx, cudaGetLastError());
     if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev[6], stream)); ctx->ev_valid = true; }
@@ -598,15 +588,15 @@ int bv_create(int device, const bv_params* params, bv_ctx** out_ctx) {
         cudaDeviceProp prop;
         if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { rc = set_err(nullptr, BV_ERR_CUDA, "cudaGetDeviceProperties failed"); break; }
         ctx->num_sms = prop.multiProcessorCount;
-        if (cudaFuncSetAttribute(bv::bv_count_kernel<BV_COUNT_WARPS, BV_COUNT_STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)bv::count_smem_bytes<BV_COUNT_WARPS, BV_COUNT_STAGES>()) != cudaSuccess ||
-            cudaFuncSetAttribute(bv::bv_count_kernel<BV_COUNT_WARPS_LONG, BV_COUNT_STAGES_LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)bv::count_smem_bytes<BV_COUNT_WARPS_LONG, BV_COUNT_STAGES_LONG>()) != cudaSuccess ||
+        if (cudaFuncSetAttribute(bv::bv_count_kernel<bv::kCountWarpsShort, bv::kCountStagesShort>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)bv::count_smem_bytes<bv::kCountWarpsShort, bv::kCountStagesShort>()) != cudaSuccess ||
+            cudaFuncSetAttribute(bv::bv_count_kernel<bv::kCountWarpsLong, bv::kCountStagesLong>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)bv::count_smem_bytes<bv::kCountWarpsLong, bv::kCountStagesLong>()) != cudaSuccess ||
             cudaFuncSetAttribute(bv::bv_bound_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kBoundSmemBytes) != cudaSuccess ||
             cudaFuncSetAttribute(bv::bv_hist_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes) != cudaSuccess ||
             cudaFuncSetAttribute(bv::bv_hist_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kHistLongSmemBytes) != cudaSuccess ||
-            cudaFuncSetAttribute(bv::bv_em_task_kernel<BV_TASK_LO_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kTaskSmemBytes) != cudaSuccess ||
-            cudaFuncSetAttribute(bv::bv_em_task_kernel<BV_TASK_HI_CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kTaskSmemBytes) != cudaSuccess ||
+            cudaFuncSetAttribute(bv::bv_em_task_kernel<bv::kTaskLoCtas>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kTaskSmemBytes) != cudaSuccess ||
+            cudaFuncSetAttribute(bv::bv_em_task_kernel<bv::kTaskHiCtas>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kTaskSmemBytes) != cudaSuccess ||
             cudaFuncSetAttribute(bv::bv_em_iter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kTaskSmemBytes) != cudaSuccess ||
             cudaFuncSetAttribute(bv::bv_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes) != cudaSuccess ||
             cudaFuncSetAttribute(bv::bv_ranksum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kCallSmemBytes) != cudaSuccess ||
@@ -618,23 +608,15 @@ int bv_create(int device, const bv_params* params, bv_ctx** out_ctx) {
         }
         {   // the EM task kernel's grid: what is resident at once (registers / shared memory decide)
             int nb = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, bv::bv_em_task_kernel<BV_TASK_LO_CTAS>, bv::kTaskThreads, bv::kTaskSmemBytes) == cudaSuccess && nb > 0)
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, bv::bv_em_task_kernel<bv::kTaskLoCtas>, bv::kTaskThreads, bv::kTaskSmemBytes) == cudaSuccess && nb > 0)
                 ctx->task_ctas_per_sm = nb;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, bv::bv_em_task_kernel<BV_TASK_HI_CTAS>, bv::kTaskThreads, bv::kTaskSmemBytes) == cudaSuccess && nb > 0)
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, bv::bv_em_task_kernel<bv::kTaskHiCtas>, bv::kTaskThreads, bv::kTaskSmemBytes) == cudaSuccess && nb > 0)
                 ctx->task_ctas_per_sm_hi = nb;
             cudaGetLastError();
         }
         {
-            const char* z = getenv("BASEVAR_B200_TASK_SPLIT");
-            if (z && z[0]) ctx->task_split_override = atoll(z);
-        }
-        {
             const char* z = getenv("BASEVAR_B200_TRACE");
             ctx->trace = z && z[0] == '1';
-        }
-        {
-            const char* z = getenv("BASEVAR_B200_ZERO_COPY_QUAL");
-            if (z && z[0] == '0') ctx->zero_copy_qual = false;
         }
         rc = upload_tables(ctx);
         if (rc != BV_OK) break;
@@ -815,7 +797,7 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
         // When it lives in pinned host memory the kernels fetch exactly those rows over PCIe themselves (zero copy),
         // and the plane is not uploaded at all; pageable memory is copied like the other planes.
         const uint8_t* qual_zero_copy = nullptr;
-        if (ctx->zero_copy_qual && tile->n_sites) qual_zero_copy = static_cast<const uint8_t*>(host_device_pointer(tile->qual));
+        if (tile->n_sites) qual_zero_copy = static_cast<const uint8_t*>(host_device_pointer(tile->qual));
         for (int k = 0; k < 3 && tile->n_sites; ++k) {
             if (k == 1 && qual_zero_copy) continue;
             if (dp == tile->pitch)
@@ -1290,7 +1272,7 @@ uint32_t bv_suggest_tile_sites(const bv_ctx* ctx, uint32_t n_samples, uint64_t m
     if (fit < 1) fit = 1;
     if (fit > 0xffffffffull) fit = 0xffffffffull;
     const uint64_t sms = ctx && ctx->num_sms > 0 ? (uint64_t)ctx->num_sms : 148;
-    const uint64_t unit = sms * (n_samples > (uint32_t)bv::kLongRowSamples ? BV_COUNT_WARPS_LONG : BV_COUNT_WARPS);
+    const uint64_t unit = sms * (n_samples > (uint32_t)bv::kLongRowSamples ? bv::kCountWarpsLong : bv::kCountWarpsShort);
     return (uint32_t)(fit >= unit ? fit / unit * unit : fit);
 }
 

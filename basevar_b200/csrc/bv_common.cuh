@@ -54,7 +54,7 @@ constexpr uint32_t kStateScalar = 1;         // counts are final, K2 has to fini
 constexpr uint32_t kStateBound = 2;          // result depends on base qualities; K3 tries the likelihood-ratio bound
 constexpr uint32_t kStateEM = 3;             // result depends on base qualities; K4 runs EM + LRT
 
-constexpr int kCntSlow = 0, kCntBound = 1, kCntEm = 2, kCntEmNext = 3;   // SiteKernelArgs::counters
+constexpr int kCntSlow = 0, kCntBound = 1, kCntEm = 2;                    // SiteKernelArgs::counters (3 is unused)
 constexpr int kCntCalled = 4, kCntGroupNext = 5;                          // called sites (K4 -> K5, K6)
 constexpr int kCntBadCell = 6;                                            // malformed sparse input (K0, bv_expand_kernel.cuh)
 constexpr int kCntEmHdr = 7, kCntEmPool = 8;                              // K4a -> K4b: EM sites and the pool of their bins
@@ -116,7 +116,7 @@ struct SiteKernelArgs {
     uint32_t em_task_cap[3];
     // compact record transport (BV_OUT_COMPACT): null unless the tile asked for it
     uint32_t em_resume;      // bv_em_task_kernel: the EM iterations were run by bv_em_iter_kernel, start from its frequencies
-    uint32_t em_task_split;  // tiles with more EM tasks than this run bv_em_task_kernel<4>, the others bv_em_task_kernel<1>
+    uint32_t em_task_split;  // tiles with more EM tasks than this run bv_em_task_kernel<kTaskHiCtas>, the others <kTaskLoCtas>
     uint2* brief;            // [n_sites] device copy of the briefs: K1 writes them, bv_pack_kernel completes them
     bv_site_out* full_out;   // pinned host memory (mapped): the full records, written by bv_pack_kernel
     // called sites (n_alt > 0): rank sums (K5) and population-group frequencies (K6); all null / 0 when not asked for

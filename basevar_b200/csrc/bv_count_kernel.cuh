@@ -23,19 +23,9 @@ namespace bv {
 // B200 (profiles/history/r01o_k1_ring_shapes.txt): rows of <= 1,000 samples want many warps (per-site work is short, 32 warps
 // keep the issue slots 82 % busy), rows of 10,000 samples want deeper rings on fewer warps (0.66 ms vs 0.93 ms per
 // 10^9 cells).
-#ifndef BV_COUNT_WARPS
-#define BV_COUNT_WARPS 32
-#endif
-#ifndef BV_COUNT_STAGES
-#define BV_COUNT_STAGES 3
-#endif
-#ifndef BV_COUNT_WARPS_LONG
-#define BV_COUNT_WARPS_LONG 16
-#endif
-#ifndef BV_COUNT_STAGES_LONG
-#define BV_COUNT_STAGES_LONG 4
-#endif
-constexpr int kLongRowSamples = 4096;         // rows longer than this use the *_LONG shape
+constexpr int kCountWarpsShort = 32, kCountStagesShort = 3;
+constexpr int kCountWarpsLong = 16, kCountStagesLong = 4;
+constexpr int kLongRowSamples = 4096;         // rows longer than this use the *Long shape
 constexpr int kChunk = 1024;                  // cells per stage and plane: two 16-cell vectors per lane
 constexpr int kSlowBatch = 16;                // one atomicAdd on the list counter per this many sites
 
@@ -55,8 +45,8 @@ struct __align__(128) CountWarp {
 
 template <int kCountWarps, int kCountStages>
 constexpr size_t count_smem_bytes() { return (size_t)kCountWarps * sizeof(CountWarp<kCountStages>); }
-static_assert(count_smem_bytes<BV_COUNT_WARPS, BV_COUNT_STAGES>() <= 232448, "shared memory of the count kernel exceeds 227 KB");
-static_assert(count_smem_bytes<BV_COUNT_WARPS_LONG, BV_COUNT_STAGES_LONG>() <= 232448, "shared memory of the count kernel exceeds 227 KB");
+static_assert(count_smem_bytes<kCountWarpsShort, kCountStagesShort>() <= 232448, "shared memory of the count kernel exceeds 227 KB");
+static_assert(count_smem_bytes<kCountWarpsLong, kCountStagesLong>() <= 232448, "shared memory of the count kernel exceeds 227 KB");
 
 struct ScanAcc {
     uint32_t nref;     // 128 * (# cells holding the reference base)

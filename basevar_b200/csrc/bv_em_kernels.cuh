@@ -29,14 +29,6 @@
 #pragma once
 #include "bv_finish_kernels.cuh"
 
-#ifndef BV_HIST_STATIC
-#define BV_HIST_STATIC 1        // 0: the EM list is dealt out through a shared fetch counter (tuning builds)
-#endif
-#ifndef BV_TASK_WARP_ROUNDS
-#define BV_TASK_WARP_ROUNDS 0   // 1: bv_em_task_kernel works in rounds of one warp, no barriers, decisions queued per warp (tuning builds:
-                                // 2-4 % faster on C3 / C4 / C5 with fabs, 1.5 % slower on C2, see DESIGN.md)
-#endif
-
 namespace bv {
 
 // ---- K4a: one site in state kStateEM -----------------------------------------------------------------------------------------
@@ -193,7 +185,7 @@ __device__ __noinline__ void hist_site(uint32_t site) {
     if (W.vcf_n == 32) vcf_flush();
 }
 
-// Persistent warps with dynamic work distribution over the EM list.  LONG: the shape for rows of more than kLongRowSamples
+// Persistent warps over the EM list.  LONG: the shape for rows of more than kLongRowSamples
 // samples (kLongWarps warps per CTA, build_hist_long).
 template <bool LONG>
 __global__ void __launch_bounds__((LONG ? kLongWarps : kQualWarps) * 32, 1) bv_hist_kernel(const __grid_constant__ SiteKernelArgs a) {
@@ -216,7 +208,6 @@ __global__ void __launch_bounds__((LONG ? kLongWarps : kQualWarps) * 32, 1) bv_h
     // entry is read while this one is worked on.  (A shared fetch counter cost every site a round trip to one L2 address that
     // 4,736 warps queue on: 17 % of the kernel's stall samples on deep pileups.)
     const uint32_t n_em = a.counters[kCntEm];
-#if BV_HIST_STATIC
     const uint32_t total_warps = gridDim.x * (blockDim.x >> 5);
     uint32_t i = (threadIdx.x >> 5) * gridDim.x + blockIdx.x;
     uint32_t site_next = i < n_em ? a.list_em[i] : 0u;
@@ -225,40 +216,19 @@ __global__ void __launch_bounds__((LONG ? kLongWarps : kQualWarps) * 32, 1) bv_h
         if (i + total_warps < n_em) site_next = a.list_em[i + total_warps];
         hist_site<LONG>(site);
     }
-#else
-    for (;;) {
-        uint32_t i = 0;
-        if (lane == 0) i = atomicAdd(a.counters + kCntEmNext, 1u);
-        i = __shfl_sync(kFull, i, 0);
-        if (i >= n_em) break;
-        hist_site<LONG>(a.list_em[i]);
-    }
-#endif
     if (W.vcf_n) vcf_flush();
 }
 
 // =====================================================================================================================
 // K4b: one thread per EM task; the thread that finishes a site's last task decides the site.
 // =====================================================================================================================
-#ifndef BV_TASK_THREADS
-#define BV_TASK_THREADS 128
-#endif
-#ifndef BV_TASK_LO_CTAS
-#define BV_TASK_LO_CTAS 3       // resident CTAs per SM the two builds of bv_em_task_kernel are compiled for: tiles with few EM tasks ...
-#endif
-#ifndef BV_TASK_HI_CTAS
-#define BV_TASK_HI_CTAS 4       // ... and tiles with many
-#endif
-static_assert(BV_TASK_LO_CTAS != BV_TASK_HI_CTAS, "the two builds of bv_em_task_kernel are told apart by their CTA count");
-#ifndef BV_TASK_STAGE_BINS
-#define BV_TASK_STAGE_BINS 96
-#endif
-#ifndef BV_TASK_G4_MAX_TASKS
-#define BV_TASK_G4_MAX_TASKS 12288
-#endif
-constexpr int kTaskThreads = BV_TASK_THREADS;
-constexpr int kStageBins = BV_TASK_STAGE_BINS;     // bins per site staged in shared memory; longer lists are read from the pool
+constexpr int kTaskThreads = 128;
+constexpr int kTaskLoCtas = 3;                     // resident CTAs per SM the two builds of bv_em_task_kernel are compiled for: tiles with few EM tasks ...
+constexpr int kTaskHiCtas = 4;                     // ... and tiles with many
+static_assert(kTaskLoCtas != kTaskHiCtas, "the two builds of bv_em_task_kernel are told apart by their CTA count");
+constexpr int kStageBins = 96;                     // bins per site staged in shared memory; longer lists are read from the pool
 constexpr int kStageStride = kStageBins + 1;       // odd: the rows of 32 different sites start in 32 different banks
+constexpr uint32_t kG4MaxTasks = 12288;            // tiles with at most this many EM tasks give each task four lanes
 
 struct __align__(16) TaskCta {
     double lut[4][kQSlots];           // 1 - eps(q), eps(q) / 3, log(1 - eps(q)), log(eps(q) / 3)
@@ -267,9 +237,6 @@ struct __align__(16) TaskCta {
     uint32_t decide_hdr[kTaskThreads];   // ... their headers: decided one thread per site after the round
     uint32_t n_fs;                    // Fisher tests of the VCF rows of decided sites, listed by decide_site ...
     uint32_t fs_site[2 * kTaskThreads];  // ... on their way to list_fisher, a CTA of them at a time
-#if BV_TASK_WARP_ROUNDS
-    uint32_t dq[kTaskThreads / 32][64];  // per warp: headers of completed sites waiting for their decision
-#endif
     uint32_t bins[kTaskThreads * kStageStride];   // one row per task of the round
 };
 constexpr size_t kTaskSmemBytes = sizeof(TaskCta);
@@ -291,18 +258,6 @@ struct LaneGroup {
     __device__ __forceinline__ bool any(bool p) const { return (__ballot_sync(mask, p) & mask) != 0u; }
 };
 __device__ __forceinline__ double sum4(const double (&p)[4]) { return (p[0] + p[2]) + (p[1] + p[3]); }
-
-// 1 / m to ~1 ulp: the hardware's 20-bit estimate and two Newton steps (the correctly rounded division costs twice as
-// many FP64 instructions; the posteriors it feeds are inside the stated tolerance either way).  m == 0 gives NaN, where
-// 1.0 / 0 gives inf: the posteriors 0 * inf the reference then forms are NaN as well.
-__device__ __forceinline__ double rcp_fast(double m) {
-    double r;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(m));
-    double e = fma(-m, r, 1.0);
-    r = fma(r, e, r);
-    e = fma(-m, r, 1.0);
-    return fma(r, e, r);
-}
 
 // log(r) for the ratio of two marginals of consecutive E-steps: once the EM settles r is within 2^-10 of 1 for every bin,
 // and t - t^2/2 + t^3/3 - t^4/4 (t = r - 1, exact) is then good to 2e-16 of t -- below the rounding of a full logarithm,
@@ -869,16 +824,16 @@ __device__ __noinline__ void decide_site(const SiteKernelArgs& a, const EmSiteHd
 }
 
 // Two builds of the kernel, launched one after the other; the task count (known on the device only) picks the one that works,
-// the other leaves at once.  kMinCtas = 1: the compiler takes the registers it wants (154: three CTAs per SM), fastest while
-// the tasks of a tile fit one round of resident threads.  kMinCtas = 4: 126 registers, four CTAs per SM, 12 % faster once
-// they do not (deep multi-allelic pileups: 185,000 tasks per 200,000 sites of C5) and 7-14 % slower below
-// (gpurun r2u, profiles/r02_em_task_occupancy.txt).
+// the other leaves at once.  kMinCtas = kTaskLoCtas (3): 168 registers, three CTAs per SM, fastest while the tasks of a tile
+// fit one round of resident threads.  kMinCtas = kTaskHiCtas (4): 128 registers (and 384 bytes of spill stores), four CTAs per
+// SM, 12 % faster once they do not (deep multi-allelic pileups: 185,000 tasks per 200,000 sites of C5) and 7-14 % slower below
+// (register counts from ptxas -v; timings on a B200 in profiles/r02_em_task_occupancy.txt).
 template <int kMinCtas>
 __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(const __grid_constant__ SiteKernelArgs a) {
     {
         const uint64_t n_all = (uint64_t)min(a.counters[kCntEmTask2], a.em_task_cap[0]) + min(a.counters[kCntEmTask3], a.em_task_cap[1]) +
                                min(a.counters[kCntEmTask4], a.em_task_cap[2]);
-        if ((n_all > (uint64_t)a.em_task_split) != (kMinCtas == BV_TASK_HI_CTAS)) return;
+        if ((n_all > (uint64_t)a.em_task_split) != (kMinCtas == kTaskHiCtas)) return;
     }
     TaskCta& cs = *reinterpret_cast<TaskCta*>(bv_smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
@@ -897,100 +852,11 @@ __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(cons
     LaneGroup lg;
     {
         const uint64_t n_tasks = (uint64_t)n_list[0] + n_list[1] + n_list[2];
-        int G = n_tasks <= (uint64_t)BV_TASK_G4_MAX_TASKS ? 4 : 1;
-#ifdef BV_TASK_FORCE_G
-        G = BV_TASK_FORCE_G;   // tuning builds (1 or 4)
-#endif
+        const int G = n_tasks <= (uint64_t)kG4MaxTasks ? 4 : 1;
         lg.G = G;
         lg.gl = lane & (G - 1);
         lg.mask = (G == 1 ? 1u : 0xfu) << (lane & ~(G - 1));
     }
-#if BV_TASK_WARP_ROUNDS
-    // Tuning build (off by default).  Rounds of ONE WARP: 32 / G tasks of one list, staged into the warp's own 32 rows, run, and
-    // the sites they complete queued for decision by the same warp -- nothing in a round waits for another warp, where rounds of
-    // a whole CTA cost a barrier per phase (a fifth of the kernel's stall samples).  Measured (profiles/r02_variants.txt): 2-4 %
-    // faster on C3 / C4 / C5 with fabs, even on C5, 1.5 % slower on C2 -- the CTA's warps in lockstep share the instruction
-    // cache better than warps in different phases.  Round v of the three lists taken together goes to warp v mod (all warps).
-    __syncthreads();   // the tables are written
-    const uint32_t tpw = 32u / (uint32_t)lg.G;                 // tasks per round
-    const uint32_t slot = (uint32_t)lane / (uint32_t)lg.G;      // this lane's task of the round
-    blk_end[0] = (n_list[0] + tpw - 1) / tpw;
-    blk_end[1] = blk_end[0] + (n_list[1] + tpw - 1) / tpw;
-    blk_end[2] = blk_end[1] + (n_list[2] + tpw - 1) / tpw;
-    const uint32_t warps_per_cta = kTaskThreads / 32, total_warps = gridDim.x * warps_per_cta;
-    const uint32_t row0 = (uint32_t)(tid & ~31);
-    uint32_t dq_n = 0;   // (warp-uniform) completed sites waiting in cs.dq[warp]
-#pragma unroll 1
-    for (uint32_t v = (uint32_t)(tid >> 5) * gridDim.x + blockIdx.x; v < blk_end[2]; v += total_warps) {
-        const int li = v < blk_end[0] ? 0 : v < blk_end[1] ? 1 : 2;   // (warp-uniform) tasks of one subset size per round
-        const uint32_t idx = (v - (li ? blk_end[li - 1] : 0u)) * tpw + slot;
-        const uint32_t t = base[li] + idx;
-        const uint32_t word = idx < n_list[li] ? a.em_tasks[t] : kEmTaskInvalid;
-        const bool valid = word != kEmTaskInvalid;
-        const uint32_t hdr = word & 0x0fffffffu, subset = word >> 28;
-        EmSiteHdr* const Hg = a.em_hdr + hdr;
-        uint32_t h_nb = 0, h_off = 0;   // (only these two words of the header are needed here)
-        if (valid) { h_off = Hg->bins_off; h_nb = Hg->nb; }
-        // Staging: the tasks of a site are neighbours in the list, so one row serves a run of lanes with the same header; all 32
-        // lanes copy it (coalesced), one run after the other.  Lists longer than a row are read from the pool.
-        const uint32_t hdr_prev = __shfl_up_sync(kFull, valid ? hdr : kEmTaskInvalid, 1);
-        const bool leader = valid && (lane == 0 || hdr_prev != hdr);
-        const uint32_t lead = __ballot_sync(kFull, leader);
-        const uint32_t row = row0 + (uint32_t)__popc(lead & ((2u << lane) - 1u)) - 1u;   // row of the last leader up to this lane
-        __syncwarp();   // the previous round's readers of the warp's rows are done
-        for (uint32_t todo = lead; todo; todo &= todo - 1u) {
-            const int src = __ffs(todo) - 1;
-            const uint32_t nb = __shfl_sync(kFull, h_nb, src), off = __shfl_sync(kFull, h_off, src);
-            const uint32_t r = row0 + (uint32_t)__popc(lead & ((2u << src) - 1u)) - 1u;
-            if (nb <= (uint32_t)kStageBins)
-                for (uint32_t i = lane; i < nb; i += 32) cs.bins[r * kStageStride + i] = a.em_pool[off + i];
-        }
-        const uint32_t* bins = nullptr;
-        if (valid) bins = h_nb <= (uint32_t)kStageBins ? cs.bins + row * kStageStride : a.em_pool + h_off;
-        __syncwarp();
-        bool last = false;
-        if (valid) {
-            double* res = a.em_res + (size_t)t * kEmResDoubles;
-            if (li == 0) em_task<2>(a, lut, cs.ltab, Hg, bins, subset, res, lg);
-            else if (li == 1) em_task<3>(a, lut, cs.ltab, Hg, bins, subset, res, lg);
-            else em_task<4>(a, lut, cs.ltab, Hg, bins, subset, res, lg);
-            if (lg.gl == 0) {
-                __threadfence();
-                last = atomicSub(&Hg->remaining, 1u) == 1u;   // every task of the site has stored its result
-            }
-        }
-        // The sites this round completed wait in the warp's queue until 32 of them are there: the decision is scalar work (one lane
-        // per site), and a 4-allele site completes once per 11 tasks -- decided round by round, 3 lanes in 32 would run it.
-        // (A decision needs the task results and the single-allele log-likelihoods K4a left with the header, not the bins.)
-        const uint32_t dm = __ballot_sync(kFull, last);
-        if (dm) {
-            if (last) cs.dq[tid >> 5][dq_n + (uint32_t)__popc(dm & ((1u << lane) - 1u))] = hdr;
-            dq_n += (uint32_t)__popc(dm);
-            __syncwarp();
-            if (dq_n >= 32u) {
-                dq_n -= 32u;
-                const uint32_t d_hdr = cs.dq[tid >> 5][dq_n + (uint32_t)lane];
-                __threadfence();
-                const EmSiteHdr Hd = a.em_hdr[d_hdr];
-                uint32_t e = 0;
-                decide_site(a, Hd, d_hdr, e);
-                __syncwarp();
-                fisher_push(a, e != 0u, (e & kFisherWide) != 0u, e & ~kFisherWide);
-            }
-        }
-    }
-    {
-        uint32_t e = 0;
-        if ((uint32_t)lane < dq_n) {
-            const uint32_t d_hdr = cs.dq[tid >> 5][lane];
-            __threadfence();
-            const EmSiteHdr Hd = a.em_hdr[d_hdr];
-            decide_site(a, Hd, d_hdr, e);
-        }
-        __syncwarp();
-        fisher_push(a, e != 0u, (e & kFisherWide) != 0u, e & ~kFisherWide);
-    }
-#else
     const uint32_t tpc = (uint32_t)(kTaskThreads / lg.G);   // tasks per CTA and round
     const uint32_t slot = (uint32_t)tid / (uint32_t)lg.G;    // this thread's task of the round = its staging row
     blk_end[0] = (n_list[0] + tpc - 1) / tpc;
@@ -1059,7 +925,6 @@ __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(cons
         const uint32_t e = have ? cs.fs_site[k0 + (uint32_t)tid] : 0u;
         fisher_push(a, have, (e & kFisherWide) != 0u, e & ~kFisherWide);
     }
-#endif
 }
 
 }  // namespace bv

@@ -54,16 +54,14 @@ __device__ __forceinline__ void fisher_push(const SiteKernelArgs& a, bool pred, 
         if (pred && wide) a.list_fisher[2u * a.n_sites - 1u - (pos + __popc(mw & below))] = entry;
     }
 }
-// Which end of the list: is the support [max(0, n1_ + n_1 - n), min(n1_, n_1)] of the table (a b / c d) wider than BV_FISHER_LIST_WIDE
+// Which end of the list: is the support [max(0, n1_ + n_1 - n), min(n1_, n_1)] of the table (a b / c d) wider than kFisherListWide
 // outcomes?  24 = where the algorithm changes (fisher_fast_applicable): the reference's walk on one end, bisection + tails on the
 // other.  Splitting later (48, 96, 200: the cheap bisections with the walks, only the long tails apart) measured slower on deep pileups
 // (bv_fisher_kernel on C5: 0.256 / 0.279 / 0.315 / 0.342 ms per 10^6 sites), equal elsewhere (profiles/r02_fisher_queues.txt).
-#ifndef BV_FISHER_LIST_WIDE
-#define BV_FISHER_LIST_WIDE 24
-#endif
+constexpr int kFisherListWide = 24;
 __device__ __forceinline__ bool fisher_support_wide(int t11, int t12, int t21, int t22) {
     const int n1_ = t11 + t12, n_1 = t11 + t21, n = n1_ + t21 + t22;
-    return min(n1_, n_1) - max(0, n1_ + n_1 - n) > BV_FISHER_LIST_WIDE;
+    return min(n1_, n_1) - max(0, n1_ + n_1 - n) > kFisherListWide;
 }
 
 // The two strand tables of a site from its record: ref vs every non-reference base (CVG row, basetype_caller.cpp:1236-1245) and ref
@@ -265,10 +263,7 @@ __global__ void __launch_bounds__(256) bv_pack_kernel(const __grid_constant__ Si
 // Light kernel, high occupancy: the row's base + qual planes come through two TMA-filled buffers per warp, the next
 // unit (also the next site's first one) in flight while the current one is scanned with SIMD byte arithmetic.
 // =====================================================================================================================
-#ifndef BV_BOUND_WARPS
-#define BV_BOUND_WARPS 32
-#endif
-constexpr int kBoundWarps = BV_BOUND_WARPS;
+constexpr int kBoundWarps = 32;
 constexpr int kBChunk = 1024;                 // cells per buffer and plane: two 16-cell vectors per lane
 constexpr uint32_t kBoundLimit = 12530483u;   // floor(11.95 * 2^20)
 
@@ -413,18 +408,9 @@ __global__ void __launch_bounds__(kBoundWarps * 32, 1) bv_bound_kernel(const __g
 // =====================================================================================================================
 // K4: one warp per site of the EM list.
 // =====================================================================================================================
-#ifndef BV_QUAL_WARPS
-#define BV_QUAL_WARPS 32
-#endif
-constexpr int kQualWarps = BV_QUAL_WARPS;
-#ifndef BV_P2_CHUNK
-#define BV_P2_CHUNK 512
-#endif
-constexpr int kP2Chunk = BV_P2_CHUNK;        // cells per buffer and plane: kP2Chunk / 512 16-cell vectors per lane
-#ifndef BV_P2_BUFS
-#define BV_P2_BUFS 2
-#endif
-constexpr int kP2Bufs = BV_P2_BUFS;          // ring of row chunks per warp: kP2Bufs - 1 TMA fetches in flight ahead of the scan
+constexpr int kQualWarps = 32;
+constexpr int kP2Chunk = 512;                // cells per buffer and plane: kP2Chunk / 512 16-cell vectors per lane
+constexpr int kP2Bufs = 2;                   // ring of row chunks per warp: kP2Bufs - 1 TMA fetches in flight ahead of the scan
 
 struct __align__(128) P2Buf {                // one chunk of the base and qual planes
     uint8_t base[kP2Chunk];
@@ -551,9 +537,7 @@ __device__ __forceinline__ uint32_t hist_phred_range() {
 //   dense (deep pileups): all 16 cells straight from the registers that hold the vector, the mask bit as the predicate of
 //     the shared-memory atomic: 5 instructions per cell instead of 10 per trip.
 // The phred range is read off the histogram afterwards (96 slots, three per lane) instead of being tracked per cell.
-#ifndef BV_HIST_DENSE_TRIPS
-#define BV_HIST_DENSE_TRIPS 7
-#endif
+constexpr int kHistDenseTrips = 7;   // the dense loop once the fullest lane of a vector has this many counted cells
 // hist[idx] += 1 for the lanes with `on`, as ONE predicated instruction (no branch around it)
 __device__ __forceinline__ void hist_add_if(uint32_t hist_s, uint32_t idx, uint32_t on) {
     asm volatile(
@@ -591,7 +575,7 @@ __device__ __noinline__ uint32_t build_hist(uint32_t site, const uint8_t* grp, u
         uint32_t t = ((n0 >> 7) | (n1 >> 6) | (n2 >> 5) | (n3 >> 4)) ^ 0x0f0f0f0fu;
         // warp-uniform trip count, lanes that run out are predicated off: the warp never splits
         const int n = (int)__reduce_max_sync(kFull, (uint32_t)__popc(t));
-        if (n >= BV_HIST_DENSE_TRIPS) {
+        if (n >= kHistDenseTrips) {
             // phred > 95 shares the last slot (bytes >= 0x80 never occur next to a counted base in a valid tile; they clamp too)
             const uint4 vq = *reinterpret_cast<const uint4*>(cellp + kP2Chunk);
             const uint32_t hist_s = smem_u32(W.hist);
@@ -625,16 +609,10 @@ __device__ __noinline__ uint32_t build_hist(uint32_t site, const uint8_t* grp, u
 // vectors of a 2,048-cell chunk and walks one 64-bit mask of their 64 cells: the fullest of 32 lanes then has ~12 cells
 // where the mean is 6.4, the fetch / wait / loop overhead of a chunk is paid once per four vectors, and the warp count
 // per SM is halved to make room for the larger buffers (16 warps x 2 buffers x 4 KB).
-#ifndef BV_LONG_WARPS
-#define BV_LONG_WARPS 16
-#endif
-#ifndef BV_LONG_VPL
-#define BV_LONG_VPL 4
-#endif
-constexpr int kLongWarps = BV_LONG_WARPS;
-constexpr int kLongVpl = BV_LONG_VPL;         // 16-cell vectors per lane and chunk: 2 or 4
+constexpr int kLongWarps = 16;
+constexpr int kLongVpl = 4;                   // 16-cell vectors per lane and chunk: 2 or 4
 constexpr int kLongChunk = 512 * kLongVpl;    // cells per buffer and plane
-static_assert(kLongVpl == 2 || kLongVpl == 4, "BV_LONG_VPL must be 2 or 4");
+static_assert(kLongVpl == 2 || kLongVpl == 4, "kLongVpl must be 2 or 4");
 struct __align__(128) LongBuf {
     uint8_t base[kLongChunk];
     uint8_t qual[kLongChunk];
@@ -701,7 +679,7 @@ __device__ __noinline__ uint32_t build_hist_long(uint32_t site) {
             if (v < 2) lo |= tv; else hi |= tv;
         }
         const int n = (int)__reduce_max_sync(kFull, (uint32_t)(__popc(lo) + __popc(hi)));
-        if (n >= kLongVpl * BV_HIST_DENSE_TRIPS) {
+        if (n >= kLongVpl * kHistDenseTrips) {
 #pragma unroll
             for (int v = 0; v < kLongVpl; ++v) {
                 const uint4 vq = *reinterpret_cast<const uint4*>(cb + 512 * v + kLongChunk);
@@ -819,10 +797,8 @@ __device__ __noinline__ double em_bins(const uint32_t* bins, double* lml, int nb
 //     at least 1, i.e. when a marginal changed by a factor e: decided exactly from the ratio of the marginals -- inside
 //     (1/2.5, 2.5) no logarithm is needed, otherwise the logarithms themselves decide -- so that `log` runs once per
 //     bin and EM call (for the reported log-likelihoods) instead of once per bin and iteration.
-// out of line: the inlined libdevice log is ~90 instructions per call site and this kernel is instruction-fetch sensitive
-#ifndef BV_EM_LOG
-#define BV_EM_LOG nlog
-#endif
+// Logarithms through nlog, out of line: the inlined libdevice log is ~90 instructions per call site and this kernel is
+// instruction-fetch sensitive.
 template <int NS>
 __device__ __noinline__ double em_bins_reg(const uint32_t* bins, int nb, int subset, double total) {
     QualWarp& W = warp_smem();
@@ -891,7 +867,7 @@ __device__ __noinline__ double em_bins_reg(const uint32_t* bins, int nb, int sub
         } else {
 #pragma unroll
             for (int k = 0; k < NS; ++k) {
-                const double llh = BV_EM_LOG(mk[k]);
+                const double llh = nlog(mk[k]);
                 if (!first && on[k]) delta += cd[k] * fabs(llh - prev[k]);
                 prev[k] = llh;
             }
@@ -911,7 +887,7 @@ __device__ __noinline__ double em_bins_reg(const uint32_t* bins, int nb, int sub
     double ll = 0;
 #pragma unroll
     for (int k = 0; k < NS; ++k) {
-        const double lml = int_mode ? BV_EM_LOG(prev[k]) : prev[k];
+        const double lml = int_mode ? nlog(prev[k]) : prev[k];
         if (on[k]) ll += cd[k] * lml;
     }
     if (lane == 0) { W.emf[0] = f0; W.emf[1] = f1; W.emf[2] = f2; W.emf[3] = f3; }

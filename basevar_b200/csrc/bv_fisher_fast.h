@@ -32,21 +32,26 @@ BV_FN double ff_lbinom(const LF& lf, int n, int k) {   // kfunc.c:197-201
     return lf(n) - lf(k) - lf(n - k);
 }
 
-// num / den in the tail recurrences.  On the device: num * (1 / den) with the reciprocal from the hardware's estimate and two
-// Newton steps (~1 ulp; the correctly rounded FP64 division costs six times as many instructions and the tails are hundreds
-// of steps long on deep pileups).  The difference, a few ulp per step, is far inside the 1e-8 slack of every decision here.
-#ifndef BV_FF_RCP
-#define BV_FF_RCP 1
-#endif
-BV_FN double ff_div(double num, double den) {
-#if defined(__CUDA_ARCH__) && BV_FF_RCP
+#if defined(__CUDACC__)
+// 1 / m to ~1 ulp: the hardware's 20-bit estimate and two Newton steps (the correctly rounded division costs twice as
+// many FP64 instructions).  m == 0 gives NaN, where 1.0 / 0 gives inf: the EM posteriors 0 * inf the reference then forms
+// (bv_em_kernels.cuh) are NaN as well.
+__device__ __forceinline__ double rcp_fast(double m) {
     double r;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(den));
-    double e = fma(-den, r, 1.0);
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(m));
+    double e = fma(-m, r, 1.0);
     r = fma(r, e, r);
-    e = fma(-den, r, 1.0);
-    r = fma(r, e, r);
-    return num * r;
+    e = fma(-m, r, 1.0);
+    return fma(r, e, r);
+}
+#endif
+
+// num / den in the tail recurrences.  On the device: num * rcp_fast(den) (the correctly rounded FP64 division costs six times
+// as many instructions and the tails are hundreds of steps long on deep pileups).  The difference, a few ulp per step, is far
+// inside the 1e-8 slack of every decision here.
+BV_FN double ff_div(double num, double den) {
+#if defined(__CUDA_ARCH__)
+    return num * rcp_fast(den);
 #else
     return num / den;
 #endif

@@ -103,28 +103,17 @@ __device__ __noinline__ double hypergeo_tab(const double* __restrict__ lf, int n
 
 // kfunc.c:220-243 with only n11 moving.  The step's factor a / n11 * b / n22 is formed as (a * b) * (1 / (n11 * n22)) -- integer
 // products below 2^53, exact, and a Newton reciprocal (ff_div) -- where the reference divides twice: a few ulp per step, far inside
-// the 1e-8 slack of the comparisons the walk feeds, at a third of the instructions (BV_HG_RCP=0: the divisions).
-#ifndef BV_HG_RCP
-#define BV_HG_RCP 1
-#endif
+// the 1e-8 slack of the comparisons the walk feeds, at a third of the instructions.
 __device__ __noinline__ double hg_move(const double* __restrict__ lf, HgState& st, int n11) {
     int n22 = n11 + st.n - st.n1_ - st.n_1;
     if ((n11 % 11) && n22) {
         if (n11 == st.n11 + 1) {
-#if BV_HG_RCP
             st.p *= ff_div((double)(st.n1_ - st.n11) * (double)(st.n_1 - st.n11), (double)n11 * (double)n22);
-#else
-            st.p *= (double)(st.n1_ - st.n11) / n11 * (st.n_1 - st.n11) / n22;
-#endif
             st.n11 = n11;
             return st.p;
         }
         if (n11 == st.n11 - 1) {
-#if BV_HG_RCP
             st.p *= ff_div((double)st.n11 * (double)(st.n11 + st.n - st.n1_ - st.n_1), (double)(st.n1_ - n11) * (double)(st.n_1 - n11));
-#else
-            st.p *= (double)st.n11 / (st.n1_ - n11) * (st.n11 + st.n - st.n1_ - st.n_1) / (st.n_1 - n11);
-#endif
             st.n11 = n11;
             return st.p;
         }
