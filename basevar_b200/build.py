@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbasevar_b200.so")
 SOURCES = [os.path.join(CSRC, "bv_api.cu"), os.path.join(CSRC, "bv_encode16.cpp")]   # the .cpp goes to the host compiler as is
-DEPS = SOURCES + [os.path.join(CSRC, f) for f in ("bv_common.cuh", "bv_count_kernel.cuh", "bv_finish_kernels.cuh", "bv_em_kernels.cuh", "bv_call_kernels.cuh", "bv_expand_kernel.cuh", "bv_math.cuh",
+DEPS = SOURCES + [os.path.join(CSRC, f) for f in ("bv_common.cuh", "bv_count_kernel.cuh", "bv_finish_kernels.cuh", "bv_em_kernels.cuh", "bv_call_kernels.cuh", "bv_list_kernel.cuh", "bv_expand_kernel.cuh", "bv_math.cuh",
                                                   "bv_fisher_fast.h", "bv_synth.cuh")] + [
     os.path.join(HERE, "..", "include", "basevar_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
@@ -47,7 +47,7 @@ HOST_DEPS = HOST_SRC + [os.path.join(HERE, "host", f) for f in ("bv_host.hpp", "
 CLI = os.path.join(HERE, "bin", "basevar")   # `basevar basetype ...` over BAM files (host/bv_main.cpp)
 ROOT = os.path.dirname(HERE)
 CPP_TESTS = {"test_host_cpu": [], "test_host_gpu": ["-ldl"], "test_fisher_fast": ["-ldl", "-lm"], "test_caller_cpu": [],
-             "test_caller_gpu": ["-lz"], "pileup_dump": ["-lz"]}
+             "test_caller_gpu": ["-lz"], "pileup_dump": ["-lz"], "test_lists_gpu": ["-ldl", "-lm"]}
 
 
 def build_host(force=False):

@@ -49,6 +49,11 @@ CALL_OUT_DTYPE = np.dtype([("site", "<u4"), ("mq_rank_sum", "<i4"), ("read_pos_r
 GROUP_OUT_DTYPE = np.dtype([("n_alt", "u1"), ("alt", "u1", (4,)), ("flags", "u1"), ("reserved", "u1", (2,)), ("af", "<f8", (4,))])
 assert CALL_OUT_DTYPE.itemsize == 16 and GROUP_OUT_DTYPE.itemsize == 40
 GROUP_NONE = 255
+# struct bv_lrt_out (64 bytes): BaseType::lrt(list) of one site; lists are uint8 [n_sites][4] ended early by LIST_END
+LRT_OUT_DTYPE = np.dtype([("n_alt", "u1"), ("alt", "u1", (4,)), ("n_active", "u1"), ("flags", "u1"), ("em_calls", "u1"),
+                          ("af", "<f8", (4,)), ("qual", "<f8"), ("chi2", "<f8"), ("fs", "<f8")])
+assert LRT_OUT_DTYPE.itemsize == 64
+LIST_END = 255
 
 
 class BvParams(C.Structure):
@@ -150,6 +155,10 @@ _SIGNATURES = [
     ("bv_tile_submit_calls", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvTile), C.POINTER(BvTileAux)]),
     ("bv_tile_wait_calls", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_void_p]),
     ("bv_tile_run_device_calls", C.c_int, [C.c_void_p, C.POINTER(BvTile), C.POINTER(BvTileAux)] + [C.c_void_p] * 5),
+    ("bv_last_list_kernel_time", C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
+    ("bv_tile_submit_lists", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvTile), C.c_void_p]),
+    ("bv_tile_wait_lists", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    ("bv_tile_run_device_lists", C.c_int, [C.c_void_p, C.POINTER(BvTile)] + [C.c_void_p] * 4),
     ("bv_synth_fill_rpr_device", C.c_int, [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p, C.c_void_p]),
     ("bv_synth_fill_rpr_host", C.c_int, [C.POINTER(BvSynthModel), C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p]),
     ("bv_synth_set_model", C.c_int, [C.c_void_p, C.POINTER(BvSynthModel)]),

@@ -20,6 +20,7 @@
 #include "bv_finish_kernels.cuh"
 #include "bv_em_kernels.cuh"
 #include "bv_call_kernels.cuh"
+#include "bv_list_kernel.cuh"
 #include "bv_expand_kernel.cuh"
 #include "bv_synth.cuh"
 
@@ -138,6 +139,12 @@ struct bv_slot {
     uint32_t* h_counters = nullptr;       // copy of the scratch counters (kCntCalled = number of calls)
     uint8_t* d_aux = nullptr;             // mapq | rpr planes of pageable host tiles (allocated on first use)
     bool with_calls = false;
+    // per-site candidate lists (bv_tile_submit_lists): allocated on first use
+    uint32_t* h_lists = nullptr;          // [max_sites] pinned staging of the tile's lists, one word per site
+    uint32_t* d_lists = nullptr;          // [max_sites]
+    bv_lrt_out* d_lrt = nullptr;          // [max_sites]
+    bv_lrt_out* h_lrt = nullptr;          // [max_sites] pinned
+    bool with_lists = false;
     // sparse tiles (bv_tile_submit_sparse): the covered cells as uploaded, expanded into d_planes by K0
     uint32_t* d_cells = nullptr;          // [cells_cap] cells, then [cells_cap] aux words
     uint32_t* d_site_start = nullptr;     // [max_sites + 1]
@@ -180,6 +187,9 @@ struct bv_ctx {
     uint32_t n_groups = 0;
     cudaEvent_t ev_call[3] = {nullptr, nullptr, nullptr};
     bool ev_call_valid = false;
+    cudaEvent_t ev_list[2] = {nullptr, nullptr};   // around K8 bv_list_kernel
+    bool ev_list_valid = false;
+    bool list_kernel_ready = false;   // bv_list_kernel's shared-memory attribute is set (first lists tile)
     cudaStream_t copy_stream = nullptr;   // uploads of sparse host tiles, in submit order (see tile_submit_sparse_impl)
     bool trace = false;               // BASEVAR_B200_TRACE=1: one line per sparse host tile on stderr at its wait
     cudaEvent_t ev_trace0 = nullptr;  // recorded at the first traced submit: the origin of the timeline
@@ -421,6 +431,41 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
     return BV_OK;
 }
 
+// K8 after the standard kernels of the tile (it reads their records): one warp per site with a non-empty list.
+static int launch_list_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const uint32_t* d_lists, bv_lrt_out* d_lrt, cudaStream_t stream) {
+    BvRange range("bv: launch K8 list");
+    if (a.n_sites == 0) return BV_OK;
+    if (a.n_samples == 0) {   // no reads anywhere: every entry is all-zero
+        BV_CUDA(ctx, cudaMemsetAsync(d_lrt, 0, (size_t)a.n_sites * sizeof(bv_lrt_out), stream));
+        return BV_OK;
+    }
+    if (!ctx->list_kernel_ready) {   // on first use: a context that never runs K8 loads and sets up exactly what it did without it
+        BV_CUDA(ctx, cudaFuncSetAttribute(bv::bv_list_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
+        ctx->list_kernel_ready = true;
+    }
+    const bool prof = ctx->profiling;
+    if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[0], stream));
+    uint32_t grid = (a.n_sites + bv::kQualWarps - 1) / bv::kQualWarps;
+    if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;   // (the bin spill rows are sized for this grid)
+    bv::bv_list_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_lists, d_lrt);
+    BV_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[1], stream)); ctx->ev_list_valid = true; }
+    return BV_OK;
+}
+
+// Host check of a tile's lists (what the kernel would otherwise treat as empty): BV_OK or BV_ERR_ARG.
+static int check_lists(bv_ctx* ctx, const uint8_t (*lists)[4], uint32_t n_sites) {
+    for (uint32_t i = 0; i < n_sites; ++i) {
+        uint32_t w, order;
+        memcpy(&w, lists[i], 4);
+        if (bv::list_decode(w, order) < 0)
+            return set_err(ctx, BV_ERR_ARG, "lists[%u] = {%u, %u, %u, %u}: a base repeats or a code is neither 0..3 nor BV_LIST_END", i,
+                           lists[i][0], lists[i][1], lists[i][2], lists[i][3]);
+    }
+    return BV_OK;
+}
+
 // The cells of one site, words16 known to have room for the worst case.  The common cell -- ascending, gap < 31, strand + or - --
 // is one load, a few shifts and one store; everything else leaves through the slow path of the caller.
 template <bool AUX>
@@ -489,10 +534,12 @@ int bv_set_profiling(bv_ctx* ctx, int on) {
     if (on && !ctx->ev[0]) {
         for (int i = 0; i < 7; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev[i]));
         for (int i = 0; i < 3; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev_call[i]));
+        for (int i = 0; i < 2; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev_list[i]));
     }
     ctx->profiling = on != 0;
     ctx->ev_valid = false;
     ctx->ev_call_valid = false;
+    ctx->ev_list_valid = false;
     return BV_OK;
 }
 
@@ -502,6 +549,15 @@ int bv_last_call_kernel_times(bv_ctx* ctx, float ms[2]) {
     BV_CUDA(ctx, cudaSetDevice(ctx->device));
     BV_CUDA(ctx, cudaEventSynchronize(ctx->ev_call[2]));
     for (int i = 0; i < 2; ++i) BV_CUDA(ctx, cudaEventElapsedTime(&ms[i], ctx->ev_call[i], ctx->ev_call[i + 1]));
+    return BV_OK;
+}
+
+int bv_last_list_kernel_time(bv_ctx* ctx, float* ms) {
+    if (!ctx || !ms) return set_err(ctx, BV_ERR_ARG, "null argument");
+    if (!ctx->ev_list_valid) return set_err(ctx, BV_ERR_STATE, "no profiled tile with the list kernel yet");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    BV_CUDA(ctx, cudaEventSynchronize(ctx->ev_list[1]));
+    BV_CUDA(ctx, cudaEventElapsedTime(ms, ctx->ev_list[0], ctx->ev_list[1]));
     return BV_OK;
 }
 
@@ -665,6 +721,9 @@ void bv_destroy(bv_ctx* ctx) {
             if (s.h_groups) cudaFreeHost(s.h_groups);
             if (s.h_counters) cudaFreeHost(s.h_counters);
             cudaFree(s.d_aux);
+            if (s.h_lists) cudaFreeHost(s.h_lists);
+            if (s.h_lrt) cudaFreeHost(s.h_lrt);
+            cudaFree(s.d_lists); cudaFree(s.d_lrt);
             cudaFree(s.d_cells); cudaFree(s.d_site_start);
             for (int k = 0; k < 4; ++k) if (s.ev_trace[k]) cudaEventDestroy(s.ev_trace[k]);
             if (s.ev_up) cudaEventDestroy(s.ev_up);
@@ -675,6 +734,7 @@ void bv_destroy(bv_ctx* ctx) {
     scratch_free(ctx->dev_scratch);
     for (int i = 0; i < 7; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 3; ++i) if (ctx->ev_call[i]) cudaEventDestroy(ctx->ev_call[i]);
+    for (int i = 0; i < 2; ++i) if (ctx->ev_list[i]) cudaEventDestroy(ctx->ev_list[i]);
     if (ctx->ev_trace0) cudaEventDestroy(ctx->ev_trace0);
     if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
     delete ctx;
@@ -751,7 +811,8 @@ int bv_set_groups(bv_ctx* ctx, const uint8_t* sample_group, uint32_t n_samples, 
     return BV_OK;
 }
 
-static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls);
+static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls,
+                            const uint8_t (*lists)[4] = nullptr);
 
 int bv_tile_submit(bv_ctx* ctx, int slot, const bv_tile* tile) { return tile_submit_impl(ctx, slot, tile, nullptr, false); }
 
@@ -768,7 +829,8 @@ static const void* host_device_pointer(const void* p) {
     return nullptr;
 }
 
-static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls) {
+static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls,
+                            const uint8_t (*lists)[4]) {
     BvRange range("bv_tile_submit (dense tile: H2D, kernels, D2H)");
     if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
     if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
@@ -783,6 +845,19 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
     s.compact = tile->location == BV_LOC_HOST && tile->out_mode == BV_OUT_COMPACT;
     s.h_ref = tile->location == BV_LOC_HOST ? tile->ref_base : nullptr;
     if (s.compact && with_calls) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT is not available with the called-site kernels");
+    if (lists) {   // checked and staged before anything is queued: a refused tile leaves the slot as it was
+        if (tile->out_mode != BV_OUT_RECORDS) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: out_mode must be BV_OUT_RECORDS");
+        int rc = check_lists(ctx, lists, tile->n_sites);
+        if (rc != BV_OK) return rc;
+        if (!s.h_lists) {
+            const size_t n = ctx->prm.max_sites;
+            BV_CUDA(ctx, cudaHostAlloc(&s.h_lists, n * sizeof(uint32_t), cudaHostAllocDefault));
+            BV_CUDA(ctx, cudaHostAlloc(&s.h_lrt, n * sizeof(bv_lrt_out), cudaHostAllocDefault));
+            BV_CUDA(ctx, cudaMalloc(&s.d_lists, n * sizeof(uint32_t)));
+            BV_CUDA(ctx, cudaMalloc(&s.d_lrt, n * sizeof(bv_lrt_out)));
+        }
+        if (tile->n_sites) memcpy(s.h_lists, lists, (size_t)tile->n_sites * sizeof(uint32_t));
+    }
     bv_tile dev = *tile;
     if (tile->location == BV_LOC_HOST) {
         if (!tile->base || !tile->qual || !tile->strand || !tile->ref_base) return set_err(ctx, BV_ERR_ARG, "bv_tile: null pointer");
@@ -848,6 +923,12 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
     }
     rc = launch_site_kernel(ctx, a, s.stream);
     if (rc != BV_OK) return rc;
+    if (lists && tile->n_sites) {
+        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, (size_t)tile->n_sites * sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
+        rc = launch_list_kernel(ctx, a, s.d_lists, s.d_lrt, s.stream);
+        if (rc != BV_OK) return rc;
+        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)tile->n_sites * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
+    }
     rc = return_records(ctx, s, a, tile->n_sites, s.h_out);
     if (rc != BV_OK) return rc;
     if (with_calls || s.compact) {
@@ -856,6 +937,7 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
             BV_CUDA(ctx, cudaMemcpyAsync(s.h_counters, a.counters, bv::kNumCounters * sizeof(uint32_t), cudaMemcpyDeviceToHost, s.stream));
     }
     s.with_calls = with_calls;
+    s.with_lists = lists != nullptr;
     s.n_sites = tile->n_sites;
     s.busy = true;
     if (tile->location == BV_LOC_HOST) ctx->h2d_bytes_total += s.h2d_bytes;
@@ -979,6 +1061,7 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
     }
     if (trace) BV_CUDA(ctx, cudaEventRecord(s.ev_trace[3], s.stream));
     s.with_calls = with_calls;
+    s.with_lists = false;
     s.n_sites = t->n_sites;
     s.busy = true;
     ctx->h2d_bytes_total += s.h2d_bytes;
@@ -1158,6 +1241,39 @@ int bv_tile_wait_calls(bv_ctx* ctx, int slot, bv_site_out* out, bv_call_out* cal
     if (n && calls) memcpy(calls, s.h_calls, (size_t)n * sizeof(bv_call_out));
     if (n && groups && ctx->n_groups && s.h_groups) memcpy(groups, s.h_groups, (size_t)n * ctx->n_groups * sizeof(bv_group_out));
     return BV_OK;
+}
+
+int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8_t (*lists)[4]) {
+    if (!lists) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: null lists");
+    return tile_submit_impl(ctx, slot, tile, nullptr, false, lists);
+}
+
+int bv_tile_wait_lists(bv_ctx* ctx, int slot, bv_site_out* out, bv_lrt_out* lrt_out) {
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    if (!lrt_out) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists: null lrt_out");
+    bv_slot& s = ctx->slots[slot];
+    if (s.busy && !s.with_lists) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without lists", slot);
+    int rc = bv_tile_wait(ctx, slot, out);
+    if (rc != BV_OK) return rc;
+    if (s.n_sites) memcpy(lrt_out, s.h_lrt, (size_t)s.n_sites * sizeof(bv_lrt_out));
+    return BV_OK;
+}
+
+int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d_lists)[4], bv_site_out* d_out,
+                             bv_lrt_out* d_lrt_out, void* stream) {
+    BvRange range("bv_tile_run_device_lists");
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: tile must be device resident");
+    if (tile && tile->n_sites && (!d_lists || !d_lrt_out)) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: null lists / output");
+    if (((uintptr_t)d_lists) & 3) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: d_lists must be 4-byte aligned");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    bv::SiteKernelArgs a;
+    int rc = fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, &a);
+    if (rc != BV_OK) return rc;
+    rc = launch_site_kernel(ctx, a, (cudaStream_t)stream);
+    if (rc != BV_OK) return rc;
+    return launch_list_kernel(ctx, a, reinterpret_cast<const uint32_t*>(d_lists), d_lrt_out, (cudaStream_t)stream);
 }
 
 int bv_synth_fill_rpr_device(bv_ctx* ctx, uint64_t site0, uint32_t n_sites, uint32_t n_samples, uint64_t rpr_pitch,

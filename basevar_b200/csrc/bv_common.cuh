@@ -24,7 +24,7 @@
 //        (one per tail), the tests over wide supports (bisection + tail sums) apart from those over narrow ones (the
 //        reference's walk), so that every warp runs one path.
 //   K5 / K6 (bv_call_kernels.cuh) rank sums and population-group frequencies of the called sites; K7 bv_pack_kernel
-//        (bv_finish_kernels.cuh) the compact result transport.
+//        (bv_finish_kernels.cuh) the compact result transport; K8 bv_list_kernel (bv_list_kernel.cuh) lrt(list) per site.
 //
 // Work moves between the kernels through compact lists of site indices (appended with warp-aggregated atomics, so their
 // order varies from run to run; every site is independent, so the records do not).  The record's `reserved0` word

@@ -11,7 +11,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .capi import BvError, BvSparseTile, BvTile, BvTileAux, CALL_OUT_DTYPE, GROUP_OUT_DTYPE, SITE_OUT_DTYPE
+from .capi import BvError, BvSparseTile, BvTile, BvTileAux, CALL_OUT_DTYPE, GROUP_OUT_DTYPE, LRT_OUT_DTYPE, SITE_OUT_DTYPE
 
 
 def _ptr(a):
@@ -309,6 +309,49 @@ class BaseTypeEngine:
         groups = np.concatenate(groups) if groups else np.zeros((0, G), GROUP_OUT_DTYPE)
         order = np.argsort(calls["site"], kind="stable")
         return out, calls[order], groups[order]
+
+    # -- lrt(specific_bases): per-site ordered candidate lists -------------------------------------------
+    def call_host_lists(self, base, qual, strand, ref_base, lists, n_samples):
+        """Like call_host, plus BaseType::lrt(list) of every site.  lists: uint8 [S][4], 1..4 distinct base codes per site
+        in caller order, ended early by capi.LIST_END (a row of LIST_END skips the site).
+        Returns (records, lrt_out: capi.LRT_OUT_DTYPE [S])."""
+        S, pitch = base.shape
+        lists = np.ascontiguousarray(lists, np.uint8)
+        assert lists.shape == (S, 4)
+        out = np.zeros(S, dtype=SITE_OUT_DTYPE)
+        lrt = np.zeros(S, dtype=LRT_OUT_DTYPE)
+        n_slots, step = self.params.n_slots, self.params.max_sites
+        assert n_slots >= 1 and step >= 1, "engine was created without slots"
+        pending, slot = [], 0
+
+        def wait(ps, p0):
+            self._check(self.lib.bv_tile_wait_lists(self._ctx, ps, out[p0:].ctypes.data, lrt[p0:].ctypes.data), "bv_tile_wait_lists")
+
+        for s0 in range(0, max(S, 1), step):
+            ns = min(step, S - s0)
+            if len(pending) == n_slots:
+                wait(*pending.pop(0))
+            t = BvTile(base[s0:].ctypes.data, qual[s0:].ctypes.data, strand[s0:].ctypes.data, ref_base[s0:].ctypes.data, pitch, ns,
+                       n_samples, capi.BV_LOC_HOST, 0)
+            self._check(self.lib.bv_tile_submit_lists(self._ctx, slot, C.byref(t), lists[s0:].ctypes.data), "bv_tile_submit_lists")
+            pending.append((slot, s0))
+            slot = (slot + 1) % n_slots
+        for ps, p0 in pending:
+            wait(ps, p0)
+        return out, lrt
+
+    def call_device_lists(self, d_base, d_qual, d_strand, d_ref, d_lists, n_sites, n_samples, pitch, d_out, d_lrt_out, stream=0):
+        """Device-resident call_host_lists: every argument a device pointer (int); d_lists uint8 [n_sites][4], d_lrt_out
+        n_sites LRT_OUT_DTYPE entries.  Asynchronous on `stream` (a cudaStream_t handle)."""
+        t = BvTile(int(d_base), int(d_qual), int(d_strand), int(d_ref), pitch, n_sites, n_samples, capi.BV_LOC_DEVICE, 0)
+        self._check(self.lib.bv_tile_run_device_lists(self._ctx, C.byref(t), C.c_void_p(int(d_lists)), C.c_void_p(int(d_out)),
+                                                      C.c_void_p(int(d_lrt_out)), C.c_void_p(int(stream))), "bv_tile_run_device_lists")
+
+    def last_list_kernel_time(self):
+        """Duration (ms) of K8 bv_list_kernel of the most recent lists tile (profiling must be on); waits for it."""
+        ms = C.c_float(0.0)
+        self._check(self.lib.bv_last_list_kernel_time(self._ctx, C.byref(ms)), "bv_last_list_kernel_time")
+        return float(ms.value)
 
     # -- device-resident tiles ---------------------------------------------------------------------
     def call_device(self, d_base, d_qual, d_strand, d_ref, n_sites, n_samples, pitch, d_out, stream=0):

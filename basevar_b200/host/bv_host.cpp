@@ -174,6 +174,12 @@ std::vector<bv_site_out> Context::run(const bv_sparse_tile& tile) {
     wait(0, out.data());
     return out;
 }
+void Context::submit_lists(int slot, const bv_tile& tile, const uint8_t (*lists)[4]) {
+    check(bv_tile_submit_lists(ctx_, slot, &tile, lists), ctx_, "bv_tile_submit_lists");
+}
+void Context::wait_lists(int slot, bv_site_out* out, bv_lrt_out* lrt_out) {
+    check(bv_tile_wait_lists(ctx_, slot, out, lrt_out), ctx_, "bv_tile_wait_lists");
+}
 uint64_t Context::launch_count() const { return bv_launch_count(ctx_); }
 double Context::fisher_fs(int ref_fwd, int ref_rev, int alt_fwd, int alt_rev) {
     const int32_t t[4] = {ref_fwd, ref_rev, alt_fwd, alt_rev};
@@ -197,12 +203,9 @@ struct OneSite {   // the calling thread's default context for the one-site drop
     uint32_t n = 0;
 };
 thread_local OneSite t_one;
-}  // namespace
 
-BaseType::BaseType(const BatchInfo* bi, double af)
-    : ref_id_(bi->ref_id), ref_base_(bi->ref_base), ref_pos_(bi->ref_pos) {
-    const float maf = (float)af;
-    const uint32_t n = (uint32_t)bi->n;
+// the calling thread's one-site context and packer, made fit for min_af `maf` and rows of n samples
+void one_site_prepare(float maf, uint32_t n) {
     if (!t_one.ctx || t_one.min_af != maf || t_one.n < n) {
         const char* d = getenv("BASEVAR_B200_DEVICE");
         t_one.ctx.reset();
@@ -214,19 +217,68 @@ BaseType::BaseType(const BatchInfo* bi, double af)
     }
     if (!t_one.packer || t_one.packer->n_samples() != n) t_one.packer.reset(new TilePacker(n, 1));
     t_one.packer->clear();
+}
+}  // namespace
+
+BaseType::BaseType(const BatchInfo* bi, double af)
+    : ref_id_(bi->ref_id), ref_base_(bi->ref_base), ref_pos_(bi->ref_pos) {
+    const float maf = (float)af;
+    const uint32_t n = (uint32_t)bi->n;
+    one_site_prepare(maf, n);
     t_one.packer->add_site(*bi);   // throws on a malformed base string, like the reference's constructor
-    rec_ = t_one.ctx->run(t_one.packer->tile())[0];
+    const bv_tile t = t_one.packer->tile();
+    rec_ = t_one.ctx->run(t)[0];
+    row_base_.assign(t.base, t.base + n);
+    row_qual_.assign(t.qual, t.qual + n);
+    row_strand_.assign(t.strand, t.strand + n);
+    row_ref_ = (char)t.ref_base[0];
+    min_af_ = maf;
+    has_row_ = true;
     // the constructor gives depths; ALT / AF / QUAL appear with lrt() (src/basetype.cpp:130)
     total_depth_ = (int)(rec_.depth[0] + rec_.depth[1] + rec_.depth[2] + rec_.depth[3] + rec_.depth_other);
 }
 
 void BaseType::lrt(const std::vector<char>& specific_bases) {
-    if (specific_bases != BASES)
-        throw std::invalid_argument("[ERROR] lrt() over a subset of bases is not computed on the device (pop-group path)");
+    if (specific_bases != BASES) {
+        if (!has_row_)
+            throw std::invalid_argument("[ERROR] lrt() over a list other than A,C,G,T needs the site's reads: build the BaseType "
+                                        "from a BatchInfo and min_af");
+        lrt_list(specific_bases);
+        return;
+    }
     if (rec_.flags & BV_FLAG_ZERO_SUBSET)   // src/basetype.cpp:113-115
         throw std::runtime_error("[ERROR] The sum of frequence of active bases must always > 0. Check: ");
     if (lrt_done_) return;   // (the reference appends the ALT alleles again on a second call; nobody relies on that)
     fill_from_record();
+    lrt_done_ = true;
+}
+
+void BaseType::lrt_list(const std::vector<char>& specific_bases) {
+    uint8_t list[1][4] = {{BV_LIST_END, BV_LIST_END, BV_LIST_END, BV_LIST_END}};
+    int n = 0;
+    for (size_t i = 0; i < specific_bases.size(); ++i) {
+        const char c = specific_bases[i];
+        for (size_t j = 0; j < i; ++j)
+            if (specific_bases[j] == c) throw std::invalid_argument(std::string("[ERROR] lrt(): base '") + c + "' is listed twice");
+        const int code = c == 'A' ? 0 : c == 'C' ? 1 : c == 'G' ? 2 : c == 'T' ? 3 : -1;
+        if (code >= 0) list[0][n++] = (uint8_t)code;   // any other character has no depth entry: never active (basetype.cpp:137)
+    }
+    const uint32_t N = (uint32_t)row_base_.size();
+    one_site_prepare(min_af_, N);
+    t_one.packer->add_site_cells(row_ref_, row_base_.data(), row_qual_.data(), row_strand_.data(), nullptr);
+    bv_lrt_out lo;
+    t_one.ctx->submit_lists(0, t_one.packer->tile(), list);
+    t_one.ctx->wait_lists(0, nullptr, &lo);
+    if (lo.flags & BV_FLAG_ZERO_SUBSET)   // src/basetype.cpp:113-115
+        throw std::runtime_error("[ERROR] The sum of frequence of active bases must always > 0. Check: ");
+    alt_bases_.clear();
+    af_by_lrt_.clear();
+    for (int k = 0; k < lo.n_alt && k < 4; ++k) {
+        const char b = BASES[lo.alt[k] & 3];
+        alt_bases_.push_back(b);
+        af_by_lrt_[b] = lo.af[k];
+    }
+    var_qual_ = lo.qual;
     lrt_done_ = true;
 }
 

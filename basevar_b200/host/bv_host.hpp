@@ -156,6 +156,9 @@ public:
     std::vector<bv_site_out> run(const bv_tile& tile);   // submit + wait on slot 0
     void submit(int slot, const bv_sparse_tile& tile);   // sparse transport of the same tile (kernel K0 expands it)
     std::vector<bv_site_out> run(const bv_sparse_tile& tile);
+    // the same plus BaseType::lrt(list) per site (bv_tile_submit_lists): lists[n_sites][4], BV_LIST_END-terminated
+    void submit_lists(int slot, const bv_tile& tile, const uint8_t (*lists)[4]);
+    void wait_lists(int slot, bv_site_out* out, bv_lrt_out* lrt_out);
     uint32_t n_slots() const { return n_slots_; }
     uint64_t launch_count() const;
     bv_ctx* raw() { return ctx_; }
@@ -180,7 +183,11 @@ public:
     BaseType(const BatchInfo* smp_bi, double af);
 
     void lrt() { lrt(BASES); }                              // src/basetype.h:117
-    void lrt(const std::vector<char>& specific_bases);      // only the full set {A,C,G,T} is computed on the device
+    // Any ordered list (src/basetype.h:118, the population-group path's lrt([REF, ALT...])): the site's row runs again with
+    // the list on the calling thread's context (bv_tile_submit_lists).  A/C/G/T map to base codes; any other character is
+    // never active (it has no depth entry).  A repeated character throws std::invalid_argument.  Needs the reads: a
+    // BaseType built from a record alone throws std::invalid_argument for any list other than {A,C,G,T}.
+    void lrt(const std::vector<char>& specific_bases);
 
     bool is_only_snp() const { return true; }
     const std::string& get_ref_id() const { return ref_id_; }
@@ -195,6 +202,7 @@ public:
 
 private:
     void fill_from_record();
+    void lrt_list(const std::vector<char>& specific_bases);
     std::string ref_id_, ref_base_;
     uint32_t ref_pos_ = 0;
     std::vector<char> alt_bases_;
@@ -203,6 +211,11 @@ private:
     int total_depth_ = 0;
     bool lrt_done_ = false;
     bv_site_out rec_{};
+    // drop-in path: the site's encoded row, kept for lrt(list) (the reference's BatchInfo is only borrowed by the ctor)
+    std::vector<uint8_t> row_base_, row_qual_, row_strand_;
+    char row_ref_ = 'N';
+    float min_af_ = 0.f;
+    bool has_row_ = false;
 };
 
 // strand_bias(ref, ALT string) from a device record (src/basetype.cpp:244-295).  The counts come from the record's 2x4

@@ -24,6 +24,8 @@
  *     (MQRankSum/ReadPosRankSum/BaseQRankSum of the VCF row, src/basetype_caller.cpp:1151-1157)
  *   __gb(): BaseType on one population  src/basetype_caller.cpp:767-797   bv_set_groups + bv_tile_submit_calls
  *     group + lrt([REF, ALT...])        src/basetype_caller.cpp:747-760   (group kernel), bv_group_out
+ *   BaseType::lrt(specific_bases)       src/basetype.h:118               bv_tile_submit_lists / bv_tile_run_device_lists
+ *     (any ordered candidate list)      src/basetype.cpp:130-199         (list kernel K8), bv_lrt_out
  *
  * Everything is `extern "C"`, plain pointers and sizes, POD structs; no exception crosses the
  * boundary.  Every entry point returns BV_OK (0) or a negative status; bv_last_error() gives text.
@@ -197,6 +199,33 @@ typedef struct bv_group_out {
 #define BV_GROUP_NONE 255    /* sample belongs to no population group */
 #define BV_MAX_GROUPS 254
 
+/* One per site of a lists submit: BaseType(row, min_af) + lrt(list) over that site's ordered candidate list
+ * (src/basetype.h:117-118, src/basetype.cpp:130-199).  64 bytes.
+ *   active  = the list entries with depth/total >= min_af, in LIST order (total includes depth_other; 0 => none);
+ *   EM + backward elimination over `active`, subsets in list order (src/external/combinations.h), first minimum kept;
+ *   ALT     = active bases, in list order, that are not toupper(REF); af[k] = get_lrt_af(alt[k]);
+ *   qual    = get_var_qual(): 5000 (BV_FLAG_MONO_QUAL) for one active base at total > 10 and depth/total > 0.5,
+ *             else -10 log10 of the chi-square survival function of `chi2`; 0 when n_alt == 0;
+ *   fs      = FS of strand_bias(REF, ALT set) from the record's strand table, as bv_fisher_fs computes it; 0 if !n_alt.
+ * flags: BV_FLAG_ZERO_SUBSET / NEAR_LRT / LRT_TIE / EM_MAXITER / MONO_QUAL of this call, plus the row's BAD_QUAL and
+ * BAD_STRAND.  A site with an empty list, or without counted reads, gets an all-zero entry.
+ * Departure from the reference (which does not define the case): a list with a repeated base or a code outside
+ * BV_BASE_A..BV_BASE_T is refused with BV_ERR_ARG by bv_tile_submit_lists. */
+typedef struct bv_lrt_out {
+    uint8_t n_alt;
+    uint8_t alt[4];          /* base codes, in list order                                                          */
+    uint8_t n_active;        /* |active set| after backward elimination                                            */
+    uint8_t flags;           /* BV_FLAG_*                                                                          */
+    uint8_t em_calls;        /* EM invocations of this call (saturating)                                           */
+    double  af[4];
+    double  qual;
+    double  chi2;            /* last chi_sqrt_value of the elimination loop (0 when it did not run)                 */
+    double  fs;
+} bv_lrt_out;
+
+/* lists[site][4]: 1..4 distinct base codes in caller order, ended early by BV_LIST_END (an empty list skips the site) */
+#define BV_LIST_END 255
+
 typedef struct bv_ctx bv_ctx;
 
 /* ---- lifecycle --------------------------------------------------------------------------------- */
@@ -216,6 +245,7 @@ int         bv_last_kernel_times(bv_ctx* ctx, float ms[4]);
 int         bv_last_em_kernel_times(bv_ctx* ctx, float ms[2]);
 int         bv_last_fisher_kernel_time(bv_ctx* ctx, float* ms);
 int         bv_last_call_kernel_times(bv_ctx* ctx, float ms[2]);   /* K5 rank sums, K6 population groups */
+int         bv_last_list_kernel_time(bv_ctx* ctx, float* ms);      /* K8 bv_list_kernel of the last lists tile */
 
 /* ---- tile pipeline (replaces: BatchInfo -> BaseType ctor -> lrt() -> strand_bias per site) ------ */
 /* Asynchronous.  Host tiles are copied H2D on the slot's stream (pinned memory makes the copy truly
@@ -319,6 +349,20 @@ int bv_tile_wait_calls(bv_ctx* ctx, int slot, bv_site_out* out, bv_call_out* cal
  * are device pointers; d_groups may be NULL when no groups are set).  Stream ordered. */
 int bv_tile_run_device_calls(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux* aux, bv_site_out* d_out,
                              bv_call_out* d_calls, bv_group_out* d_groups, uint32_t* d_n_calls, void* stream);
+
+/* ---- lrt(specific_bases): per-site ordered candidate lists ----------------------------------------------- */
+/* bv_tile_submit + the list kernel (K8 bv_list_kernel), which runs after the standard kernels and reads the depths and
+ * strand counts of their records.  The records are the same bytes a plain bv_tile_submit gives.  lists: n_sites x 4
+ * bytes in host memory, read during the call.  BV_ERR_ARG (nothing submitted, the slot stays free) for a repeated
+ * base or a code that is neither BV_BASE_A..T nor BV_LIST_END.  Dense tiles with out_mode BV_OUT_RECORDS only. */
+int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8_t (*lists)[4]);
+/* Blocks; `out` receives n_sites records (may be NULL), `lrt_out` n_sites bv_lrt_out entries. */
+int bv_tile_wait_lists(bv_ctx* ctx, int slot, bv_site_out* out, bv_lrt_out* lrt_out);
+/* Device-resident variant: tile planes, d_lists [n_sites][4] (4-byte aligned), d_out and d_lrt_out are device pointers.
+ * Stream ordered, so the lists are not seen before the kernel runs: a list the host entry points would refuse is treated
+ * as an empty one here (all-zero entry). */
+int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d_lists)[4], bv_site_out* d_out,
+                             bv_lrt_out* d_lrt_out, void* stream);
 
 /* ---- synthetic pileups --------------------------------------------------------------------------- */
 int bv_synth_set_model(bv_ctx* ctx, const bv_synth_model* model);
