@@ -47,7 +47,8 @@ HOST_DEPS = HOST_SRC + [os.path.join(HERE, "host", f) for f in ("bv_host.hpp", "
 CLI = os.path.join(HERE, "bin", "basevar")   # `basevar basetype ...` over BAM files (host/bv_main.cpp)
 ROOT = os.path.dirname(HERE)
 CPP_TESTS = {"test_host_cpu": [], "test_host_gpu": ["-ldl"], "test_fisher_fast": ["-ldl", "-lm"], "test_caller_cpu": [],
-             "test_caller_gpu": ["-lz"], "pileup_dump": ["-lz"], "test_lists_gpu": ["-ldl", "-lm"]}
+             "test_caller_gpu": ["-lz"], "pileup_dump": ["-lz"], "test_lists_gpu": ["-ldl", "-lm"],
+             "test_ranksum_gpu": ["-ldl", "-lm"]}
 
 
 def build_host(force=False):

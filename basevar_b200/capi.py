@@ -173,6 +173,8 @@ _SIGNATURES = [
                                             C.c_uint64, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]),
     ("bv_suggest_tile_sites", C.c_uint32, [C.c_void_p, C.c_uint32, C.c_uint64]),
     ("bv_fisher_fs", C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
+    ("bv_ranksum_test", C.c_int, [C.c_void_p] * 6 + [C.c_uint32, C.c_void_p]),
+    ("bv_last_ranksum_kernel_time", C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     ("bv_host_alloc", C.c_int, [C.POINTER(C.c_void_p), C.c_size_t]),
     ("bv_host_free", C.c_int, [C.c_void_p]),
 ]

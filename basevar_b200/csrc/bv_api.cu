@@ -190,6 +190,17 @@ struct bv_ctx {
     cudaEvent_t ev_list[2] = {nullptr, nullptr};   // around K8 bv_list_kernel
     bool ev_list_valid = false;
     bool list_kernel_ready = false;   // bv_list_kernel's shared-memory attribute is set (first lists tile)
+    // free-standing rank-sum tests (bv_ranksum_test): stream and device scratch made on first use, grown only
+    cudaStream_t rs_stream = nullptr;
+    uint8_t* d_rs_bases = nullptr;    // [rs_entries_cap]
+    int32_t* d_rs_values = nullptr;   // [rs_entries_cap]
+    uint64_t* d_rs_start = nullptr;   // [rs_problems_cap + 1]
+    uint8_t* d_rs_ref = nullptr;      // [rs_problems_cap] REF characters, then [rs_problems_cap] ALT masks
+    double* d_rs_out = nullptr;       // [rs_problems_cap]
+    uint64_t rs_entries_cap = 0;
+    uint32_t rs_problems_cap = 0;
+    cudaEvent_t ev_rs[2] = {nullptr, nullptr};   // around K9 bv_ranksum_test_kernel
+    bool ev_rs_valid = false;
     cudaStream_t copy_stream = nullptr;   // uploads of sparse host tiles, in submit order (see tile_submit_sparse_impl)
     bool trace = false;               // BASEVAR_B200_TRACE=1: one line per sparse host tile on stderr at its wait
     cudaEvent_t ev_trace0 = nullptr;  // recorded at the first traced submit: the origin of the timeline
@@ -535,11 +546,13 @@ int bv_set_profiling(bv_ctx* ctx, int on) {
         for (int i = 0; i < 7; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev[i]));
         for (int i = 0; i < 3; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev_call[i]));
         for (int i = 0; i < 2; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev_list[i]));
+        for (int i = 0; i < 2; ++i) BV_CUDA(ctx, cudaEventCreate(&ctx->ev_rs[i]));
     }
     ctx->profiling = on != 0;
     ctx->ev_valid = false;
     ctx->ev_call_valid = false;
     ctx->ev_list_valid = false;
+    ctx->ev_rs_valid = false;
     return BV_OK;
 }
 
@@ -558,6 +571,15 @@ int bv_last_list_kernel_time(bv_ctx* ctx, float* ms) {
     BV_CUDA(ctx, cudaSetDevice(ctx->device));
     BV_CUDA(ctx, cudaEventSynchronize(ctx->ev_list[1]));
     BV_CUDA(ctx, cudaEventElapsedTime(ms, ctx->ev_list[0], ctx->ev_list[1]));
+    return BV_OK;
+}
+
+int bv_last_ranksum_kernel_time(bv_ctx* ctx, float* ms) {
+    if (!ctx || !ms) return set_err(ctx, BV_ERR_ARG, "null argument");
+    if (!ctx->ev_rs_valid) return set_err(ctx, BV_ERR_STATE, "no profiled bv_ranksum_test call yet");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    BV_CUDA(ctx, cudaEventSynchronize(ctx->ev_rs[1]));
+    BV_CUDA(ctx, cudaEventElapsedTime(ms, ctx->ev_rs[0], ctx->ev_rs[1]));
     return BV_OK;
 }
 
@@ -735,6 +757,9 @@ void bv_destroy(bv_ctx* ctx) {
     for (int i = 0; i < 7; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 3; ++i) if (ctx->ev_call[i]) cudaEventDestroy(ctx->ev_call[i]);
     for (int i = 0; i < 2; ++i) if (ctx->ev_list[i]) cudaEventDestroy(ctx->ev_list[i]);
+    for (int i = 0; i < 2; ++i) if (ctx->ev_rs[i]) cudaEventDestroy(ctx->ev_rs[i]);
+    if (ctx->rs_stream) { cudaStreamSynchronize(ctx->rs_stream); cudaStreamDestroy(ctx->rs_stream); }
+    cudaFree(ctx->d_rs_bases); cudaFree(ctx->d_rs_values); cudaFree(ctx->d_rs_start); cudaFree(ctx->d_rs_ref); cudaFree(ctx->d_rs_out);
     if (ctx->ev_trace0) cudaEventDestroy(ctx->ev_trace0);
     if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
     delete ctx;
@@ -1379,6 +1404,64 @@ int bv_fisher_fs(bv_ctx* ctx, const int32_t* tables, uint32_t n, double* fs_out)
     if (e == cudaSuccess) e = cudaMemcpy(fs_out, d_fs, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost);
     cudaFree(d_t); cudaFree(d_fs);
     BV_CUDA(ctx, e);
+    return BV_OK;
+}
+
+int bv_ranksum_test(bv_ctx* ctx, const uint8_t* bases, const int32_t* values, const uint64_t* start, const uint8_t* ref_base,
+                    const uint8_t* alt_mask, uint32_t n, double* phred_out) {
+    BvRange range("bv_ranksum_test (H2D, K9, D2H)");
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (n == 0) return BV_OK;
+    if (!start || !ref_base || !alt_mask || !phred_out) return set_err(ctx, BV_ERR_ARG, "bv_ranksum_test: null argument");
+    if (start[0] != 0) return set_err(ctx, BV_ERR_ARG, "bv_ranksum_test: start[0] = %llu, not 0", (unsigned long long)start[0]);
+    for (uint32_t p = 0; p < n; ++p) {
+        if (start[p + 1] < start[p]) return set_err(ctx, BV_ERR_ARG, "bv_ranksum_test: start[%u] < start[%u]", p + 1, p);
+        if (start[p + 1] - start[p] > ctx->prm.max_samples)
+            return set_err(ctx, BV_ERR_ARG, "bv_ranksum_test: problem %u has %llu entries > max_samples %u", p,
+                           (unsigned long long)(start[p + 1] - start[p]), ctx->prm.max_samples);
+        if (alt_mask[p] > 15) return set_err(ctx, BV_ERR_ARG, "bv_ranksum_test: alt_mask[%u] = %u > 15", p, alt_mask[p]);
+    }
+    const uint64_t total = start[n];
+    if (total && (!bases || !values)) return set_err(ctx, BV_ERR_ARG, "bv_ranksum_test: null bases / values");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!ctx->rs_stream) {   // on first use: a context that never calls this sets up exactly what it did without it
+        BV_CUDA(ctx, cudaFuncSetAttribute(bv::bv_ranksum_test_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kRsSmemBytes));
+        BV_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->rs_stream, cudaStreamNonBlocking));
+    }
+    if (total > ctx->rs_entries_cap) {   // (a failed allocation leaves the scratch empty, so the next call allocates again)
+        cudaFree(ctx->d_rs_bases); cudaFree(ctx->d_rs_values);
+        ctx->d_rs_bases = nullptr; ctx->d_rs_values = nullptr; ctx->rs_entries_cap = 0;
+        BV_CUDA(ctx, cudaMalloc(&ctx->d_rs_bases, total));
+        BV_CUDA(ctx, cudaMalloc(&ctx->d_rs_values, total * sizeof(int32_t)));
+        ctx->rs_entries_cap = total;
+    }
+    if (n > ctx->rs_problems_cap) {
+        cudaFree(ctx->d_rs_start); cudaFree(ctx->d_rs_ref); cudaFree(ctx->d_rs_out);
+        ctx->d_rs_start = nullptr; ctx->d_rs_ref = nullptr; ctx->d_rs_out = nullptr; ctx->rs_problems_cap = 0;
+        BV_CUDA(ctx, cudaMalloc(&ctx->d_rs_start, ((size_t)n + 1) * sizeof(uint64_t)));
+        BV_CUDA(ctx, cudaMalloc(&ctx->d_rs_ref, 2 * (size_t)n));
+        BV_CUDA(ctx, cudaMalloc(&ctx->d_rs_out, (size_t)n * sizeof(double)));
+        ctx->rs_problems_cap = n;
+    }
+    cudaStream_t st = ctx->rs_stream;
+    uint8_t* d_mask = ctx->d_rs_ref + ctx->rs_problems_cap;
+    if (total) {
+        BV_CUDA(ctx, cudaMemcpyAsync(ctx->d_rs_bases, bases, total, cudaMemcpyHostToDevice, st));
+        BV_CUDA(ctx, cudaMemcpyAsync(ctx->d_rs_values, values, total * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    }
+    BV_CUDA(ctx, cudaMemcpyAsync(ctx->d_rs_start, start, ((size_t)n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    BV_CUDA(ctx, cudaMemcpyAsync(ctx->d_rs_ref, ref_base, n, cudaMemcpyHostToDevice, st));
+    BV_CUDA(ctx, cudaMemcpyAsync(d_mask, alt_mask, n, cudaMemcpyHostToDevice, st));
+    const bool prof = ctx->profiling;
+    if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev_rs[0], st));
+    const uint32_t max_grid = (uint32_t)ctx->num_sms * bv::kRsCtasPerSm;
+    bv::bv_ranksum_test_kernel<<<n < max_grid ? n : max_grid, bv::kRsThreads, bv::kRsSmemBytes, st>>>(
+        ctx->d_rs_bases, ctx->d_rs_values, ctx->d_rs_start, ctx->d_rs_ref, d_mask, n, ctx->d_rs_out);
+    BV_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev_rs[1], st)); ctx->ev_rs_valid = true; }
+    BV_CUDA(ctx, cudaMemcpyAsync(phred_out, ctx->d_rs_out, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    BV_CUDA(ctx, cudaStreamSynchronize(st));
     return BV_OK;
 }
 

@@ -66,9 +66,10 @@ __device__ __noinline__ double erfc_as66(double x) {
     return x > 0. ? 2. * p : 2. * (1. - p);
 }
 
-// From 2 * smp1_ranksum to the INFO value: src/algorithm.h:130-135, src/basetype.cpp:224-236,
-// (int) at src/basetype_caller.cpp:1151-1157
-__device__ __noinline__ int ranksum_phred(unsigned long long twice_ranksum, unsigned long long n1, unsigned long long n2) {
+// From 2 * smp1_ranksum to the value of ref_vs_alt_ranksumtest: src/algorithm.h:130-135, src/basetype.cpp:224-236
+// (n1, n2 > 0).  The sign of a zero result is left as the arithmetic gives it (-0.0 when every value ties).
+__device__ __noinline__ double ranksum_phred_double(unsigned long long twice_ranksum, unsigned long long n1,
+                                                    unsigned long long n2) {
     const double smp1_ranksum = (double)twice_ranksum / 2.0;
     const double e = (double)(n1 * (n1 + n2 + 1)) / 2.0;
     const double z = (smp1_ranksum - e) / sqrt((double)(n1 * n2 * (n1 + n2 + 1)) / 12.0);
@@ -76,13 +77,20 @@ __device__ __noinline__ int ranksum_phred(unsigned long long twice_ranksum, unsi
     const double p = 2 * nd;
     double v = -10 * nlog10(p);
     if (isinf(v)) v = 10000;
-    return (int)v;
+    return v;
 }
 
-// 2 * (rank sum of class 0) from the two class histograms over values [vmin, vmax]; the bins are zeroed on the way.
-__device__ __forceinline__ unsigned long long hist_twice_ranksum(uint32_t* h0, uint32_t* h1, int vmin, int vmax) {
+// the INFO value: (int) at src/basetype_caller.cpp:1151-1157
+__device__ __noinline__ int ranksum_phred(unsigned long long twice_ranksum, unsigned long long n1, unsigned long long n2) {
+    return (int)ranksum_phred_double(twice_ranksum, n1, n2);
+}
+
+// 2 * (rank sum of class 0) from the two class histograms over bins [vmin, vmax] (a larger bin is a larger value); the bins
+// are zeroed on the way.  above_io (optional): reads with a value above bin vmax on entry, all reads counted so far on exit.
+__device__ __forceinline__ unsigned long long hist_twice_ranksum(uint32_t* h0, uint32_t* h1, int vmin, int vmax,
+                                                                 unsigned long long* above_io = nullptr) {
     const int lane = threadIdx.x & 31;
-    unsigned long long acc = 0, above = 0;   // above: reads with a value greater than this step's 32 bins
+    unsigned long long acc = 0, above = above_io ? *above_io : 0ull;   // above: reads with a value greater than this step's 32 bins
 #pragma unroll 1
     for (int top = vmax; top >= vmin; top -= 32) {
         const int v = top - lane;
@@ -104,6 +112,7 @@ __device__ __forceinline__ unsigned long long hist_twice_ranksum(uint32_t* h0, u
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
+    if (above_io) *above_io = above;
     return acc;
 }
 
@@ -280,6 +289,151 @@ __global__ void __launch_bounds__(kCallWarps * 32, 1) bv_ranksum_kernel(const __
             *reinterpret_cast<uint4*>(a.calls + k) = *reinterpret_cast<const uint4*>(&o);
         }
         __syncwarp();
+    }
+}
+
+// =====================================================================================================================
+// K9: free-standing rank-sum tests (bv_ranksum_test), ref_vs_alt_ranksumtest (src/basetype.cpp:201-242) for a batch of
+// problems.  A problem is a list of (base code, int32 value) entries, a REF character and an ALT mask; its entries are
+// classified by call_class as in K5, and the result is ranksum_phred_double of the exact 2 * (REF rank sum) as K5 forms
+// it.  One CTA per problem (grid-stride): a 100,000-read call of the C++ mirror is spread over 256 threads.  Pass 1 counts
+// the classes and finds the value range R = vmax - vmin + 1 of the classified entries; then one of three exact paths:
+//   narrow    R <= kRsBins: one histogram pass over the entries, then hist_twice_ranksum over R bins (warp 0);
+//   windows   the range cut into W = ceil(R / kRsBins) windows from the top, one histogram pass per window, the count of
+//             values above the window carried to the next: cost ~ W * (n / kRsThreads + kRsBins / 32) thread steps;
+//   pairwise  the smaller class, kRsOwn values per thread in registers, against every classified entry, swept through
+//             shared memory (rpr_pairwise's sum): cost ~ ceil(min(n1, n2) / (kRsThreads * kRsOwn)) * n thread steps.
+// Between windows and pairwise the kernel takes the smaller estimate; the bound of a problem is that minimum.
+// =====================================================================================================================
+constexpr int kRsThreads = 256;
+constexpr int kRsWarps = kRsThreads / 32;
+constexpr int kRsBins = 8192;      // histogram bins per class
+constexpr int kRsTile = 2048;      // entries per shared tile of the pairwise sweep
+constexpr int kRsOwn = 8;          // values of the owned class a thread holds per sweep
+constexpr int kRsCtasPerSm = 3;
+
+struct __align__(128) RsCta {
+    uint32_t h[2][kRsBins];        // [class][value - window base], all-zero between problems
+    int32_t tv[kRsTile];
+    uint8_t tc[kRsTile];
+    unsigned long long red_cnt[kRsWarps], red_acc[kRsWarps];
+    int32_t red_lo[kRsWarps], red_hi[kRsWarps];
+};
+constexpr size_t kRsSmemBytes = sizeof(RsCta);
+static_assert(kRsCtasPerSm * (kRsSmemBytes + 1024) <= 233472, "K9: kRsCtasPerSm CTAs do not fit the shared memory of an SM");
+
+__device__ __forceinline__ unsigned long long rs_block_sum(unsigned long long x, unsigned long long* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(kFull, x, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = x;
+    __syncthreads();
+    x = 0;
+#pragma unroll
+    for (int w = 0; w < kRsWarps; ++w) x += red[w];
+    return x;
+}
+
+__global__ void __launch_bounds__(kRsThreads) bv_ranksum_test_kernel(const uint8_t* __restrict__ bases,
+                                                                     const int32_t* __restrict__ values,
+                                                                     const uint64_t* __restrict__ start,
+                                                                     const uint8_t* __restrict__ ref_base,
+                                                                     const uint8_t* __restrict__ alt_mask, uint32_t n,
+                                                                     double* __restrict__ out) {
+    RsCta& S = *reinterpret_cast<RsCta*>(bv_smem_raw);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int i = tid; i < 2 * kRsBins; i += kRsThreads) (&S.h[0][0])[i] = 0;
+    __syncthreads();
+#pragma unroll 1
+    for (uint32_t p = blockIdx.x; p < n; p += gridDim.x) {
+        const uint64_t s0 = start[p], s1 = start[p + 1];
+        const int ref_code = ref_code_of(ref_base[p]);
+        const uint32_t mask = alt_mask[p];
+        // pass 1: class counts (n1 low word, n2 high word) and the value range of the classified entries
+        unsigned long long cnt = 0;
+        int lo = INT_MAX, hi = INT_MIN;
+#pragma unroll 1
+        for (uint64_t i = s0 + tid; i < s1; i += kRsThreads) {
+            const uint32_t c = call_class(bases[i], ref_code, mask);
+            if (c < 2u) {
+                const int v = values[i];
+                cnt += c == 0u ? 1ull : 1ull << 32;
+                lo = min(lo, v); hi = max(hi, v);
+            }
+        }
+        lo = __reduce_min_sync(kFull, lo); hi = __reduce_max_sync(kFull, hi);
+        if (lane == 0) { S.red_lo[warp] = lo; S.red_hi[warp] = hi; }
+        cnt = rs_block_sum(cnt, S.red_cnt);   // (its barrier publishes red_lo / red_hi too)
+#pragma unroll
+        for (int w = 0; w < kRsWarps; ++w) { lo = min(lo, S.red_lo[w]); hi = max(hi, S.red_hi[w]); }
+        const unsigned long long n1 = cnt & 0xffffffffull, n2 = cnt >> 32, nent = s1 - s0;
+        unsigned long long twice = 0;   // 2 * REF rank sum: in warp 0 (histogram paths) or every thread (pairwise)
+        if (n1 > 0 && n2 > 0) {
+            const unsigned long long range = (unsigned long long)((long long)hi - (long long)lo) + 1ull;
+            const unsigned long long wins = (range + kRsBins - 1) / kRsBins;
+            const unsigned long long sweeps = (min(n1, n2) + kRsThreads * kRsOwn - 1) / (kRsThreads * kRsOwn);
+            if (wins == 1 || wins * ((nent + kRsThreads - 1) / kRsThreads + kRsBins / 32) <= sweeps * nent) {
+                unsigned long long above = 0;
+#pragma unroll 1
+                for (long long top = hi; top >= lo; top -= kRsBins) {   // windows [wlo, top], from the largest values down
+                    const long long wlo = max((long long)lo, top - (kRsBins - 1));
+#pragma unroll 1
+                    for (uint64_t i = s0 + tid; i < s1; i += kRsThreads) {
+                        const uint32_t c = call_class(bases[i], ref_code, mask);
+                        if (c < 2u) {
+                            const long long v = values[i];
+                            if (v >= wlo && v <= top) atomicAdd(&S.h[c][(uint32_t)(v - wlo)], 1u);
+                        }
+                    }
+                    __syncthreads();
+                    if (warp == 0) twice += hist_twice_ranksum(S.h[0], S.h[1], 0, (int)(top - wlo), &above);
+                    __syncthreads();
+                }
+            } else {
+                // pairwise: for every entry i of the owned class, 2 * #{j: v_j > v_i} + #{j: v_j == v_i} + 1 over the
+                // classified entries j (i included) is twice its rank
+                const uint32_t own = n1 <= n2 ? 0u : 1u;
+                unsigned long long acc = 0;
+                uint64_t cur = s0 + tid;   // this thread's next entry (stride kRsThreads)
+#pragma unroll 1
+                for (;;) {
+                    int va[kRsOwn];
+                    int nk = 0;
+#pragma unroll
+                    for (int k = 0; k < kRsOwn; ++k) {
+                        va[k] = 0;
+                        while (cur < s1 && call_class(bases[cur], ref_code, mask) != own) cur += kRsThreads;
+                        if (cur < s1) { va[k] = values[cur]; cur += kRsThreads; nk = k + 1; }
+                    }
+                    if (!__syncthreads_or(nk > 0)) break;
+                    acc += (unsigned long long)nk;
+#pragma unroll 1
+                    for (uint64_t t0 = s0; t0 < s1; t0 += kRsTile) {
+                        const uint32_t len = (uint32_t)min((uint64_t)kRsTile, s1 - t0);
+                        for (uint32_t j = tid; j < len; j += kRsThreads) {
+                            S.tc[j] = (uint8_t)call_class(bases[t0 + j], ref_code, mask);
+                            S.tv[j] = values[t0 + j];
+                        }
+                        __syncthreads();
+                        uint32_t a32 = 0;   // <= 2 * kRsTile * kRsOwn
+#pragma unroll 1
+                        for (uint32_t j = 0; j < len; ++j) {
+                            if (S.tc[j] > 1u) continue;   // the same j for every thread
+                            const int vj = S.tv[j];
+#pragma unroll
+                            for (int k = 0; k < kRsOwn; ++k)
+                                if (k < nk) a32 += vj > va[k] ? 2u : (vj == va[k] ? 1u : 0u);
+                        }
+                        acc += a32;
+                        __syncthreads();
+                    }
+                }
+                acc = rs_block_sum(acc, S.red_acc);
+                const unsigned long long nn = n1 + n2;
+                twice = own == 0u ? acc : nn * (nn + 1ull) - acc;   // the ranks 1..nn sum to nn (nn + 1) / 2
+            }
+        }
+        if (tid == 0) out[p] = n1 > 0 && n2 > 0 ? ranksum_phred_double(twice, n1, n2) : 10000.0;   // src/basetype.cpp:233-236
+        __syncthreads();
     }
 }
 

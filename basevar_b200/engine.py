@@ -353,6 +353,30 @@ class BaseTypeEngine:
         self._check(self.lib.bv_last_list_kernel_time(self._ctx, C.byref(ms)), "bv_last_list_kernel_time")
         return float(ms.value)
 
+    # -- ref_vs_alt_ranksumtest of free-standing problems ------------------------------------------------
+    def ranksum_test(self, bases, values, start, ref_base, alt_mask):
+        """ref_vs_alt_ranksumtest (src/basetype.cpp:201-242) of n problems on the device (bv_ranksum_test).  Problem p is
+        entries start[p]:start[p+1] of bases (uint8 BV_BASE_* codes) and values (int32), ref_base[p] its REF character
+        (ASCII code) and alt_mask[p] its ALT bases (bit b = base code b).  Returns float64 [n], not truncated."""
+        bases = np.ascontiguousarray(bases, np.uint8)
+        values = np.ascontiguousarray(values, np.int32)
+        start = np.ascontiguousarray(start, np.uint64)
+        ref_base = np.ascontiguousarray(ref_base, np.uint8)
+        alt_mask = np.ascontiguousarray(alt_mask, np.uint8)
+        n = len(ref_base)
+        assert start.shape == (n + 1,) and alt_mask.shape == (n,) and bases.shape == values.shape
+        assert int(start[-1]) <= len(bases)
+        out = np.zeros(n, np.float64)
+        self._check(self.lib.bv_ranksum_test(self._ctx, _ptr(bases), _ptr(values), _ptr(start), _ptr(ref_base), _ptr(alt_mask), n,
+                                             _ptr(out)), "bv_ranksum_test")
+        return out
+
+    def last_ranksum_kernel_time(self):
+        """Duration (ms) of K9 bv_ranksum_test_kernel of the most recent ranksum_test (profiling must be on); waits for it."""
+        ms = C.c_float(0.0)
+        self._check(self.lib.bv_last_ranksum_kernel_time(self._ctx, C.byref(ms)), "bv_last_ranksum_kernel_time")
+        return float(ms.value)
+
     # -- device-resident tiles ---------------------------------------------------------------------
     def call_device(self, d_base, d_qual, d_strand, d_ref, n_sites, n_samples, pitch, d_out, stream=0):
         """All arguments are device pointers (ints); stream is a cudaStream_t handle (int).  Asynchronous."""

@@ -188,6 +188,11 @@ double Context::fisher_fs(int ref_fwd, int ref_rev, int alt_fwd, int alt_rev) {
     return fs;
 }
 
+void Context::ranksum_test(const uint8_t* bases, const int32_t* values, const uint64_t* start, const uint8_t* ref_base,
+                           const uint8_t* alt_mask, uint32_t n, double* phred_out) {
+    check(bv_ranksum_test(ctx_, bases, values, start, ref_base, alt_mask, n, phred_out), ctx_, "bv_ranksum_test");
+}
+
 // ---- BaseType ---------------------------------------------------------------------------------------------------------
 BaseType::BaseType(const BatchInfo* bi, const bv_site_out& rec)
     : ref_id_(bi->ref_id), ref_base_(bi->ref_base), ref_pos_(bi->ref_pos), rec_(rec) {
@@ -306,6 +311,19 @@ double BaseType::get_lrt_af(char b) const {
     return it->second;
 }
 
+// The calling thread's default context for the free functions, made again when it has room for fewer than max_samples samples.
+static Context* thread_context(uint32_t max_samples) {
+    if (!t_one.ctx || t_one.ctx->max_samples() < max_samples) {
+        const char* d = getenv("BASEVAR_B200_DEVICE");
+        t_one.ctx.reset();
+        t_one.packer.reset();
+        t_one.n = std::max<uint32_t>(max_samples, 1);
+        t_one.min_af = 0.01f;
+        t_one.ctx.reset(new Context(d ? atoi(d) : 0, t_one.min_af, t_one.n, 1, 1));
+    }
+    return t_one.ctx.get();
+}
+
 // ---- strand_bias -------------------------------------------------------------------------------------------------------
 static int code_of(char c) { return c == 'A' ? 0 : c == 'C' ? 1 : c == 'G' ? 2 : c == 'T' ? 3 : -1; }
 
@@ -336,22 +354,56 @@ StrandBiasInfo strand_bias(const char ref_base, const std::string alt_bases_stri
     else {
         // neither of the two sets the record carries FS for: the 2x2 table goes to the device (bv_fisher_fs, the code of bv_fisher_kernel)
         const uint32_t reads = (uint32_t)(s.ref_fwd + s.ref_rev + s.alt_fwd + s.alt_rev);
-        if (!ctx) {
-            if (!t_one.ctx || t_one.ctx->max_samples() + 1 < reads) {
-                const char* d = getenv("BASEVAR_B200_DEVICE");
-                t_one.ctx.reset();
-                t_one.packer.reset();
-                t_one.n = std::max<uint32_t>(reads, 1);
-                t_one.min_af = 0.01f;
-                t_one.ctx.reset(new Context(d ? atoi(d) : 0, t_one.min_af, t_one.n, 1, 1));
-            }
-            ctx = t_one.ctx.get();
-        }
+        if (!ctx) ctx = thread_context(reads - 1);   // the log-factorial table covers max_samples + 1 reads
         s.fs = ctx->fisher_fs(s.ref_fwd, s.ref_rev, s.alt_fwd, s.alt_rev);
     }
     // src/basetype.cpp:286, int32 products as in the reference
     s.sor = (s.ref_rev * s.alt_fwd > 0) ? (double)(s.ref_fwd * s.alt_rev) / (double)(s.ref_rev * s.alt_fwd) : 10000;
     return s;
+}
+
+// ---- ref_vs_alt_ranksumtest ---------------------------------------------------------------------------------------------
+static double ranksum_one(const char ref_base, const std::string& alt_bases_string, const std::vector<char>& bases,
+                          const std::vector<int32_t>& values, Context* ctx) {
+    if (ref_base >= 'a' && ref_base <= 'z')
+        throw std::invalid_argument(std::string("[ERROR] ref_vs_alt_ranksumtest: lowercase ref_base '") + ref_base + "'");
+    uint8_t alt_mask = 0;
+    for (char c : alt_bases_string) {
+        const int k = code_of(c);
+        if (k < 0) throw std::invalid_argument(std::string("[ERROR] ref_vs_alt_ranksumtest: ALT base '") + c + "' is not A/C/G/T");
+        alt_mask |= (uint8_t)(1u << k);
+    }
+    const bool ref_is_code = code_of(ref_base) >= 0 || ref_base == 'N';
+    std::vector<uint8_t> codes(bases.size());
+    for (size_t i = 0; i < bases.size(); ++i) {
+        const char c = bases[i];
+        if (!ref_is_code && c == ref_base)
+            throw std::invalid_argument(std::string("[ERROR] ref_vs_alt_ranksumtest: ref_base '") + ref_base +
+                                        "' is not A/C/G/T/N and a base equals it");
+        const int k = code_of(c);
+        codes[i] = (uint8_t)(k >= 0 ? k : c == 'N' ? BV_BASE_N : c == '+' ? BV_BASE_INS : c == '-' ? BV_BASE_DEL : BV_BASE_OTHER);
+    }
+    const uint32_t n = (uint32_t)bases.size();
+    if (!ctx) ctx = thread_context(n);
+    const uint64_t start[2] = {0, n};
+    const uint8_t ref = (uint8_t)ref_base;
+    double v = 0.0;
+    ctx->ranksum_test(codes.data(), values.data(), start, &ref, &alt_mask, 1, &v);
+    return v;
+}
+
+double ref_vs_alt_ranksumtest(const char ref_base, const std::string alt_bases_string, const std::vector<char>& bases,
+                              const std::vector<int>& values, Context* ctx) {
+    if (bases.size() != values.size()) throw std::invalid_argument("[ERROR] ref_vs_alt_ranksumtest: bases and values differ in size");
+    return ranksum_one(ref_base, alt_bases_string, bases, std::vector<int32_t>(values.begin(), values.end()), ctx);
+}
+
+double ref_vs_alt_ranksumtest(const char ref_base, const std::string alt_bases_string, const std::vector<char>& bases,
+                              const std::vector<char>& values, Context* ctx) {
+    if (bases.size() != values.size()) throw std::invalid_argument("[ERROR] ref_vs_alt_ranksumtest: bases and values differ in size");
+    std::vector<int32_t> v(values.size());
+    for (size_t i = 0; i < values.size(); ++i) v[i] = (int32_t)(signed char)values[i];   // as g++ on x86-64 widens a char
+    return ranksum_one(ref_base, alt_bases_string, bases, v, ctx);
 }
 
 // ---- region sharding ----------------------------------------------------------------------------------------------------

@@ -9,6 +9,7 @@
 //   class BaseType, ctor + lrt() + getters :64-153          BaseType: filled from a device record (batch path), or
 //                                                           BaseType(const BatchInfo*, double) + lrt() for one site
 //   strand_bias(ref, alts, bases, strands) :178-181         strand_bias(ref, alts, record)
+//   ref_vs_alt_ranksumtest(...)           :168-176          ref_vs_alt_ranksumtest (same arguments; bv_ranksum_test)
 //   BatchInfo rows -> BaseType per site,                    TilePacker (BatchInfo -> packed SoA planes in pinned memory)
 //     src/basetype_caller.cpp:686-743                       Context (slots: H2D copy, kernels, D2H copy per tile)
 //   100-kb tasks over a ThreadPool,                         shard_region / run_region: contiguous region shards, one host
@@ -165,6 +166,9 @@ public:
     uint32_t max_samples() const { return max_samples_; }
     // FS of free-standing 2x2 strand tables {ref_fwd, ref_rev, alt_fwd, alt_rev} on the device (bv_fisher_fs)
     double fisher_fs(int ref_fwd, int ref_rev, int alt_fwd, int alt_rev);
+    // ref_vs_alt_ranksumtest of n free-standing problems on the device (bv_ranksum_test; arguments as there, host memory)
+    void ranksum_test(const uint8_t* bases, const int32_t* values, const uint64_t* start, const uint8_t* ref_base,
+                      const uint8_t* alt_mask, uint32_t n, double* phred_out);
 
 private:
     bv_ctx* ctx_ = nullptr;
@@ -224,6 +228,22 @@ private:
 // set (bv_fisher_fs; `ctx`, or the calling thread's default context, created on first use on device BASEVAR_B200_DEVICE or 0).
 // A record flagged BV_FLAG_BAD_STRAND throws the reference's "[ERROR] Get strange strand symbol" error.
 StrandBiasInfo strand_bias(const char ref_base, const std::string alt_bases_string, const bv_site_out& rec, Context* ctx = nullptr);
+
+// ref_vs_alt_ranksumtest (src/basetype.h:168-176, src/basetype.cpp:201-242): -10 log10 of the two-sided Wilcoxon rank-sum p of
+// the values of REF reads vs those of ALT reads, classified by the first character of each read's base, as a double (the
+// caller truncates); 10000 when a class is empty or p == 0.  Computed on the device (bv_ranksum_test) on `ctx`, or on the
+// calling thread's default context (device BASEVAR_B200_DEVICE or 0, made on first use and again for a longer list).
+// Characters map to base codes: A/C/G/T, 'N', '+' (insertion), '-' (deletion), anything else BV_BASE_OTHER; N, indels and
+// other characters are in neither class, a base equal to ref_base is a REF read, one in alt_bases_string an ALT read.
+// The char overload widens each value as a signed char.  std::invalid_argument when bases and values differ in size.
+// Departures from the reference, which compares raw characters where the packed codes cannot (std::invalid_argument):
+//   - alt_bases_string holds a character other than A/C/G/T;
+//   - ref_base is lowercase;
+//   - ref_base is a character other than A/C/G/T/N and some entry of bases equals it.
+double ref_vs_alt_ranksumtest(const char ref_base, const std::string alt_bases_string, const std::vector<char>& bases,
+                              const std::vector<int>& values, Context* ctx = nullptr);
+double ref_vs_alt_ranksumtest(const char ref_base, const std::string alt_bases_string, const std::vector<char>& bases,
+                              const std::vector<char>& values, Context* ctx = nullptr);
 
 // ---- region sharding over the GPUs of one box ---------------------------------------------------------------------------
 struct Shard {

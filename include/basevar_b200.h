@@ -26,6 +26,8 @@
  *     group + lrt([REF, ALT...])        src/basetype_caller.cpp:747-760   (group kernel), bv_group_out
  *   BaseType::lrt(specific_bases)       src/basetype.h:118               bv_tile_submit_lists / bv_tile_run_device_lists
  *     (any ordered candidate list)      src/basetype.cpp:130-199         (list kernel K8), bv_lrt_out
+ *   ref_vs_alt_ranksumtest(...) for any src/basetype.h:168-176           bv_ranksum_test (rank-sum test kernel K9), one double
+ *     ALT set and value list            src/basetype.cpp:201-242         per free-standing problem
  *
  * Everything is `extern "C"`, plain pointers and sizes, POD structs; no exception crosses the
  * boundary.  Every entry point returns BV_OK (0) or a negative status; bv_last_error() gives text.
@@ -246,6 +248,7 @@ int         bv_last_em_kernel_times(bv_ctx* ctx, float ms[2]);
 int         bv_last_fisher_kernel_time(bv_ctx* ctx, float* ms);
 int         bv_last_call_kernel_times(bv_ctx* ctx, float ms[2]);   /* K5 rank sums, K6 population groups */
 int         bv_last_list_kernel_time(bv_ctx* ctx, float* ms);      /* K8 bv_list_kernel of the last lists tile */
+int         bv_last_ranksum_kernel_time(bv_ctx* ctx, float* ms);   /* K9 bv_ranksum_test_kernel of the last bv_ranksum_test */
 
 /* ---- tile pipeline (replaces: BatchInfo -> BaseType ctor -> lrt() -> strand_bias per site) ------ */
 /* Asynchronous.  Host tiles are copied H2D on the slot's stream (pinned memory makes the copy truly
@@ -388,6 +391,20 @@ int bv_synth_fill_host(const bv_synth_model* model, uint64_t site0, uint32_t n_s
  * alt_fwd, alt_rev} in host memory, every table's total <= bv_params::max_samples + 1; fs_out: n doubles (host).
  * Blocking; a table with an empty row gives 0 (one possible outcome, p == 1). */
 int bv_fisher_fs(bv_ctx* ctx, const int32_t* tables, uint32_t n, double* fs_out);
+
+/* ---- rank-sum test of arbitrary REF / ALT classes ---------------------------------------------------------- */
+/* ref_vs_alt_ranksumtest (src/basetype.h:168-176, src/basetype.cpp:201-242) for n free-standing problems, on the device.
+ * Problem p: entries [start[p], start[p+1]) of bases (BV_BASE_* codes) and values; ref_base[p] raw ASCII (upper-cased as the
+ * tile's REF is); alt_mask[p] bit b = base code b is an ALT.  phred_out[p]: the function's double, not truncated.
+ * An entry whose base code is above BV_BASE_T is in neither class; one equal to the upper-cased REF is a REF read (whatever
+ * the mask says); otherwise it is an ALT read when its bit is set.  The value is -10 log10 of the two-sided p of the Wilcoxon
+ * rank-sum test (normal approximation, no tie correction, kf_erfc), 10000 when a class is empty or p == 0; a zero keeps the
+ * sign the arithmetic gives (-0.0 when every value ties).  Exact for any int32 values.
+ * Host memory, blocking.  BV_ERR_ARG (checked before anything is queued): null pointer (bases and values may be null when
+ * start[n] == 0), start[0] != 0 or not ascending, a problem longer than max_samples, alt_mask > 15.  Nothing is launched for
+ * n == 0. */
+int bv_ranksum_test(bv_ctx* ctx, const uint8_t* bases, const int32_t* values, const uint64_t* start,
+                    const uint8_t* ref_base, const uint8_t* alt_mask, uint32_t n, double* phred_out);
 
 /* ---- tile sizing --------------------------------------------------------------------------------- */
 /* The count kernel is persistent: num_SMs x W warps take one site row each (W = 32, or 16 for rows longer than 4,096
