@@ -48,7 +48,7 @@ CLI = os.path.join(HERE, "bin", "basevar")   # `basevar basetype ...` over BAM f
 ROOT = os.path.dirname(HERE)
 CPP_TESTS = {"test_host_cpu": [], "test_host_gpu": ["-ldl"], "test_fisher_fast": ["-ldl", "-lm"], "test_caller_cpu": [],
              "test_caller_gpu": ["-lz"], "pileup_dump": ["-lz"], "test_lists_gpu": ["-ldl", "-lm"],
-             "test_ranksum_gpu": ["-ldl", "-lm"]}
+             "test_ranksum_gpu": ["-ldl", "-lm"], "test_vcf_row_gpu": ["-ldl", "-lm"]}
 
 
 def build_host(force=False):

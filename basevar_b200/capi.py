@@ -154,6 +154,8 @@ _SIGNATURES = [
     ("bv_set_groups", C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32]),
     ("bv_tile_submit_calls", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvTile), C.POINTER(BvTileAux)]),
     ("bv_tile_wait_calls", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_void_p]),
+    ("bv_tile_wait_calls_compact", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint32),
+                                             C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_void_p]),
     ("bv_tile_run_device_calls", C.c_int, [C.c_void_p, C.POINTER(BvTile), C.POINTER(BvTileAux)] + [C.c_void_p] * 5),
     ("bv_last_list_kernel_time", C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     ("bv_tile_submit_lists", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvTile), C.c_void_p]),
@@ -166,6 +168,9 @@ _SIGNATURES = [
     ("bv_synth_fill_host", C.c_int, [C.POINTER(BvSynthModel), C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64] + [C.c_void_p] * 5),
     ("bv_tile_submit_sparse", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvSparseTile)]),
     ("bv_tile_submit_sparse_calls", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvSparseTile)]),
+    ("bv_tile_submit_sparse_lists", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvSparseTile), C.c_void_p]),
+    ("bv_tile_wait_lists_compact", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint32),
+                                             C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
     ("bv_sparse_encode16_bound", C.c_uint64, [C.c_uint64, C.c_uint32, C.c_uint32]),
     ("bv_sparse_encode16", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
                                      C.POINTER(C.c_uint64)]),

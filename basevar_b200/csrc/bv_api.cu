@@ -139,12 +139,15 @@ struct bv_slot {
     uint32_t* h_counters = nullptr;       // copy of the scratch counters (kCntCalled = number of calls)
     uint8_t* d_aux = nullptr;             // mapq | rpr planes of pageable host tiles (allocated on first use)
     bool with_calls = false;
-    // per-site candidate lists (bv_tile_submit_lists): allocated on first use
-    uint32_t* h_lists = nullptr;          // [max_sites] pinned staging of the tile's lists, one word per site
-    uint32_t* d_lists = nullptr;          // [max_sites]
+    // per-site candidate lists (bv_tile_submit_lists / bv_tile_submit_sparse_lists): allocated on first use
+    uint32_t* h_lists = nullptr;          // [2 * max_sites] pinned staging of the tile's lists: one word per site, or with
+                                          // compact results {site, list word} per listed site
+    uint32_t* d_lists = nullptr;          // [2 * max_sites]
     bv_lrt_out* d_lrt = nullptr;          // [max_sites]
     bv_lrt_out* h_lrt = nullptr;          // [max_sites] pinned
     bool with_lists = false;
+    bool lists_packed = false;            // h_lrt holds n_listed entries, one per site with a non-empty list, in site order
+    uint32_t n_listed = 0;
     // sparse tiles (bv_tile_submit_sparse): the covered cells as uploaded, expanded into d_planes by K0
     uint32_t* d_cells = nullptr;          // [cells_cap] cells, then [cells_cap] aux words
     uint32_t* d_site_start = nullptr;     // [max_sites + 1]
@@ -190,6 +193,7 @@ struct bv_ctx {
     cudaEvent_t ev_list[2] = {nullptr, nullptr};   // around K8 bv_list_kernel
     bool ev_list_valid = false;
     bool list_kernel_ready = false;   // bv_list_kernel's shared-memory attribute is set (first lists tile)
+    bool list_packed_ready = false;   // the same for bv_list_packed_kernel (first sparse lists tile with compact results)
     // free-standing rank-sum tests (bv_ranksum_test): stream and device scratch made on first use, grown only
     cudaStream_t rs_stream = nullptr;
     uint8_t* d_rs_bases = nullptr;    // [rs_entries_cap]
@@ -462,6 +466,41 @@ static int launch_list_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const ui
     BV_CUDA(ctx, cudaGetLastError());
     ctx->launches += 1;
     if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[1], stream)); ctx->ev_list_valid = true; }
+    return BV_OK;
+}
+
+// K8 over the packed list of a compact tile (bv_list_packed_kernel): one warp per listed site, entry k for pair k.
+static int launch_list_packed_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const uint2* d_pairs, uint32_t n_pairs, bv_lrt_out* d_lrt,
+                                     cudaStream_t stream) {
+    BvRange range("bv: launch K8 list (packed)");
+    if (n_pairs == 0) return BV_OK;
+    if (a.n_samples == 0) {   // no reads anywhere: every entry is all-zero
+        BV_CUDA(ctx, cudaMemsetAsync(d_lrt, 0, (size_t)n_pairs * sizeof(bv_lrt_out), stream));
+        return BV_OK;
+    }
+    if (!ctx->list_packed_ready) {
+        BV_CUDA(ctx, cudaFuncSetAttribute(bv::bv_list_packed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
+        ctx->list_packed_ready = true;
+    }
+    const bool prof = ctx->profiling;
+    if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[0], stream));
+    uint32_t grid = (n_pairs + bv::kQualWarps - 1) / bv::kQualWarps;
+    if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;   // (the bin spill rows are sized for this grid)
+    bv::bv_list_packed_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_pairs, n_pairs, d_lrt);
+    BV_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[1], stream)); ctx->ev_list_valid = true; }
+    return BV_OK;
+}
+
+// The slot's list staging and results, allocated on the first lists tile.
+static int lists_reserve(bv_ctx* ctx, bv_slot& s) {
+    if (s.h_lists) return BV_OK;
+    const size_t n = ctx->prm.max_sites;
+    BV_CUDA(ctx, cudaHostAlloc(&s.h_lists, 2 * n * sizeof(uint32_t), cudaHostAllocDefault));
+    BV_CUDA(ctx, cudaHostAlloc(&s.h_lrt, n * sizeof(bv_lrt_out), cudaHostAllocDefault));
+    BV_CUDA(ctx, cudaMalloc(&s.d_lists, 2 * n * sizeof(uint32_t)));
+    BV_CUDA(ctx, cudaMalloc(&s.d_lrt, n * sizeof(bv_lrt_out)));
     return BV_OK;
 }
 
@@ -791,6 +830,7 @@ int bv_tile_run_device_calls(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux
     if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
     if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_calls: tile must be device resident");
     if (!d_n_calls) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_calls: null d_n_calls");
+    if (tile && tile->out_mode == BV_OUT_COMPACT) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
     BV_CUDA(ctx, cudaSetDevice(ctx->device));
     bv::SiteKernelArgs a;
     int rc = fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, &a);
@@ -869,18 +909,14 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
     s.sparse = false; s.out_direct = false; s.out_user = nullptr;
     s.compact = tile->location == BV_LOC_HOST && tile->out_mode == BV_OUT_COMPACT;
     s.h_ref = tile->location == BV_LOC_HOST ? tile->ref_base : nullptr;
-    if (s.compact && with_calls) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT is not available with the called-site kernels");
+    if (with_calls && tile->location == BV_LOC_DEVICE && tile->out_mode == BV_OUT_COMPACT)
+        return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
     if (lists) {   // checked and staged before anything is queued: a refused tile leaves the slot as it was
         if (tile->out_mode != BV_OUT_RECORDS) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: out_mode must be BV_OUT_RECORDS");
         int rc = check_lists(ctx, lists, tile->n_sites);
         if (rc != BV_OK) return rc;
-        if (!s.h_lists) {
-            const size_t n = ctx->prm.max_sites;
-            BV_CUDA(ctx, cudaHostAlloc(&s.h_lists, n * sizeof(uint32_t), cudaHostAllocDefault));
-            BV_CUDA(ctx, cudaHostAlloc(&s.h_lrt, n * sizeof(bv_lrt_out), cudaHostAllocDefault));
-            BV_CUDA(ctx, cudaMalloc(&s.d_lists, n * sizeof(uint32_t)));
-            BV_CUDA(ctx, cudaMalloc(&s.d_lrt, n * sizeof(bv_lrt_out)));
-        }
+        rc = lists_reserve(ctx, s);
+        if (rc != BV_OK) return rc;
         if (tile->n_sites) memcpy(s.h_lists, lists, (size_t)tile->n_sites * sizeof(uint32_t));
     }
     bv_tile dev = *tile;
@@ -963,6 +999,8 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
     }
     s.with_calls = with_calls;
     s.with_lists = lists != nullptr;
+    s.lists_packed = false;
+    s.n_listed = 0;
     s.n_sites = tile->n_sites;
     s.busy = true;
     if (tile->location == BV_LOC_HOST) ctx->h2d_bytes_total += s.h2d_bytes;
@@ -971,8 +1009,9 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
 
 // Sparse host tile: upload the covered cells (4 bytes each), expand them into the slot's dense planes (K0), then the
 // same kernels as for a dense tile.  The qual plane -- and for the called-site kernels the mapq / rpr planes -- are
-// device resident here (there is no host plane to read in place).
-static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* t, bool with_calls) {
+// device resident here (there is no host plane to read in place).  With lists, K8 follows on the expanded planes.
+static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* t, bool with_calls,
+                                   const uint8_t (*lists)[4] = nullptr) {
     BvRange range("bv_tile_submit_sparse (H2D of the cells, K0 expand, kernels, D2H)");
     if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
     if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
@@ -997,7 +1036,25 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
     s.sparse = true; s.out_direct = false; s.out_user = t->out;
     s.compact = t->out_mode == BV_OUT_COMPACT;
     s.h_ref = t->ref_base;
-    if (s.compact && (with_calls || t->out)) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: `out` must be NULL and the called-site kernels are not available");
+    if (s.compact && t->out) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: `out` must be NULL");
+    uint32_t n_listed = 0;
+    if (lists) {   // checked and staged before anything is queued: a refused tile leaves the slot as it was
+        int rc = check_lists(ctx, lists, t->n_sites);
+        if (rc != BV_OK) return rc;
+        rc = lists_reserve(ctx, s);
+        if (rc != BV_OK) return rc;
+        if (s.compact) {   // the listed sites only, as {site, list word} pairs in site order
+            uint2* pairs = reinterpret_cast<uint2*>(s.h_lists);
+            for (uint32_t i = 0; i < t->n_sites; ++i) {
+                if (lists[i][0] == BV_LIST_END) continue;
+                uint32_t w;
+                memcpy(&w, lists[i], 4);
+                pairs[n_listed++] = make_uint2(i, w);
+            }
+        } else if (t->n_sites) {
+            memcpy(s.h_lists, lists, (size_t)t->n_sites * sizeof(uint32_t));
+        }
+    }
     if (n_cells > s.cells_cap) {   // grows only; sized by the first tiles of a run
         if (s.d_cells) BV_CUDA(ctx, cudaFree(s.d_cells));
         s.d_cells = nullptr; s.cells_cap = 0;
@@ -1075,6 +1132,19 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
     }
     rc = launch_site_kernel(ctx, a, s.stream, /*counters_zeroed=*/true);
     if (rc != BV_OK) return rc;
+    if (lists && s.compact && n_listed) {
+        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, (size_t)n_listed * sizeof(uint2), cudaMemcpyHostToDevice, s.stream));
+        rc = launch_list_packed_kernel(ctx, a, reinterpret_cast<const uint2*>(s.d_lists), n_listed, s.d_lrt, s.stream);
+        if (rc != BV_OK) return rc;
+        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)n_listed * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
+        s.h2d_bytes += (size_t)n_listed * sizeof(uint2);
+    } else if (lists && !s.compact && t->n_sites) {
+        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, (size_t)t->n_sites * sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
+        rc = launch_list_kernel(ctx, a, s.d_lists, s.d_lrt, s.stream);
+        if (rc != BV_OK) return rc;
+        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)t->n_sites * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
+        s.h2d_bytes += (size_t)t->n_sites * sizeof(uint32_t);
+    }
     if (trace) BV_CUDA(ctx, cudaEventRecord(s.ev_trace[2], s.stream));
     if (t->n_sites) {
         bv_site_out* dst = s.h_out;
@@ -1086,7 +1156,9 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
     }
     if (trace) BV_CUDA(ctx, cudaEventRecord(s.ev_trace[3], s.stream));
     s.with_calls = with_calls;
-    s.with_lists = false;
+    s.with_lists = lists != nullptr;
+    s.lists_packed = lists && s.compact;
+    s.n_listed = n_listed;
     s.n_sites = t->n_sites;
     s.busy = true;
     ctx->h2d_bytes_total += s.h2d_bytes;
@@ -1095,6 +1167,11 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
 
 int bv_tile_submit_sparse(bv_ctx* ctx, int slot, const bv_sparse_tile* tile) { return tile_submit_sparse_impl(ctx, slot, tile, false); }
 int bv_tile_submit_sparse_calls(bv_ctx* ctx, int slot, const bv_sparse_tile* tile) { return tile_submit_sparse_impl(ctx, slot, tile, true); }
+int bv_tile_submit_sparse_lists(bv_ctx* ctx, int slot, const bv_sparse_tile* tile, const uint8_t (*lists)[4]) {
+    if (tile && tile->n_sites && !lists) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_sparse_lists: null lists");
+    static const uint8_t no_lists[1][4] = {{BV_LIST_END, BV_LIST_END, BV_LIST_END, BV_LIST_END}};   // (an empty tile may pass NULL)
+    return tile_submit_sparse_impl(ctx, slot, tile, false, lists ? lists : no_lists);
+}
 
 uint64_t bv_sparse_encode16_bound(uint64_t n_cells, uint32_t n_sites, uint32_t n_samples) {
     return n_cells + (uint64_t)n_sites * (n_samples / BV_CELL16_GAP_SKIP + 1u);   // at most n_samples / 31 skips per site
@@ -1251,6 +1328,16 @@ void bv_site_expand(const bv_site_brief* b, uint8_t ref_base, float min_af, bv_s
     out->em_calls = n_active;
 }
 
+// The called-site outputs of a waited-for slot into the caller's arrays.
+static int copy_calls(bv_ctx* ctx, const bv_slot& s, bv_call_out* calls, uint32_t max_calls, uint32_t* n_calls, bv_group_out* groups) {
+    const uint32_t n = s.h_counters[bv::kCntCalled];
+    *n_calls = n;
+    if (n > max_calls) return set_err(ctx, BV_ERR_ARG, "tile has %u called sites > max_calls %u", n, max_calls);
+    if (n && calls) memcpy(calls, s.h_calls, (size_t)n * sizeof(bv_call_out));
+    if (n && groups && ctx->n_groups && s.h_groups) memcpy(groups, s.h_groups, (size_t)n * ctx->n_groups * sizeof(bv_group_out));
+    return BV_OK;
+}
+
 int bv_tile_wait_calls(bv_ctx* ctx, int slot, bv_site_out* out, bv_call_out* calls, uint32_t max_calls,
                        uint32_t* n_calls, bv_group_out* groups) {
     if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
@@ -1260,12 +1347,19 @@ int bv_tile_wait_calls(bv_ctx* ctx, int slot, bv_site_out* out, bv_call_out* cal
     if (s.busy && !s.with_calls) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without called-site kernels", slot);
     int rc = bv_tile_wait(ctx, slot, out);
     if (rc != BV_OK) return rc;
-    const uint32_t n = s.h_counters[bv::kCntCalled];
-    *n_calls = n;
-    if (n > max_calls) return set_err(ctx, BV_ERR_ARG, "tile has %u called sites > max_calls %u", n, max_calls);
-    if (n && calls) memcpy(calls, s.h_calls, (size_t)n * sizeof(bv_call_out));
-    if (n && groups && ctx->n_groups && s.h_groups) memcpy(groups, s.h_groups, (size_t)n * ctx->n_groups * sizeof(bv_group_out));
-    return BV_OK;
+    return copy_calls(ctx, s, calls, max_calls, n_calls, groups);
+}
+
+int bv_tile_wait_calls_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full,
+                               bv_call_out* calls, uint32_t max_calls, uint32_t* n_calls, bv_group_out* groups) {
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    if (!n_calls) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_calls_compact: null n_calls");
+    bv_slot& s = ctx->slots[slot];
+    if (s.busy && !s.with_calls) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without called-site kernels", slot);
+    int rc = bv_tile_wait_compact(ctx, slot, brief, full, n_full);
+    if (rc != BV_OK) return rc;
+    return copy_calls(ctx, s, calls, max_calls, n_calls, groups);
 }
 
 int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8_t (*lists)[4]) {
@@ -1279,9 +1373,27 @@ int bv_tile_wait_lists(bv_ctx* ctx, int slot, bv_site_out* out, bv_lrt_out* lrt_
     if (!lrt_out) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists: null lrt_out");
     bv_slot& s = ctx->slots[slot];
     if (s.busy && !s.with_lists) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without lists", slot);
+    if (s.busy && s.lists_packed) return set_err(ctx, BV_ERR_STATE, "slot %d has compact results: collect with bv_tile_wait_lists_compact", slot);
     int rc = bv_tile_wait(ctx, slot, out);
     if (rc != BV_OK) return rc;
     if (s.n_sites) memcpy(lrt_out, s.h_lrt, (size_t)s.n_sites * sizeof(bv_lrt_out));
+    return BV_OK;
+}
+
+int bv_tile_wait_lists_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full,
+                               bv_lrt_out* lrt_out, uint32_t max_lrt, uint32_t* n_lrt) {
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    if (!n_lrt) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists_compact: null n_lrt");
+    bv_slot& s = ctx->slots[slot];
+    if (s.busy && !s.lists_packed) return set_err(ctx, BV_ERR_STATE, "slot %d was not submitted with lists and BV_OUT_COMPACT", slot);
+    int rc = bv_tile_wait_compact(ctx, slot, brief, full, n_full);
+    if (rc != BV_OK) return rc;
+    const uint32_t n = s.n_listed;
+    *n_lrt = n;
+    if (n > max_lrt) return set_err(ctx, BV_ERR_ARG, "tile has %u listed sites > max_lrt %u", n, max_lrt);
+    if (n && !lrt_out) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists_compact: null lrt_out");
+    if (n) memcpy(lrt_out, s.h_lrt, (size_t)n * sizeof(bv_lrt_out));
     return BV_OK;
 }
 
@@ -1292,6 +1404,7 @@ int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d
     if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: tile must be device resident");
     if (tile && tile->n_sites && (!d_lists || !d_lrt_out)) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: null lists / output");
     if (((uintptr_t)d_lists) & 3) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: d_lists must be 4-byte aligned");
+    if (tile && tile->out_mode == BV_OUT_COMPACT) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
     BV_CUDA(ctx, cudaSetDevice(ctx->device));
     bv::SiteKernelArgs a;
     int rc = fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, &a);

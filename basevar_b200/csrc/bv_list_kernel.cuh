@@ -30,6 +30,8 @@ __host__ __device__ __forceinline__ int list_decode(uint32_t w, uint32_t& order)
     return 4;
 }
 
+// kPacked: lrt_out is the site's own entry (the packed list of bv_list_packed_kernel), else the tile's array indexed by site.
+template <bool kPacked>
 __device__ __noinline__ void list_site(uint32_t site, uint32_t w, bv_lrt_out* __restrict__ lrt_out) {
     QualWarp& W = warp_smem();
     const QualCta& cs = cta_shared();
@@ -41,7 +43,7 @@ __device__ __noinline__ void list_site(uint32_t site, uint32_t w, bv_lrt_out* __
     const uint32_t dep[4] = {W.rec.depth[0], W.rec.depth[1], W.rec.depth[2], W.rec.depth[3]};
     const uint32_t total = dep[0] + dep[1] + dep[2] + dep[3] + W.rec.depth_other;
     if (n_list <= 0 || total == 0) {   // skipped, or src/basetype.cpp:132 returns at once: all-zero entry
-        if (lane < 4) reinterpret_cast<uint4*>(lrt_out + site)[lane] = make_uint4(0u, 0u, 0u, 0u);
+        if (lane < 4) reinterpret_cast<uint4*>(kPacked ? lrt_out : lrt_out + site)[lane] = make_uint4(0u, 0u, 0u, 0u);
         __syncwarp();
         return;
     }
@@ -120,14 +122,14 @@ __device__ __noinline__ void list_site(uint32_t site, uint32_t w, bv_lrt_out* __
             if ((vf | vr) != 0 && (rf | rr) != 0) o.fs = fs_from_table(cs.a.logfact, rf, rr, vf, vr);
         }
         o.flags = (uint8_t)flags;
-        lrt_out[site] = o;
+        if (kPacked) *lrt_out = o;
+        else lrt_out[site] = o;
     }
     __syncwarp();
 }
 
-__global__ void __launch_bounds__(kQualWarps * 32, 1) bv_list_kernel(const __grid_constant__ SiteKernelArgs a,
-                                                                     const uint32_t* __restrict__ lists,
-                                                                     bv_lrt_out* __restrict__ lrt_out) {
+// shared state of K8's CTA: the tile's arguments, the LUT, every warp's histogram at zero, its mbarriers
+__device__ __forceinline__ void list_cta_setup(const SiteKernelArgs& a) {
     QualCta& cs = cta_shared();
     QualWarp& W = warp_smem();
     const int lane = threadIdx.x & 31;
@@ -141,10 +143,29 @@ __global__ void __launch_bounds__(kQualWarps * 32, 1) bv_list_kernel(const __gri
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
+}
+
+__global__ void __launch_bounds__(kQualWarps * 32, 1) bv_list_kernel(const __grid_constant__ SiteKernelArgs a,
+                                                                     const uint32_t* __restrict__ lists,
+                                                                     bv_lrt_out* __restrict__ lrt_out) {
+    list_cta_setup(a);
     // every site of the tile, dealt out statically (a site costs one pass over its row; empty lists cost nothing)
     const uint32_t total_warps = gridDim.x * (blockDim.x >> 5);
     for (uint32_t site = (threadIdx.x >> 5) * gridDim.x + blockIdx.x; site < a.n_sites; site += total_warps)
-        list_site(site, __ldg(lists + site), lrt_out);
+        list_site<false>(site, __ldg(lists + site), lrt_out);
+}
+
+// K8 over a packed list (compact results of bv_tile_submit_sparse_lists): pairs[k] = {site, list word} of the k-th listed site,
+// its entry goes to lrt_out[k].  The same per-site code as bv_list_kernel, so entry k is the bytes bv_list_kernel gives its site.
+__global__ void __launch_bounds__(kQualWarps * 32, 1) bv_list_packed_kernel(const __grid_constant__ SiteKernelArgs a,
+                                                                            const uint2* __restrict__ pairs, uint32_t n_pairs,
+                                                                            bv_lrt_out* __restrict__ lrt_out) {
+    list_cta_setup(a);
+    const uint32_t total_warps = gridDim.x * (blockDim.x >> 5);
+    for (uint32_t k = (threadIdx.x >> 5) * gridDim.x + blockIdx.x; k < n_pairs; k += total_warps) {
+        const uint2 p = __ldg(pairs + k);
+        list_site<true>(p.x, p.y, lrt_out + k);
+    }
 }
 
 }  // namespace bv

@@ -198,6 +198,22 @@ class BaseTypeEngine:
         for p in pending:
             wait(*p)
 
+    def _compact_views(self, pb, pf, nf, ns):
+        """numpy views of a compact tile's briefs and full records (the slot's pinned staging)."""
+        briefs = np.ctypeslib.as_array(C.cast(pb, C.POINTER(C.c_uint32)), shape=(ns * 2,)).view(capi.SITE_BRIEF_DTYPE) if ns else \
+            np.zeros(0, capi.SITE_BRIEF_DTYPE)
+        full = (np.ctypeslib.as_array(C.cast(pf, C.POINTER(C.c_uint8)), shape=(nf * 128,)).view(SITE_OUT_DTYPE)
+                if nf else np.zeros(0, SITE_OUT_DTYPE))
+        return briefs, full
+
+    def _collect_compact(self, pb, pf, nf, ref_base, out):
+        """Expand a compact tile into `out` (n_sites records) and note (n_full, briefs that point at a full record)."""
+        ns = len(out)
+        briefs, full = self._compact_views(pb, pf, nf.value, ns)
+        if ns:
+            self.expand_compact(briefs, full, ref_base, out)
+        self.compact_tiles.append((int(nf.value), int(((briefs["w0"] & 0x80000000) != 0).sum())))
+
     def expand_compact(self, briefs, full, ref_base, out):
         """Records of one compact tile into out[:n] (host helper bv_site_expand for the brief-only sites)."""
         is_full = (briefs["w0"] & 0x80000000) != 0
@@ -210,8 +226,27 @@ class BaseTypeEngine:
             out[i] = tmp[0]
         return out
 
-    def call_sparse_calls(self, cells, cells_aux, site_start, ref_base, n_samples):
-        """call_sparse plus the called-site outputs; returns what call_host_calls returns."""
+    def _wait_calls(self, ps, p0, ns, out, ref_base, tmp_calls, tmp_groups, G, compact):
+        """Collect a called-site tile; returns (calls with GLOBAL site indices, groups[n_calls][G])."""
+        n, step = C.c_uint32(0), len(tmp_calls)
+        gp = tmp_groups.ctypes.data if G else None
+        if compact:
+            pb, pf, nf = C.c_void_p(), C.c_void_p(), C.c_uint32(0)
+            self._check(self.lib.bv_tile_wait_calls_compact(self._ctx, ps, C.byref(pb), C.byref(pf), C.byref(nf), tmp_calls.ctypes.data,
+                                                            step, C.byref(n), gp), "bv_tile_wait_calls_compact")
+            self._collect_compact(pb, pf, nf, ref_base[p0:p0 + ns], out[p0:p0 + ns])
+        else:
+            self._check(self.lib.bv_tile_wait_calls(self._ctx, ps, out[p0:].ctypes.data, tmp_calls.ctypes.data, step, C.byref(n), gp),
+                        "bv_tile_wait_calls")
+        c = tmp_calls[:n.value].copy()
+        c["site"] += p0
+        g = tmp_groups.reshape(-1)[:n.value * G].reshape(n.value, G).copy() if G else np.zeros((n.value, 0), GROUP_OUT_DTYPE)
+        return c, g
+
+    def call_sparse_calls(self, cells, cells_aux, site_start, ref_base, n_samples, compact=False):
+        """call_sparse plus the called-site outputs; returns what call_host_calls returns.  compact=True: the tiles ask for
+        BV_OUT_COMPACT (briefs + the full records of the sites that need one), expanded here; self.compact_tiles receives
+        (n_full, briefs pointing at a full record) per tile."""
         S = ref_base.shape[0]
         assert cells.dtype in (np.uint32, np.uint16) and cells_aux.dtype == np.uint32 and site_start.dtype == np.uint32
         fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32
@@ -222,15 +257,12 @@ class BaseTypeEngine:
         tmp_calls = np.zeros(step, CALL_OUT_DTYPE)
         tmp_groups = np.zeros((step, max(G, 1)), GROUP_OUT_DTYPE)
         pending, slot, keep = [], 0, {}
+        self.compact_tiles = []
 
-        def wait(ps, p0):
-            n = C.c_uint32(0)
-            self._check(self.lib.bv_tile_wait_calls(self._ctx, ps, out[p0:].ctypes.data, tmp_calls.ctypes.data, step, C.byref(n),
-                                                    tmp_groups.ctypes.data if G else None), "bv_tile_wait_calls")
-            c = tmp_calls[:n.value].copy()
-            c["site"] += p0
+        def wait(ps, p0, ns):
+            c, g = self._wait_calls(ps, p0, ns, out, ref_base, tmp_calls, tmp_groups, G, compact)
             calls.append(c)
-            groups.append(tmp_groups.reshape(-1)[:n.value * G].reshape(n.value, G).copy() if G else np.zeros((n.value, 0), GROUP_OUT_DTYPE))
+            groups.append(g)
 
         for s0 in range(0, max(S, 1), step):
             ns = min(step, S - s0)
@@ -241,12 +273,12 @@ class BaseTypeEngine:
             keep[slot] = st
             off = min(c0, max(cells.shape[0] - 1, 0))
             t = BvSparseTile(cells[off:].ctypes.data, cells_aux[off:].ctypes.data, st.ctypes.data, ref_base[s0:].ctypes.data, None, ns, n_samples,
-                             fmt, 0)
+                             fmt, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
             self._check(self.lib.bv_tile_submit_sparse_calls(self._ctx, slot, C.byref(t)), "bv_tile_submit_sparse_calls")
-            pending.append((slot, s0))
+            pending.append((slot, s0, ns))
             slot = (slot + 1) % n_slots
-        for ps, p0 in pending:
-            wait(ps, p0)
+        for p in pending:
+            wait(*p)
         calls = np.concatenate(calls) if calls else np.zeros(0, CALL_OUT_DTYPE)
         groups = np.concatenate(groups) if groups else np.zeros((0, G), GROUP_OUT_DTYPE)
         order = np.argsort(calls["site"], kind="stable")
@@ -269,9 +301,9 @@ class BaseTypeEngine:
         else:
             self._check(self.lib.bv_set_groups(self._ctx, None, 0, 0), "bv_set_groups")
 
-    def call_host_calls(self, base, qual, strand, ref_base, mapq, rpr, n_samples):
+    def call_host_calls(self, base, qual, strand, ref_base, mapq, rpr, n_samples, compact=False):
         """Like call_host, plus the called-site outputs.  mapq: uint8 [S][pitch]; rpr: uint16 [S][rpr_pitch].
-        Returns (records, calls sorted by GLOBAL site index, groups[n_calls][n_groups])."""
+        Returns (records, calls sorted by GLOBAL site index, groups[n_calls][n_groups]).  compact: as in call_sparse_calls."""
         S, pitch = base.shape
         assert mapq.shape == base.shape and mapq.dtype == np.uint8 and rpr.dtype == np.uint16 and rpr.shape[0] == S
         rpr_pitch = rpr.shape[1]
@@ -283,28 +315,25 @@ class BaseTypeEngine:
         tmp_calls = np.zeros(step, CALL_OUT_DTYPE)
         tmp_groups = np.zeros((step, max(G, 1)), GROUP_OUT_DTYPE)
         pending, slot = [], 0
+        self.compact_tiles = []
 
-        def wait(ps, p0):
-            n = C.c_uint32(0)
-            self._check(self.lib.bv_tile_wait_calls(self._ctx, ps, out[p0:].ctypes.data, tmp_calls.ctypes.data, step, C.byref(n),
-                                                    tmp_groups.ctypes.data if G else None), "bv_tile_wait_calls")
-            c = tmp_calls[:n.value].copy()
-            c["site"] += p0
+        def wait(ps, p0, ns):
+            c, g = self._wait_calls(ps, p0, ns, out, ref_base, tmp_calls, tmp_groups, G, compact)
             calls.append(c)
-            groups.append(tmp_groups.reshape(-1)[:n.value * G].reshape(n.value, G).copy() if G else np.zeros((n.value, 0), GROUP_OUT_DTYPE))
+            groups.append(g)
 
         for s0 in range(0, max(S, 1), step):
             ns = min(step, S - s0)
             if len(pending) == n_slots:
                 wait(*pending.pop(0))
             t = BvTile(base[s0:].ctypes.data, qual[s0:].ctypes.data, strand[s0:].ctypes.data, ref_base[s0:].ctypes.data, pitch, ns,
-                       n_samples, capi.BV_LOC_HOST, 0)
+                       n_samples, capi.BV_LOC_HOST, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
             a = BvTileAux(mapq[s0:].ctypes.data, rpr[s0:].ctypes.data, rpr_pitch)
             self._check(self.lib.bv_tile_submit_calls(self._ctx, slot, C.byref(t), C.byref(a)), "bv_tile_submit_calls")
-            pending.append((slot, s0))
+            pending.append((slot, s0, ns))
             slot = (slot + 1) % n_slots
-        for ps, p0 in pending:
-            wait(ps, p0)
+        for p in pending:
+            wait(*p)
         calls = np.concatenate(calls) if calls else np.zeros(0, CALL_OUT_DTYPE)
         groups = np.concatenate(groups) if groups else np.zeros((0, G), GROUP_OUT_DTYPE)
         order = np.argsort(calls["site"], kind="stable")
@@ -340,6 +369,54 @@ class BaseTypeEngine:
             wait(ps, p0)
         return out, lrt
 
+    def call_sparse_lists(self, cells, site_start, ref_base, lists, n_samples, fmt=None, compact=False):
+        """call_sparse plus BaseType::lrt(list) per site (bv_tile_submit_sparse_lists).  lists as in call_host_lists; fmt:
+        capi.CELLS_U32 / CELLS_U16, or None to take it from cells.dtype.  Returns (records, lrt): lrt is LRT_OUT_DTYPE [S]
+        (compact=False), or with compact=True one entry per site whose list is non-empty, in site order (the records are then
+        expanded from the compact form; self.compact_tiles as in call_sparse_calls)."""
+        S = ref_base.shape[0]
+        assert cells.dtype in (np.uint32, np.uint16) and site_start.dtype == np.uint32 and site_start.shape[0] == S + 1
+        if fmt is None:
+            fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32
+        lists = np.ascontiguousarray(lists, np.uint8)
+        assert lists.shape == (S, 4)
+        out = np.zeros(S, dtype=SITE_OUT_DTYPE)
+        n_slots, step = self.params.n_slots, self.params.max_sites
+        assert n_slots >= 1 and step >= 1, "engine was created without slots"
+        lrt = np.zeros(S, dtype=LRT_OUT_DTYPE)
+        packed, tmp = [], np.zeros(step, LRT_OUT_DTYPE)
+        pending, slot, keep = [], 0, {}
+        self.compact_tiles = []
+
+        def wait(ps, p0, ns):
+            if not compact:
+                self._check(self.lib.bv_tile_wait_lists(self._ctx, ps, out[p0:].ctypes.data, lrt[p0:].ctypes.data), "bv_tile_wait_lists")
+                return
+            pb, pf, nf, n = C.c_void_p(), C.c_void_p(), C.c_uint32(0), C.c_uint32(0)
+            self._check(self.lib.bv_tile_wait_lists_compact(self._ctx, ps, C.byref(pb), C.byref(pf), C.byref(nf), tmp.ctypes.data, step,
+                                                            C.byref(n)), "bv_tile_wait_lists_compact")
+            self._collect_compact(pb, pf, nf, ref_base[p0:p0 + ns], out[p0:p0 + ns])
+            packed.append(tmp[:n.value].copy())
+
+        for s0 in range(0, max(S, 1), step):
+            ns = min(step, S - s0)
+            if len(pending) == n_slots:
+                wait(*pending.pop(0))
+            c0 = int(site_start[s0])
+            st = site_start[s0:s0 + ns + 1] - np.uint32(c0)
+            keep[slot] = st
+            off = min(c0, max(cells.shape[0] - 1, 0))
+            t = BvSparseTile(cells[off:].ctypes.data, None, st.ctypes.data, ref_base[s0:].ctypes.data, None, ns, n_samples, fmt,
+                             capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
+            self._check(self.lib.bv_tile_submit_sparse_lists(self._ctx, slot, C.byref(t), lists[s0:].ctypes.data), "bv_tile_submit_sparse_lists")
+            pending.append((slot, s0, ns))
+            slot = (slot + 1) % n_slots
+        for p in pending:
+            wait(*p)
+        if compact:
+            lrt = np.concatenate(packed) if packed else np.zeros(0, LRT_OUT_DTYPE)
+        return out, lrt
+
     def call_device_lists(self, d_base, d_qual, d_strand, d_ref, d_lists, n_sites, n_samples, pitch, d_out, d_lrt_out, stream=0):
         """Device-resident call_host_lists: every argument a device pointer (int); d_lists uint8 [n_sites][4], d_lrt_out
         n_sites LRT_OUT_DTYPE entries.  Asynchronous on `stream` (a cudaStream_t handle)."""
@@ -348,7 +425,8 @@ class BaseTypeEngine:
                                                       C.c_void_p(int(d_lrt_out)), C.c_void_p(int(stream))), "bv_tile_run_device_lists")
 
     def last_list_kernel_time(self):
-        """Duration (ms) of K8 bv_list_kernel of the most recent lists tile (profiling must be on); waits for it."""
+        """Duration (ms) of K8 (bv_list_kernel, or bv_list_packed_kernel for compact sparse lists) of the most recent lists tile
+        (profiling must be on); waits for it."""
         ms = C.c_float(0.0)
         self._check(self.lib.bv_last_list_kernel_time(self._ctx, C.byref(ms)), "bv_last_list_kernel_time")
         return float(ms.value)

@@ -55,12 +55,13 @@ TilePacker::TilePacker(uint32_t n_samples, uint32_t max_sites, bool pinned)
     qual_ = plane_alloc(plane, pinned_);
     strand_ = plane_alloc(plane, pinned_);
     mapq_ = plane_alloc(plane, pinned_);
+    rpr_ = reinterpret_cast<uint16_t*>(plane_alloc(plane * sizeof(uint16_t), pinned_));
     ref_ = plane_alloc(max_sites_, pinned_);
 }
 
 TilePacker::~TilePacker() {
     plane_free(base_, pinned_); plane_free(qual_, pinned_); plane_free(strand_, pinned_); plane_free(mapq_, pinned_);
-    plane_free(ref_, pinned_);
+    plane_free(reinterpret_cast<uint8_t*>(rpr_), pinned_); plane_free(ref_, pinned_);
 }
 
 void TilePacker::next_row(char ref_base, uint8_t** b, uint8_t** q, uint8_t** s, uint8_t** m) {
@@ -71,6 +72,7 @@ void TilePacker::next_row(char ref_base, uint8_t** b, uint8_t** q, uint8_t** s, 
     memset(qual_ + row, 0, pitch_);
     memset(strand_ + row, BV_STRAND_NONE, pitch_);
     memset(mapq_ + row, 0, pitch_);
+    memset(rpr_ + row, 0, pitch_ * sizeof(uint16_t));
     ref_[n_sites_] = (uint8_t)ref_base;
     *b = base_ + row; *q = qual_ + row; *s = strand_ + row; *m = mapq_ + row;
     ++n_sites_;
@@ -89,6 +91,12 @@ bv_tile TilePacker::tile() const {
     t.pitch = pitch_; t.n_sites = n_sites_; t.n_samples = n_samples_;
     t.location = BV_LOC_HOST; t.out_mode = BV_OUT_RECORDS;
     return t;
+}
+
+bv_tile_aux TilePacker::aux() const {
+    bv_tile_aux a;
+    a.mapq = mapq_; a.rpr = rpr_; a.rpr_pitch = pitch_;
+    return a;
 }
 
 // ---- SparsePacker -----------------------------------------------------------------------------------------------------
@@ -157,6 +165,9 @@ Context::Context(int device, float min_af, uint32_t max_samples, uint32_t max_si
     p.n_slots = n_slots;
     check(bv_create(device, &p, &ctx_), nullptr, "bv_create");
     max_samples_ = max_samples;
+    max_sites_ = max_sites;
+    min_af_ = min_af;
+    slot_tiles_.resize(n_slots);
 }
 Context::~Context() { bv_destroy(ctx_); }
 void Context::submit(int slot, const bv_tile& tile) { check(bv_tile_submit(ctx_, slot, &tile), ctx_, "bv_tile_submit"); }
@@ -176,10 +187,148 @@ std::vector<bv_site_out> Context::run(const bv_sparse_tile& tile) {
 }
 void Context::submit_lists(int slot, const bv_tile& tile, const uint8_t (*lists)[4]) {
     check(bv_tile_submit_lists(ctx_, slot, &tile, lists), ctx_, "bv_tile_submit_lists");
+    note_tile(slot, tile.n_sites, BV_OUT_RECORDS, tile.ref_base);
 }
 void Context::wait_lists(int slot, bv_site_out* out, bv_lrt_out* lrt_out) {
     check(bv_tile_wait_lists(ctx_, slot, out, lrt_out), ctx_, "bv_tile_wait_lists");
 }
+void Context::submit_lists(int slot, const bv_sparse_tile& tile, const uint8_t (*lists)[4]) {
+    check(bv_tile_submit_sparse_lists(ctx_, slot, &tile, lists), ctx_, "bv_tile_submit_sparse_lists");
+    note_tile(slot, tile.n_sites, (int)tile.out_mode, tile.ref_base);
+}
+
+void Context::note_tile(int slot, uint32_t n_sites, int out_mode, const uint8_t* ref_base) {
+    SlotTile& st = slot_tiles_.at((size_t)slot);
+    st.n_sites = n_sites; st.compact = out_mode == BV_OUT_COMPACT; st.ref_base = ref_base;
+}
+
+// the records part of a result: the compact views (and a copy of the REF bases they expand against), else nothing to do
+void Context::take_records(int slot, TileResult& r, const bv_site_brief* brief, const bv_site_out* full, uint32_t n_full) {
+    const SlotTile& st = slot_tiles_.at((size_t)slot);
+    r.n_sites = st.n_sites;
+    r.compact = st.compact;
+    r.min_af = min_af_;
+    if (!st.compact) return;
+    r.brief = brief; r.full = full; r.n_full = n_full;
+    if (st.n_sites) r.ref_base.assign(st.ref_base, st.ref_base + st.n_sites);
+}
+
+// the context's staging for what a wait copies out before TileResult gets its share: grown once, never zero-filled again
+template <class T>
+static T* staging(std::vector<T>& v, size_t n) {
+    if (v.size() < n) v.resize(n);
+    return v.data();
+}
+
+TileResult Context::wait_lists(int slot) {
+    TileResult r;
+    const SlotTile& st = slot_tiles_.at((size_t)slot);
+    if (!st.compact) {
+        r.records.resize(st.n_sites);
+        r.lrt.resize(st.n_sites);
+        check(bv_tile_wait_lists(ctx_, slot, r.records.data(), r.lrt.data()), ctx_, "bv_tile_wait_lists");
+        take_records(slot, r, nullptr, nullptr, 0);
+        return r;
+    }
+    const bv_site_brief* brief = nullptr;
+    const bv_site_out* full = nullptr;
+    uint32_t n_full = 0, n_lrt = 0;
+    const bv_lrt_out* lrt = staging(lrt_stage_, st.n_sites);
+    check(bv_tile_wait_lists_compact(ctx_, slot, &brief, &full, &n_full, lrt_stage_.data(), st.n_sites, &n_lrt), ctx_,
+          "bv_tile_wait_lists_compact");
+    r.lrt.assign(lrt, lrt + n_lrt);
+    take_records(slot, r, brief, full, n_full);
+    return r;
+}
+
+void Context::set_groups(const std::map<std::string, std::vector<size_t>>& group_smp_idx) {
+    if (group_smp_idx.size() > BV_MAX_GROUPS)
+        throw std::invalid_argument("[ERROR] set_groups: more than " + std::to_string(BV_MAX_GROUPS) + " population groups");
+    std::vector<uint8_t> sg(max_samples_, (uint8_t)BV_GROUP_NONE);
+    uint32_t g = 0;
+    for (const auto& kv : group_smp_idx) {   // std::map: ascending name, the reference's order
+        for (size_t i : kv.second) {
+            if (i >= max_samples_)
+                throw std::invalid_argument("[ERROR] set_groups: sample " + std::to_string(i) + " of group " + kv.first + " is out of range");
+            if (sg[i] != BV_GROUP_NONE)
+                throw std::invalid_argument("[ERROR] set_groups: sample " + std::to_string(i) + " is listed twice");
+            sg[i] = (uint8_t)g;
+        }
+        ++g;
+    }
+    check(bv_set_groups(ctx_, sg.data(), max_samples_, g), ctx_, "bv_set_groups");
+    n_groups_ = g;
+}
+
+void Context::submit_calls(int slot, const bv_tile& tile, const bv_tile_aux& aux) {
+    check(bv_tile_submit_calls(ctx_, slot, &tile, &aux), ctx_, "bv_tile_submit_calls");
+    note_tile(slot, tile.n_sites, tile.location == BV_LOC_HOST ? tile.out_mode : BV_OUT_RECORDS, tile.ref_base);
+}
+
+void Context::submit_calls(int slot, const bv_sparse_tile& tile) {
+    check(bv_tile_submit_sparse_calls(ctx_, slot, &tile), ctx_, "bv_tile_submit_sparse_calls");
+    note_tile(slot, tile.n_sites, (int)tile.out_mode, tile.ref_base);
+}
+
+TileResult Context::wait_calls(int slot) {
+    TileResult r;
+    const SlotTile& st = slot_tiles_.at((size_t)slot);
+    const bv_call_out* calls = staging(calls_stage_, st.n_sites);
+    const bv_group_out* groups = staging(groups_stage_, (size_t)st.n_sites * n_groups_);
+    uint32_t n_calls = 0;
+    bv_group_out* gp = n_groups_ ? groups_stage_.data() : nullptr;
+    if (st.compact) {
+        const bv_site_brief* brief = nullptr;
+        const bv_site_out* full = nullptr;
+        uint32_t n_full = 0;
+        check(bv_tile_wait_calls_compact(ctx_, slot, &brief, &full, &n_full, calls_stage_.data(), st.n_sites, &n_calls, gp), ctx_,
+              "bv_tile_wait_calls_compact");
+        take_records(slot, r, brief, full, n_full);
+    } else {
+        r.records.resize(st.n_sites);
+        check(bv_tile_wait_calls(ctx_, slot, r.records.data(), calls_stage_.data(), st.n_sites, &n_calls, gp), ctx_, "bv_tile_wait_calls");
+        take_records(slot, r, nullptr, nullptr, 0);
+    }
+    // the device lists the called sites in no particular order: ascending site, groups alongside
+    std::vector<uint32_t> order(n_calls);
+    for (uint32_t k = 0; k < n_calls; ++k) order[k] = k;
+    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return calls[a].site < calls[b].site; });
+    r.n_groups = n_groups_;
+    r.calls.resize(n_calls);
+    r.groups.resize((size_t)n_calls * n_groups_);
+    for (uint32_t k = 0; k < n_calls; ++k) {
+        r.calls[k] = calls[order[k]];
+        for (uint32_t g = 0; g < n_groups_; ++g) r.groups[(size_t)k * n_groups_ + g] = groups[(size_t)order[k] * n_groups_ + g];
+    }
+    return r;
+}
+
+// ---- TileResult -------------------------------------------------------------------------------------------------------
+bv_site_out TileResult::record(uint32_t site) const {
+    if (site >= n_sites) throw std::out_of_range("[ERROR] TileResult::record: site out of range");
+    if (!compact) return records[site];
+    const bv_site_brief& b = brief[site];
+    if (b.w0 & 0x80000000u) {
+        const uint32_t k = b.w0 & 0x7fffffffu;
+        if (k >= n_full) throw std::runtime_error("[ERROR] TileResult::record: compact record index out of range");
+        return full[k];
+    }
+    bv_site_out rec;
+    bv_site_expand(&b, ref_base[site], min_af, &rec);
+    return rec;
+}
+
+const bv_call_out* TileResult::call(uint32_t site) const {
+    auto it = std::lower_bound(calls.begin(), calls.end(), site, [](const bv_call_out& c, uint32_t s) { return c.site < s; });
+    return it != calls.end() && it->site == site ? &*it : nullptr;
+}
+
+const bv_group_out* TileResult::group(uint32_t site, uint32_t g) const {
+    const bv_call_out* c = call(site);
+    if (!c || g >= n_groups) return nullptr;
+    return &groups[(size_t)(c - calls.data()) * n_groups + g];
+}
+
 uint64_t Context::launch_count() const { return bv_launch_count(ctx_); }
 double Context::fisher_fs(int ref_fwd, int ref_rev, int alt_fwd, int alt_rev) {
     const int32_t t[4] = {ref_fwd, ref_rev, alt_fwd, alt_rev};
@@ -197,6 +346,29 @@ void Context::ranksum_test(const uint8_t* bases, const int32_t* values, const ui
 BaseType::BaseType(const BatchInfo* bi, const bv_site_out& rec)
     : ref_id_(bi->ref_id), ref_base_(bi->ref_base), ref_pos_(bi->ref_pos), rec_(rec) {
     fill_from_record();
+    lrt_done_ = true;
+}
+
+BaseType::BaseType(const BatchInfo* bi, const bv_group_out& g) : ref_id_(bi->ref_id), ref_base_(bi->ref_base), ref_pos_(bi->ref_pos) {
+    fill_alts(g.flags, g.n_alt, g.alt, g.af);
+}
+
+BaseType::BaseType(const BatchInfo* bi, const bv_lrt_out& lo) : ref_id_(bi->ref_id), ref_base_(bi->ref_base), ref_pos_(bi->ref_pos) {
+    fill_alts(lo.flags, lo.n_alt, lo.alt, lo.af);
+    var_qual_ = lo.qual;
+}
+
+// ALT set and AFs of an lrt(list) result (bv_lrt_out, bv_group_out)
+void BaseType::fill_alts(uint8_t flags, int n_alt, const uint8_t* alt, const double* af) {
+    if (flags & BV_FLAG_ZERO_SUBSET)   // src/basetype.cpp:113-115
+        throw std::runtime_error("[ERROR] The sum of frequence of active bases must always > 0. Check: ");
+    alt_bases_.clear();
+    af_by_lrt_.clear();
+    for (int k = 0; k < n_alt && k < 4; ++k) {
+        const char b = BASES[alt[k] & 3];
+        alt_bases_.push_back(b);
+        af_by_lrt_[b] = af[k];
+    }
     lrt_done_ = true;
 }
 
@@ -274,17 +446,8 @@ void BaseType::lrt_list(const std::vector<char>& specific_bases) {
     bv_lrt_out lo;
     t_one.ctx->submit_lists(0, t_one.packer->tile(), list);
     t_one.ctx->wait_lists(0, nullptr, &lo);
-    if (lo.flags & BV_FLAG_ZERO_SUBSET)   // src/basetype.cpp:113-115
-        throw std::runtime_error("[ERROR] The sum of frequence of active bases must always > 0. Check: ");
-    alt_bases_.clear();
-    af_by_lrt_.clear();
-    for (int k = 0; k < lo.n_alt && k < 4; ++k) {
-        const char b = BASES[lo.alt[k] & 3];
-        alt_bases_.push_back(b);
-        af_by_lrt_[b] = lo.af[k];
-    }
+    fill_alts(lo.flags, lo.n_alt, lo.alt, lo.af);
     var_qual_ = lo.qual;
-    lrt_done_ = true;
 }
 
 void BaseType::fill_from_record() {

@@ -82,11 +82,14 @@ public:
         if (bi.n != n_samples_) throw std::runtime_error("[ERROR] BatchInfo::n does not match the tile's sample count");
         uint8_t *b, *q, *s, *m;
         next_row(bi.ref_base.empty() ? 'N' : bi.ref_base[0], &b, &q, &s, &m);
+        uint16_t* r = rpr_ + (size_t)(n_sites_ - 1) * pitch_;
         for (size_t i = 0; i < bi.n; ++i) {
             b[i] = encode_base(bi.align_bases[i]);
             q[i] = (uint8_t)(bi.align_base_quals[i] - 33);
             s[i] = encode_strand(bi.map_strands[i]);
             m[i] = (uint8_t)(bi.mapqs[i] > 255 ? 255 : bi.mapqs[i] < 0 ? 0 : bi.mapqs[i]);
+            const int rp = bi.base_pos_ranks.empty() ? 0 : bi.base_pos_ranks[i];   // clamped as SparsePacker::add_site does
+            r[i] = (uint16_t)(rp < 0 ? 0 : rp > 65535 ? 65535 : rp);
         }
     }
     // One site of already encoded cells (row pointers of n_samples bytes each; mapq may be null).
@@ -95,6 +98,9 @@ public:
     void next_row(char ref_base, uint8_t** base, uint8_t** qual, uint8_t** strand, uint8_t** mapq);
 
     bv_tile tile() const;   // BV_LOC_HOST tile over the packed sites
+    // the called-site kernels' planes of the same sites: mapqs, and base_pos_ranks clamped to 0..65535 (rows next_row() /
+    // add_site_cells() start are all zero); rpr_pitch = pitch()
+    bv_tile_aux aux() const;
     const uint8_t* mapq_plane() const { return mapq_; }
 
 private:
@@ -102,6 +108,7 @@ private:
     uint64_t pitch_;
     bool pinned_;
     uint8_t *base_ = nullptr, *qual_ = nullptr, *strand_ = nullptr, *mapq_ = nullptr, *ref_ = nullptr;
+    uint16_t* rpr_ = nullptr;
 };
 
 // ---- sparse packer: only the covered cells of a site travel (bv_sparse_tile) ----------------------------------------------
@@ -143,6 +150,29 @@ private:
     uint8_t* ref_ = nullptr;
 };
 
+// ---- the batch results of one tile --------------------------------------------------------------------------------------
+// What Context::wait_calls / wait_lists collect: the records (all of them, or the compact form), the called-site outputs and
+// the list results.  The compact views point into the slot's pinned staging: valid until the slot's next submit.
+struct TileResult {
+    uint32_t n_sites = 0;
+    bool compact = false;
+    std::vector<bv_site_out> records;        // BV_OUT_RECORDS: one per site
+    const bv_site_brief* brief = nullptr;    // BV_OUT_COMPACT: one per site (bv_tile_wait_compact) ...
+    const bv_site_out* full = nullptr;       // ... and the n_full records they point into
+    uint32_t n_full = 0;
+    std::vector<uint8_t> ref_base;           // BV_OUT_COMPACT: the tile's REF bases, for bv_site_expand
+    float min_af = 0.f;
+    std::vector<bv_call_out> calls;          // called sites (n_alt > 0), ascending site
+    uint32_t n_groups = 0;
+    std::vector<bv_group_out> groups;        // [calls.size()][n_groups], groups[k * n_groups + g] belongs to calls[k]
+    std::vector<bv_lrt_out> lrt;             // lists tiles: one per site (BV_OUT_RECORDS), or one per site whose list is
+                                             // non-empty, in site order (BV_OUT_COMPACT)
+
+    bv_site_out record(uint32_t site) const;                      // the site's record (all-REF sites expanded)
+    const bv_call_out* call(uint32_t site) const;                 // null when the site is not called
+    const bv_group_out* group(uint32_t site, uint32_t g) const;   // null when the site is not called
+};
+
 // ---- a context bound to one GPU ---------------------------------------------------------------------------------------
 class Context {
 public:
@@ -160,6 +190,19 @@ public:
     // the same plus BaseType::lrt(list) per site (bv_tile_submit_lists): lists[n_sites][4], BV_LIST_END-terminated
     void submit_lists(int slot, const bv_tile& tile, const uint8_t (*lists)[4]);
     void wait_lists(int slot, bv_site_out* out, bv_lrt_out* lrt_out);
+    // sparse tiles (bv_tile_submit_sparse_lists), BV_OUT_RECORDS or BV_OUT_COMPACT (tile.out_mode); cells_aux is not read
+    void submit_lists(int slot, const bv_sparse_tile& tile, const uint8_t (*lists)[4]);
+    TileResult wait_lists(int slot);   // records or compact view, and `lrt`
+    // Population groups of the called-site kernels (bv_set_groups), as _out_vcf_line's group_smp_idx holds them: group g is the
+    // g-th name in map order (ascending, as basetype_caller.cpp:756 iterates them); samples in no group belong to none.
+    // std::invalid_argument: more than BV_MAX_GROUPS groups, a sample listed twice, a sample index >= max_samples.
+    void set_groups(const std::map<std::string, std::vector<size_t>>& group_smp_idx);
+    uint32_t n_groups() const { return n_groups_; }
+    // The VCF row's batch outputs (bv_tile_submit_calls / bv_tile_submit_sparse_calls): rank sums and population groups of
+    // every called site.  BV_OUT_COMPACT (tile.out_mode) for host tiles; collect with wait_calls.
+    void submit_calls(int slot, const bv_tile& tile, const bv_tile_aux& aux);
+    void submit_calls(int slot, const bv_sparse_tile& tile);
+    TileResult wait_calls(int slot);   // records or compact view, `calls` and `groups`
     uint32_t n_slots() const { return n_slots_; }
     uint64_t launch_count() const;
     bv_ctx* raw() { return ctx_; }
@@ -171,9 +214,20 @@ public:
                       const uint8_t* alt_mask, uint32_t n, double* phred_out);
 
 private:
+    struct SlotTile { uint32_t n_sites = 0; bool compact = false; const uint8_t* ref_base = nullptr; };
+    void note_tile(int slot, uint32_t n_sites, int out_mode, const uint8_t* ref_base);
+    void take_records(int slot, TileResult& r, const bv_site_brief* brief, const bv_site_out* full, uint32_t n_full);
     bv_ctx* ctx_ = nullptr;
     uint32_t n_slots_;
     uint32_t max_samples_ = 0;
+    uint32_t max_sites_ = 0;
+    float min_af_ = 0.f;
+    uint32_t n_groups_ = 0;
+    std::vector<SlotTile> slot_tiles_;
+    // what the waits copy out of the slots before a TileResult takes the tile's share (sized by the largest tile waited for)
+    std::vector<bv_call_out> calls_stage_;
+    std::vector<bv_group_out> groups_stage_;
+    std::vector<bv_lrt_out> lrt_stage_;
 };
 
 // ---- per-site mirror of the reference's class --------------------------------------------------------------------------
@@ -182,6 +236,11 @@ public:
     BaseType() {}
     // Batch path: the record the device produced for this site.
     BaseType(const BatchInfo* smp_bi, const bv_site_out& rec);
+    // Batch path of lrt(list): a population group's result (K6, TileResult::group) or a list's (K8, TileResult::lrt).  The
+    // getters give the ALT set, get_lrt_af and (lists only; 0 for a group) get_var_qual as BaseType(&bi, af).lrt(list) does;
+    // depths are not carried (get_total_depth 0).  Throws like lrt(list) when the EM met a zero-frequency subset.
+    BaseType(const BatchInfo* smp_bi, const bv_group_out& group);
+    BaseType(const BatchInfo* smp_bi, const bv_lrt_out& lrt);
     // Drop-in path (src/basetype.h:105): one site through a one-row tile on the calling thread's default context
     // (device BASEVAR_B200_DEVICE or 0).  `af` is the CLI's float min_af widened to double (basetype_caller.cpp:506).
     BaseType(const BatchInfo* smp_bi, double af);
@@ -206,6 +265,7 @@ public:
 
 private:
     void fill_from_record();
+    void fill_alts(uint8_t flags, int n_alt, const uint8_t* alt, const double* af);
     void lrt_list(const std::vector<char>& specific_bases);
     std::string ref_id_, ref_base_;
     uint32_t ref_pos_ = 0;

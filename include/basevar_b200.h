@@ -28,6 +28,11 @@
  *     (any ordered candidate list)      src/basetype.cpp:130-199         (list kernel K8), bv_lrt_out
  *   ref_vs_alt_ranksumtest(...) for any src/basetype.h:168-176           bv_ranksum_test (rank-sum test kernel K9), one double
  *     ALT set and value list            src/basetype.cpp:201-242         per free-standing problem
+ *   the VCF row of a tile in batch:     src/basetype_caller.cpp:1151-1194 bv_tile_submit_sparse_calls / bv_tile_submit_calls with
+ *     rank sums + groups, compact form                                    BV_OUT_COMPACT, bv_tile_wait_calls_compact
+ *   lrt([REF, ALT...]) at called sites  src/basetype_caller.cpp:747-760   bv_tile_submit_sparse_lists (K8 on the expanded planes);
+ *     of a sparse tile                                                    with BV_OUT_COMPACT one packed entry per listed site,
+ *                                                                         bv_tile_wait_lists_compact
  *
  * Everything is `extern "C"`, plain pointers and sizes, POD structs; no exception crosses the
  * boundary.  Every entry point returns BV_OK (0) or a negative status; bv_last_error() gives text.
@@ -118,6 +123,9 @@ typedef struct bv_tile {
     int32_t  location;       /* BV_LOC_HOST (pinned or pageable) or BV_LOC_DEVICE                         */
     int32_t  out_mode;       /* BV_OUT_RECORDS, or BV_OUT_COMPACT (host tiles; collect with bv_tile_wait_compact) */
 } bv_tile;
+/* Device-resident tiles have no compact form.  bv_tile_submit_calls (device tile), bv_tile_run_device_calls and
+ * bv_tile_run_device_lists refuse out_mode BV_OUT_COMPACT with BV_ERR_ARG; bv_tile_run_device, and bv_tile_submit of a device
+ * tile, do not read out_mode and return records. */
 
 /* ---- per-site result record: fixed 128 bytes --------------------------------------------------- */
 typedef struct bv_site_out {
@@ -247,7 +255,8 @@ int         bv_last_kernel_times(bv_ctx* ctx, float ms[4]);
 int         bv_last_em_kernel_times(bv_ctx* ctx, float ms[2]);
 int         bv_last_fisher_kernel_time(bv_ctx* ctx, float* ms);
 int         bv_last_call_kernel_times(bv_ctx* ctx, float ms[2]);   /* K5 rank sums, K6 population groups */
-int         bv_last_list_kernel_time(bv_ctx* ctx, float* ms);      /* K8 bv_list_kernel of the last lists tile */
+int         bv_last_list_kernel_time(bv_ctx* ctx, float* ms);      /* K8 (bv_list_kernel, or bv_list_packed_kernel for compact
+                                                                    * sparse lists) of the last lists tile */
 int         bv_last_ranksum_kernel_time(bv_ctx* ctx, float* ms);   /* K9 bv_ranksum_test_kernel of the last bv_ranksum_test */
 
 /* ---- tile pipeline (replaces: BatchInfo -> BaseType ctor -> lrt() -> strand_bias per site) ------ */
@@ -319,8 +328,22 @@ typedef struct bv_sparse_tile {
 
 /* Asynchronous, like bv_tile_submit (host memory only; pinned memory makes the copies truly asynchronous). */
 int bv_tile_submit_sparse(bv_ctx* ctx, int slot, const bv_sparse_tile* tile);
-/* The same plus the called-site kernels; collect with bv_tile_wait_calls. */
+/* The same plus the called-site kernels; collect with bv_tile_wait_calls, or with bv_tile_wait_calls_compact when
+ * out_mode is BV_OUT_COMPACT. */
 int bv_tile_submit_sparse_calls(bv_ctx* ctx, int slot, const bv_sparse_tile* tile);
+/* The same as bv_tile_submit_sparse plus lrt(list) per site (K8 on the planes K0 expanded, after the standard kernels); the
+ * records are the bytes bv_tile_submit_sparse gives.  lists: n_sites x 4 bytes in host memory, read during the call, checked
+ * as bv_tile_submit_lists checks them (BV_ERR_ARG, nothing submitted, the slot stays free).  Either cell format.
+ *   out_mode BV_OUT_RECORDS: collect with bv_tile_wait_lists, one bv_lrt_out per site;
+ *   out_mode BV_OUT_COMPACT: only the sites whose list is non-empty travel, 8 bytes up ({site, list}) and one bv_lrt_out
+ *                            down each, packed in site order; collect with bv_tile_wait_lists_compact.
+ * cells_aux is not read: lists and the called-site kernels do not run in one submit. */
+int bv_tile_submit_sparse_lists(bv_ctx* ctx, int slot, const bv_sparse_tile* tile, const uint8_t (*lists)[4]);
+/* For a lists tile with BV_OUT_COMPACT: blocks; brief / full / n_full as bv_tile_wait_compact gives them; lrt_out receives
+ * *n_lrt entries, entry k belonging to the k-th site (in site order) whose list is non-empty.  BV_ERR_ARG (nothing copied to
+ * lrt_out) when *n_lrt exceeds max_lrt. */
+int bv_tile_wait_lists_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full,
+                               bv_lrt_out* lrt_out, uint32_t max_lrt, uint32_t* n_lrt);
 /* BV_CELLS_U32 -> BV_CELLS_U16 on the host (plain C loop): the cells of every site must ascend by sample.  words16 has
  * room for max_words words (bv_sparse_encode16_bound() is always enough; pass words16 == NULL to count only);
  * start16[n_sites + 1] receives the word offsets, *n_words the word count.  BV_ERR_ARG: cells not ascending, a strand
@@ -341,15 +364,22 @@ int bv_synth_fill_sparse_host(const bv_synth_model* model, uint64_t site0, uint3
  * n_groups == 0 turns the group kernel off.  Not allowed while a slot is busy. */
 int bv_set_groups(bv_ctx* ctx, const uint8_t* sample_group, uint32_t n_samples, uint32_t n_groups);
 /* bv_tile_submit + the kernels of the called sites.  `aux` planes live where the tile lives (host or device);
- * pageable host planes are uploaded whole, pinned ones are read in place for the called rows only. */
+ * pageable host planes are uploaded whole, pinned ones are read in place for the called rows only.  Host tiles may ask for
+ * BV_OUT_COMPACT (collect with bv_tile_wait_calls_compact); a device-resident tile that asks for it is refused (BV_ERR_ARG):
+ * there is no device-resident compact form. */
 int bv_tile_submit_calls(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux);
 /* Blocks; `out` receives n_sites records, `calls` up to max_calls entries, `groups` (may be NULL when no groups are
  * set) n_groups entries per call, groups[k * n_groups + g] belonging to calls[k].  *n_calls = number of called sites
  * of the tile; BV_ERR_ARG (nothing copied to calls/groups) when it exceeds max_calls. */
 int bv_tile_wait_calls(bv_ctx* ctx, int slot, bv_site_out* out, bv_call_out* calls, uint32_t max_calls,
                        uint32_t* n_calls, bv_group_out* groups);
+/* For a called-site tile with BV_OUT_COMPACT: blocks; brief / full / n_full as bv_tile_wait_compact gives them, calls / n_calls /
+ * groups as bv_tile_wait_calls.  A called site is never all-REF, so its record is always among `full`; bv_call_out::site is the
+ * site's row index, as in records mode. */
+int bv_tile_wait_calls_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full,
+                               bv_call_out* calls, uint32_t max_calls, uint32_t* n_calls, bv_group_out* groups);
 /* Device-resident variant (tile, aux planes, d_out, d_calls [n_sites], d_groups [n_sites * n_groups] and d_n_calls
- * are device pointers; d_groups may be NULL when no groups are set).  Stream ordered. */
+ * are device pointers; d_groups may be NULL when no groups are set).  Stream ordered.  out_mode must be BV_OUT_RECORDS. */
 int bv_tile_run_device_calls(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux* aux, bv_site_out* d_out,
                              bv_call_out* d_calls, bv_group_out* d_groups, uint32_t* d_n_calls, void* stream);
 
@@ -357,13 +387,15 @@ int bv_tile_run_device_calls(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux
 /* bv_tile_submit + the list kernel (K8 bv_list_kernel), which runs after the standard kernels and reads the depths and
  * strand counts of their records.  The records are the same bytes a plain bv_tile_submit gives.  lists: n_sites x 4
  * bytes in host memory, read during the call.  BV_ERR_ARG (nothing submitted, the slot stays free) for a repeated
- * base or a code that is neither BV_BASE_A..T nor BV_LIST_END.  Dense tiles with out_mode BV_OUT_RECORDS only. */
+ * base or a code that is neither BV_BASE_A..T nor BV_LIST_END.  Dense tiles with out_mode BV_OUT_RECORDS only (sparse tiles,
+ * also with compact results: bv_tile_submit_sparse_lists).  Lists and the called-site kernels do not run in one submit:
+ * bv_tile_wait_calls / bv_tile_wait_calls_compact on a lists slot return BV_ERR_STATE. */
 int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8_t (*lists)[4]);
 /* Blocks; `out` receives n_sites records (may be NULL), `lrt_out` n_sites bv_lrt_out entries. */
 int bv_tile_wait_lists(bv_ctx* ctx, int slot, bv_site_out* out, bv_lrt_out* lrt_out);
 /* Device-resident variant: tile planes, d_lists [n_sites][4] (4-byte aligned), d_out and d_lrt_out are device pointers.
  * Stream ordered, so the lists are not seen before the kernel runs: a list the host entry points would refuse is treated
- * as an empty one here (all-zero entry). */
+ * as an empty one here (all-zero entry).  out_mode must be BV_OUT_RECORDS (there is no device-resident compact form). */
 int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d_lists)[4], bv_site_out* d_out,
                              bv_lrt_out* d_lrt_out, void* stream);
 
