@@ -205,7 +205,7 @@ struct bv_ctx {
     uint32_t rs_problems_cap = 0;
     cudaEvent_t ev_rs[2] = {nullptr, nullptr};   // around K9 bv_ranksum_test_kernel
     bool ev_rs_valid = false;
-    cudaStream_t copy_stream = nullptr;   // uploads of sparse host tiles, in submit order (see tile_submit_sparse_impl)
+    cudaStream_t copy_stream = nullptr;   // uploads of sparse host tiles, in submit order (see upload_sparse)
     bool trace = false;               // BASEVAR_B200_TRACE=1: one line per sparse host tile on stderr at its wait
     cudaEvent_t ev_trace0 = nullptr;  // recorded at the first traced submit: the origin of the timeline
     uint64_t tiles_traced = 0;
@@ -446,47 +446,30 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
     return BV_OK;
 }
 
-// K8 after the standard kernels of the tile (it reads their records): one warp per site with a non-empty list.
-static int launch_list_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const uint32_t* d_lists, bv_lrt_out* d_lrt, cudaStream_t stream) {
-    BvRange range("bv: launch K8 list");
-    if (a.n_sites == 0) return BV_OK;
+// K8 after the standard kernels of the tile (it reads their records), one warp per listed site: over the n = n_sites words of
+// d_lists (bv_list_kernel), or over the n {site, list word} pairs of a compact tile's packed list, entry k for pair k
+// (bv_list_packed_kernel, d_pairs).
+static int launch_list_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const uint32_t* d_lists, const uint2* d_pairs, uint32_t n,
+                              bv_lrt_out* d_lrt, cudaStream_t stream) {
+    BvRange range(d_pairs ? "bv: launch K8 list (packed)" : "bv: launch K8 list");
+    if (n == 0) return BV_OK;
     if (a.n_samples == 0) {   // no reads anywhere: every entry is all-zero
-        BV_CUDA(ctx, cudaMemsetAsync(d_lrt, 0, (size_t)a.n_sites * sizeof(bv_lrt_out), stream));
+        BV_CUDA(ctx, cudaMemsetAsync(d_lrt, 0, (size_t)n * sizeof(bv_lrt_out), stream));
         return BV_OK;
     }
-    if (!ctx->list_kernel_ready) {   // on first use: a context that never runs K8 loads and sets up exactly what it did without it
-        BV_CUDA(ctx, cudaFuncSetAttribute(bv::bv_list_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
-        ctx->list_kernel_ready = true;
+    // on first use: a context that never runs K8 loads and sets up exactly what it did without it
+    bool& ready = d_pairs ? ctx->list_packed_ready : ctx->list_kernel_ready;
+    if (!ready) {
+        BV_CUDA(ctx, cudaFuncSetAttribute(d_pairs ? (const void*)bv::bv_list_packed_kernel : (const void*)bv::bv_list_kernel,
+                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
+        ready = true;
     }
     const bool prof = ctx->profiling;
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[0], stream));
-    uint32_t grid = (a.n_sites + bv::kQualWarps - 1) / bv::kQualWarps;
+    uint32_t grid = (n + bv::kQualWarps - 1) / bv::kQualWarps;
     if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;   // (the bin spill rows are sized for this grid)
-    bv::bv_list_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_lists, d_lrt);
-    BV_CUDA(ctx, cudaGetLastError());
-    ctx->launches += 1;
-    if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[1], stream)); ctx->ev_list_valid = true; }
-    return BV_OK;
-}
-
-// K8 over the packed list of a compact tile (bv_list_packed_kernel): one warp per listed site, entry k for pair k.
-static int launch_list_packed_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const uint2* d_pairs, uint32_t n_pairs, bv_lrt_out* d_lrt,
-                                     cudaStream_t stream) {
-    BvRange range("bv: launch K8 list (packed)");
-    if (n_pairs == 0) return BV_OK;
-    if (a.n_samples == 0) {   // no reads anywhere: every entry is all-zero
-        BV_CUDA(ctx, cudaMemsetAsync(d_lrt, 0, (size_t)n_pairs * sizeof(bv_lrt_out), stream));
-        return BV_OK;
-    }
-    if (!ctx->list_packed_ready) {
-        BV_CUDA(ctx, cudaFuncSetAttribute(bv::bv_list_packed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
-        ctx->list_packed_ready = true;
-    }
-    const bool prof = ctx->profiling;
-    if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[0], stream));
-    uint32_t grid = (n_pairs + bv::kQualWarps - 1) / bv::kQualWarps;
-    if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;   // (the bin spill rows are sized for this grid)
-    bv::bv_list_packed_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_pairs, n_pairs, d_lrt);
+    if (d_pairs) bv::bv_list_packed_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_pairs, n, d_lrt);
+    else bv::bv_list_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_lists, d_lrt);
     BV_CUDA(ctx, cudaGetLastError());
     ctx->launches += 1;
     if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[1], stream)); ctx->ev_list_valid = true; }
@@ -814,13 +797,21 @@ int bv_set_params(bv_ctx* ctx, const bv_params* p) {
     return BV_OK;
 }
 
+// The prologue of the device-resident entry points: the tile's kernel arguments over the context's own scratch.
+// no_compact: the entry point refuses BV_OUT_COMPACT (bv_tile_run_device ignores out_mode).
+static int device_tile_args(bv_ctx* ctx, const bv_tile* tile, bv_site_out* d_out, bool no_compact, bv::SiteKernelArgs* a) {
+    if (no_compact && tile && tile->out_mode == BV_OUT_COMPACT)
+        return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    return fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, a);
+}
+
 int bv_tile_run_device(bv_ctx* ctx, const bv_tile* tile, bv_site_out* d_out, void* stream) {
     BvRange range("bv_tile_run_device");
     if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
     if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device: tile must be device resident");
-    BV_CUDA(ctx, cudaSetDevice(ctx->device));
     bv::SiteKernelArgs a;
-    int rc = fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, &a);
+    int rc = device_tile_args(ctx, tile, d_out, false, &a);
     if (rc != BV_OK) return rc;
     return launch_site_kernel(ctx, a, (cudaStream_t)stream);
 }
@@ -830,10 +821,8 @@ int bv_tile_run_device_calls(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux
     if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
     if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_calls: tile must be device resident");
     if (!d_n_calls) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_calls: null d_n_calls");
-    if (tile && tile->out_mode == BV_OUT_COMPACT) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
-    BV_CUDA(ctx, cudaSetDevice(ctx->device));
     bv::SiteKernelArgs a;
-    int rc = fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, &a);
+    int rc = device_tile_args(ctx, tile, d_out, true, &a);
     if (rc != BV_OK) return rc;
     rc = set_call_args(ctx, tile, aux, ctx->dev_scratch, d_calls, d_groups, &a);
     if (rc != BV_OK) return rc;
@@ -845,6 +834,21 @@ int bv_tile_run_device_calls(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux
     if (rc != BV_OK) return rc;
     BV_CUDA(ctx, cudaMemcpyAsync(d_n_calls, a.counters + bv::kCntCalled, sizeof(uint32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return BV_OK;
+}
+
+int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d_lists)[4], bv_site_out* d_out,
+                             bv_lrt_out* d_lrt_out, void* stream) {
+    BvRange range("bv_tile_run_device_lists");
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: tile must be device resident");
+    if (tile && tile->n_sites && (!d_lists || !d_lrt_out)) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: null lists / output");
+    if (((uintptr_t)d_lists) & 3) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: d_lists must be 4-byte aligned");
+    bv::SiteKernelArgs a;
+    int rc = device_tile_args(ctx, tile, d_out, true, &a);
+    if (rc != BV_OK) return rc;
+    rc = launch_site_kernel(ctx, a, (cudaStream_t)stream);
+    if (rc != BV_OK) return rc;
+    return launch_list_kernel(ctx, a, reinterpret_cast<const uint32_t*>(d_lists), nullptr, a.n_sites, d_lrt_out, (cudaStream_t)stream);
 }
 
 int bv_set_groups(bv_ctx* ctx, const uint8_t* sample_group, uint32_t n_samples, uint32_t n_groups) {
@@ -876,16 +880,6 @@ int bv_set_groups(bv_ctx* ctx, const uint8_t* sample_group, uint32_t n_samples, 
     return BV_OK;
 }
 
-static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls,
-                            const uint8_t (*lists)[4] = nullptr);
-
-int bv_tile_submit(bv_ctx* ctx, int slot, const bv_tile* tile) { return tile_submit_impl(ctx, slot, tile, nullptr, false); }
-
-int bv_tile_submit_calls(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux) {
-    if (!aux) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_calls: null aux");
-    return tile_submit_impl(ctx, slot, tile, aux, true);
-}
-
 // pinned (or otherwise device-accessible) host memory: the pointer the kernels can use, else null
 static const void* host_device_pointer(const void* p) {
     cudaPointerAttributes at;
@@ -894,31 +888,38 @@ static const void* host_device_pointer(const void* p) {
     return nullptr;
 }
 
-static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls,
-                            const uint8_t (*lists)[4]) {
-    BvRange range("bv_tile_submit (dense tile: H2D, kernels, D2H)");
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
-    if (!tile) return set_err(ctx, BV_ERR_ARG, "null tile");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy) return set_err(ctx, BV_ERR_STATE, "slot %d is busy: call bv_tile_wait first", slot);
-    if (tile->n_sites > ctx->prm.max_sites) return set_err(ctx, BV_ERR_ARG, "tile has %u sites > max_sites %u", tile->n_sites, ctx->prm.max_sites);
-    BV_CUDA(ctx, cudaSetDevice(ctx->device));
-    s.qual_host = nullptr;
-    s.h2d_bytes = 0;
-    s.sparse = false; s.out_direct = false; s.out_user = nullptr;
-    s.compact = tile->location == BV_LOC_HOST && tile->out_mode == BV_OUT_COMPACT;
-    s.h_ref = tile->location == BV_LOC_HOST ? tile->ref_base : nullptr;
-    if (with_calls && tile->location == BV_LOC_DEVICE && tile->out_mode == BV_OUT_COMPACT)
-        return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
-    if (lists) {   // checked and staged before anything is queued: a refused tile leaves the slot as it was
-        if (tile->out_mode != BV_OUT_RECORDS) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: out_mode must be BV_OUT_RECORDS");
-        int rc = check_lists(ctx, lists, tile->n_sites);
-        if (rc != BV_OK) return rc;
-        rc = lists_reserve(ctx, s);
-        if (rc != BV_OK) return rc;
-        if (tile->n_sites) memcpy(s.h_lists, lists, (size_t)tile->n_sites * sizeof(uint32_t));
+// The slot of a submit or a wait; null for a null context or a bad slot index, with the error (BV_ERR_ARG) set.
+static bv_slot* slot_of(bv_ctx* ctx, int slot) {
+    if (!ctx) { set_err(nullptr, BV_ERR_ARG, "null context"); return nullptr; }
+    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) { set_err(ctx, BV_ERR_ARG, "bad slot %d", slot); return nullptr; }
+    return &ctx->slots[slot];
+}
+
+// A tile's lists, checked and staged in the slot's pinned memory before anything is queued (a refused tile leaves the slot as it
+// was): one word per site, or for packed results {site, list word} pairs of the sites with a non-empty list, in site order.
+static int stage_lists(bv_ctx* ctx, bv_slot& s, const uint8_t (*lists)[4], uint32_t n_sites, bool packed, uint32_t* n_listed) {
+    int rc = check_lists(ctx, lists, n_sites);
+    if (rc != BV_OK) return rc;
+    rc = lists_reserve(ctx, s);
+    if (rc != BV_OK) return rc;
+    *n_listed = 0;
+    if (packed) {
+        uint2* pairs = reinterpret_cast<uint2*>(s.h_lists);
+        for (uint32_t i = 0; i < n_sites; ++i) {
+            if (lists[i][0] == BV_LIST_END) continue;
+            uint32_t w;
+            memcpy(&w, lists[i], 4);
+            pairs[(*n_listed)++] = make_uint2(i, w);
+        }
+    } else if (n_sites) {
+        memcpy(s.h_lists, lists, (size_t)n_sites * sizeof(uint32_t));
     }
+    return BV_OK;
+}
+
+// Dense tile: the planes of a host tile go up on the slot's stream; a device-resident tile is read where it is.  Fills `a` and
+// s.h2d_bytes.
+static int upload_dense(bv_ctx* ctx, bv_slot& s, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls, bv::SiteKernelArgs* a) {
     bv_tile dev = *tile;
     if (tile->location == BV_LOC_HOST) {
         if (!tile->base || !tile->qual || !tile->strand || !tile->ref_base) return set_err(ctx, BV_ERR_ARG, "bv_tile: null pointer");
@@ -949,112 +950,43 @@ static int tile_submit_impl(bv_ctx* ctx, int slot, const bv_tile* tile, const bv
         dev.pitch = dp;
         dev.location = BV_LOC_DEVICE;
     }
-    bv::SiteKernelArgs a;
-    int rc = fill_kernel_args(ctx, &dev, s.d_out, s.scratch, &a);
+    int rc = fill_kernel_args(ctx, &dev, s.d_out, s.scratch, a);
     if (rc != BV_OK) return rc;
-    if (tile->location == BV_LOC_HOST && s.qual_host) { a.qual = s.qual_host; a.qual_pitch = tile->pitch; }
-    if (s.compact) { a.brief = s.d_brief; a.full_out = static_cast<bv_site_out*>(const_cast<void*>(host_device_pointer(s.h_out))); }
-    if (s.compact && !a.full_out) return set_err(ctx, BV_ERR_CUDA, "pinned staging is not device accessible");
-    if (with_calls) {
-        bv_tile_aux dev_aux = *aux;
-        if (tile->location == BV_LOC_HOST && tile->n_sites) {
-            // the aux planes are read for the called rows only: in place when pinned, else uploaded whole
-            const uint8_t* zm = static_cast<const uint8_t*>(host_device_pointer(aux->mapq));
-            const uint16_t* zr = static_cast<const uint16_t*>(host_device_pointer(aux->rpr));
-            if (aux->rpr_pitch % 8 != 0 || aux->rpr_pitch < tile->n_samples) return set_err(ctx, BV_ERR_ARG, "bv_tile_aux: bad rpr_pitch");
-            if (zm && zr) {
-                dev_aux.mapq = zm; dev_aux.rpr = zr;
-                rc = set_call_args(ctx, &dev, &dev_aux, s.scratch, s.h_calls, s.h_groups, &a);
-                a.aux_pitch = tile->pitch;
-            } else {
-                const size_t plane = (size_t)ctx->prm.max_sites * ctx->pitch_cap;
-                if (!s.d_aux) BV_CUDA(ctx, cudaMalloc(&s.d_aux, 3 * plane));
-                const uint64_t dp = dev.pitch;
-                BV_CUDA(ctx, cudaMemcpy2DAsync(s.d_aux, dp, aux->mapq, tile->pitch, dp, tile->n_sites, cudaMemcpyHostToDevice, s.stream));
-                BV_CUDA(ctx, cudaMemcpy2DAsync(s.d_aux + plane, 2 * dp, aux->rpr, 2 * aux->rpr_pitch, 2 * (size_t)tile->n_samples, tile->n_sites,
-                                               cudaMemcpyHostToDevice, s.stream));
-                s.h2d_bytes += (size_t)tile->n_sites * (dp + 2 * (size_t)tile->n_samples);
-                dev_aux.mapq = s.d_aux; dev_aux.rpr = reinterpret_cast<const uint16_t*>(s.d_aux + plane); dev_aux.rpr_pitch = dp;
-                rc = set_call_args(ctx, &dev, &dev_aux, s.scratch, s.h_calls, s.h_groups, &a);
-            }
+    if (s.qual_host) { a->qual = s.qual_host; a->qual_pitch = tile->pitch; }
+    if (!with_calls) return BV_OK;
+    bv_tile_aux dev_aux = *aux;
+    bool aux_in_place = false;
+    if (tile->location == BV_LOC_HOST && tile->n_sites) {
+        // the aux planes are read for the called rows only: in place when pinned, else uploaded whole
+        const uint8_t* zm = static_cast<const uint8_t*>(host_device_pointer(aux->mapq));
+        const uint16_t* zr = static_cast<const uint16_t*>(host_device_pointer(aux->rpr));
+        if (aux->rpr_pitch % 8 != 0 || aux->rpr_pitch < tile->n_samples) return set_err(ctx, BV_ERR_ARG, "bv_tile_aux: bad rpr_pitch");
+        aux_in_place = zm && zr;
+        if (aux_in_place) {
+            dev_aux.mapq = zm; dev_aux.rpr = zr;
         } else {
-            rc = set_call_args(ctx, &dev, &dev_aux, s.scratch, s.h_calls, s.h_groups, &a);
+            const size_t plane = (size_t)ctx->prm.max_sites * ctx->pitch_cap;
+            if (!s.d_aux) BV_CUDA(ctx, cudaMalloc(&s.d_aux, 3 * plane));
+            const uint64_t dp = dev.pitch;
+            BV_CUDA(ctx, cudaMemcpy2DAsync(s.d_aux, dp, aux->mapq, tile->pitch, dp, tile->n_sites, cudaMemcpyHostToDevice, s.stream));
+            BV_CUDA(ctx, cudaMemcpy2DAsync(s.d_aux + plane, 2 * dp, aux->rpr, 2 * aux->rpr_pitch, 2 * (size_t)tile->n_samples, tile->n_sites,
+                                           cudaMemcpyHostToDevice, s.stream));
+            s.h2d_bytes += (size_t)tile->n_sites * (dp + 2 * (size_t)tile->n_samples);
+            dev_aux.mapq = s.d_aux; dev_aux.rpr = reinterpret_cast<const uint16_t*>(s.d_aux + plane); dev_aux.rpr_pitch = dp;
         }
-        if (rc != BV_OK) return rc;
     }
-    rc = launch_site_kernel(ctx, a, s.stream);
-    if (rc != BV_OK) return rc;
-    if (lists && tile->n_sites) {
-        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, (size_t)tile->n_sites * sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
-        rc = launch_list_kernel(ctx, a, s.d_lists, s.d_lrt, s.stream);
-        if (rc != BV_OK) return rc;
-        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)tile->n_sites * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
-    }
-    rc = return_records(ctx, s, a, tile->n_sites, s.h_out);
-    if (rc != BV_OK) return rc;
-    if (with_calls || s.compact) {
-        s.h_counters[bv::kCntCalled] = 0; s.h_counters[bv::kCntFull] = 0;
-        if (tile->n_sites && tile->n_samples)
-            BV_CUDA(ctx, cudaMemcpyAsync(s.h_counters, a.counters, bv::kNumCounters * sizeof(uint32_t), cudaMemcpyDeviceToHost, s.stream));
-    }
-    s.with_calls = with_calls;
-    s.with_lists = lists != nullptr;
-    s.lists_packed = false;
-    s.n_listed = 0;
-    s.n_sites = tile->n_sites;
-    s.busy = true;
-    if (tile->location == BV_LOC_HOST) ctx->h2d_bytes_total += s.h2d_bytes;
-    return BV_OK;
+    rc = set_call_args(ctx, &dev, &dev_aux, s.scratch, s.h_calls, s.h_groups, a);
+    if (aux_in_place) a->aux_pitch = tile->pitch;   // (the caller's planes keep the caller's pitch)
+    return rc;
 }
 
-// Sparse host tile: upload the covered cells (4 bytes each), expand them into the slot's dense planes (K0), then the
-// same kernels as for a dense tile.  The qual plane -- and for the called-site kernels the mapq / rpr planes -- are
-// device resident here (there is no host plane to read in place).  With lists, K8 follows on the expanded planes.
-static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* t, bool with_calls,
-                                   const uint8_t (*lists)[4] = nullptr) {
-    BvRange range("bv_tile_submit_sparse (H2D of the cells, K0 expand, kernels, D2H)");
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
-    if (!t) return set_err(ctx, BV_ERR_ARG, "null tile");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy) return set_err(ctx, BV_ERR_STATE, "slot %d is busy: call bv_tile_wait first", slot);
-    if (t->n_sites > ctx->prm.max_sites) return set_err(ctx, BV_ERR_ARG, "tile has %u sites > max_sites %u", t->n_sites, ctx->prm.max_sites);
-    if (t->n_samples > ctx->prm.max_samples || t->n_samples > BV_CELL_MAX_SAMPLES)
-        return set_err(ctx, BV_ERR_ARG, "sparse tile: n_samples %u > max_samples %u or > %u", t->n_samples, ctx->prm.max_samples, BV_CELL_MAX_SAMPLES);
-    if (t->n_sites && (!t->site_start || !t->ref_base)) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: null pointer");
-    if (t->format != BV_CELLS_U32 && t->format != BV_CELLS_U16) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: unknown format %u", t->format);
+// Sparse host tile: upload the covered cells (4 or 2 bytes each) and expand them into the slot's dense planes (K0).  The qual
+// plane -- and for the called-site kernels the mapq / rpr planes -- are device resident here (there is no host plane to read in
+// place).  Fills `a` and s.h2d_bytes; trace: records the first two events of the tile's timeline.
+static int upload_sparse(bv_ctx* ctx, bv_slot& s, const bv_sparse_tile* t, bool with_calls, bool trace, bv::SiteKernelArgs* a) {
     const bool u16 = t->format == BV_CELLS_U16;
     const size_t word_bytes = u16 ? sizeof(uint16_t) : sizeof(uint32_t);
     const uint64_t n_cells = t->n_sites ? t->site_start[t->n_sites] : 0;   // words of `format`
-    if (t->n_sites && t->site_start[0] != 0) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: site_start[0] must be 0");
-    if (n_cells && (!t->cells || (with_calls && !t->cells_aux))) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: null cells");
-    if (n_cells > (uint64_t)t->n_sites * ((uint64_t)t->n_samples + (u16 ? t->n_samples / BV_CELL16_GAP_SKIP + 2u : 0u)))
-        return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: more cells than sample-sites");
-    BV_CUDA(ctx, cudaSetDevice(ctx->device));
-    s.qual_host = nullptr;
-    s.h2d_bytes = 0;
-    s.sparse = true; s.out_direct = false; s.out_user = t->out;
-    s.compact = t->out_mode == BV_OUT_COMPACT;
-    s.h_ref = t->ref_base;
-    if (s.compact && t->out) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: `out` must be NULL");
-    uint32_t n_listed = 0;
-    if (lists) {   // checked and staged before anything is queued: a refused tile leaves the slot as it was
-        int rc = check_lists(ctx, lists, t->n_sites);
-        if (rc != BV_OK) return rc;
-        rc = lists_reserve(ctx, s);
-        if (rc != BV_OK) return rc;
-        if (s.compact) {   // the listed sites only, as {site, list word} pairs in site order
-            uint2* pairs = reinterpret_cast<uint2*>(s.h_lists);
-            for (uint32_t i = 0; i < t->n_sites; ++i) {
-                if (lists[i][0] == BV_LIST_END) continue;
-                uint32_t w;
-                memcpy(&w, lists[i], 4);
-                pairs[n_listed++] = make_uint2(i, w);
-            }
-        } else if (t->n_sites) {
-            memcpy(s.h_lists, lists, (size_t)t->n_sites * sizeof(uint32_t));
-        }
-    }
     if (n_cells > s.cells_cap) {   // grows only; sized by the first tiles of a run
         if (s.d_cells) BV_CUDA(ctx, cudaFree(s.d_cells));
         s.d_cells = nullptr; s.cells_cap = 0;
@@ -1069,21 +1001,14 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
     bv_tile dev;
     dev.base = s.d_planes; dev.qual = s.d_planes + plane; dev.strand = s.d_planes + 2 * plane; dev.ref_base = s.d_ref;
     dev.pitch = dp; dev.n_sites = t->n_sites; dev.n_samples = t->n_samples; dev.location = BV_LOC_DEVICE; dev.out_mode = BV_OUT_RECORDS;
-    bv::SiteKernelArgs a;
-    int rc = fill_kernel_args(ctx, &dev, s.d_out, s.scratch, &a);
+    int rc = fill_kernel_args(ctx, &dev, s.d_out, s.scratch, a);
     if (rc != BV_OK) return rc;
-    if (s.compact) {
-        a.brief = s.d_brief; a.full_out = static_cast<bv_site_out*>(const_cast<void*>(host_device_pointer(s.h_out)));
-        if (!a.full_out) return set_err(ctx, BV_ERR_CUDA, "pinned staging is not device accessible");
-    }
     if (with_calls) {
         bv_tile_aux dev_aux;
         dev_aux.mapq = s.d_aux; dev_aux.rpr = reinterpret_cast<const uint16_t*>(s.d_aux + plane); dev_aux.rpr_pitch = dp;
-        rc = set_call_args(ctx, &dev, &dev_aux, s.scratch, s.h_calls, s.h_groups, &a);
+        rc = set_call_args(ctx, &dev, &dev_aux, s.scratch, s.h_calls, s.h_groups, a);
         if (rc != BV_OK) return rc;
     }
-    memset(s.h_counters, 0, bv::kNumCounters * sizeof(uint32_t));
-    const bool trace = ctx->trace && t->n_sites && t->n_samples;
     // Uploads go through ONE stream, in submit order.  On the slots' own streams the uploads of the tiles in flight run side by
     // side and share the link: they all finish together, then their kernels run with the link idle, and the pipeline moves in
     // waves (100,000-sample tiles, 4 slots: 75 % of the bare-copy rate; profiles/r02_tile_timeline.txt).  First in, first out,
@@ -1114,13 +1039,13 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
         if (trace) BV_CUDA(ctx, cudaEventRecord(s.ev_trace[1], up));
         BV_CUDA(ctx, cudaEventRecord(s.ev_up, up));
         BV_CUDA(ctx, cudaStreamWaitEvent(s.stream, s.ev_up, 0));
-        BV_CUDA(ctx, cudaMemsetAsync(a.counters, 0, bv::kNumCounters * sizeof(uint32_t), s.stream));
+        BV_CUDA(ctx, cudaMemsetAsync(a->counters, 0, bv::kNumCounters * sizeof(uint32_t), s.stream));
         bv::ExpandArgs x;
         x.cells = s.d_cells; x.cells_aux = with_calls ? s.d_cells + s.cells_cap : nullptr; x.site_start = s.d_site_start;
         x.base = s.d_planes; x.qual = s.d_planes + plane; x.strand = s.d_planes + 2 * plane;
         x.mapq = with_calls ? s.d_aux : nullptr;
         x.rpr = with_calls ? reinterpret_cast<uint16_t*>(s.d_aux + plane) : nullptr;
-        x.counters = a.counters;
+        x.counters = a->counters;
         x.pitch = dp; x.rpr_pitch = dp; x.n_cells = n_cells; x.n_sites = t->n_sites; x.n_samples = t->n_samples;
         uint32_t grid = (t->n_sites + bv::kExpandWarps - 1) / bv::kExpandWarps;
         const uint32_t cap = (uint32_t)ctx->num_sms * 2u;   // persistent: 2 CTAs of 16 warps per SM (96 KB of staging each)
@@ -1130,47 +1055,139 @@ static int tile_submit_sparse_impl(bv_ctx* ctx, int slot, const bv_sparse_tile* 
         BV_CUDA(ctx, cudaGetLastError());
         ctx->launches += 1;
     }
-    rc = launch_site_kernel(ctx, a, s.stream, /*counters_zeroed=*/true);
+    return BV_OK;
+}
+
+// Everything after the upload of a slot's tile, on the slot's stream: K1..K6; with lists their upload, K8 (per site, or over the
+// packed list of a compact tile) and its results back; the records back into dst; the counters back for the slots whose wait reads
+// them (sparse, called-site or compact tiles); and the slot's bookkeeping.  trace: the last two events of a traced tile.
+static int submit_tail(bv_ctx* ctx, bv_slot& s, bv::SiteKernelArgs& a, bool with_calls, bool with_lists, uint32_t n_listed,
+                       bool counters_zeroed, bool trace, bv_site_out* dst) {
+    const uint32_t n_sites = a.n_sites;
+    if (s.compact) {
+        a.brief = s.d_brief;
+        a.full_out = static_cast<bv_site_out*>(const_cast<void*>(host_device_pointer(s.h_out)));
+        if (!a.full_out) return set_err(ctx, BV_ERR_CUDA, "pinned staging is not device accessible");
+    }
+    int rc = launch_site_kernel(ctx, a, s.stream, counters_zeroed);
     if (rc != BV_OK) return rc;
-    if (lists && s.compact && n_listed) {
-        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, (size_t)n_listed * sizeof(uint2), cudaMemcpyHostToDevice, s.stream));
-        rc = launch_list_packed_kernel(ctx, a, reinterpret_cast<const uint2*>(s.d_lists), n_listed, s.d_lrt, s.stream);
+    const bool packed = with_lists && s.compact;
+    const uint32_t n_lrt = packed ? n_listed : n_sites;
+    if (with_lists && n_lrt) {
+        const size_t list_bytes = (size_t)n_lrt * (packed ? sizeof(uint2) : sizeof(uint32_t));
+        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, list_bytes, cudaMemcpyHostToDevice, s.stream));
+        rc = launch_list_kernel(ctx, a, s.d_lists, packed ? reinterpret_cast<const uint2*>(s.d_lists) : nullptr, n_lrt, s.d_lrt, s.stream);
         if (rc != BV_OK) return rc;
-        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)n_listed * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
-        s.h2d_bytes += (size_t)n_listed * sizeof(uint2);
-    } else if (lists && !s.compact && t->n_sites) {
-        BV_CUDA(ctx, cudaMemcpyAsync(s.d_lists, s.h_lists, (size_t)t->n_sites * sizeof(uint32_t), cudaMemcpyHostToDevice, s.stream));
-        rc = launch_list_kernel(ctx, a, s.d_lists, s.d_lrt, s.stream);
-        if (rc != BV_OK) return rc;
-        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)t->n_sites * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
-        s.h2d_bytes += (size_t)t->n_sites * sizeof(uint32_t);
+        BV_CUDA(ctx, cudaMemcpyAsync(s.h_lrt, s.d_lrt, (size_t)n_lrt * sizeof(bv_lrt_out), cudaMemcpyDeviceToHost, s.stream));
+        s.h2d_bytes += list_bytes;
     }
     if (trace) BV_CUDA(ctx, cudaEventRecord(s.ev_trace[2], s.stream));
-    if (t->n_sites) {
-        bv_site_out* dst = s.h_out;
-        if (t->out && host_device_pointer(t->out)) { dst = t->out; s.out_direct = true; }
-        rc = return_records(ctx, s, a, t->n_sites, dst);
-        if (rc != BV_OK) return rc;
-        if (t->n_samples)
+    rc = return_records(ctx, s, a, n_sites, dst);
+    if (rc != BV_OK) return rc;
+    if (s.sparse || with_calls || s.compact) {   // (a tile without cells leaves them zero)
+        memset(s.h_counters, 0, bv::kNumCounters * sizeof(uint32_t));
+        if (n_sites && a.n_samples)
             BV_CUDA(ctx, cudaMemcpyAsync(s.h_counters, a.counters, bv::kNumCounters * sizeof(uint32_t), cudaMemcpyDeviceToHost, s.stream));
     }
     if (trace) BV_CUDA(ctx, cudaEventRecord(s.ev_trace[3], s.stream));
     s.with_calls = with_calls;
-    s.with_lists = lists != nullptr;
-    s.lists_packed = lists && s.compact;
+    s.with_lists = with_lists;
+    s.lists_packed = packed;
     s.n_listed = n_listed;
-    s.n_sites = t->n_sites;
+    s.n_sites = n_sites;
     s.busy = true;
     ctx->h2d_bytes_total += s.h2d_bytes;
     return BV_OK;
 }
 
-int bv_tile_submit_sparse(bv_ctx* ctx, int slot, const bv_sparse_tile* tile) { return tile_submit_sparse_impl(ctx, slot, tile, false); }
-int bv_tile_submit_sparse_calls(bv_ctx* ctx, int slot, const bv_sparse_tile* tile) { return tile_submit_sparse_impl(ctx, slot, tile, true); }
+// Dense tile, host or device resident (bv_tile_submit, _calls, _lists).
+static int tile_submit_dense(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux, bool with_calls,
+                             const uint8_t (*lists)[4] = nullptr) {
+    BvRange range("bv_tile_submit (dense tile: H2D, kernels, D2H)");
+    bv_slot* sp = slot_of(ctx, slot);
+    if (!sp) return BV_ERR_ARG;
+    if (!tile) return set_err(ctx, BV_ERR_ARG, "null tile");
+    bv_slot& s = *sp;
+    if (s.busy) return set_err(ctx, BV_ERR_STATE, "slot %d is busy: call bv_tile_wait first", slot);
+    if (tile->n_sites > ctx->prm.max_sites) return set_err(ctx, BV_ERR_ARG, "tile has %u sites > max_sites %u", tile->n_sites, ctx->prm.max_sites);
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    s.qual_host = nullptr;
+    s.h2d_bytes = 0;
+    s.sparse = false; s.out_direct = false; s.out_user = nullptr;
+    s.compact = tile->location == BV_LOC_HOST && tile->out_mode == BV_OUT_COMPACT;
+    s.h_ref = tile->location == BV_LOC_HOST ? tile->ref_base : nullptr;
+    if (with_calls && tile->location == BV_LOC_DEVICE && tile->out_mode == BV_OUT_COMPACT)
+        return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
+    uint32_t n_listed = 0;
+    if (lists) {
+        if (tile->out_mode != BV_OUT_RECORDS) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: out_mode must be BV_OUT_RECORDS");
+        const int rc = stage_lists(ctx, s, lists, tile->n_sites, false, &n_listed);
+        if (rc != BV_OK) return rc;
+    }
+    bv::SiteKernelArgs a;
+    int rc = upload_dense(ctx, s, tile, aux, with_calls, &a);
+    if (rc != BV_OK) return rc;
+    return submit_tail(ctx, s, a, with_calls, lists != nullptr, n_listed, false, false, s.h_out);
+}
+
+// Sparse host tile (bv_tile_submit_sparse, _calls, _lists): the cells up, K0 expand, then what a dense tile runs.
+static int tile_submit_sparse(bv_ctx* ctx, int slot, const bv_sparse_tile* t, bool with_calls, const uint8_t (*lists)[4] = nullptr) {
+    BvRange range("bv_tile_submit_sparse (H2D of the cells, K0 expand, kernels, D2H)");
+    bv_slot* sp = slot_of(ctx, slot);
+    if (!sp) return BV_ERR_ARG;
+    if (!t) return set_err(ctx, BV_ERR_ARG, "null tile");
+    bv_slot& s = *sp;
+    if (s.busy) return set_err(ctx, BV_ERR_STATE, "slot %d is busy: call bv_tile_wait first", slot);
+    if (t->n_sites > ctx->prm.max_sites) return set_err(ctx, BV_ERR_ARG, "tile has %u sites > max_sites %u", t->n_sites, ctx->prm.max_sites);
+    if (t->n_samples > ctx->prm.max_samples || t->n_samples > BV_CELL_MAX_SAMPLES)
+        return set_err(ctx, BV_ERR_ARG, "sparse tile: n_samples %u > max_samples %u or > %u", t->n_samples, ctx->prm.max_samples, BV_CELL_MAX_SAMPLES);
+    if (t->n_sites && (!t->site_start || !t->ref_base)) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: null pointer");
+    if (t->format != BV_CELLS_U32 && t->format != BV_CELLS_U16) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: unknown format %u", t->format);
+    const bool u16 = t->format == BV_CELLS_U16;
+    const uint64_t n_cells = t->n_sites ? t->site_start[t->n_sites] : 0;   // words of `format`
+    if (t->n_sites && t->site_start[0] != 0) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: site_start[0] must be 0");
+    if (n_cells && (!t->cells || (with_calls && !t->cells_aux))) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: null cells");
+    if (n_cells > (uint64_t)t->n_sites * ((uint64_t)t->n_samples + (u16 ? t->n_samples / BV_CELL16_GAP_SKIP + 2u : 0u)))
+        return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: more cells than sample-sites");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    s.qual_host = nullptr;
+    s.h2d_bytes = 0;
+    s.sparse = true; s.out_direct = false; s.out_user = t->out;
+    s.compact = t->out_mode == BV_OUT_COMPACT;
+    s.h_ref = t->ref_base;
+    if (s.compact && t->out) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: `out` must be NULL");
+    uint32_t n_listed = 0;
+    if (lists) {
+        const int rc = stage_lists(ctx, s, lists, t->n_sites, s.compact, &n_listed);
+        if (rc != BV_OK) return rc;
+    }
+    const bool trace = ctx->trace && t->n_sites && t->n_samples;
+    bv::SiteKernelArgs a;
+    int rc = upload_sparse(ctx, s, t, with_calls, trace, &a);
+    if (rc != BV_OK) return rc;
+    // pinned records of the caller: the D2H copy goes straight into them
+    s.out_direct = t->n_sites && t->out && host_device_pointer(t->out);
+    return submit_tail(ctx, s, a, with_calls, lists != nullptr, n_listed, true, trace, s.out_direct ? t->out : s.h_out);
+}
+
+int bv_tile_submit(bv_ctx* ctx, int slot, const bv_tile* tile) { return tile_submit_dense(ctx, slot, tile, nullptr, false); }
+
+int bv_tile_submit_calls(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux) {
+    if (!aux) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_calls: null aux");
+    return tile_submit_dense(ctx, slot, tile, aux, true);
+}
+
+int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8_t (*lists)[4]) {
+    if (!lists) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: null lists");
+    return tile_submit_dense(ctx, slot, tile, nullptr, false, lists);
+}
+
+int bv_tile_submit_sparse(bv_ctx* ctx, int slot, const bv_sparse_tile* tile) { return tile_submit_sparse(ctx, slot, tile, false); }
+int bv_tile_submit_sparse_calls(bv_ctx* ctx, int slot, const bv_sparse_tile* tile) { return tile_submit_sparse(ctx, slot, tile, true); }
 int bv_tile_submit_sparse_lists(bv_ctx* ctx, int slot, const bv_sparse_tile* tile, const uint8_t (*lists)[4]) {
     if (tile && tile->n_sites && !lists) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_sparse_lists: null lists");
     static const uint8_t no_lists[1][4] = {{BV_LIST_END, BV_LIST_END, BV_LIST_END, BV_LIST_END}};   // (an empty tile may pass NULL)
-    return tile_submit_sparse_impl(ctx, slot, tile, false, lists ? lists : no_lists);
+    return tile_submit_sparse(ctx, slot, tile, false, lists ? lists : no_lists);
 }
 
 uint64_t bv_sparse_encode16_bound(uint64_t n_cells, uint32_t n_sites, uint32_t n_samples) {
@@ -1259,11 +1276,11 @@ int bv_synth_fill_sparse_host(const bv_synth_model* model, uint64_t site0, uint3
     return BV_OK;
 }
 
-int bv_tile_wait(bv_ctx* ctx, int slot, bv_site_out* out) {
+// The wait of every form: synchronise the slot, print its trace line, report bad cells; then the records into `out` (and into the
+// sparse tile's `out`), or with `brief` the views of a compact tile's pinned staging.
+static int wait_slot(bv_ctx* ctx, int slot, bv_slot& s, bv_site_out* out, const bv_site_brief** brief = nullptr,
+                     const bv_site_out** full = nullptr, uint32_t* n_full = nullptr) {
     BvRange range("bv_tile_wait");
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
-    bv_slot& s = ctx->slots[slot];
     if (!s.busy) return set_err(ctx, BV_ERR_STATE, "slot %d has nothing submitted", slot);
     BV_CUDA(ctx, cudaSetDevice(ctx->device));
     const double t_wait0 = ctx->trace ? host_seconds() - ctx->t_trace0 : 0.0;
@@ -1281,7 +1298,9 @@ int bv_tile_wait(bv_ctx* ctx, int slot, bv_site_out* out) {
     if (s.sparse && s.n_sites && s.h_counters[bv::kCntBadCell])
         return set_err(ctx, BV_ERR_ARG, "sparse tile: cell with sample >= n_samples or site_start not ascending / beyond the cell count");
     if (s.compact) {   // collected in compact form (bv_tile_wait_compact), or expanded here for a caller that wants records
-        if (out) {
+        if (brief) {
+            *brief = s.h_brief; *full = s.h_out; *n_full = s.n_sites ? s.h_counters[bv::kCntFull] : 0;
+        } else if (out) {
             const uint32_t n_full = s.h_counters[bv::kCntFull];
             for (uint32_t i = 0; i < s.n_sites; ++i) {
                 const bv_site_brief& b = s.h_brief[i];
@@ -1300,16 +1319,17 @@ int bv_tile_wait(bv_ctx* ctx, int slot, bv_site_out* out) {
     return BV_OK;
 }
 
+int bv_tile_wait(bv_ctx* ctx, int slot, bv_site_out* out) {
+    bv_slot* s = slot_of(ctx, slot);
+    return s ? wait_slot(ctx, slot, *s, out) : BV_ERR_ARG;
+}
+
 int bv_tile_wait_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full) {
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    bv_slot* s = slot_of(ctx, slot);
+    if (!s) return BV_ERR_ARG;
     if (!brief || !full || !n_full) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_compact: null argument");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy && !s.compact) return set_err(ctx, BV_ERR_STATE, "slot %d was not submitted with BV_OUT_COMPACT", slot);
-    int rc = bv_tile_wait(ctx, slot, nullptr);
-    if (rc != BV_OK) return rc;
-    *brief = s.h_brief; *full = s.h_out; *n_full = s.n_sites ? s.h_counters[bv::kCntFull] : 0;
-    return BV_OK;
+    if (s->busy && !s->compact) return set_err(ctx, BV_ERR_STATE, "slot %d was not submitted with BV_OUT_COMPACT", slot);
+    return wait_slot(ctx, slot, *s, nullptr, brief, full, n_full);
 }
 
 void bv_site_expand(const bv_site_brief* b, uint8_t ref_base, float min_af, bv_site_out* out) {
@@ -1340,78 +1360,52 @@ static int copy_calls(bv_ctx* ctx, const bv_slot& s, bv_call_out* calls, uint32_
 
 int bv_tile_wait_calls(bv_ctx* ctx, int slot, bv_site_out* out, bv_call_out* calls, uint32_t max_calls,
                        uint32_t* n_calls, bv_group_out* groups) {
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    bv_slot* s = slot_of(ctx, slot);
+    if (!s) return BV_ERR_ARG;
     if (!n_calls) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_calls: null n_calls");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy && !s.with_calls) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without called-site kernels", slot);
-    int rc = bv_tile_wait(ctx, slot, out);
+    if (s->busy && !s->with_calls) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without called-site kernels", slot);
+    int rc = wait_slot(ctx, slot, *s, out);
     if (rc != BV_OK) return rc;
-    return copy_calls(ctx, s, calls, max_calls, n_calls, groups);
+    return copy_calls(ctx, *s, calls, max_calls, n_calls, groups);
 }
 
 int bv_tile_wait_calls_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full,
                                bv_call_out* calls, uint32_t max_calls, uint32_t* n_calls, bv_group_out* groups) {
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    bv_slot* s = slot_of(ctx, slot);
+    if (!s) return BV_ERR_ARG;
     if (!n_calls) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_calls_compact: null n_calls");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy && !s.with_calls) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without called-site kernels", slot);
+    if (s->busy && !s->with_calls) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without called-site kernels", slot);
     int rc = bv_tile_wait_compact(ctx, slot, brief, full, n_full);
     if (rc != BV_OK) return rc;
-    return copy_calls(ctx, s, calls, max_calls, n_calls, groups);
-}
-
-int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8_t (*lists)[4]) {
-    if (!lists) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_lists: null lists");
-    return tile_submit_impl(ctx, slot, tile, nullptr, false, lists);
+    return copy_calls(ctx, *s, calls, max_calls, n_calls, groups);
 }
 
 int bv_tile_wait_lists(bv_ctx* ctx, int slot, bv_site_out* out, bv_lrt_out* lrt_out) {
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    bv_slot* s = slot_of(ctx, slot);
+    if (!s) return BV_ERR_ARG;
     if (!lrt_out) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists: null lrt_out");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy && !s.with_lists) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without lists", slot);
-    if (s.busy && s.lists_packed) return set_err(ctx, BV_ERR_STATE, "slot %d has compact results: collect with bv_tile_wait_lists_compact", slot);
-    int rc = bv_tile_wait(ctx, slot, out);
+    if (s->busy && !s->with_lists) return set_err(ctx, BV_ERR_STATE, "slot %d was submitted without lists", slot);
+    if (s->busy && s->lists_packed) return set_err(ctx, BV_ERR_STATE, "slot %d has compact results: collect with bv_tile_wait_lists_compact", slot);
+    int rc = wait_slot(ctx, slot, *s, out);
     if (rc != BV_OK) return rc;
-    if (s.n_sites) memcpy(lrt_out, s.h_lrt, (size_t)s.n_sites * sizeof(bv_lrt_out));
+    if (s->n_sites) memcpy(lrt_out, s->h_lrt, (size_t)s->n_sites * sizeof(bv_lrt_out));
     return BV_OK;
 }
 
 int bv_tile_wait_lists_compact(bv_ctx* ctx, int slot, const bv_site_brief** brief, const bv_site_out** full, uint32_t* n_full,
                                bv_lrt_out* lrt_out, uint32_t max_lrt, uint32_t* n_lrt) {
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (slot < 0 || (uint32_t)slot >= ctx->prm.n_slots || !ctx->slots) return set_err(ctx, BV_ERR_ARG, "bad slot %d", slot);
+    bv_slot* s = slot_of(ctx, slot);
+    if (!s) return BV_ERR_ARG;
     if (!n_lrt) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists_compact: null n_lrt");
-    bv_slot& s = ctx->slots[slot];
-    if (s.busy && !s.lists_packed) return set_err(ctx, BV_ERR_STATE, "slot %d was not submitted with lists and BV_OUT_COMPACT", slot);
+    if (s->busy && !s->lists_packed) return set_err(ctx, BV_ERR_STATE, "slot %d was not submitted with lists and BV_OUT_COMPACT", slot);
     int rc = bv_tile_wait_compact(ctx, slot, brief, full, n_full);
     if (rc != BV_OK) return rc;
-    const uint32_t n = s.n_listed;
+    const uint32_t n = s->n_listed;
     *n_lrt = n;
     if (n > max_lrt) return set_err(ctx, BV_ERR_ARG, "tile has %u listed sites > max_lrt %u", n, max_lrt);
     if (n && !lrt_out) return set_err(ctx, BV_ERR_ARG, "bv_tile_wait_lists_compact: null lrt_out");
-    if (n) memcpy(lrt_out, s.h_lrt, (size_t)n * sizeof(bv_lrt_out));
+    if (n) memcpy(lrt_out, s->h_lrt, (size_t)n * sizeof(bv_lrt_out));
     return BV_OK;
-}
-
-int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d_lists)[4], bv_site_out* d_out,
-                             bv_lrt_out* d_lrt_out, void* stream) {
-    BvRange range("bv_tile_run_device_lists");
-    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
-    if (tile && tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: tile must be device resident");
-    if (tile && tile->n_sites && (!d_lists || !d_lrt_out)) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: null lists / output");
-    if (((uintptr_t)d_lists) & 3) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_lists: d_lists must be 4-byte aligned");
-    if (tile && tile->out_mode == BV_OUT_COMPACT) return set_err(ctx, BV_ERR_ARG, "BV_OUT_COMPACT: device-resident tiles have no compact form");
-    BV_CUDA(ctx, cudaSetDevice(ctx->device));
-    bv::SiteKernelArgs a;
-    int rc = fill_kernel_args(ctx, tile, d_out, ctx->dev_scratch, &a);
-    if (rc != BV_OK) return rc;
-    rc = launch_site_kernel(ctx, a, (cudaStream_t)stream);
-    if (rc != BV_OK) return rc;
-    return launch_list_kernel(ctx, a, reinterpret_cast<const uint32_t*>(d_lists), d_lrt_out, (cudaStream_t)stream);
 }
 
 int bv_synth_fill_rpr_device(bv_ctx* ctx, uint64_t site0, uint32_t n_sites, uint32_t n_samples, uint64_t rpr_pitch,

@@ -6,6 +6,7 @@
 what ``BaseType`` + ``strand_bias`` would have produced.  Tiles are pipelined over ``n_slots`` CUDA
 streams (H2D copy, kernel, D2H copy per slot).
 """
+import collections
 import ctypes as C
 
 import numpy as np
@@ -62,7 +63,7 @@ class BaseTypeEngine:
 
     @property
     def h2d_bytes(self):
-        """Bytes uploaded by bv_tile_submit so far (host tiles)."""
+        """Bytes uploaded by the bv_tile_submit* calls so far (planes or cells of host tiles, lists of lists tiles)."""
         return int(self.lib.bv_h2d_bytes(self._ctx))
 
     KERNEL_NAMES = ("bv_count_kernel", "bv_scalar_kernel", "bv_bound_kernel", "bv_em_kernel")
@@ -86,6 +87,53 @@ class BaseTypeEngine:
         self._check(self.lib.bv_last_fisher_kernel_time(self._ctx, C.cast(C.byref(ms, 8), C.POINTER(C.c_float))), "bv_last_fisher_kernel_time")
         return dict(zip(self.EM_KERNEL_NAMES, (float(x) for x in ms)))
 
+    # -- the slot pipeline -------------------------------------------------------------------------
+    def _site_ranges(self, S):
+        """(site0, n_sites) of the tiles of S sites, max_sites each; no sites is one empty tile."""
+        step = self.params.max_sites
+        assert step >= 1, "engine was created without slots"
+        return [(s0, min(step, S - s0)) for s0 in range(0, max(S, 1), step)]
+
+    def _pipeline(self, tiles, submit, wait):
+        """submit(slot, tile) each tile on the slots in turn, at most n_slots in flight, and wait(slot, tile) for each in submit
+        order: the oldest before its slot takes the next tile, the rest at the end.  A tile stays referenced until its wait, and
+        with it the arrays its descriptor points into."""
+        n_slots = self.params.n_slots
+        assert n_slots >= 1, "engine was created without slots"
+        pending, slot = collections.deque(), 0
+        for tile in tiles:
+            if len(pending) == n_slots:
+                wait(*pending.popleft())
+            submit(slot, tile)
+            pending.append((slot, tile))
+            slot = (slot + 1) % n_slots
+        for p in pending:
+            wait(*p)
+
+    def _dense_tiles(self, base, qual, strand, ref_base, n_samples, out_mode=capi.OUT_RECORDS):
+        """(BvTile, site0, None) of each tile of host planes [S][pitch]."""
+        S, pitch = base.shape
+        return ((BvTile(base[s0:].ctypes.data, qual[s0:].ctypes.data, strand[s0:].ctypes.data, ref_base[s0:].ctypes.data, pitch, ns,
+                        n_samples, capi.BV_LOC_HOST, out_mode), s0, None) for s0, ns in self._site_ranges(S))
+
+    def _sparse_tiles(self, cells, cells_aux, site_start, ref_base, n_samples, fmt=None, out_mode=capi.OUT_RECORDS, out=None,
+                      pinned=False):
+        """(BvSparseTile, site0, its site_start) of each tile: the per-tile offsets start at 0, rebased from the whole-run array (a
+        packer writes them so), and must live until the tile's wait.  out: records array the D2H copy writes in place.  pinned:
+        the rebased offsets are pinned (a pageable source makes cudaMemcpyAsync wait for the uploads queued in front of it)."""
+        if fmt is None:
+            fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32   # uint16: the delta-coded compact form
+        for s0, ns in self._site_ranges(ref_base.shape[0]):
+            c0 = int(site_start[s0])
+            st = site_start[s0:s0 + ns + 1]
+            if c0 or pinned:
+                st = _alloc(ns + 1, np.uint32, pinned)
+                st[:] = site_start[s0:s0 + ns + 1] - np.uint32(c0)
+            # (cells[c0:] of a tile without cells is the end of the array, which the tile never reads)
+            t = BvSparseTile(cells[c0:].ctypes.data, cells_aux[c0:].ctypes.data if cells_aux is not None else None, st.ctypes.data,
+                             ref_base[s0:].ctypes.data, out[s0:].ctypes.data if out is not None else None, ns, n_samples, fmt, out_mode)
+            yield t, s0, st
+
     # -- tiles from host memory --------------------------------------------------------------------
     def call_host(self, base, qual, strand, ref_base, n_samples, out=None):
         """Run planes [S][pitch] (numpy uint8, ideally pinned) through the slot pipeline.
@@ -97,22 +145,14 @@ class BaseTypeEngine:
             assert a.dtype == np.uint8 and a.flags["C_CONTIGUOUS"]
         if out is None:
             out = np.zeros(S, dtype=SITE_OUT_DTYPE)
-        n_slots, step = self.params.n_slots, self.params.max_sites
-        assert n_slots >= 1 and step >= 1, "engine was created without slots"
-        pending = []  # (slot, site0)
-        slot = 0
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            if len(pending) == n_slots:
-                ps, p0 = pending.pop(0)
-                self._check(self.lib.bv_tile_wait(self._ctx, ps, out[p0:].ctypes.data), "bv_tile_wait")
-            t = BvTile(base[s0:].ctypes.data, qual[s0:].ctypes.data, strand[s0:].ctypes.data,
-                       ref_base[s0:].ctypes.data, pitch, ns, n_samples, capi.BV_LOC_HOST, 0)
-            self._check(self.lib.bv_tile_submit(self._ctx, slot, C.byref(t)), "bv_tile_submit")
-            pending.append((slot, s0))
-            slot = (slot + 1) % n_slots
-        for ps, p0 in pending:
-            self._check(self.lib.bv_tile_wait(self._ctx, ps, out[p0:].ctypes.data), "bv_tile_wait")
+
+        def submit(slot, tile):
+            self._check(self.lib.bv_tile_submit(self._ctx, slot, C.byref(tile[0])), "bv_tile_submit")
+
+        def wait(slot, tile):
+            self._check(self.lib.bv_tile_wait(self._ctx, slot, out[tile[1]:].ctypes.data), "bv_tile_wait")
+
+        self._pipeline(self._dense_tiles(base, qual, strand, ref_base, n_samples), submit, wait)
         return out
 
     # -- sparse tiles from host memory: only the covered cells cross PCIe ---------------------------------
@@ -123,28 +163,10 @@ class BaseTypeEngine:
         records).  With out_pinned=True `out` is pinned host memory and the D2H DMA writes the records in place."""
         S = ref_base.shape[0]
         assert cells.dtype in (np.uint32, np.uint16) and site_start.dtype == np.uint32 and site_start.shape[0] == S + 1
-        fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32   # uint16: the delta-coded compact form
         if out is None:
             out = np.zeros(S, dtype=SITE_OUT_DTYPE)
-        n_slots, step = self.params.n_slots, self.params.max_sites
-        assert n_slots >= 1 and step >= 1, "engine was created without slots"
-        pending, slot, keep = [], 0, {}
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            if len(pending) == n_slots:
-                ps, p0 = pending.pop(0)
-                self._check(self.lib.bv_tile_wait(self._ctx, ps, None if out_pinned else out[p0:].ctypes.data), "bv_tile_wait")
-            c0 = int(site_start[s0])
-            # per-tile offsets start at 0 (a packer writes them so; here they are rebased from the whole-run array)
-            st = site_start[s0:s0 + ns + 1] - np.uint32(c0) if c0 else site_start[s0:s0 + ns + 1]
-            keep[slot] = st
-            t = BvSparseTile(cells[c0:].ctypes.data if c0 < cells.shape[0] else cells.ctypes.data, None, st.ctypes.data,
-                             ref_base[s0:].ctypes.data, out[s0:].ctypes.data if out_pinned else None, ns, n_samples, fmt, 0)
-            self._check(self.lib.bv_tile_submit_sparse(self._ctx, slot, C.byref(t)), "bv_tile_submit_sparse")
-            pending.append((slot, s0))
-            slot = (slot + 1) % n_slots
-        for ps, p0 in pending:
-            self._check(self.lib.bv_tile_wait(self._ctx, ps, None if out_pinned else out[p0:].ctypes.data), "bv_tile_wait")
+        tiles = self._sparse_tiles(cells, None, site_start, ref_base, n_samples, out=out if out_pinned else None)
+        self.run_sparse_tiles(tiles, out=None if out_pinned else out)
         return out
 
     def sparse_tiles(self, cells, site_start, ref_base, n_samples, out_pinned=None, compact=False):
@@ -153,50 +175,29 @@ class BaseTypeEngine:
         site + the full records of the sites that need one; collect with run_sparse_tiles(..., compact=...))."""
         S = ref_base.shape[0]
         assert cells.dtype in (np.uint32, np.uint16) and site_start.dtype == np.uint32 and site_start.shape[0] == S + 1
-        fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32
-        step = self.params.max_sites
-        tiles = []
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            c0 = int(site_start[s0])
-            # (pinned when the records are: a pageable source makes cudaMemcpyAsync wait for the uploads queued in front of it)
-            st = _alloc(ns + 1, np.uint32, out_pinned is not None)
-            st[:] = site_start[s0:s0 + ns + 1] - np.uint32(c0)
-            t = BvSparseTile(cells[c0:].ctypes.data if c0 < cells.shape[0] else cells.ctypes.data, None, st.ctypes.data,
-                             ref_base[s0:].ctypes.data, out_pinned[s0:].ctypes.data if out_pinned is not None and not compact else None,
-                             ns, n_samples, fmt, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
-            tiles.append((t, s0, st))
-        return tiles
+        return list(self._sparse_tiles(cells, None, site_start, ref_base, n_samples, out_mode=capi.OUT_COMPACT if compact else capi.OUT_RECORDS,
+                                       out=out_pinned if not compact else None, pinned=out_pinned is not None))
 
     def run_sparse_tiles(self, tiles, repeats=1, out=None, compact=None):
         """Submit the tiles `repeats` times over the slots without draining the pipeline in between (the steps of a
         benchmark run, or the tiles of a long region); every slot is waited for before its next submit and at the end.
         compact: for BV_OUT_COMPACT tiles a callable (site0, n_sites, briefs, full_records) that consumes a tile's compact
         result (numpy views of the slot's pinned staging, valid during the call only); None drops them (timing runs)."""
-        n_slots = self.params.n_slots
-        pending, slot = [], 0
+        def submit(slot, tile):
+            self._check(self.lib.bv_tile_submit_sparse(self._ctx, slot, C.byref(tile[0])), "bv_tile_submit_sparse")
 
-        def wait(ps, p0, ns, is_compact):
-            if not is_compact:
-                self._check(self.lib.bv_tile_wait(self._ctx, ps, out[p0:].ctypes.data if out is not None else None), "bv_tile_wait")
+        def wait(slot, tile):
+            t, s0, _ = tile
+            if t.out_mode != capi.OUT_COMPACT:
+                self._check(self.lib.bv_tile_wait(self._ctx, slot, out[s0:].ctypes.data if out is not None else None), "bv_tile_wait")
                 return
             pb, pf, nf = C.c_void_p(), C.c_void_p(), C.c_uint32(0)
-            self._check(self.lib.bv_tile_wait_compact(self._ctx, ps, C.byref(pb), C.byref(pf), C.byref(nf)), "bv_tile_wait_compact")
+            self._check(self.lib.bv_tile_wait_compact(self._ctx, slot, C.byref(pb), C.byref(pf), C.byref(nf)), "bv_tile_wait_compact")
+            ns = int(t.n_sites)
             if compact is not None and ns:
-                briefs = np.ctypeslib.as_array(C.cast(pb, C.POINTER(C.c_uint32)), shape=(ns * 2,)).view(capi.SITE_BRIEF_DTYPE)
-                full = (np.ctypeslib.as_array(C.cast(pf, C.POINTER(C.c_uint8)), shape=(nf.value * 128,)).view(SITE_OUT_DTYPE)
-                        if nf.value else np.zeros(0, SITE_OUT_DTYPE))
-                compact(p0, ns, briefs, full)
+                compact(s0, ns, *self._compact_views(pb, pf, nf.value, ns))
 
-        for _ in range(repeats):
-            for t, s0, _keep in tiles:
-                if len(pending) == n_slots:
-                    wait(*pending.pop(0))
-                self._check(self.lib.bv_tile_submit_sparse(self._ctx, slot, C.byref(t)), "bv_tile_submit_sparse")
-                pending.append((slot, s0, int(t.n_sites), t.out_mode == capi.OUT_COMPACT))
-                slot = (slot + 1) % n_slots
-        for p in pending:
-            wait(*p)
+        self._pipeline((tile for _ in range(repeats) for tile in tiles), submit, wait)
 
     def _compact_views(self, pb, pf, nf, ns):
         """numpy views of a compact tile's briefs and full records (the slot's pinned staging)."""
@@ -226,22 +227,40 @@ class BaseTypeEngine:
             out[i] = tmp[0]
         return out
 
-    def _wait_calls(self, ps, p0, ns, out, ref_base, tmp_calls, tmp_groups, G, compact):
-        """Collect a called-site tile; returns (calls with GLOBAL site indices, groups[n_calls][G])."""
-        n, step = C.c_uint32(0), len(tmp_calls)
+    def _run_calls(self, S, tiles, submit, ref_base, compact):
+        """The slot pipeline of tiles with the called-site kernels.  Returns (records, calls sorted by GLOBAL site index,
+        groups[n_calls][n_groups]); with compact=True the records are expanded from the compact form and self.compact_tiles
+        receives (n_full, briefs pointing at a full record) per tile."""
+        G = getattr(self, "n_groups", 0)
+        step = self.params.max_sites
+        out = np.zeros(S, dtype=SITE_OUT_DTYPE)
+        calls, groups = [], []
+        tmp_calls = np.zeros(step, CALL_OUT_DTYPE)
+        tmp_groups = np.zeros((step, max(G, 1)), GROUP_OUT_DTYPE)
         gp = tmp_groups.ctypes.data if G else None
-        if compact:
-            pb, pf, nf = C.c_void_p(), C.c_void_p(), C.c_uint32(0)
-            self._check(self.lib.bv_tile_wait_calls_compact(self._ctx, ps, C.byref(pb), C.byref(pf), C.byref(nf), tmp_calls.ctypes.data,
-                                                            step, C.byref(n), gp), "bv_tile_wait_calls_compact")
-            self._collect_compact(pb, pf, nf, ref_base[p0:p0 + ns], out[p0:p0 + ns])
-        else:
-            self._check(self.lib.bv_tile_wait_calls(self._ctx, ps, out[p0:].ctypes.data, tmp_calls.ctypes.data, step, C.byref(n), gp),
-                        "bv_tile_wait_calls")
-        c = tmp_calls[:n.value].copy()
-        c["site"] += p0
-        g = tmp_groups.reshape(-1)[:n.value * G].reshape(n.value, G).copy() if G else np.zeros((n.value, 0), GROUP_OUT_DTYPE)
-        return c, g
+        self.compact_tiles = []
+
+        def wait(slot, tile):
+            t, s0, _ = tile
+            ns, n = int(t.n_sites), C.c_uint32(0)
+            if compact:
+                pb, pf, nf = C.c_void_p(), C.c_void_p(), C.c_uint32(0)
+                self._check(self.lib.bv_tile_wait_calls_compact(self._ctx, slot, C.byref(pb), C.byref(pf), C.byref(nf), tmp_calls.ctypes.data,
+                                                                step, C.byref(n), gp), "bv_tile_wait_calls_compact")
+                self._collect_compact(pb, pf, nf, ref_base[s0:s0 + ns], out[s0:s0 + ns])
+            else:
+                self._check(self.lib.bv_tile_wait_calls(self._ctx, slot, out[s0:].ctypes.data, tmp_calls.ctypes.data, step, C.byref(n), gp),
+                            "bv_tile_wait_calls")
+            c = tmp_calls[:n.value].copy()
+            c["site"] += s0
+            calls.append(c)
+            groups.append(tmp_groups.reshape(-1)[:n.value * G].reshape(n.value, G).copy() if G else np.zeros((n.value, 0), GROUP_OUT_DTYPE))
+
+        self._pipeline(tiles, submit, wait)
+        calls = np.concatenate(calls) if calls else np.zeros(0, CALL_OUT_DTYPE)
+        groups = np.concatenate(groups) if groups else np.zeros((0, G), GROUP_OUT_DTYPE)
+        order = np.argsort(calls["site"], kind="stable")
+        return out, calls[order], groups[order]
 
     def call_sparse_calls(self, cells, cells_aux, site_start, ref_base, n_samples, compact=False):
         """call_sparse plus the called-site outputs; returns what call_host_calls returns.  compact=True: the tiles ask for
@@ -249,40 +268,12 @@ class BaseTypeEngine:
         (n_full, briefs pointing at a full record) per tile."""
         S = ref_base.shape[0]
         assert cells.dtype in (np.uint32, np.uint16) and cells_aux.dtype == np.uint32 and site_start.dtype == np.uint32
-        fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32
-        G = getattr(self, "n_groups", 0)
-        out = np.zeros(S, dtype=SITE_OUT_DTYPE)
-        n_slots, step = self.params.n_slots, self.params.max_sites
-        calls, groups = [], []
-        tmp_calls = np.zeros(step, CALL_OUT_DTYPE)
-        tmp_groups = np.zeros((step, max(G, 1)), GROUP_OUT_DTYPE)
-        pending, slot, keep = [], 0, {}
-        self.compact_tiles = []
 
-        def wait(ps, p0, ns):
-            c, g = self._wait_calls(ps, p0, ns, out, ref_base, tmp_calls, tmp_groups, G, compact)
-            calls.append(c)
-            groups.append(g)
+        def submit(slot, tile):
+            self._check(self.lib.bv_tile_submit_sparse_calls(self._ctx, slot, C.byref(tile[0])), "bv_tile_submit_sparse_calls")
 
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            if len(pending) == n_slots:
-                wait(*pending.pop(0))
-            c0 = int(site_start[s0])
-            st = site_start[s0:s0 + ns + 1] - np.uint32(c0)
-            keep[slot] = st
-            off = min(c0, max(cells.shape[0] - 1, 0))
-            t = BvSparseTile(cells[off:].ctypes.data, cells_aux[off:].ctypes.data, st.ctypes.data, ref_base[s0:].ctypes.data, None, ns, n_samples,
-                             fmt, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
-            self._check(self.lib.bv_tile_submit_sparse_calls(self._ctx, slot, C.byref(t)), "bv_tile_submit_sparse_calls")
-            pending.append((slot, s0, ns))
-            slot = (slot + 1) % n_slots
-        for p in pending:
-            wait(*p)
-        calls = np.concatenate(calls) if calls else np.zeros(0, CALL_OUT_DTYPE)
-        groups = np.concatenate(groups) if groups else np.zeros((0, G), GROUP_OUT_DTYPE)
-        order = np.argsort(calls["site"], kind="stable")
-        return out, calls[order], groups[order]
+        tiles = self._sparse_tiles(cells, cells_aux, site_start, ref_base, n_samples, out_mode=capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
+        return self._run_calls(S, tiles, submit, ref_base, compact)
 
     # -- called sites: rank sums + population groups ---------------------------------------------------
     CALL_KERNEL_NAMES = ("bv_ranksum_kernel", "bv_group_kernel")
@@ -307,37 +298,14 @@ class BaseTypeEngine:
         S, pitch = base.shape
         assert mapq.shape == base.shape and mapq.dtype == np.uint8 and rpr.dtype == np.uint16 and rpr.shape[0] == S
         rpr_pitch = rpr.shape[1]
-        G = getattr(self, "n_groups", 0)
-        out = np.zeros(S, dtype=SITE_OUT_DTYPE)
-        n_slots, step = self.params.n_slots, self.params.max_sites
-        assert n_slots >= 1 and step >= 1, "engine was created without slots"
-        calls, groups = [], []
-        tmp_calls = np.zeros(step, CALL_OUT_DTYPE)
-        tmp_groups = np.zeros((step, max(G, 1)), GROUP_OUT_DTYPE)
-        pending, slot = [], 0
-        self.compact_tiles = []
 
-        def wait(ps, p0, ns):
-            c, g = self._wait_calls(ps, p0, ns, out, ref_base, tmp_calls, tmp_groups, G, compact)
-            calls.append(c)
-            groups.append(g)
-
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            if len(pending) == n_slots:
-                wait(*pending.pop(0))
-            t = BvTile(base[s0:].ctypes.data, qual[s0:].ctypes.data, strand[s0:].ctypes.data, ref_base[s0:].ctypes.data, pitch, ns,
-                       n_samples, capi.BV_LOC_HOST, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
+        def submit(slot, tile):
+            t, s0, _ = tile
             a = BvTileAux(mapq[s0:].ctypes.data, rpr[s0:].ctypes.data, rpr_pitch)
             self._check(self.lib.bv_tile_submit_calls(self._ctx, slot, C.byref(t), C.byref(a)), "bv_tile_submit_calls")
-            pending.append((slot, s0, ns))
-            slot = (slot + 1) % n_slots
-        for p in pending:
-            wait(*p)
-        calls = np.concatenate(calls) if calls else np.zeros(0, CALL_OUT_DTYPE)
-        groups = np.concatenate(groups) if groups else np.zeros((0, G), GROUP_OUT_DTYPE)
-        order = np.argsort(calls["site"], kind="stable")
-        return out, calls[order], groups[order]
+
+        tiles = self._dense_tiles(base, qual, strand, ref_base, n_samples, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
+        return self._run_calls(S, tiles, submit, ref_base, compact)
 
     # -- lrt(specific_bases): per-site ordered candidate lists -------------------------------------------
     def call_host_lists(self, base, qual, strand, ref_base, lists, n_samples):
@@ -349,24 +317,15 @@ class BaseTypeEngine:
         assert lists.shape == (S, 4)
         out = np.zeros(S, dtype=SITE_OUT_DTYPE)
         lrt = np.zeros(S, dtype=LRT_OUT_DTYPE)
-        n_slots, step = self.params.n_slots, self.params.max_sites
-        assert n_slots >= 1 and step >= 1, "engine was created without slots"
-        pending, slot = [], 0
 
-        def wait(ps, p0):
-            self._check(self.lib.bv_tile_wait_lists(self._ctx, ps, out[p0:].ctypes.data, lrt[p0:].ctypes.data), "bv_tile_wait_lists")
+        def submit(slot, tile):
+            self._check(self.lib.bv_tile_submit_lists(self._ctx, slot, C.byref(tile[0]), lists[tile[1]:].ctypes.data), "bv_tile_submit_lists")
 
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            if len(pending) == n_slots:
-                wait(*pending.pop(0))
-            t = BvTile(base[s0:].ctypes.data, qual[s0:].ctypes.data, strand[s0:].ctypes.data, ref_base[s0:].ctypes.data, pitch, ns,
-                       n_samples, capi.BV_LOC_HOST, 0)
-            self._check(self.lib.bv_tile_submit_lists(self._ctx, slot, C.byref(t), lists[s0:].ctypes.data), "bv_tile_submit_lists")
-            pending.append((slot, s0))
-            slot = (slot + 1) % n_slots
-        for ps, p0 in pending:
-            wait(ps, p0)
+        def wait(slot, tile):
+            s0 = tile[1]
+            self._check(self.lib.bv_tile_wait_lists(self._ctx, slot, out[s0:].ctypes.data, lrt[s0:].ctypes.data), "bv_tile_wait_lists")
+
+        self._pipeline(self._dense_tiles(base, qual, strand, ref_base, n_samples), submit, wait)
         return out, lrt
 
     def call_sparse_lists(self, cells, site_start, ref_base, lists, n_samples, fmt=None, compact=False):
@@ -376,43 +335,32 @@ class BaseTypeEngine:
         expanded from the compact form; self.compact_tiles as in call_sparse_calls)."""
         S = ref_base.shape[0]
         assert cells.dtype in (np.uint32, np.uint16) and site_start.dtype == np.uint32 and site_start.shape[0] == S + 1
-        if fmt is None:
-            fmt = capi.CELLS_U16 if cells.dtype == np.uint16 else capi.CELLS_U32
         lists = np.ascontiguousarray(lists, np.uint8)
         assert lists.shape == (S, 4)
         out = np.zeros(S, dtype=SITE_OUT_DTYPE)
-        n_slots, step = self.params.n_slots, self.params.max_sites
-        assert n_slots >= 1 and step >= 1, "engine was created without slots"
         lrt = np.zeros(S, dtype=LRT_OUT_DTYPE)
+        step = self.params.max_sites
         packed, tmp = [], np.zeros(step, LRT_OUT_DTYPE)
-        pending, slot, keep = [], 0, {}
         self.compact_tiles = []
 
-        def wait(ps, p0, ns):
+        def submit(slot, tile):
+            self._check(self.lib.bv_tile_submit_sparse_lists(self._ctx, slot, C.byref(tile[0]), lists[tile[1]:].ctypes.data),
+                        "bv_tile_submit_sparse_lists")
+
+        def wait(slot, tile):
+            t, s0, _ = tile
             if not compact:
-                self._check(self.lib.bv_tile_wait_lists(self._ctx, ps, out[p0:].ctypes.data, lrt[p0:].ctypes.data), "bv_tile_wait_lists")
+                self._check(self.lib.bv_tile_wait_lists(self._ctx, slot, out[s0:].ctypes.data, lrt[s0:].ctypes.data), "bv_tile_wait_lists")
                 return
+            ns = int(t.n_sites)
             pb, pf, nf, n = C.c_void_p(), C.c_void_p(), C.c_uint32(0), C.c_uint32(0)
-            self._check(self.lib.bv_tile_wait_lists_compact(self._ctx, ps, C.byref(pb), C.byref(pf), C.byref(nf), tmp.ctypes.data, step,
+            self._check(self.lib.bv_tile_wait_lists_compact(self._ctx, slot, C.byref(pb), C.byref(pf), C.byref(nf), tmp.ctypes.data, step,
                                                             C.byref(n)), "bv_tile_wait_lists_compact")
-            self._collect_compact(pb, pf, nf, ref_base[p0:p0 + ns], out[p0:p0 + ns])
+            self._collect_compact(pb, pf, nf, ref_base[s0:s0 + ns], out[s0:s0 + ns])
             packed.append(tmp[:n.value].copy())
 
-        for s0 in range(0, max(S, 1), step):
-            ns = min(step, S - s0)
-            if len(pending) == n_slots:
-                wait(*pending.pop(0))
-            c0 = int(site_start[s0])
-            st = site_start[s0:s0 + ns + 1] - np.uint32(c0)
-            keep[slot] = st
-            off = min(c0, max(cells.shape[0] - 1, 0))
-            t = BvSparseTile(cells[off:].ctypes.data, None, st.ctypes.data, ref_base[s0:].ctypes.data, None, ns, n_samples, fmt,
-                             capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
-            self._check(self.lib.bv_tile_submit_sparse_lists(self._ctx, slot, C.byref(t), lists[s0:].ctypes.data), "bv_tile_submit_sparse_lists")
-            pending.append((slot, s0, ns))
-            slot = (slot + 1) % n_slots
-        for p in pending:
-            wait(*p)
+        tiles = self._sparse_tiles(cells, None, site_start, ref_base, n_samples, fmt, capi.OUT_COMPACT if compact else capi.OUT_RECORDS)
+        self._pipeline(tiles, submit, wait)
         if compact:
             lrt = np.concatenate(packed) if packed else np.zeros(0, LRT_OUT_DTYPE)
         return out, lrt
@@ -549,23 +497,16 @@ def sparse_encode16(cells, site_start, aux=None, pinned=False):
 def synth_fill_sparse_host(model, site0, n_sites, n_samples, with_aux=False, pinned=False):
     """Host twin of the generator in sparse form.  Returns (cells, cells_aux | None, site_start, ref_base)."""
     lib = capi.load_library()
-
-    def alloc(k, dt):
-        if pinned:
-            import torch
-            return torch.empty(max(k, 1), dtype={np.uint32: torch.int32, np.uint8: torch.uint8}[dt], pin_memory=True).numpy().view(dt)[:k]
-        return np.empty(k, dt)
-
-    site_start = alloc(n_sites + 1, np.uint32)
-    ref = alloc(n_sites, np.uint8)
+    site_start = _alloc(n_sites + 1, np.uint32, pinned)
+    ref = _alloc(n_sites, np.uint8, pinned)
     total = n_sites * n_samples
     # one pass with room for the expected number of cells + 6 sigma; a second, exact one if that was too small
     exp = total * (model.cov_thr / 2.0 ** 32)
     cap = int(min(total, exp + 6.0 * np.sqrt(exp + 1.0) + 64))
     n = C.c_uint64(0)
     for attempt in range(2):
-        cells = alloc(cap, np.uint32)
-        aux = alloc(cap, np.uint32) if with_aux else None
+        cells = _alloc(cap, np.uint32, pinned)
+        aux = _alloc(cap, np.uint32, pinned) if with_aux else None
         rc = lib.bv_synth_fill_sparse_host(C.byref(model), site0, n_sites, n_samples, cells.ctypes.data,
                                            aux.ctypes.data if with_aux else None, cap, site_start.ctypes.data, ref.ctypes.data, C.byref(n))
         if rc == capi.BV_OK:

@@ -245,7 +245,8 @@ void        bv_destroy(bv_ctx* ctx);
 const char* bv_last_error(const bv_ctx* ctx);                  /* ctx may be NULL: last global error */
 int         bv_set_params(bv_ctx* ctx, const bv_params* params); /* change min_af / em mode; capacities fixed */
 uint64_t    bv_launch_count(const bv_ctx* ctx);                /* kernels launched by this context so far */
-uint64_t    bv_h2d_bytes(const bv_ctx* ctx);                   /* bytes uploaded by bv_tile_submit so far (host tiles) */
+uint64_t    bv_h2d_bytes(const bv_ctx* ctx);                   /* bytes uploaded by the bv_tile_submit* calls so far: the planes
+                                                                  or cells of host tiles, and the lists of lists tiles */
 /* Instrumentation: with profiling on, every tile records CUDA events between its kernels (K1 count, K2 scalar,
  * K3 bound, K4 = K4a row histograms + K4b EM tasks and decisions, then the Fisher tests K2 and K4b listed);
  * bv_last_kernel_times() waits for the most recent tile and returns the durations of K1..K4 in ms,
