@@ -24,7 +24,8 @@
 #include "bv_expand_kernel.cuh"
 #include "bv_synth.cuh"
 
-constexpr uint32_t kScalarCtasPerSm = 8;      // grid cap of K2 and of bv_fisher_kernel, per SM
+constexpr uint32_t kScalarCtasPerSm = 2;      // grid cap of K2, per SM (98 registers: two CTAs resident)
+constexpr uint32_t kFisherCtasPerSm = 8;      // grid cap of bv_fisher_kernel, per SM
 constexpr uint32_t kEmPoolBinsPerSite = 64;   // EM bin pool per site of the tile (see scratch_reserve)
 
 // NVTX range over a scope (SURVEY.md section 5, "Tracing"): nsys / ncu timelines show the host side of every tile
@@ -345,6 +346,35 @@ static int set_call_args(bv_ctx* ctx, const bv_tile* t, const bv_tile_aux* aux, 
     return BV_OK;
 }
 
+// K2..KF of launch_site_kernel.  pdl: K3..KF with programmatic stream serialization (griddepcontrol, see bv_common.cuh):
+// the kernel is launched once every CTA of the kernel before it has triggered, which each does when it has no work left,
+// and its CTAs run their prologue (shared-memory tables from constant inputs) on the SMs that kernel has left, while its
+// last CTAs finish; their reads of its results wait in grid_dep_wait for its completion.  That takes the launch gap
+// (1-2 us) and the prologue off the critical path of every link of the chain.  No deadlock: the dependents are released
+// only when every CTA of the primary has triggered or exited, i.e. is resident or gone, so a waiting dependent CTA never
+// holds resources that a primary CTA still needs in order to start, even where the primary takes more than one wave.
+// Measured on a B200 (profiles/r06_bench_ab.json), two choices:
+//   * triggering on the kernels' first lines was slower (C2 step +0.019 ms): the dependents' CTAs then sat waiting on the
+//     SMs for the whole of the primary, and K4b's idle build for the whole of the working one;
+//   * K2 is launched plainly: chained behind K1 its CTAs land on the SMs in the order K1's CTAs finish, two per SM, and
+//     it ran 8 us longer than it does behind a drained K1.
+// Profiled tiles launch every kernel without the attribute, with the events between them: per-kernel times of a
+// serialised chain, comparable over the history of the project.
+static cudaError_t launch_chained(bool pdl, void (*kernel)(bv::SiteKernelArgs), uint32_t grid, uint32_t block, size_t smem,
+                                  cudaStream_t stream, const bv::SiteKernelArgs& a) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kernel, a);
+}
+
 // The basetype core of one tile: K1 (counts, every cell), K2 (scalar finish, one thread per site), K3 / K4 (sites whose
 // result depends on base qualities: likelihood-ratio bound, then EM + LRT).  Stream ordered; see csrc/bv_common.cuh.
 static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStream_t stream, bool counters_zeroed = false) {
@@ -373,29 +403,28 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
     }
     BV_CUDA(ctx, cudaGetLastError());
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[1], stream));
-    grid = (a.n_sites + 255) / 256;   // grid-stride over K1's work list
+    // K1 and K2 are launched plainly: K1 stays behind the counter memset and the previous tile's KF.  K3..KF are chained.
+    const bool pdl = !prof;
+    grid = (a.n_sites + bv::kScalarThreads - 1) / bv::kScalarThreads;   // CTAs split K1's work list into equal slices
     if (grid > (uint32_t)ctx->num_sms * kScalarCtasPerSm) grid = (uint32_t)ctx->num_sms * kScalarCtasPerSm;
-    bv::bv_scalar_kernel<<<grid, 256, 0, stream>>>(a);
-    BV_CUDA(ctx, cudaGetLastError());
+    BV_CUDA(ctx, launch_chained(false, bv::bv_scalar_kernel, grid, bv::kScalarThreads, 0, stream, a));
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[2], stream));
     // K3 and K4, persistent: each warp strides over groups of 32 sites
     grid = ((a.n_sites + 31) / 32 + bv::kBoundWarps - 1) / bv::kBoundWarps;
     if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;
-    bv::bv_bound_kernel<<<grid, bv::kBoundWarps * 32, bv::kBoundSmemBytes, stream>>>(a);
-    BV_CUDA(ctx, cudaGetLastError());
+    BV_CUDA(ctx, launch_chained(pdl, bv::bv_bound_kernel, grid, bv::kBoundWarps * 32, bv::kBoundSmemBytes, stream, a));
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[3], stream));
     // K4a: one warp per site of the EM list, whose length the host does not know: up to every site of the tile (deep pileups
     // with a small min_af: half of the sites of a 100,000-sample tile), so the grid covers that; warps without work leave at once
     if (a.n_samples > (uint32_t)bv::kLongRowSamples) {
         grid = (a.n_sites + bv::kLongWarps - 1) / bv::kLongWarps;
         if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;
-        bv::bv_hist_kernel<true><<<grid, bv::kLongWarps * 32, bv::kHistLongSmemBytes, stream>>>(a);
+        BV_CUDA(ctx, launch_chained(pdl, bv::bv_hist_kernel<true>, grid, bv::kLongWarps * 32, bv::kHistLongSmemBytes, stream, a));
     } else {
         grid = (a.n_sites + bv::kQualWarps - 1) / bv::kQualWarps;
         if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;
-        bv::bv_hist_kernel<false><<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a);
+        BV_CUDA(ctx, launch_chained(pdl, bv::bv_hist_kernel<false>, grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream, a));
     }
-    BV_CUDA(ctx, cudaGetLastError());
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[4], stream));
     // K4b: groups of lanes per EM task, CTAs stride over the task lists (their lengths are only known on the device, where the
     // kernel picks the group size from them): always the grid that fills the GPU, CTAs without work leave at once
@@ -405,23 +434,19 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
     if (a.abs_mode != BV_EM_ABS_INT_TRUNC) {
         // fabs in the convergence test: EMs of very different lengths; their iterations run with the lanes fed task by task
         // (bv_em_iter_kernel), the rest of every task -- log-likelihood sums, decisions -- from the frequencies that leaves
-        bv::bv_em_iter_kernel<<<grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(a);
-        BV_CUDA(ctx, cudaGetLastError());
+        BV_CUDA(ctx, launch_chained(pdl, bv::bv_em_iter_kernel, grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream, a));
         ctx->launches += 1;
         b.em_resume = 1;
     }
     // two builds of the kernel (registers / occupancy); the tile's task count decides on the device which of them works
-    bv::bv_em_task_kernel<bv::kTaskLoCtas><<<grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(b);
-    BV_CUDA(ctx, cudaGetLastError());
-    bv::bv_em_task_kernel<bv::kTaskHiCtas><<<grid_hi, bv::kTaskThreads, bv::kTaskSmemBytes, stream>>>(b);
+    BV_CUDA(ctx, launch_chained(pdl, bv::bv_em_task_kernel<bv::kTaskLoCtas>, grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream, b));
+    BV_CUDA(ctx, launch_chained(pdl, bv::bv_em_task_kernel<bv::kTaskHiCtas>, grid_hi, bv::kTaskThreads, bv::kTaskSmemBytes, stream, b));
     ctx->launches += 1;
-    BV_CUDA(ctx, cudaGetLastError());
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev[5], stream));
     // the Fisher tests K2 and K4 listed (as many as two per site; the counts are on the device): grid-stride
     grid = (4u * a.n_sites + bv::kFisherThreads - 1) / bv::kFisherThreads;   // (a pair of lanes per test)
-    if (grid > (uint32_t)ctx->num_sms * kScalarCtasPerSm) grid = (uint32_t)ctx->num_sms * kScalarCtasPerSm;
-    bv::bv_fisher_kernel<<<grid, bv::kFisherThreads, 0, stream>>>(a);
-    BV_CUDA(ctx, cudaGetLastError());
+    if (grid > (uint32_t)ctx->num_sms * kFisherCtasPerSm) grid = (uint32_t)ctx->num_sms * kFisherCtasPerSm;
+    BV_CUDA(ctx, launch_chained(pdl, bv::bv_fisher_kernel, grid, bv::kFisherThreads, 0, stream, a));
     if (prof) { BV_CUDA(ctx, cudaEventRecord(ctx->ev[6], stream)); ctx->ev_valid = true; }
     ctx->launches += 6;
     if (a.list_called) {

@@ -177,6 +177,15 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                  : "memory");
 }
 
+// ---- programmatic dependent launch (griddepcontrol, sm_90+) along K2 -> K3 -> ... -> KF (launch_site_kernel, bv_api.cu) ------
+// K3..KF are launched with programmatic stream serialization: a kernel's CTAs may start while the kernel before it still
+// runs, once every CTA of that kernel has called grid_dep_launch (or exited).  Everything a kernel reads that an earlier
+// kernel of the tile wrote (counters, work lists, records, the EM tables) comes after grid_dep_wait, which returns once
+// the kernel before has completed and its writes are visible; every CTA calls it, also those with no work, so that a
+// kernel never completes before the one it follows.  Both are no-ops for a kernel launched without the attribute.
+__device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void grid_dep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 // valid = number of real cells in this 16-cell vector (>= 16 for all but the row's last vector): padding cells
 // are turned into 'N'
 __device__ __forceinline__ void mask_tail(uint4& vb, int valid) {

@@ -203,6 +203,7 @@ __global__ void __launch_bounds__((LONG ? kLongWarps : kQualWarps) * 32, 1) bv_h
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
+    grid_dep_wait();
     // The EM list is final (K3 is done).  A site costs one pass over its row, the same for every site of a tile, so the sites
     // are dealt out statically -- entry i to warp i mod (all warps), neighbours in the list to different SMs -- and the next
     // entry is read while this one is worked on.  (A shared fetch counter cost every site a round trip to one L2 address that
@@ -216,6 +217,7 @@ __global__ void __launch_bounds__((LONG ? kLongWarps : kQualWarps) * 32, 1) bv_h
         if (i + total_warps < n_em) site_next = a.list_em[i + total_warps];
         hist_site<LONG>(site);
     }
+    grid_dep_launch();
     if (W.vcf_n) vcf_flush();
 }
 
@@ -681,12 +683,14 @@ __global__ void __launch_bounds__(kTaskThreads) bv_em_iter_kernel(const __grid_c
     for (int i = threadIdx.x; i < 4 * kQSlots; i += kTaskThreads) cs.lut[i / kQSlots][i % kQSlots] = a.lut[(i / kQSlots) * kQStride + i % kQSlots];
     for (int i = threadIdx.x; i < kLogTabEntries; i += kTaskThreads) cs.ltab[i] = a.logtab[i];
     __syncthreads();
+    grid_dep_wait();
     const double* lut = &cs.lut[0][0];
     const uint32_t n2 = min(a.counters[kCntEmTask2], a.em_task_cap[0]), n3 = min(a.counters[kCntEmTask3], a.em_task_cap[1]),
                    n4 = min(a.counters[kCntEmTask4], a.em_task_cap[2]);
     em_iter_list<2>(a, cs, lut, 0u, n2, a.counters + kCntEmFetch2);
     em_iter_list<3>(a, cs, lut, a.em_task_cap[0], n3, a.counters + kCntEmFetch3);
     em_iter_list<4>(a, cs, lut, a.em_task_cap[0] + a.em_task_cap[1], n4, a.counters + kCntEmFetch4);
+    grid_dep_launch();
 }
 
 // ---- the site's decision, after its last task has finished ----------------------------------------------------------------------
@@ -830,16 +834,17 @@ __device__ __noinline__ void decide_site(const SiteKernelArgs& a, const EmSiteHd
 // (register counts from ptxas -v; timings on a B200 in profiles/r02_em_task_occupancy.txt).
 template <int kMinCtas>
 __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(const __grid_constant__ SiteKernelArgs a) {
-    {
-        const uint64_t n_all = (uint64_t)min(a.counters[kCntEmTask2], a.em_task_cap[0]) + min(a.counters[kCntEmTask3], a.em_task_cap[1]) +
-                               min(a.counters[kCntEmTask4], a.em_task_cap[2]);
-        if ((n_all > (uint64_t)a.em_task_split) != (kMinCtas == kTaskHiCtas)) return;
-    }
     TaskCta& cs = *reinterpret_cast<TaskCta*>(bv_smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
     for (int i = tid; i < 4 * kQSlots; i += kTaskThreads) cs.lut[i / kQSlots][i % kQSlots] = a.lut[(i / kQSlots) * kQStride + i % kQSlots];
     for (int i = tid; i < kLogTabEntries; i += kTaskThreads) cs.ltab[i] = a.logtab[i];
     if (tid == 0) cs.n_fs = 0;
+    grid_dep_wait();
+    {
+        const uint64_t n_all = (uint64_t)min(a.counters[kCntEmTask2], a.em_task_cap[0]) + min(a.counters[kCntEmTask3], a.em_task_cap[1]) +
+                               min(a.counters[kCntEmTask4], a.em_task_cap[2]);
+        if ((n_all > (uint64_t)a.em_task_split) != (kMinCtas == kTaskHiCtas)) return;
+    }
     const double* lut = &cs.lut[0][0];
     // the three task lists, one after the other
     uint32_t n_list[3], blk_end[3], base[3];
@@ -920,6 +925,7 @@ __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(cons
         }
     }
     __syncthreads();
+    grid_dep_launch();
     for (uint32_t k0 = 0; k0 < cs.n_fs; k0 += (uint32_t)kTaskThreads) {   // the tests still listed here
         const bool have = k0 + (uint32_t)tid < cs.n_fs;
         const uint32_t e = have ? cs.fs_site[k0 + (uint32_t)tid] : 0u;

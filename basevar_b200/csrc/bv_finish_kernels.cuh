@@ -18,7 +18,8 @@ namespace bv {
 // can decide (REF with >= 22 reads plus one minor allele with <= 4; the minor allele's code travels in the alt word),
 // else state kStateEM.
 // =====================================================================================================================
-// append `site` to a work list for the lanes with `pred`; one atomicAdd per warp (all 32 lanes must call)
+// append `site` to a work list (global, or a CTA's staging list in shared memory) for the lanes with `pred`; one atomicAdd
+// per warp (all 32 lanes must call)
 __device__ __forceinline__ void list_append(uint32_t* list, uint32_t* counter, bool pred, uint32_t site) {
     const int lane = threadIdx.x & 31;
     const uint32_t m = __ballot_sync(kFull, pred);
@@ -111,6 +112,7 @@ __device__ __forceinline__ void fisher_job(const SiteKernelArgs& a, bool have, u
 
 constexpr int kFisherThreads = 256;
 __global__ void __launch_bounds__(kFisherThreads) bv_fisher_kernel(const __grid_constant__ SiteKernelArgs a) {
+    grid_dep_wait();
     const uint32_t n_wide = a.counters[kCntFisherWide], n_narrow = a.counters[kCntFisherNarrow];
     const uint32_t threads = gridDim.x * blockDim.x;
     const bool pair = 2u * (n_wide + n_narrow + 32u) <= threads;      // a pair of lanes per test while that still is one trip
@@ -127,33 +129,86 @@ __global__ void __launch_bounds__(kFisherThreads) bv_fisher_kernel(const __grid_
     }
 }
 
-__device__ __forceinline__ uint32_t scalar_site(const SiteKernelArgs& a, uint32_t site, bool& fs_job, bool& fs_wide);
+// K2 works in passes of kScalarSites sites per thread: the list entries of a pass, then the records and REF bases of all
+// of its sites are loaded before the first site is finished, so that a thread has kScalarSites scattered 64-byte reads in
+// flight instead of one.  Its appends to the four work lists (bound, EM, narrow and wide Fisher tests) are gathered in
+// shared memory and go out with one global atomicAdd per list and CTA: per warp they were four returning atomics in a row
+// on four counters that every warp of the tile hit.
+constexpr int kScalarThreads = 256;
+constexpr int kScalarSites = 4;
+constexpr uint32_t kScalarPass = (uint32_t)kScalarThreads * kScalarSites;   // sites per CTA and pass
 
-__global__ void __launch_bounds__(256) bv_scalar_kernel(const __grid_constant__ SiteKernelArgs a) {
+__device__ __forceinline__ uint32_t scalar_site(const SiteKernelArgs& a, uint32_t site, const uint4 (&w)[4], uint32_t ref_char,
+                                                bool& fs_job, bool& fs_wide);
+
+__global__ void __launch_bounds__(kScalarThreads) bv_scalar_kernel(const __grid_constant__ SiteKernelArgs a) {
+    __shared__ uint32_t s_list[4][kScalarPass];   // staged appends: bound, EM, narrow Fisher, wide Fisher
+    __shared__ uint32_t s_cnt[4], s_n[4], s_base[4];
+    const int tid = threadIdx.x;
+    if (tid < 4) s_cnt[tid] = 0;
+    // every CTA takes an equal slice of the list (all SMs get work however few sites are listed), in passes
     const uint32_t n_slow = a.counters[kCntSlow];
-    const uint32_t stride = gridDim.x * blockDim.x;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; (i & ~31u) < n_slow; i += stride) {   // warp-uniform trips
-        const bool valid = i < n_slow;
-        const uint32_t site = valid ? a.list_slow[i] : 0u;
-        bool fs_job = false, fs_wide = false;
-        const uint32_t state = valid ? scalar_site(a, site, fs_job, fs_wide) : kStateDone;
-        list_append(a.list_bound, a.counters + kCntBound, state == kStateBound, site);
-        list_append(a.list_em, a.counters + kCntEm, state == kStateEM, site);
-        fisher_push(a, fs_job, fs_wide, site);
+    const uint32_t slice = ((n_slow + gridDim.x - 1u) / gridDim.x + 31u) & ~31u;
+    const uint32_t end = min(n_slow, (blockIdx.x + 1u) * slice);
+#pragma unroll 1
+    for (uint32_t p0 = blockIdx.x * slice; p0 < end; p0 += kScalarPass) {   // CTA-uniform trips
+        uint32_t site[kScalarSites], ref_char[kScalarSites];
+        uint4 w[kScalarSites][4];
+#pragma unroll
+        for (int k = 0; k < kScalarSites; ++k) {
+            const uint32_t i = p0 + (uint32_t)(k * kScalarThreads + tid);
+            site[k] = i < end ? a.list_slow[i] : 0xffffffffu;
+        }
+#pragma unroll
+        for (int k = 0; k < kScalarSites; ++k) {
+            if (site[k] != 0xffffffffu) {
+                const uint4* rec = reinterpret_cast<const uint4*>(a.out + site[k]);
+                w[k][0] = rec[0]; w[k][1] = rec[1]; w[k][2] = rec[2]; w[k][3] = rec[3];
+                ref_char[k] = a.ref_base[site[k]];
+            }
+        }
+        __syncthreads();   // s_cnt is zero and the previous pass's staging lists are written out
+#pragma unroll
+        for (int k = 0; k < kScalarSites; ++k) {
+            const bool valid = site[k] != 0xffffffffu;
+            bool fs_job = false, fs_wide = false;
+            const uint32_t state = valid ? scalar_site(a, site[k], w[k], ref_char[k], fs_job, fs_wide) : kStateDone;
+            list_append(s_list[0], &s_cnt[0], state == kStateBound, site[k]);
+            list_append(s_list[1], &s_cnt[1], state == kStateEM, site[k]);
+            list_append(s_list[2], &s_cnt[2], fs_job && !fs_wide, site[k]);
+            list_append(s_list[3], &s_cnt[3], fs_job && fs_wide, site[k]);
+        }
+        __syncthreads();
+        if (tid < 4) {
+            const int cnt = tid == 0 ? kCntBound : tid == 1 ? kCntEm : tid == 2 ? kCntFisherNarrow : kCntFisherWide;
+            const uint32_t n = s_cnt[tid];
+            s_n[tid] = n;
+            s_base[tid] = n ? atomicAdd(a.counters + cnt, n) : 0u;
+            s_cnt[tid] = 0;
+        }
+        __syncthreads();
+        for (uint32_t j = tid; j < s_n[0]; j += kScalarThreads) a.list_bound[s_base[0] + j] = s_list[0][j];
+        for (uint32_t j = tid; j < s_n[1]; j += kScalarThreads) a.list_em[s_base[1] + j] = s_list[1][j];
+        // narrow tests from the front of list_fisher, wide ones from the back (bv_fisher_kernel)
+        for (uint32_t j = tid; j < s_n[2]; j += kScalarThreads) a.list_fisher[s_base[2] + j] = s_list[2][j];
+        for (uint32_t j = tid; j < s_n[3]; j += kScalarThreads) a.list_fisher[2u * a.n_sites - 1u - (s_base[3] + j)] = s_list[3][j];
     }
+    grid_dep_launch();
 }
 
 // returns the site's new state
-__device__ __forceinline__ uint32_t scalar_site(const SiteKernelArgs& a, uint32_t site, bool& fs_job, bool& fs_wide) {
+// w: the first 64 bytes of the site's record, ref_char: its REF base
+__device__ __forceinline__ uint32_t scalar_site(const SiteKernelArgs& a, uint32_t site, const uint4 (&w)[4], uint32_t ref_char,
+                                                bool& fs_job, bool& fs_wide) {
     uint32_t* rec = reinterpret_cast<uint32_t*>(a.out + site);
-    const uint4 w0 = reinterpret_cast<const uint4*>(rec)[0];   // depth[4]
-    const uint4 w1 = reinterpret_cast<const uint4*>(rec)[1];   // other, state, fwd[0..1]
-    const uint4 w2 = reinterpret_cast<const uint4*>(rec)[2];   // fwd[2..3], rev[0..1]
-    const uint4 w3 = reinterpret_cast<const uint4*>(rec)[3];   // rev[2..3], alt word, info word
+    const uint4 w0 = w[0];   // depth[4]
+    const uint4 w1 = w[1];   // other, state, fwd[0..1]
+    const uint4 w2 = w[2];   // fwd[2..3], rev[0..1]
+    const uint4 w3 = w[3];   // rev[2..3], alt word, info word
     const uint32_t d0 = w0.x, d1 = w0.y, d2 = w0.z, d3 = w0.w, other = w1.x;
     const uint32_t f0 = w1.z, f1 = w1.w, f2 = w2.x, f3 = w2.y, r0 = w2.z, r1 = w2.w, r2 = w3.x, r3 = w3.y;
     const uint32_t flags = (w3.w >> 16) & 0xffu;
-    const int ref_code = ref_code_of(a.ref_base[site]);
+    const int ref_code = ref_code_of(ref_char);
     const uint32_t total = d0 + d1 + d2 + d3 + other;
     const double dtot = (double)total;
 
@@ -295,6 +350,7 @@ __global__ void __launch_bounds__(kBoundWarps * 32, 1) bv_bound_kernel(const __g
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
+    grid_dep_wait();   // (the prologue above reads constant inputs only)
 
     const uint32_t N = a.n_samples;
     const uint32_t row_bytes = (N + 15u) & ~15u;
@@ -403,6 +459,7 @@ __global__ void __launch_bounds__(kBoundWarps * 32, 1) bv_bound_kernel(const __g
             }
         }
     }
+    grid_dep_launch();
 }
 
 // =====================================================================================================================
