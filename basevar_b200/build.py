@@ -51,6 +51,15 @@ CPP_TESTS = {"test_host_cpu": [], "test_host_gpu": ["-ldl"], "test_fisher_fast":
              "test_ranksum_gpu": ["-ldl", "-lm"], "test_vcf_row_gpu": ["-ldl", "-lm"]}
 
 
+# What the programs linked against the host layer compile in: they are linked again when their source or one of these changes.
+# A library rebuilt behind an unchanged interface is picked up at load time (both libraries are shared), without a relink.
+PROGRAM_HEADERS = [h for h in HOST_DEPS if h.endswith((".hpp", ".h"))] + [os.path.join(CSRC, "bv_fisher_fast.h")]
+
+
+def _stale(target, sources):
+    return not os.path.exists(target) or any(os.path.getmtime(d) > os.path.getmtime(target) for d in sources)
+
+
 def build_host(force=False):
     """The C++ host layer (g++) over the C ABI, and its test programs under tests/cpp/bin/."""
     build(force=False)
@@ -63,12 +72,12 @@ def build_host(force=False):
     for name, extra in CPP_TESTS.items():
         src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
         exe = os.path.join(bindir, name)
-        if force or not os.path.exists(exe) or os.path.getmtime(exe) < max(os.path.getmtime(src), os.path.getmtime(HOST_LIB)):
+        if force or _stale(exe, [src] + PROGRAM_HEADERS):
             subprocess.check_call([cxx, "-std=c++17", "-O2", "-Wall", "-o", exe, src, "-L" + HERE, "-lbasevar_b200_host",
                                    "-lbasevar_b200", "-Wl,-rpath," + HERE, "-lpthread"] + extra)
     main_src = os.path.join(HERE, "host", "bv_main.cpp")
     os.makedirs(os.path.dirname(CLI), exist_ok=True)
-    if force or not os.path.exists(CLI) or os.path.getmtime(CLI) < max(os.path.getmtime(main_src), os.path.getmtime(HOST_LIB)):
+    if force or _stale(CLI, [main_src] + PROGRAM_HEADERS):
         subprocess.check_call([cxx, "-std=c++17", "-O2", "-Wall", "-o", CLI, main_src, "-L" + HERE, "-lbasevar_b200_host",
                                "-lbasevar_b200", "-Wl,-rpath," + HERE, "-Wl,-rpath,$ORIGIN/..", "-lpthread", "-lz"])
     return HOST_LIB

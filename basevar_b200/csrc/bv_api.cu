@@ -26,7 +26,8 @@
 
 constexpr uint32_t kScalarCtasPerSm = 2;      // grid cap of K2, per SM (98 registers: two CTAs resident)
 constexpr uint32_t kFisherCtasPerSm = 8;      // grid cap of bv_fisher_kernel, per SM
-constexpr uint32_t kEmPoolBinsPerSite = 64;   // EM bin pool per site of the tile (see scratch_reserve)
+constexpr uint32_t kMaxTileSites = 1u << 22;  // sites of one tile at most (EM header indices have 28 bits)
+static_assert((uint64_t)bv::kMaxBins * kMaxTileSites < (1ull << 31), "EM bin pool offsets of a tile fit 31 bits");
 
 // NVTX range over a scope (SURVEY.md section 5, "Tracing"): nsys / ncu timelines show the host side of every tile
 // (submit, wait) and the launch sequence K0, K1, K2, K3, K4a, K4b, K5, K6 under these names.
@@ -119,7 +120,7 @@ struct bv_scratch {
     uint32_t* d_em_tasks = nullptr;
     double* d_em_res = nullptr;
     double* d_em_single = nullptr;    // [cap][4] log-likelihoods of the single-allele models of the EM sites (K4a -> K4b)
-    uint32_t em_pool_cap = 0, em_task_cap[3] = {0, 0, 0};
+    uint32_t em_task_cap[3] = {0, 0, 0};
     uint32_t cap = 0;
 };
 
@@ -259,21 +260,21 @@ static int scratch_reserve(bv_ctx* ctx, bv_scratch& sc, uint32_t n_sites) {
         sc.d_lists = nullptr;
         sc.cap = 0;
         BV_CUDA(ctx, cudaMalloc(&sc.d_lists, 6 * (size_t)n_sites * sizeof(uint32_t)));
-        // EM scratch: room for every site to be an EM site; 64 bins and 3 tasks per site of the tile on average (a deep,
-        // multi-allelic pileup needs 25 and 1; what does not fit is finished inside K4a, see bv_em_kernels.cuh)
+        // EM scratch: room for every site of a tile to be an EM site with kMaxBins bins and all 11 tasks (6, 4 and 1 over subsets
+        // of 2, 3 and 4 alleles), so that K4a's allocations cannot fail and every EM site is decided by K4b (bv_em_kernels.cuh):
+        // 2,940 bytes per site and slot -- pool 1,920, task results 880, header 64, single-allele log-likelihoods 32, task
+        // list 44.  No tile has more than kMaxTileSites sites.
         cudaFree(sc.d_em_hdr); cudaFree(sc.d_em_pool); cudaFree(sc.d_em_tasks); cudaFree(sc.d_em_res); cudaFree(sc.d_em_single);
         sc.d_em_hdr = nullptr; sc.d_em_pool = nullptr; sc.d_em_tasks = nullptr; sc.d_em_res = nullptr; sc.d_em_single = nullptr;
         cudaGetLastError();
-        const uint64_t pool = (uint64_t)n_sites * kEmPoolBinsPerSite + 4096;
-        sc.em_pool_cap = (uint32_t)(pool < 0x7ffffff0ull ? pool : 0x7ffffff0ull);
-        // task slots for subsets of 2, 3 and 4 alleles: 2, 1 and 1/2 per site of the tile (header indices have 28 bits)
-        sc.em_task_cap[0] = 2u * n_sites + 1024u; sc.em_task_cap[1] = n_sites + 512u; sc.em_task_cap[2] = n_sites / 2u + 256u;
-        const size_t n_task = (size_t)sc.em_task_cap[0] + sc.em_task_cap[1] + sc.em_task_cap[2];
-        BV_CUDA(ctx, cudaMalloc(&sc.d_em_hdr, (size_t)n_sites * sizeof(bv::EmSiteHdr)));
-        BV_CUDA(ctx, cudaMalloc(&sc.d_em_pool, (size_t)sc.em_pool_cap * sizeof(uint32_t)));
+        const uint32_t em_sites = n_sites < kMaxTileSites ? n_sites : kMaxTileSites;
+        sc.em_task_cap[0] = 6u * em_sites; sc.em_task_cap[1] = 4u * em_sites; sc.em_task_cap[2] = em_sites;
+        const size_t n_task = (size_t)11 * em_sites;
+        BV_CUDA(ctx, cudaMalloc(&sc.d_em_hdr, (size_t)em_sites * sizeof(bv::EmSiteHdr)));
+        BV_CUDA(ctx, cudaMalloc(&sc.d_em_pool, (size_t)em_sites * bv::kMaxBins * sizeof(uint32_t)));
         BV_CUDA(ctx, cudaMalloc(&sc.d_em_tasks, n_task * sizeof(uint32_t)));
         BV_CUDA(ctx, cudaMalloc(&sc.d_em_res, n_task * bv::kEmResDoubles * sizeof(double)));
-        BV_CUDA(ctx, cudaMalloc(&sc.d_em_single, (size_t)n_sites * 4 * sizeof(double)));
+        BV_CUDA(ctx, cudaMalloc(&sc.d_em_single, (size_t)em_sites * 4 * sizeof(double)));
         sc.cap = n_sites;
     }
     return BV_OK;
@@ -287,7 +288,7 @@ static int fill_kernel_args(bv_ctx* ctx, const bv_tile* t, bv_site_out* d_out, b
                        (unsigned long long)t->pitch, t->n_samples);
     if (t->n_samples > ctx->prm.max_samples)
         return set_err(ctx, BV_ERR_ARG, "bv_tile: n_samples %u > max_samples %u", t->n_samples, ctx->prm.max_samples);
-    if (t->n_sites > (1u << 22)) return set_err(ctx, BV_ERR_ARG, "bv_tile: more than 2^22 sites in one tile");
+    if (t->n_sites > kMaxTileSites) return set_err(ctx, BV_ERR_ARG, "bv_tile: more than 2^22 sites in one tile");
     if ((((uintptr_t)t->base) | ((uintptr_t)t->qual) | ((uintptr_t)t->strand)) & 15)
         return set_err(ctx, BV_ERR_ARG, "bv_tile: plane pointers must be 16-byte aligned");
     a->base = t->base; a->qual = t->qual; a->strand = t->strand; a->ref_base = t->ref_base;
@@ -307,7 +308,6 @@ static int fill_kernel_args(bv_ctx* ctx, const bv_tile* t, bv_site_out* d_out, b
     a->list_fisher = sc.d_lists + 4 * (size_t)sc.cap;   // [2 * n_sites] of its 2 * cap words
     a->counters = sc.d_counters;
     a->em_hdr = sc.d_em_hdr; a->em_pool = sc.d_em_pool; a->em_tasks = sc.d_em_tasks; a->em_res = sc.d_em_res; a->em_single = sc.d_em_single;
-    a->em_pool_cap = sc.em_pool_cap;
     for (int k = 0; k < 3; ++k) a->em_task_cap[k] = sc.em_task_cap[k];
     a->brief = nullptr; a->full_out = nullptr;   // set by the submit paths of compact tiles
     a->em_resume = 0;

@@ -54,13 +54,12 @@ constexpr uint32_t kStateScalar = 1;         // counts are final, K2 has to fini
 constexpr uint32_t kStateBound = 2;          // result depends on base qualities; K3 tries the likelihood-ratio bound
 constexpr uint32_t kStateEM = 3;             // result depends on base qualities; K4 runs EM + LRT
 
-constexpr int kCntSlow = 0, kCntBound = 1, kCntEm = 2;                    // SiteKernelArgs::counters (3 is unused)
+constexpr int kCntSlow = 0, kCntBound = 1, kCntEm = 2;                    // SiteKernelArgs::counters (3 and 10 are unused)
 constexpr int kCntCalled = 4, kCntGroupNext = 5;                          // called sites (K4 -> K5, K6)
 constexpr int kCntBadCell = 6;                                            // malformed sparse input (K0, bv_expand_kernel.cuh)
 constexpr int kCntEmHdr = 7, kCntEmPool = 8;                              // K4a -> K4b: EM sites and the pool of their bins
 constexpr int kCntEmTask2 = 9, kCntEmTask3 = 11, kCntEmTask4 = 12;        // EM tasks by number of alleles in the candidate subset
 constexpr int kCntFull = 13;                                              // full records of a compact tile (bv_pack_kernel)
-constexpr int kCntEmFallback = 10;                                        // EM sites finished inside K4a (scratch pools full)
 constexpr int kCntFisherNarrow = 14, kCntFisherWide = 15;                   // queued Fisher tests (K2, K4b -> bv_fisher_kernel)
 constexpr int kCntEmFetch2 = 16, kCntEmFetch3 = 17, kCntEmFetch4 = 18;      // next task of each list (bv_em_iter_kernel)
 constexpr int kNumCounters = 24;
@@ -107,12 +106,11 @@ struct SiteKernelArgs {
     uint32_t* counters;      // [kNumCounters], zeroed before K1
     // K4a -> K4b (bv_em_kernels.cuh)
     EmSiteHdr* em_hdr;       // [n_sites]
-    uint32_t* em_pool;       // [em_pool_cap] compact bins of the EM sites, allocated with kCntEmPool
+    uint32_t* em_pool;       // [n_sites][kMaxBins] compact bins of the EM sites, allocated with kCntEmPool
     uint32_t* em_tasks;      // hdr index | subset << 28; three lists one after the other: 2-, 3- and 4-allele subsets,
-                             // em_task_cap[k] slots each, allocated with kCntEmTask2 / 3 / 4
+                             // em_task_cap[k] slots each (6 / 4 / 1 per site), allocated with kCntEmTask2 / 3 / 4
     double* em_res;          // [sum of em_task_cap][kEmResDoubles], indexed like em_tasks
     double* em_single;       // [n_sites][4], indexed like em_hdr: log-likelihood of the single-allele model of each ACTIVE base
-    uint32_t em_pool_cap;
     uint32_t em_task_cap[3];
     // compact record transport (BV_OUT_COMPACT): null unless the tile asked for it
     uint32_t em_resume;      // bv_em_task_kernel: the EM iterations were run by bv_em_iter_kernel, start from its frequencies

@@ -24,8 +24,11 @@
 //
 // At most 3 of the 11 tasks of a 4-allele site are never consulted (the elimination needs <= 8 EMs); evaluating them
 // anyway removes every dependency between EMs.  A flag an unconsulted task raises (BV_FLAG_EM_MAXITER) is not reported.
-// Scratch (headers, bin pool, task lists) is sized per tile; a site that does not fit any more is finished inside K4a by
-// the warp-per-site code K6 also uses (lrt_on_bins), so that the records never depend on the pool size.
+// Scratch (headers, bin pool, task lists, results) has room for every site of the largest tile to be an EM site with kMaxBins
+// bins and all 11 tasks (scratch_reserve, bv_api.cu), so every EM site of every tile takes this one path: its records do not
+// depend on the context's max_sites nor on the order in which K4a's warps allocate.  (A fallback that finished the sites that
+// did not fit inside K4a with lrt_on_bins associated its sums differently: AF / QUAL / chi2 then differed in the last bits
+// between a small and a large context, and from run to run.)
 #pragma once
 #include "bv_finish_kernels.cuh"
 
@@ -43,8 +46,7 @@ __device__ __noinline__ void hist_site(uint32_t site) {
     const uint32_t d0 = W.rec.depth[0], d1 = W.rec.depth[1], d2 = W.rec.depth[2], d3 = W.rec.depth[3];
     const uint32_t total = d0 + d1 + d2 + d3 + W.rec.depth_other;
     // ---- lrt (src/basetype.cpp:130-199): the active set (total > 0 here) was worked out by K2 ----
-    uint32_t act = (reinterpret_cast<const uint32_t*>(&W.rec)[kWAlt] >> 8) & 0xfu;
-    int n_act = __popc(act);
+    const uint32_t act = (reinterpret_cast<const uint32_t*>(&W.rec)[kWAlt] >> 8) & 0xfu;
     if (lane == 0) W.flag_word = W.rec.flags;
     __syncwarp();
 
@@ -53,9 +55,7 @@ __device__ __noinline__ void hist_site(uint32_t site) {
     const uint32_t qmin = h & 0xffu, qmax = (h >> 8) & 0xffu;
     if (lane == 0) W.flag_word |= h >> 16;
     __syncwarp();
-    double chi = 0.0;
-    uint32_t em_calls = 0;
-    if (n_act >= 2) {
+    if (__popc(act) >= 2) {
         const int nb = compact_bins(qmin, qmax);
         // ---- hand the site to K4b: bins into the pool, one task per subset of >= 2 active alleles ----
         // lane m < 16 looks after subset m; tasks are listed by subset size (2, 3, 4 alleles), in ascending subset order
@@ -65,68 +65,60 @@ __device__ __noinline__ void hist_site(uint32_t site) {
         const uint32_t bal2 = __ballot_sync(kFull, is_task && k == 2), bal3 = __ballot_sync(kFull, is_task && k == 3),
                        bal4 = __ballot_sync(kFull, is_task && k == 4);
         const uint32_t n_k[3] = {(uint32_t)__popc(bal2), (uint32_t)__popc(bal3), (uint32_t)__popc(bal4)};
-        // five allocations at once: pool (lane 0), header (lane 1), task slots of each size (lanes 2-4)
-        uint32_t got = 0, want = 0, cap = 0;
-        if (lane == 0) { want = (uint32_t)nb; cap = cs.a.em_pool_cap; }
-        if (lane == 1) { want = 1u; cap = cs.a.n_sites; }
-        if (lane >= 2 && lane < 5) { want = n_k[lane - 2]; cap = cs.a.em_task_cap[lane - 2]; }
+        // five allocations at once: pool (lane 0), header (lane 1), task slots of each size (lanes 2-4).  They cannot fail: the
+        // scratch has kMaxBins pool entries, one header and 6 / 4 / 1 task slots per site of the tile (scratch_reserve).
+        uint32_t got = 0, want = 0;
+        if (lane == 0) want = (uint32_t)nb;
+        if (lane == 1) want = 1u;
+        if (lane >= 2 && lane < 5) want = n_k[lane - 2];
         constexpr int kCnt[5] = {kCntEmPool, kCntEmHdr, kCntEmTask2, kCntEmTask3, kCntEmTask4};
         if (lane < 5 && want) got = atomicAdd(cs.a.counters + kCnt[lane], want);
-        const bool fits = got <= cap && want <= cap - got;
-        const bool ok = __all_sync(kFull, fits);
         const uint32_t off = __shfl_sync(kFull, got, 0), hdr = __shfl_sync(kFull, got, 1);
         const uint32_t t2 = __shfl_sync(kFull, got, 2), t3 = __shfl_sync(kFull, got, 3), t4 = __shfl_sync(kFull, got, 4);
         const uint32_t base3 = cs.a.em_task_cap[0], base4 = base3 + cs.a.em_task_cap[1];
-        // slot of this lane's task (task slots that were allocated but stay unused are marked invalid)
-        const uint32_t my_t = k == 2 ? t2 + (uint32_t)__popc(bal2 & ((1u << lane) - 1u))
-                            : k == 3 ? base3 + t3 + (uint32_t)__popc(bal3 & ((1u << lane) - 1u)) : base4 + t4;
-        const uint32_t my_cap = k == 2 ? base3 : k == 3 ? base4 : base4 + cs.a.em_task_cap[2];
-        if (is_task && my_t < my_cap) cs.a.em_tasks[my_t] = ok ? (hdr | (m << 28)) : kEmTaskInvalid;
-        if (ok) {
-            const uint32_t* bins = nb <= kSmemBins ? W.bins : cs.a.bin_spill + (size_t)(blockIdx.x * kQualWarps + (threadIdx.x >> 5)) * kMaxBins;
-            for (int i = lane; i < nb; i += 32) cs.a.em_pool[off + i] = bins[i];
-            // first bin of each base (bins are sorted by base): lane b counts the bins of bases < b + 1
-            uint32_t below = 0;
-            for (int i = lane; i < nb; i += 32) {
-                const uint32_t b = bin_base(bins[i]);
-                below += (b < 1u) | ((uint32_t)(b < 2u) << 8) | ((uint32_t)(b < 3u) << 16) | ((uint32_t)(b < 4u) << 24);
-            }
-            // (a lane sees at most kMaxBins / 32 = 15 bins, so the four byte counters cannot overflow before the reduction)
-            const uint32_t s0 = __reduce_add_sync(kFull, below & 0xffu), s1 = __reduce_add_sync(kFull, (below >> 8) & 0xffu),
-                           s2 = __reduce_add_sync(kFull, (below >> 16) & 0xffu), s3 = __reduce_add_sync(kFull, below >> 24);
-            // log-likelihoods of the four single-allele models (closed form, see single_allele_ll): the last elimination round of
-            // the site's decision consults two of them
-            {
-                double sl[4];
-                single_allele_ll4(bins, nb, sl);
-                if (lane < 4) cs.a.em_single[(size_t)hdr * 4 + lane] = lane == 0 ? sl[0] : lane == 1 ? sl[1] : lane == 2 ? sl[2] : sl[3];
-            }
-            if (lane == 0) {
-                uint4 w0, w1, w2, w3;
-                w0.x = site; w0.y = off; w0.z = (uint32_t)nb; w0.w = act | (W.flag_word << 8);
-                w1.x = t2; w1.y = base3 + t3; w1.z = base4 + t4; w1.w = n_k[0] + n_k[1] + n_k[2];
-                w2.x = d0; w2.y = d1; w2.z = d2; w2.w = d3;
-                w3.x = total; w3.y = s0 | (s1 << 16); w3.z = s2 | (s3 << 16); w3.w = 0;
-                uint4* H = reinterpret_cast<uint4*>(cs.a.em_hdr + hdr);
-                H[0] = w0; H[1] = w1; H[2] = w2; H[3] = w3;
-            }
-            __syncwarp();
-            return;   // the record is completed by K4b
+        if (is_task) {
+            const uint32_t my_t = k == 2 ? t2 + (uint32_t)__popc(bal2 & ((1u << lane) - 1u))
+                                : k == 3 ? base3 + t3 + (uint32_t)__popc(bal3 & ((1u << lane) - 1u)) : base4 + t4;
+            cs.a.em_tasks[my_t] = hdr | (m << 28);
         }
-        // scratch pools full: finish the site here
-        if (lane == 0) atomicAdd(cs.a.counters + kCntEmFallback, 1u);
-        const uint32_t r = lrt_on_bins(nb, act, kOrderACGT);
-        act = r & 0xfu; n_act = (int)((r >> 4) & 0xfu); em_calls = r >> 8;
-        chi = W.res_chi;
-    } else {
-        // One active allele: the reference still runs one EM; its answer is closed form (see single_allele_ll):
-        // AF == 1.0 exactly, or NaN when a phred-0 read of that base exists.
+        const uint32_t* bins = nb <= kSmemBins ? W.bins : cs.a.bin_spill + (size_t)(blockIdx.x * kQualWarps + (threadIdx.x >> 5)) * kMaxBins;
+        for (int i = lane; i < nb; i += 32) cs.a.em_pool[off + i] = bins[i];
+        // first bin of each base (bins are sorted by base): lane b counts the bins of bases < b + 1
+        uint32_t below = 0;
+        for (int i = lane; i < nb; i += 32) {
+            const uint32_t b = bin_base(bins[i]);
+            below += (b < 1u) | ((uint32_t)(b < 2u) << 8) | ((uint32_t)(b < 3u) << 16) | ((uint32_t)(b < 4u) << 24);
+        }
+        // (a lane sees at most kMaxBins / 32 = 15 bins, so the four byte counters cannot overflow before the reduction)
+        const uint32_t s0 = __reduce_add_sync(kFull, below & 0xffu), s1 = __reduce_add_sync(kFull, (below >> 8) & 0xffu),
+                       s2 = __reduce_add_sync(kFull, (below >> 16) & 0xffu), s3 = __reduce_add_sync(kFull, below >> 24);
+        // log-likelihoods of the four single-allele models (closed form, see single_allele_ll): the last elimination round of
+        // the site's decision consults two of them
+        {
+            double sl[4];
+            single_allele_ll4(bins, nb, sl);
+            if (lane < 4) cs.a.em_single[(size_t)hdr * 4 + lane] = lane == 0 ? sl[0] : lane == 1 ? sl[1] : lane == 2 ? sl[2] : sl[3];
+        }
+        if (lane == 0) {
+            uint4 w0, w1, w2, w3;
+            w0.x = site; w0.y = off; w0.z = (uint32_t)nb; w0.w = act | (W.flag_word << 8);
+            w1.x = t2; w1.y = base3 + t3; w1.z = base4 + t4; w1.w = n_k[0] + n_k[1] + n_k[2];
+            w2.x = d0; w2.y = d1; w2.z = d2; w2.w = d3;
+            w3.x = total; w3.y = s0 | (s1 << 16); w3.z = s2 | (s3 << 16); w3.w = 0;
+            uint4* H = reinterpret_cast<uint4*>(cs.a.em_hdr + hdr);
+            H[0] = w0; H[1] = w1; H[2] = w2; H[3] = w3;
+        }
+        __syncwarp();
+        return;   // the record is completed by K4b
+    }
+    // One active allele: the reference still runs one EM; its answer is closed form (see single_allele_ll):
+    // AF == 1.0 exactly, or NaN when a phred-0 read of that base exists.
+    {
         const int b = __ffs(act) - 1;
         const bool bad = qmin == 0 && W.hist[b * kQSlots] != 0;
         const double v = bad ? __longlong_as_double(0x7ff8000000000000ll) : 1.0;
         __syncwarp();
         if (lane < 4) W.res_f[lane] = lane == b ? v : 0.0;
-        em_calls = 1;
         if (qmin <= qmax) {   // histogram back to zero
 #pragma unroll 1
             for (uint32_t q = qmin + lane; q <= qmax; q += 32) {
@@ -150,7 +142,7 @@ __device__ __noinline__ void hist_site(uint32_t site) {
     if (n_alt) {
         const int first_act = __ffs(act) - 1;
         const double r = (double)sel4u(first_act, d0, d1, d2, d3) / (double)total;
-        if (n_act == 1 && total > 10 && r > 0.5) { qual = 5000.0; flags |= BV_FLAG_MONO_QUAL; }
+        if (total > 10 && r > 0.5) { qual = 5000.0; flags |= BV_FLAG_MONO_QUAL; }
     }
 
     // ---- record ----
@@ -169,11 +161,11 @@ __device__ __noinline__ void hist_site(uint32_t site) {
         if (alt_set & 8) { r.af[k] = af[3]; alts |= 3u << (8 * k); ++k; }
         r.n_alt = (uint8_t)n_alt;
         r.alt[0] = (uint8_t)alts; r.alt[1] = (uint8_t)(alts >> 8); r.alt[2] = (uint8_t)(alts >> 16); r.alt[3] = (uint8_t)(alts >> 24);
-        r.n_active = (uint8_t)n_act;
+        r.n_active = 1;
         r.flags = (uint8_t)flags;
-        r.em_calls = (uint8_t)(em_calls > 255u ? 255u : em_calls);
+        r.em_calls = 1;
         r.qual = qual;
-        r.chi2 = chi;
+        r.chi2 = 0.0;
         r.fs_vcf = 0.0;
         // called sites go on to the rank-sum / population-group kernels (bv_call_kernels.cuh)
         if (n_alt && cs.a.list_called) cs.a.list_called[atomicAdd(cs.a.counters + kCntCalled, 1u)] = site;
@@ -636,15 +628,13 @@ __device__ __forceinline__ void em_iter_list(const SiteKernelArgs& a, TaskCta& c
                 else {
                     t = list_base + idx;
                     const uint32_t word = a.em_tasks[t];
-                    if (word != kEmTaskInvalid) {   // (a slot that was allocated but not used: the lane asks again)
-                        const EmSiteHdr H = a.em_hdr[word & 0x0fffffffu];
-                        if (H.nb <= (uint32_t)kStageBins) {
-                            for (uint32_t i = 0; i < H.nb; ++i) my_row[i] = a.em_pool[H.bins_off + i];
-                            bins = my_row;
-                        } else bins = a.em_pool + H.bins_off;
-                        em_setup<NA>(H, word >> 28, S);
-                        have = true; first = true; it = a.em_max_iter; flags = 0;
-                    }
+                    const EmSiteHdr H = a.em_hdr[word & 0x0fffffffu];
+                    if (H.nb <= (uint32_t)kStageBins) {
+                        for (uint32_t i = 0; i < H.nb; ++i) my_row[i] = a.em_pool[H.bins_off + i];
+                        bins = my_row;
+                    } else bins = a.em_pool + H.bins_off;
+                    em_setup<NA>(H, word >> 28, S);
+                    have = true; first = true; it = a.em_max_iter; flags = 0;
                 }
             }
         }
@@ -685,11 +675,9 @@ __global__ void __launch_bounds__(kTaskThreads) bv_em_iter_kernel(const __grid_c
     __syncthreads();
     grid_dep_wait();
     const double* lut = &cs.lut[0][0];
-    const uint32_t n2 = min(a.counters[kCntEmTask2], a.em_task_cap[0]), n3 = min(a.counters[kCntEmTask3], a.em_task_cap[1]),
-                   n4 = min(a.counters[kCntEmTask4], a.em_task_cap[2]);
-    em_iter_list<2>(a, cs, lut, 0u, n2, a.counters + kCntEmFetch2);
-    em_iter_list<3>(a, cs, lut, a.em_task_cap[0], n3, a.counters + kCntEmFetch3);
-    em_iter_list<4>(a, cs, lut, a.em_task_cap[0] + a.em_task_cap[1], n4, a.counters + kCntEmFetch4);
+    em_iter_list<2>(a, cs, lut, 0u, a.counters[kCntEmTask2], a.counters + kCntEmFetch2);
+    em_iter_list<3>(a, cs, lut, a.em_task_cap[0], a.counters[kCntEmTask3], a.counters + kCntEmFetch3);
+    em_iter_list<4>(a, cs, lut, a.em_task_cap[0] + a.em_task_cap[1], a.counters[kCntEmTask4], a.counters + kCntEmFetch4);
     grid_dep_launch();
 }
 
@@ -841,16 +829,15 @@ __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(cons
     if (tid == 0) cs.n_fs = 0;
     grid_dep_wait();
     {
-        const uint64_t n_all = (uint64_t)min(a.counters[kCntEmTask2], a.em_task_cap[0]) + min(a.counters[kCntEmTask3], a.em_task_cap[1]) +
-                               min(a.counters[kCntEmTask4], a.em_task_cap[2]);
+        const uint64_t n_all = (uint64_t)a.counters[kCntEmTask2] + a.counters[kCntEmTask3] + a.counters[kCntEmTask4];
         if ((n_all > (uint64_t)a.em_task_split) != (kMinCtas == kTaskHiCtas)) return;
     }
     const double* lut = &cs.lut[0][0];
     // the three task lists, one after the other
     uint32_t n_list[3], blk_end[3], base[3];
-    n_list[0] = min(a.counters[kCntEmTask2], a.em_task_cap[0]);
-    n_list[1] = min(a.counters[kCntEmTask3], a.em_task_cap[1]);
-    n_list[2] = min(a.counters[kCntEmTask4], a.em_task_cap[2]);
+    n_list[0] = a.counters[kCntEmTask2];
+    n_list[1] = a.counters[kCntEmTask3];
+    n_list[2] = a.counters[kCntEmTask4];
     base[0] = 0; base[1] = a.em_task_cap[0]; base[2] = a.em_task_cap[0] + a.em_task_cap[1];
     // Lanes per task: one -- a thread per task -- unless the tile has so few tasks that most of the GPU would stand idle
     // behind their serial chains: then four (the sums are formed the same way either way, see LaneGroup).

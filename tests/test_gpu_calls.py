@@ -28,13 +28,16 @@ def _soft_sites(recs):
     return set(np.nonzero((recs["flags"] & (capi.FLAG_NEAR_LRT | capi.FLAG_LRT_TIE)) != 0)[0].tolist())
 
 
-def _run_and_check(engine, b, q, s, r, mapq, rpr, N, grp, G, maf, abs_mode, label):
+def _run_and_check(engine, b, q, s, r, mapq, rpr, N, grp, G, maf, abs_mode, label, pin_flips=False):
+    """pin_flips: the records' listed flips are held to tests/golden/flips_r02.json under `label` (util.report_flips)."""
     engine.set_params(min_af=maf, abs_mode=abs_mode)
     engine.set_groups(grp, G)
     recs, calls, groups = engine.call_host_calls(b, q, s, r, mapq, rpr, N)
     want_recs = L.oracle_tile(b, q, s, r, N, maf, abs_mode)
     ie, fe, flips = util.compare_records(recs, want_recs)
     assert len(ie) == 0 and len(fe) == 0, f"{label}: records differ at {ie[:5]} / {fe[:5]}"
+    if pin_flips:
+        util.report_flips(label, recs, want_recs, flips)
     # every called site is listed exactly once
     assert np.array_equal(calls["site"], np.nonzero(recs["n_alt"] > 0)[0]), label
     # the oracle's called-site outputs for OUR call set (so that a listed tie flip does not cascade)
@@ -79,17 +82,28 @@ def test_calls_match_reference_fixture(engine, path, abs_mode):
         ("C5-like", 600, 2000, 3, dict(coverage=0.99326, variant_frac=0.5, multi_frac=0.5)),
         ("odd-N", 2000, 1003, 5, dict(coverage=0.3, variant_frac=0.3, multi_frac=0.5)),
         ("tiny-N", 2000, 7, 2, dict(coverage=0.8, variant_frac=0.5)),
+        ("deep-wide-phred", 120, 3000, 1, None),   # util.binned_tile: rows of more than 160 bins (K6's spill rows)
     ],
 )
 def test_calls_synthetic(engine, name, S, N, G, kw, abs_mode):
-    model = bv.synth.make_model(seed=4321 + N, **kw)
-    b, q, s, mapq, r = bv.synth_fill_host(model, 0, S, N, with_mapq=True)
-    rpr = bv.synth_fill_rpr_host(model, 0, S, N)
+    maf = bv.cli_min_af(0.01, N)
+    if kw is None:
+        rng = np.random.default_rng(S + abs_mode)
+        b, q, s, r = util.binned_tile(rng, util.deep_shape(rng, S, N, maf), N, maf)
+        mapq, rpr = util.random_aux(rng, b, N)
+    else:
+        model = bv.synth.make_model(seed=4321 + N, **kw)
+        b, q, s, mapq, r = bv.synth_fill_host(model, 0, S, N, with_mapq=True)
+        rpr = bv.synth_fill_rpr_host(model, 0, S, N)
     rng = np.random.default_rng(N)
     grp = util.random_groups(rng, N, G)
-    maf = bv.cli_min_af(0.01, N)
-    recs, calls, groups = _run_and_check(engine, b, q, s, r, mapq, rpr, N, grp, G, maf, abs_mode, name)
+    recs, calls, groups = _run_and_check(engine, b, q, s, r, mapq, rpr, N, grp, G, maf, abs_mode, f"calls {name} abs={abs_mode}",
+                                         pin_flips=kw is None)
     assert len(calls) > 0
+    if kw is None:   # the one group's rows (90 % of the samples) still pass kSmemBins at most called sites
+        g0 = np.nonzero(grp == 0)[0]
+        deep = util.bin_counts(b[:, g0], q[:, g0], len(g0))[calls["site"]] > 160
+        assert deep.sum() > len(calls) // 2 and len(calls) > 50
 
 
 def test_calls_pinned_planes_zero_copy_and_no_groups(engine):

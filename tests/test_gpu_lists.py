@@ -62,12 +62,15 @@ def compare_to_oracle(got, want, depth, label):
     return np.nonzero(call_diff & soft)[0]
 
 
-def run_and_check(engine, b, q, s, r, lists, N, maf, abs_mode, label):
+def run_and_check(engine, b, q, s, r, lists, N, maf, abs_mode, label, pin_flips=False):
+    """pin_flips: the listed flips are held to tests/golden/flips_r02.json under `label` (util.report_flips)."""
     engine.set_params(min_af=maf, abs_mode=abs_mode)
     recs, lrt = engine.call_host_lists(b, q, s, r, lists, N)
     want = OL.oracle_lists(b, q, s, r, lists, N, maf, abs_mode)
     depth = recs["depth"].sum(axis=1).astype(np.float64) + recs["depth_other"]
     flips = compare_to_oracle(lrt, want, depth, label)
+    if pin_flips:
+        util.report_flips(label, lrt, want, flips)
     return recs, lrt, flips
 
 
@@ -109,6 +112,14 @@ def test_lists_fuzz_vs_oracle(engine, min_af, abs_mode):
         r[rng.random(S) < 0.05] = ord("N")
         r[rng.random(S) < 0.05] = ord("g")
         run_and_check(engine, b, q, s, r, random_lists(rng, S), N, maf_of(min_af, N), abs_mode, f"fuzz N={N} maf={min_af}")
+    # deep rows with every phred 0..95: more than kSmemBins = 160 bins per row, so lrt_on_bins works through the spill rows
+    N = 3000
+    maf = maf_of(min_af, N)
+    b, q, s, r = util.binned_tile(rng, util.deep_shape(rng, 80, N, maf), N, maf)
+    assert (util.bin_counts(b, q, N) > 160).all()
+    _, lrt, _ = run_and_check(engine, b, q, s, r, random_lists(rng, len(r)), N, maf, abs_mode, f"lists deep-wide-phred maf={min_af} mode={abs_mode}",
+                              pin_flips=True)
+    assert (lrt["em_calls"] >= 3).sum() > 10
 
 
 @pytest.mark.parametrize("abs_mode", [0, 1])
@@ -117,9 +128,8 @@ def test_acgt_lists_equal_the_records(engine, min_af, abs_mode):
     """lrt(A,C,G,T) against the site's own record.  Bit for bit: n_alt / alt / n_active / fs, em_calls except where the bound
     of K3 decided the site without an EM (BV_FLAG_LRT_BOUND), and af / qual / chi2 wherever the record took at most one EM.
     Where it took the EMs of several subsets the record comes from K4b's thread-per-task EM, whose sums are associated
-    differently from those of lrt_on_bins (K8, K6, K4a's fallback when the scratch pools are full): there af / qual / chi2
-    agree to util's tolerance and the sites are printed -- the finding that the records of such sites depend in their last
-    bits on whether K4b or K4a's fallback decided them."""
+    differently from those of lrt_on_bins (K8, K6): there af / qual / chi2 agree to util's tolerance and the sites are printed.
+    Every EM site of a record is decided by K4b whatever the context's max_sites (tests/test_gpu_em_scratch.py)."""
     for (S, N, kw) in [(6000, 1000, dict(coverage=0.1, variant_frac=0.1)), (500, 2000, dict(coverage=0.99326, variant_frac=0.5, multi_frac=0.5)),
                        (300, 10000, dict(coverage=0.1, variant_frac=0.2)), (2000, 7, dict(coverage=0.8, variant_frac=0.5))]:
         model = bv.synth.make_model(seed=31 + N, **kw)
@@ -154,10 +164,16 @@ def test_acgt_lists_equal_the_records(engine, min_af, abs_mode):
 def test_ref_alt_lists_equal_the_group_kernel(engine, abs_mode):
     """[REF, ALT...] at the called sites with one group of every sample: K6's bv_group_out, bit for bit."""
     for (S, N, kw) in [(4000, 1000, dict(coverage=0.1, variant_frac=0.2, multi_frac=0.3)),
-                       (400, 2000, dict(coverage=0.99326, variant_frac=0.5, multi_frac=0.5))]:
-        model = bv.synth.make_model(seed=5 + N, **kw)
-        b, q, s, mapq, r = bv.synth_fill_host(model, 0, S, N, with_mapq=True)
-        rpr = bv.synth_fill_rpr_host(model, 0, S, N)
+                       (400, 2000, dict(coverage=0.99326, variant_frac=0.5, multi_frac=0.5)),
+                       (150, 3000, None)]:   # util.binned_tile: rows of more than 160 bins (K6's and K8's spill rows)
+        if kw is None:
+            rng = np.random.default_rng(abs_mode)
+            b, q, s, r = util.binned_tile(rng, util.deep_shape(rng, S, N, 0.01), N, 0.01)
+            mapq, rpr = util.random_aux(rng, b, N)
+        else:
+            model = bv.synth.make_model(seed=5 + N, **kw)
+            b, q, s, mapq, r = bv.synth_fill_host(model, 0, S, N, with_mapq=True)
+            rpr = bv.synth_fill_rpr_host(model, 0, S, N)
         engine.set_params(min_af=0.01, abs_mode=abs_mode)
         engine.set_groups(np.zeros(N, np.uint8), 1)
         recs, calls, groups = engine.call_host_calls(b, q, s, r, mapq, rpr, N)
@@ -175,6 +191,8 @@ def test_ref_alt_lists_equal_the_group_kernel(engine, abs_mode):
         assert same_f64(got["af"], g["af"]).all()
         lrt_flags = capi.FLAG_ZERO_SUBSET | capi.FLAG_NEAR_LRT | capi.FLAG_LRT_TIE | capi.FLAG_EM_MAXITER | capi.FLAG_BAD_QUAL
         assert ((got["flags"] & lrt_flags) == (g["flags"] & lrt_flags)).all()
+        if kw is None:
+            assert (util.bin_counts(b, q, N)[calls["site"]] > 160).all()
         uncalled = np.setdiff1d(np.arange(S), calls["site"])
         assert lrt[uncalled].tobytes() == bytes(64 * len(uncalled))
 

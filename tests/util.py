@@ -148,6 +148,117 @@ def random_tile(rng, S, N, cov, qlo, qhi, nalt_max=3, other=0.0, indel=0.0, bad_
     return base, qual, strand, refc
 
 
+N_QBINS = 96   # phred 0..95: the histogram slots of K4a / K6 / K8 that hold one phred each (bv_common.cuh kQSlots)
+EM_TASKS = {0: 0, 1: 0, 2: 1, 3: 4, 4: 11}   # EM tasks of a site by its number of active alleles (subsets of >= 2 of them)
+
+
+def active_threshold(T, min_af):
+    """Smallest depth d with (double)d / T >= (double)(float)min_af, the reference's compare (src/basetype.cpp:137)."""
+    maf = float(np.float32(min_af))
+    d = max(0, int(np.ceil(maf * T)) - 2)
+    while d / T < maf:
+        d += 1
+    return d
+
+
+def binned_site(rng, nb, k, T, min_af):
+    """One row of T counted reads with exactly nb distinct (base, phred) bins (bases A, C, G, T and OTHER, phred 0..95) and
+    exactly k active alleles under min_af.  Returns (bases, phreds) in random order, or None when no such row exists.
+    Two active alleles always have >= 5 reads each, so that the bound of K3 (REF plus a minor allele of <= 4 reads) never
+    settles a site meant for the EM."""
+    thr = active_threshold(T, min_af)
+    act = np.sort(rng.choice(4, k, replace=False))
+    is_act = np.isin(np.arange(5), act)
+    cap = np.where(is_act | (np.arange(5) == 4), N_QBINS, min(N_QBINS, thr - 1))
+    if k < 1 or nb < k or nb > cap.sum():
+        return None
+    cnt = is_act.astype(np.int64)
+    free = np.repeat(np.arange(5), cap - cnt)
+    cnt += np.bincount(rng.choice(free, nb - k, replace=False), minlength=5) if nb > k else 0
+    depth = cnt.copy()
+    for b in range(4):   # inactive bases: up to one read below the threshold
+        if not is_act[b] and cnt[b]:
+            depth[b] += rng.integers(0, thr - 1 - cnt[b] + 1)
+    if cnt[4]:
+        depth[4] += rng.integers(0, max(1, T // 20))
+    floor = np.where(is_act, np.maximum(np.maximum(cnt, thr), 5), 0)
+    left = T - depth[~is_act].sum() - floor.sum()
+    if left < 0:
+        depth[~is_act] = cnt[~is_act]
+        left = T - depth[~is_act].sum() - floor.sum()
+        if left < 0:
+            return None
+    w = rng.dirichlet(np.ones(k))
+    if k >= 2 and rng.random() < 0.3:   # one allele right at the threshold (or at its bin count)
+        w[-1] = 0.0
+        w /= w.sum()
+    depth[act] = floor[act] + rng.multinomial(left, w)
+    bases, phreds = [], []
+    for b in range(5):
+        if depth[b]:
+            qs = rng.choice(N_QBINS, cnt[b], replace=False)
+            phreds.append(np.concatenate([qs, rng.choice(qs, depth[b] - cnt[b])]))
+            bases.append(np.full(depth[b], b))
+    order = rng.permutation(T)
+    return np.concatenate(bases)[order].astype(np.uint8), np.concatenate(phreds)[order].astype(np.uint8)
+
+
+def max_bins(k, N, min_af):
+    """Most bins binned_tile can place in a row of N cells with k active alleles: 96 per active base and OTHER, and fewer than
+    the active threshold of the fewest reads binned_tile covers (90 % of N) per inactive base."""
+    return (k + 1) * N_QBINS + (4 - k) * min(N_QBINS, active_threshold(N - N // 10, min_af) - 1)
+
+
+def deep_shape(rng, S, N, min_af, lo=161):
+    """(nb, k) of S deep, wide-phred rows: 1-4 active alleles and more than kSmemBins = 160 bins each (up to max_bins)."""
+    ks = [int(k) for k in rng.integers(1, 5, S) if max_bins(int(k), N, min_af) >= lo]
+    return [(int(rng.integers(lo, max_bins(k, N, min_af) + 1)), k) for k in ks]
+
+
+def binned_tile(rng, shape, N, min_af, odd_ref=0.05):
+    """Dense planes [S][round16(N)] with one row per (nb, k) of `shape`: exactly nb (base, phred) bins and k active alleles
+    (binned_site), 90-100 % of the N cells covered, random strands, REF mostly one of the active alleles, a few 'N' and
+    lowercase REFs.  Returns (base, qual, strand, ref_base)."""
+    S, pitch = len(shape), (N + 15) // 16 * 16
+    base = np.full((S, pitch), 5, np.uint8)
+    qual = np.zeros((S, pitch), np.uint8)
+    strand = np.full((S, pitch), 2, np.uint8)
+    ref = np.zeros(S, np.uint8)
+    for s, (nb, k) in enumerate(shape):
+        T = N - int(rng.integers(0, N // 10 + 1))
+        row = binned_site(rng, nb, k, T, min_af)
+        assert row is not None, (nb, k, N, min_af)
+        cells = rng.choice(N, T, replace=False)
+        base[s, cells], qual[s, cells] = row
+        strand[s, cells] = rng.integers(0, 2, T)
+        bases = np.unique(row[0][row[0] < 4])
+        rc = int(rng.choice(bases)) if len(bases) and rng.random() < 0.7 else int(rng.integers(0, 4))
+        u = rng.random()
+        ref[s] = ord("N") if u < odd_ref else ord("acgt"[rc]) if u < 2 * odd_ref else ord("ACGT"[rc])
+    return base, qual, strand, ref
+
+
+def bin_counts(base, qual, N):
+    """Distinct (base, phred) pairs among the counted cells (base codes 0..4) of every row; phred must be < 96."""
+    b, q = base[:, :N].astype(np.int64), qual[:, :N].astype(np.int64)
+    counted = b < 5
+    assert (q[counted] < N_QBINS).all()
+    seen = np.zeros((base.shape[0], 5 * N_QBINS), bool)
+    rows = np.broadcast_to(np.arange(base.shape[0])[:, None], b.shape)
+    seen[rows[counted], (b * N_QBINS + q)[counted]] = True
+    return seen.sum(axis=1)
+
+
+def active_counts(base, N, min_af):
+    """Number of active alleles of every row: depth / total >= min_af (float-widened), total over base codes 0..4."""
+    b = base[:, :N]
+    depth = np.stack([(b == c).sum(axis=1) for c in range(5)], axis=1)
+    total = depth.sum(axis=1)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        act = (depth[:, :4] / np.maximum(total, 1)[:, None]) >= float(np.float32(min_af))
+    return np.where(total > 0, act.sum(axis=1), 0)
+
+
 def random_aux(rng, base, N, rpr_max=35, mapq_levels=(60, 60, 60, 37, 20, 0)):
     """mapq (u8) and read-position-rank (u16) planes for a base plane; uncovered cells get 0 like the batchfile."""
     S, pitch = base.shape
