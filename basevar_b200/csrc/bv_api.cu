@@ -431,9 +431,10 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
     grid = (uint32_t)ctx->num_sms * (uint32_t)ctx->task_ctas_per_sm;
     const uint32_t grid_hi = (uint32_t)ctx->num_sms * (uint32_t)ctx->task_ctas_per_sm_hi;
     bv::SiteKernelArgs b = a;
-    if (a.abs_mode != BV_EM_ABS_INT_TRUNC) {
+    if (a.abs_mode != BV_EM_ABS_INT_TRUNC || a.em_max_iter == 0) {
         // fabs in the convergence test: EMs of very different lengths; their iterations run with the lanes fed task by task
-        // (bv_em_iter_kernel), the rest of every task -- log-likelihood sums, decisions -- from the frequencies that leaves
+        // (bv_em_iter_kernel), the rest of every task -- log-likelihood sums, decisions -- from the frequencies that leaves.
+        // (em_max_iter 0, either mode: no iteration, and bv_em_iter_kernel leaves the frequencies of the first E-step + M-step.)
         BV_CUDA(ctx, launch_chained(pdl, bv::bv_em_iter_kernel, grid, bv::kTaskThreads, bv::kTaskSmemBytes, stream, a));
         ctx->launches += 1;
         b.em_resume = 1;
@@ -691,9 +692,20 @@ static int upload_tables(bv_ctx* ctx) {
     return BV_OK;
 }
 
+// The statistics' parameters the kernels follow exactly (include/basevar_b200.h, bv_params); nullptr when they are.
+static const char* params_error(const bv_params* p) {
+    if (!(isfinite(p->min_af) && p->min_af > 0.0f))
+        return "min_af must be finite and > 0 (at 0 a zero-frequency allele is active and the reference throws)";
+    if (p->em_max_iter < 0) return "em_max_iter must be >= 0";
+    if (isnan(p->em_eps)) return "em_eps must not be NaN";
+    if (p->em_abs_mode != BV_EM_ABS_INT_TRUNC && p->em_abs_mode != BV_EM_ABS_DOUBLE) return "em_abs_mode must be BV_EM_ABS_INT_TRUNC or BV_EM_ABS_DOUBLE";
+    return nullptr;
+}
+
 int bv_create(int device, const bv_params* params, bv_ctx** out_ctx) {
     if (!params || !out_ctx) return set_err(nullptr, BV_ERR_ARG, "bv_create: null argument");
     *out_ctx = nullptr;
+    if (const char* why = params_error(params)) return set_err(nullptr, BV_ERR_ARG, "bv_create: %s", why);
     if (params->max_samples == 0 || params->max_samples > 2000000u)
         return set_err(nullptr, BV_ERR_ARG, "bv_create: max_samples must be in 1..2000000");
     if (params->n_slots > 64) return set_err(nullptr, BV_ERR_ARG, "bv_create: n_slots > 64");
@@ -814,6 +826,7 @@ void bv_destroy(bv_ctx* ctx) {
 
 int bv_set_params(bv_ctx* ctx, const bv_params* p) {
     if (!ctx || !p) return set_err(ctx, BV_ERR_ARG, "bv_set_params: null argument");
+    if (const char* why = params_error(p)) return set_err(ctx, BV_ERR_ARG, "bv_set_params: %s", why);   // (nothing changed)
     ctx->prm.min_af = p->min_af;
     ctx->prm.lrt_threshold = p->lrt_threshold;
     ctx->prm.em_max_iter = p->em_max_iter;

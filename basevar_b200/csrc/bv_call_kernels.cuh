@@ -504,6 +504,7 @@ __device__ __noinline__ void group_unit(uint32_t k, uint32_t g) {
             const double v = bad ? __longlong_as_double(0x7ff8000000000000ll) : 1.0;
             __syncwarp();
             if (lane < 4) W.res_f[lane] = lane == b ? v : 0.0;
+            if (lane == 0) W.flag_word |= single_em_flag(dep[b], total, cs.a);
         }
         if (qmin <= qmax) {   // histogram back to zero
 #pragma unroll 1

@@ -72,7 +72,8 @@ struct __align__(16) EmSiteHdr {
     uint32_t site;
     uint32_t bins_off;       // first word of the site's bins in SiteKernelArgs::em_pool
     uint32_t nb;             // number of bins
-    uint32_t act_flags;      // active alleles before the LRT (bits 0-3) | BV_FLAG_* raised so far << 8
+    uint32_t act_flags;      // active alleles before the LRT (bits 0-3) | BV_FLAG_* raised so far << 8 | bit 16 + b: the EM of the
+                             // single-allele model {b} raises BV_FLAG_EM_MAXITER (single_em_flag; none at the default parameters)
     uint32_t task[3];        // slot of the site's first task among the 2-, 3- and 4-allele tasks (em_tasks / em_res)
     uint32_t remaining;      // tasks not finished yet: the thread that takes it to 0 decides the site
     uint32_t depth[4];
@@ -208,6 +209,30 @@ __device__ __forceinline__ bool is_active(uint32_t dep, uint32_t total, double d
     if (x < thr * 0.999999999) return false;
     return x / dtot >= min_af;
 }
+
+// BV_FLAG_EM_MAXITER of the EM of a single-allele model {b} that starts from f_b = d / total (0 < d <= total), the closed form
+// of its loop count (src/algorithm.h:210-255): the first M-step sets f_b = 1 exactly, so in the loop's first iteration every
+// log marginal moves by -log(d / total) and in every later one by 0.  The loop therefore ends after one iteration when that
+// first sum is below eps, after two when 0 < eps, and otherwise runs all em_max_iter.  (A phred-0 read of b makes the
+// marginals NaN; that loop count is not modelled, see BV_FLAG_EM_MAXITER in the header.)
+// Out of line: the kernels that call it run at the default parameters, where the answer is 0 without it.
+__device__ __noinline__ uint32_t single_em_flag_off_default(uint32_t d, uint32_t total, int max_iter, double eps, int abs_mode) {
+    if (max_iter <= 1) return BV_FLAG_EM_MAXITER;
+    double delta1 = 0.0;
+    if (d != total) {
+        const double lg = -log((double)d / (double)total);
+        delta1 = (double)total * (abs_mode == BV_EM_ABS_INT_TRUNC ? (double)(int)lg : lg);
+    }
+    const bool flag = !(delta1 < eps) && (max_iter == 2 || !(eps > 0.0));
+    return flag ? BV_FLAG_EM_MAXITER : 0u;
+}
+__device__ __forceinline__ uint32_t single_em_flag(uint32_t d, uint32_t total, const SiteKernelArgs& a) {
+    if (a.em_max_iter > 2 && a.em_eps > 0.0) return 0u;   // the defaults: done after at most two iterations
+    return single_em_flag_off_default(d, total, a.em_max_iter, a.em_eps, a.abs_mode);
+}
+// At em_max_iter 0 the EM reports the first E-step's log marginals, L * f0 with f0 = d / total: the closed form of the
+// single-allele log-likelihood (f = 1) plus this.  Out of line for the same reason.
+__device__ __noinline__ double first_estep_ll_shift(uint32_t d, double dtot) { return dtot * log((double)d / dtot); }
 
 __device__ __forceinline__ uint32_t sel4u(int j, uint32_t v0, uint32_t v1, uint32_t v2, uint32_t v3) {
     return j == 0 ? v0 : j == 1 ? v1 : j == 2 ? v2 : v3;

@@ -90,6 +90,7 @@ __global__ void __launch_bounds__(kCountWarps * 32, 1) bv_count_kernel(const __g
     const uint64_t pitch = a.pitch;
     uint32_t* const g_out = reinterpret_cast<uint32_t*>(a.out);
     const uint32_t one_active = (1.0 >= a.min_af) ? 1u : 0u;   // a site whose reads all agree has that allele active
+    const uint32_t one_flags = single_em_flag(1u, 1u, a);       // ... and its EM starts from f = 1
     const uint32_t s_stage0 = smem_u32(&W.stage[0]), s_full0 = smem_u32(&W.full[0]);
     // byte masks of the row's last 16-cell vector when N is not a multiple of 16 (one lane, once per row)
     uint32_t keep[4];
@@ -194,7 +195,7 @@ __global__ void __launch_bounds__(kCountWarps * 32, 1) bv_count_kernel(const __g
             if (lane == ref_code) w = n_ref;                          // depth[REF]
             if (lane == ref_code + kWFwd) w = n_ref - n_rev;          // fwd[REF]
             if (lane == ref_code + kWRev) w = n_rev;                  // rev[REF]
-            if (lane == kWInfo) w = (n_active << 8) | (n_active << 24);   // n_active | flags 0 | em_calls
+            if (lane == kWInfo) w = (n_active << 8) | ((n_active ? one_flags : 0u) << 16) | (n_active << 24);   // n_active | flags | em_calls
         } else {
             // counts only: words 0..13 = depth[4], other, state, fwd[4], rev[4]; flags in word 15
             const uint32_t b = lane < 4 ? lane : lane < kWRev ? lane - kWFwd : lane - kWRev;   // base of this word
@@ -215,7 +216,10 @@ __global__ void __launch_bounds__(kCountWarps * 32, 1) bv_count_kernel(const __g
         }
         g_out[(size_t)site * 32 + lane] = w;
         // compact transport: the two counts the whole record of such a site follows from; 0xffffffff = needs its full record
-        if (a.brief != nullptr && lane == 0) a.brief[site] = fl == 0 ? make_uint2(n_ref, n_rev) : make_uint2(0xffffffffu, 0u);
+        // (a brief carries no flags: a covered site whose record has one -- one_flags, at em_max_iter <= 1 or em_eps <= 0 --
+        // travels as a full record)
+        if (a.brief != nullptr && lane == 0)
+            a.brief[site] = fl == 0 && (n_ref == 0 || one_flags == 0u) ? make_uint2(n_ref, n_rev) : make_uint2(0xffffffffu, 0u);
         ref_raw = ref_next;
     }
     if (slow_n) flush_slow();

@@ -94,14 +94,26 @@ __device__ __noinline__ void hist_site(uint32_t site) {
                        s2 = __reduce_add_sync(kFull, (below >> 16) & 0xffu), s3 = __reduce_add_sync(kFull, below >> 24);
         // log-likelihoods of the four single-allele models (closed form, see single_allele_ll): the last elimination round of
         // the site's decision consults two of them
+        // (away from the default parameters: at em_max_iter 0 the log-likelihood of the first E-step, and which of these EMs raise
+        // BV_FLAG_EM_MAXITER -- worked out here, so that the decision in K4b stays as it is at the defaults)
+        uint32_t single_mi = 0;
         {
             double sl[4];
             single_allele_ll4(bins, nb, sl);
-            if (lane < 4) cs.a.em_single[(size_t)hdr * 4 + lane] = lane == 0 ? sl[0] : lane == 1 ? sl[1] : lane == 2 ? sl[2] : sl[3];
+            if (lane < 4) {
+                double v = lane == 0 ? sl[0] : lane == 1 ? sl[1] : lane == 2 ? sl[2] : sl[3];
+                const uint32_t d = sel4u(lane, d0, d1, d2, d3);
+                if (act >> lane & 1u) {
+                    if (cs.a.em_max_iter == 0) v += first_estep_ll_shift(d, (double)total);
+                    single_mi = single_em_flag(d, total, cs.a) != 0u ? 1u << lane : 0u;
+                }
+                cs.a.em_single[(size_t)hdr * 4 + lane] = v;
+            }
+            single_mi = __reduce_or_sync(kFull, single_mi);
         }
         if (lane == 0) {
             uint4 w0, w1, w2, w3;
-            w0.x = site; w0.y = off; w0.z = (uint32_t)nb; w0.w = act | (W.flag_word << 8);
+            w0.x = site; w0.y = off; w0.z = (uint32_t)nb; w0.w = act | (W.flag_word << 8) | (single_mi << 16);
             w1.x = t2; w1.y = base3 + t3; w1.z = base4 + t4; w1.w = n_k[0] + n_k[1] + n_k[2];
             w2.x = d0; w2.y = d1; w2.z = d2; w2.w = d3;
             w3.x = total; w3.y = s0 | (s1 << 16); w3.z = s2 | (s3 << 16); w3.w = 0;
@@ -128,7 +140,7 @@ __device__ __noinline__ void hist_site(uint32_t site) {
         }
     }
     __syncwarp();
-    uint32_t flags = W.flag_word;
+    uint32_t flags = W.flag_word | single_em_flag(sel4u(__ffs(act) - 1, d0, d1, d2, d3), total, cs.a);
 
     // ---- ALT / QUAL (src/basetype.cpp:170-196) ----
     // Here only the rule that needs no arithmetic (mono-allelic 5000); the chi-square survival function and the Fisher
@@ -227,6 +239,8 @@ constexpr uint32_t kG4MaxTasks = 12288;            // tiles with at most this ma
 struct __align__(16) TaskCta {
     double lut[4][kQSlots];           // 1 - eps(q), eps(q) / 3, log(1 - eps(q)), log(eps(q) / 3)
     double2 ltab[kLogTabEntries];     // log_tab()'s table
+    double em_eps;                    // SiteKernelArgs::em_eps ...
+    uint32_t unit_eps;                // ... and whether it lies in (0, 1] (em_task's convergence test; here, not in registers)
     uint32_t n_decide;                // sites whose last task finished in this round of the CTA ...
     uint32_t decide_hdr[kTaskThreads];   // ... their headers: decided one thread per site after the round
     uint32_t n_fs;                    // Fisher tests of the VCF rows of decided sites, listed by decide_site ...
@@ -448,8 +462,39 @@ __device__ __forceinline__ bool moved_by_one(double m, double mp) {
     const double diff = nlog(m) - nlog(mp);
     return fabs(diff) >= 1.0 && fabs(diff) < 2147483648.0;
 }
+// With an eps outside (0, 1] that question does not decide "sum < eps": EM()'s convergence sum itself, sum of
+// count * (double)abs((int)diff) over the bins (see iabs_trunc), formed in integers -- the same value in any order and with any
+// number of lanes per task.  Returns whether the EM goes on.
+template <int NA>
+__device__ __noinline__ bool em_int_sum_more(const uint32_t* bins, const EmState<NA>& S, const double* lut, const LaneGroup& lg, double eps) {
+    long long x = 0;
+    if (S.c_out != 0.0 && lg.gl == 0) {   // the bins outside the subset: marginals e3 * F
+        double F = S.f[0], Fp = S.fp[0];
+#pragma unroll
+        for (int k = 1; k < NA; ++k) { F += S.f[k]; Fp += S.fp[k]; }
+        x = (long long)S.c_out * iabs_trunc(nlog(F) - nlog(Fp));
+    }
+#pragma unroll 1
+    for (int k = 0; k < NA; ++k) {
+        const double fk = pick<NA>(S.f, k), fo = sum_others<NA>(S.f, k), fpk = pick<NA>(S.fp, k), fpo = sum_others<NA>(S.fp, k);
+        const int r1 = pick<NA>(S.r1, k);
+        for (int u = pick<NA>(S.r0, k) + lg.gl; u < r1; u += lg.G) {
+            const uint32_t p = bins[u];
+            const uint32_t q = bin_qual(p);
+            const double ome = lut[kLutOneMinusEps * kQSlots + q], e3 = lut[kLutEpsThird * kQSlots + q];
+            x += (long long)bin_count(p) * iabs_trunc(nlog(ome * fk + e3 * fo) - nlog(ome * fpk + e3 * fpo));
+        }
+    }
+    if (lg.G != 1) {
+        x += __shfl_xor_sync(lg.mask, x, 2);
+        x += __shfl_xor_sync(lg.mask, x, 1);
+    }
+    return !((double)x < eps);
+}
 template <int NA>
 __device__ __noinline__ bool em_moved_bin(const uint32_t* bins, const EmState<NA>& S, const double* lut, const LaneGroup& lg) {
+    const TaskCta& cs = *reinterpret_cast<const TaskCta*>(bv_smem_raw);
+    if (!cs.unit_eps) return em_int_sum_more<NA>(bins, S, lut, lg, cs.em_eps);
     if (S.c_out != 0.0) {   // the bins outside the subset: marginals e3 * F
         double F = S.f[0], Fp = S.fp[0];
 #pragma unroll
@@ -525,6 +570,7 @@ __device__ __forceinline__ void em_task(const SiteKernelArgs& a, const double* l
     }
     bool first = !resume;   // the E-step + M-step in front of EM()'s loop: no convergence test
     int it = a.em_max_iter;
+    // (em_max_iter 0 resumes after bv_em_iter_kernel in either mode: while (it--) runs no iteration, see bv_api.cu)
     for (;;) {   // (BV_EM_ABS_INT_TRUNC: with fabs the iterations are bv_em_iter_kernel's, and this function resumes after them)
         bool last = resume;
         if (!resume && !first) {
@@ -534,6 +580,7 @@ __device__ __forceinline__ void em_task(const SiteKernelArgs& a, const double* l
             // Every marginal is a non-negative combination of the frequencies, so its ratio between two E-steps lies between
             // the smallest and the largest ratio of the frequencies (e = 2.71828...): all of those inside (1/2.718, 2.718) =>
             // no log marginal moved by 1; all >= 2.7183 or all <= 1/2.7183 => every one did; otherwise the bins decide.
+            // That answers "sum < eps" exactly for 0 < eps <= 1 only; any other eps is compared with the sum itself.
             bool calm = true, up = true, down = true;
 #pragma unroll
             for (int k = 0; k < NA; ++k) {
@@ -541,6 +588,8 @@ __device__ __forceinline__ void em_task(const SiteKernelArgs& a, const double* l
                 up = up && f[k] >= 2.7183 * fp[k] && fp[k] > 0.0 && f[k] < 1e300;
                 down = down && fp[k] >= 2.7183 * f[k] && f[k] > 0.0 && fp[k] < 1e300;
             }
+            // (with eps outside (0, 1] the convergence sum itself decides: em_moved_bin; the flag is kept in shared memory)
+            if ((calm || up || down) && !reinterpret_cast<const TaskCta*>(bv_smem_raw)->unit_eps) calm = up = down = false;
             const bool more = calm ? false : (up || down) ? true : em_moved_bin<NA>(bins, S, lut, lg);
             last = !more || it == 1;
         }
@@ -651,9 +700,9 @@ __device__ __forceinline__ void em_iter_list(const SiteKernelArgs& a, TaskCta& c
             if (first) first = false;   // the E-step + M-step in front of EM()'s loop: no convergence test
             else {
                 --it;
-                if (it == 0) flags |= BV_FLAG_EM_MAXITER;
-                fin = (delta < a.em_eps) || it == 0;
+                fin = delta < a.em_eps;
             }
+            if (it == 0) { flags |= BV_FLAG_EM_MAXITER; fin = true; }   // (em_max_iter 0: right after that first E-step)
             if (fin) {
                 double* res = a.em_res + (size_t)t * kEmResDoubles;
 #pragma unroll
@@ -719,10 +768,11 @@ __device__ __noinline__ void decide_site(const SiteKernelArgs& a, const EmSiteHd
         double single_ll[2] = {0.0, 0.0};
         if (n == 1) {
             // Log-likelihoods of the two single-allele models (EMs whose answer is closed form; NaN when a phred-0 read of that
-            // base exists): K4a left them with the header (single_allele_ll4).
+            // base exists): K4a left them with the header (single_allele_ll4), and their flags in act_flags.
             const int b0 = __ffs(act) - 1, b1 = 31 - __clz(act);
             single_ll[0] = __ldcg(a.em_single + (size_t)hdr_index * 4 + b0);
             single_ll[1] = __ldcg(a.em_single + (size_t)hdr_index * 4 + b1);
+            if ((flags >> 8) & act) flags |= BV_FLAG_EM_MAXITER;   // (act_flags bits 16-19: both of them run in this round)
         }
         double best_chi = 0, best_lr = 0, best_f[4] = {0, 0, 0, 0};
         uint32_t best_set = 0;
@@ -826,7 +876,11 @@ __global__ void __launch_bounds__(kTaskThreads, kMinCtas) bv_em_task_kernel(cons
     const int tid = threadIdx.x, lane = tid & 31;
     for (int i = tid; i < 4 * kQSlots; i += kTaskThreads) cs.lut[i / kQSlots][i % kQSlots] = a.lut[(i / kQSlots) * kQStride + i % kQSlots];
     for (int i = tid; i < kLogTabEntries; i += kTaskThreads) cs.ltab[i] = a.logtab[i];
-    if (tid == 0) cs.n_fs = 0;
+    if (tid == 0) {
+        cs.n_fs = 0;
+        cs.em_eps = a.em_eps;
+        cs.unit_eps = a.em_eps > 0.0 && a.em_eps <= 1.0;
+    }
     grid_dep_wait();
     {
         const uint64_t n_all = (uint64_t)a.counters[kCntEmTask2] + a.counters[kCntEmTask3] + a.counters[kCntEmTask4];

@@ -15,8 +15,8 @@ namespace bv {
 //                                                                                        basetype_caller.cpp:1236-1245)
 // If exactly one allele is active and it is REF the record is final (the reference's single-column EM gives f = 1, no
 // ALT).  Otherwise the result depends on base qualities: state kStateBound when the site has the shape the bound of K3
-// can decide (REF with >= 22 reads plus one minor allele with <= 4; the minor allele's code travels in the alt word),
-// else state kStateEM.
+// can decide (REF with >= 22 reads plus one minor allele with <= 4, and lrt_threshold >= 24; the minor allele's code travels
+// in the alt word), else state kStateEM.
 // =====================================================================================================================
 // append `site` to a work list (global, or a CTA's staging list in shared memory) for the lanes with `pred`; one atomicAdd
 // per warp (all 32 lanes must call)
@@ -238,7 +238,8 @@ __device__ __forceinline__ uint32_t scalar_site(const SiteKernelArgs& a, uint32_
     uint32_t state = need_qual ? kStateEM : kStateDone;
     // the active set travels in bits 8-11 of the alt word (K4a), the minor allele of a bound site in bits 0-1 (K3)
     if (need_qual) rec[kWAlt] = act << 8;
-    if (n_act == 2 && (act & ref_bit)) {
+    // K3's proof ends in 2G < 23.9 < 24 <= lrt_threshold: below 24 its sites are the EM's
+    if (n_act == 2 && (act & ref_bit) && a.lrt_threshold >= 24.0) {
         const int o_code = __ffs(act & ~ref_bit) - 1;
         if (sel4u(ref_code, d0, d1, d2, d3) >= 22 && sel4u(o_code, d0, d1, d2, d3) <= 4) {
             state = kStateBound;
@@ -247,7 +248,8 @@ __device__ __forceinline__ uint32_t scalar_site(const SiteKernelArgs& a, uint32_
     }
     // n_active | flags | em_calls (a single active allele costs the reference one EM call)
     const uint32_t em_calls = (!need_qual && n_act == 1) ? 1u : 0u;
-    rec[kWInfo] = (n_act << 8) | (flags << 16) | (em_calls << 24);
+    const uint32_t em_flags = em_calls ? single_em_flag(sel4u(__ffs(act) - 1, d0, d1, d2, d3), total, a) : 0u;
+    rec[kWInfo] = (n_act << 8) | ((flags | em_flags) << 16) | (em_calls << 24);
     reinterpret_cast<double*>(rec)[14] = fs_cvg;
     rec[kWState] = state;
     return state;
@@ -314,6 +316,8 @@ __global__ void __launch_bounds__(256) bv_pack_kernel(const __grid_constant__ Si
 // single active allele REF, no ALT, whatever the EM would have returned.  Margins (23.9 vs 24, G rounded up in fixed
 // point) dwarf the 1e-12 rounding noise of the reference's sums.  A counted read with phred < 2 or > 93 voids the
 // argument; such a site goes to the EM kernel like the ones whose G is too large.
+// The last step, 23.9 < 24 <= lrt_threshold, needs lrt_threshold >= 24: below that K2 lists no site here and the EM decides
+// them all (a limit derived from the threshold would have to re-prove the depth[r] >= 22 condition for every threshold).
 //
 // Light kernel, high occupancy: the row's base + qual planes come through two TMA-filled buffers per warp, the next
 // unit (also the next site's first one) in flight while the current one is scanned with SIMD byte arithmetic.
@@ -780,6 +784,11 @@ __device__ __noinline__ uint32_t build_hist_long(uint32_t site) {
 // subset: bit j set => allele j in the candidate combination.  W.emf: initial frequencies in (NOT renormalised,
 // src/basetype.cpp:93-103), estimated frequencies out.  Returns the sum of log marginal likelihoods under the
 // second-to-last frequency vector, exactly what _f() sums (src/basetype.cpp:119-120).
+// INT_SUM, the build for parameters away from the defaults (em_subset): BV_EM_ABS_INT_TRUNC with an eps outside (0, 1] compares
+// EM()'s convergence sum itself, sum of count * (double)abs((int)diff) over the bins (see iabs_trunc), formed exactly in integers
+// ("did some |diff| reach 1" answers "sum < eps" only for 0 < eps <= 1), and em_max_iter 0 runs no iteration.  Those EMs always
+// take this build, so that the default build of it and em_bins_reg keep their registers.
+template <bool INT_SUM>
 __device__ __noinline__ double em_bins(const uint32_t* bins, double* lml, int nb, int subset, double total) {
     QualWarp& W = warp_smem();
     const QualCta& cs = cta_shared();
@@ -792,6 +801,7 @@ __device__ __noinline__ double em_bins(const uint32_t* bins, double* lml, int nb
     bool first = true;
     for (;;) {
         double s0 = 0, s1 = 0, s2 = 0, s3 = 0, delta = 0;
+        long long isum = 0;
         bool big = false;
 #pragma unroll 1
         for (int i = lane; i < nb; i += 32) {
@@ -812,7 +822,8 @@ __device__ __noinline__ double em_bins(const uint32_t* bins, double* lml, int nb
                 if (abs_mode == BV_EM_ABS_INT_TRUNC) {
                     // (double)abs((int)diff): non-zero iff |diff| >= 1; NaN/inf convert to INT_MIN whose
                     // "abs" stays negative and ends the loop (results are NaN by then)
-                    if (fabs(diff) >= 1.0 && fabs(diff) < 2147483648.0) big = true;
+                    if (INT_SUM) isum += (long long)bin_count(p) * iabs_trunc(diff);
+                    else if (fabs(diff) >= 1.0 && fabs(diff) < 2147483648.0) big = true;
                 } else {
                     delta += cd * fabs(diff);
                 }
@@ -828,10 +839,17 @@ __device__ __noinline__ double em_bins(const uint32_t* bins, double* lml, int nb
         if (subset & 2) f1 = warp_sum(s1) / total;
         if (subset & 4) f2 = warp_sum(s2) / total;
         if (subset & 8) f3 = warp_sum(s3) / total;
-        if (first) { first = false; continue; }
+        if (first) {
+            first = false;
+            if (!INT_SUM || it != 0) continue;
+            // em_max_iter 0: while (it--) { ... } (src/algorithm.h:234-251) runs no iteration after the first E-step + M-step
+            if (lane == 0) W.flag_word |= BV_FLAG_EM_MAXITER;
+            break;
+        }
         bool more;
-        if (abs_mode == BV_EM_ABS_INT_TRUNC) more = __any_sync(kFull, big);
-        else more = !(warp_sum(delta) < cs.a.em_eps);
+        if (abs_mode != BV_EM_ABS_INT_TRUNC) more = !(warp_sum(delta) < cs.a.em_eps);
+        else if (INT_SUM) more = !((double)warp_sum_ll(isum) < cs.a.em_eps);
+        else more = __any_sync(kFull, big);
         --it;
         if (it == 0 && lane == 0) W.flag_word |= BV_FLAG_EM_MAXITER;
         if (!more || it == 0) break;
@@ -954,9 +972,12 @@ __device__ __noinline__ double em_bins_reg(const uint32_t* bins, int nb, int sub
 
 // EM of one candidate subset: bins in registers when they fit (the usual case), else the loop over memory
 __device__ __forceinline__ double em_subset(const uint32_t* bins, double* lml, int nb, int subset, double total) {
+    const SiteKernelArgs& a = cta_shared().a;
+    if ((a.abs_mode == BV_EM_ABS_INT_TRUNC && !(a.em_eps > 0.0 && a.em_eps <= 1.0)) || a.em_max_iter == 0)
+        return em_bins<true>(bins, lml, nb, subset, total);
     if (nb <= 32) return em_bins_reg<1>(bins, nb, subset, total);
     if (nb <= 96) return em_bins_reg<3>(bins, nb, subset, total);
-    return em_bins(bins, lml, nb, subset, total);
+    return em_bins<false>(bins, lml, nb, subset, total);
 }
 
 // Log-likelihood of the single-allele model {b} (an EM whose answer is closed form):
@@ -1105,7 +1126,9 @@ __device__ __noinline__ uint32_t lrt_on_bins(int nb, uint32_t act, uint32_t orde
             double lr;
             if (n == 1) {
                 const int single = __ffs(sub) - 1;
+                flags |= single_em_flag(W.rec.depth[single], (uint32_t)dtot, cs.a);
                 lr = single_allele_ll(bins, nb, single);
+                if (cs.a.em_max_iter == 0) lr += first_estep_ll_shift(W.rec.depth[single], dtot);
                 const double v = (lr != lr) ? lr : 1.0;
                 __syncwarp();   // every lane has read W.emf above
                 if (lane < 4) W.emf[lane] = lane == single ? v : 0.0;

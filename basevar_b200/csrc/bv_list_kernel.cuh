@@ -79,6 +79,7 @@ __device__ __noinline__ void list_site(uint32_t site, uint32_t w, bv_lrt_out* __
             const double v = bad ? __longlong_as_double(0x7ff8000000000000ll) : 1.0;
             __syncwarp();
             if (lane < 4) W.res_f[lane] = lane == b ? v : 0.0;
+            if (lane == 0) W.flag_word |= single_em_flag(dep[b], total, cs.a);
             em_calls = 1;
         }
         if (qmin <= qmax) {   // histogram back to zero

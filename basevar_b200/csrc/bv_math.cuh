@@ -205,5 +205,19 @@ __device__ __noinline__ double warp_sum(double v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
+__device__ __forceinline__ long long warp_sum_ll(long long v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// One term of EM()'s convergence sum with BV_EM_ABS_INT_TRUNC, (double)abs((int)diff) (src/algorithm.h:245), as the x86-64
+// build computes it: cvttsd2si gives INT_MIN for NaN and out-of-range values, and abs(INT_MIN) stays INT_MIN.  The terms are
+// integers, so their sum is formed exactly in 64 bits, in any order (the reference's double sum of them is exact too).
+__device__ __forceinline__ long long iabs_trunc(double diff) {
+    if (!(diff > -2147483649.0 && diff < 2147483648.0)) return -2147483648ll;
+    const long long t = (long long)diff;
+    return t < 0 ? -t : t;
+}
 
 }  // namespace bv

@@ -46,12 +46,21 @@ class BaseTypeEngine:
         if rc != capi.BV_OK:
             raise BvError(f"{what} failed ({rc}): {self.lib.bv_last_error(self._ctx).decode()}")
 
-    def set_params(self, min_af=None, abs_mode=None):
+    def set_params(self, min_af=None, abs_mode=None, lrt_threshold=None, em_max_iter=None, em_eps=None):
+        """Change the statistics' parameters; those left at None keep their values.  A refused set changes nothing."""
+        p = capi.BvParams.from_buffer_copy(self.params)
         if min_af is not None:
-            self.params.min_af = float(np.float32(min_af))
+            p.min_af = float(np.float32(min_af))
         if abs_mode is not None:
-            self.params.em_abs_mode = abs_mode
-        self._check(self.lib.bv_set_params(self._ctx, C.byref(self.params)), "bv_set_params")
+            p.em_abs_mode = abs_mode
+        if lrt_threshold is not None:
+            p.lrt_threshold = lrt_threshold
+        if em_max_iter is not None:
+            p.em_max_iter = em_max_iter
+        if em_eps is not None:
+            p.em_eps = float(np.float32(em_eps))
+        self._check(self.lib.bv_set_params(self._ctx, C.byref(p)), "bv_set_params")
+        self.params = p
 
     def suggest_tile_sites(self, n_samples, max_bytes):
         """Largest tile (sites) that fits max_bytes of planes and that the count kernel's persistent warps split evenly."""

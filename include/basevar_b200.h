@@ -87,7 +87,11 @@ extern "C" {
 #define BV_FLAG_NEAR_LRT     0x10u /* some LRT decision had |chi2 - threshold| < 1e-9*threshold (possible flip) */
 #define BV_FLAG_LRT_BOUND    0x20u /* the LRT outcome (drop the minor allele) was proven by a bound, no EM ran:   */
                                    /* chi2 and em_calls of the record are 0 (the reference exposes neither here)  */
-#define BV_FLAG_EM_MAXITER   0x40u /* an EM used all em_max_iter iterations                                   */
+                                   /* and no EM flag is raised (the reference's EMs at em_max_iter <= 1 or       */
+                                   /* em_eps <= 0 would raise BV_FLAG_EM_MAXITER)                                 */
+#define BV_FLAG_EM_MAXITER   0x40u /* an EM used all em_max_iter iterations.  Not raised for the EM of a single   */
+                                   /* active allele with a phred-0 read of that allele: its marginals are NaN and */
+                                   /* the reference's loop count then differs (in fabs mode it always runs them all) */
 #define BV_FLAG_LRT_TIE      0x80u /* two candidate subsets had equal chi2 (to rounding): first one kept       */
 
 #define BV_EM_ABS_INT_TRUNC 0  /* as built by g++/glibc: abs() resolves to int abs(int) (algorithm.h:245)   */
@@ -99,11 +103,12 @@ extern "C" {
 /* ---- parameters ------------------------------------------------------------------------------- */
 typedef struct bv_params {
     float    min_af;         /* CLI --min-af as FLOAT (basetype_utils.h:80), widened to double inside;    */
-                             /* caller applies min(100.0f/n_bam, min_af) (basetype_caller.cpp:122)        */
-    int32_t  lrt_threshold;  /* 24  (basetype.h:21)                                                       */
-    int32_t  em_max_iter;    /* 100 (algorithm.h:213)                                                     */
-    float    em_eps;         /* 0.001f (algorithm.h:213)                                                  */
-    int32_t  em_abs_mode;    /* BV_EM_ABS_*                                                               */
+                             /* caller applies min(100.0f/n_bam, min_af) (basetype_caller.cpp:122);      */
+                             /* finite and > 0, else BV_ERR_ARG                                           */
+    int32_t  lrt_threshold;  /* 24  (basetype.h:21); any value                                            */
+    int32_t  em_max_iter;    /* 100 (algorithm.h:213); >= 0, else BV_ERR_ARG (0: no iteration)            */
+    float    em_eps;         /* 0.001f (algorithm.h:213); any value but NaN (BV_ERR_ARG)                  */
+    int32_t  em_abs_mode;    /* BV_EM_ABS_*; any other value: BV_ERR_ARG                                  */
     uint32_t max_samples;    /* capacity: largest n_samples of any tile                                   */
     uint32_t max_sites;      /* capacity: largest n_sites of any tile submitted through a slot            */
     uint32_t n_slots;        /* in-flight tile slots (each owns a stream + pinned staging); >= 1          */
@@ -243,7 +248,7 @@ int         bv_version(void);                                  /* major*1000 + m
 int         bv_create(int device, const bv_params* params, bv_ctx** out_ctx);
 void        bv_destroy(bv_ctx* ctx);
 const char* bv_last_error(const bv_ctx* ctx);                  /* ctx may be NULL: last global error */
-int         bv_set_params(bv_ctx* ctx, const bv_params* params); /* change min_af / em mode; capacities fixed */
+int         bv_set_params(bv_ctx* ctx, const bv_params* params); /* change min_af / LRT / EM parameters; capacities fixed; refused (BV_ERR_ARG): nothing changes */
 uint64_t    bv_launch_count(const bv_ctx* ctx);                /* kernels launched by this context so far */
 uint64_t    bv_h2d_bytes(const bv_ctx* ctx);                   /* bytes uploaded by the bv_tile_submit* calls so far: the planes
                                                                   or cells of host tiles, and the lists of lists tiles */

@@ -53,8 +53,8 @@ class BvParams(C.Structure):
     ]
 
 
-def make_params(min_af=0.01, abs_mode=0, max_samples=0, max_sites=0, n_slots=1):
-    return BvParams(float(np.float32(min_af)), 24, 100, float(np.float32(0.001)), abs_mode, max_samples,
+def make_params(min_af=0.01, abs_mode=0, max_samples=0, max_sites=0, n_slots=1, lrt_threshold=24, em_max_iter=100, em_eps=0.001):
+    return BvParams(float(np.float32(min_af)), lrt_threshold, em_max_iter, float(np.float32(em_eps)), abs_mode, max_samples,
                     max_sites, n_slots, 0)
 
 
@@ -107,12 +107,12 @@ def load_oracle():
     return _oracle
 
 
-def oracle_tile(base, qual, strand, ref_base, n_samples, min_af=0.01, abs_mode=0):
+def oracle_tile(base, qual, strand, ref_base, n_samples, min_af=0.01, abs_mode=0, lrt_threshold=24, em_max_iter=100, em_eps=0.001):
     """Run the C restatement over planes [S][pitch] (uint8).  Returns a SITE_OUT_DTYPE array."""
     lib = load_oracle()
     S, pitch = base.shape
     out = np.zeros(S, dtype=SITE_OUT_DTYPE)
-    prm = make_params(min_af, abs_mode)
+    prm = make_params(min_af, abs_mode, lrt_threshold=lrt_threshold, em_max_iter=em_max_iter, em_eps=em_eps)
     rc = lib.bvo_tile(_u8p(base), _u8p(qual), _u8p(strand), _u8p(ref_base), pitch, S, n_samples, C.byref(prm),
                       out.ctypes.data)
     assert rc == 0
@@ -139,7 +139,7 @@ def _group_order(ref_char, rec):
 
 
 def oracle_calls(base, qual, mapq, rpr, ref_base, n_samples, recs, sample_group=None, n_groups=0, min_af=0.01, abs_mode=0,
-                 use_ref=False):
+                 use_ref=False, lrt_threshold=24, em_max_iter=100, em_eps=0.001):
     """Rank sums and population-group calls of the called sites (recs: SITE_OUT_DTYPE of the same planes), from the C
     restatement or (use_ref) from the compiled reference.  Returns (calls sorted by site, groups[n_calls][n_groups])."""
     lib = load_ref(bool(abs_mode)) if use_ref else load_oracle()
@@ -147,7 +147,9 @@ def oracle_calls(base, qual, mapq, rpr, ref_base, n_samples, recs, sample_group=
     sites = np.nonzero(recs["n_alt"] > 0)[0]
     calls = np.zeros(len(sites), CALL_OUT_DTYPE)
     groups = np.zeros((len(sites), max(n_groups, 0)), GROUP_OUT_DTYPE)
-    prm = make_params(min_af, abs_mode)
+    # (the compiled reference has its parameters built in: it runs at the defaults only)
+    assert not use_ref or (lrt_threshold, em_max_iter, em_eps) == (24, 100, 0.001)
+    prm = make_params(min_af, abs_mode, lrt_threshold=lrt_threshold, em_max_iter=em_max_iter, em_eps=em_eps)
     u16p = C.POINTER(C.c_uint16)
     rpr = np.ascontiguousarray(rpr, np.uint16)
     for k, s in enumerate(sites):

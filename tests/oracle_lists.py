@@ -59,13 +59,14 @@ def _u8p(a):
     return a.ctypes.data_as(C.POINTER(C.c_uint8))
 
 
-def oracle_lists(base, qual, strand, ref_base, lists, n_samples, min_af=0.01, abs_mode=0):
+def oracle_lists(base, qual, strand, ref_base, lists, n_samples, min_af=0.01, abs_mode=0, lrt_threshold=24, em_max_iter=100,
+                 em_eps=0.001):
     """BaseType(row, min_af) + lrt(list) per site.  lists: uint8 [S][4], ended early by LIST_END.
     Returns a LRT_OUT_DTYPE array; a site whose list is invalid raises AssertionError."""
     lib = load()
     S = base.shape[0]
     out = np.zeros(S, LRT_OUT_DTYPE)
-    prm = L.make_params(min_af, abs_mode)
+    prm = L.make_params(min_af, abs_mode, lrt_threshold=lrt_threshold, em_max_iter=em_max_iter, em_eps=em_eps)
     for s in range(S):
         lst = np.ascontiguousarray(lists[s], np.uint8)
         n = int(np.argmax(lst == LIST_END)) if (lst == LIST_END).any() else 4
