@@ -268,8 +268,9 @@ struct LaneGroup {
 __device__ __forceinline__ double sum4(const double (&p)[4]) { return (p[0] + p[2]) + (p[1] + p[3]); }
 
 // log(r) for the ratio of two marginals of consecutive E-steps: once the EM settles r is within 2^-10 of 1 for every bin,
-// and t - t^2/2 + t^3/3 - t^4/4 (t = r - 1, exact) is then good to 2e-16 of t -- below the rounding of a full logarithm,
-// which costs ten times as many instructions.  The sum these terms go into is only compared with 0.001.
+// and t - t^2/2 + t^3/3 - t^4/4 (t = r - 1, exact) is then good to |t|^5 / 5 + 1 ulp of t: 1.8e-16 absolute (1.8e-13 of t) at
+// |t| = 2^-10, the size of the rounding of the reference's own log m - log mp wherever |log m| is of order 1 -- at a tenth of the
+// instructions of a full logarithm.  The sum these terms go into is only compared with 0.001.
 __device__ __forceinline__ double log_ratio(double r) {
     const double t = r - 1.0;
     if (fabs(t) < 0.0009765625) return t * fma(t, fma(t, fma(t, -0.25, 1.0 / 3.0), -0.5), 1.0);

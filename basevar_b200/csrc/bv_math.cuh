@@ -22,7 +22,12 @@ namespace bv {
 // ~6600 SASS instructions).  libdevice log/exp/log10 are 40-90 instructions each and get inlined at every call
 // site, so the rarely executed numerics (QUAL, Fisher) call them through these out-of-line wrappers.
 __device__ __noinline__ double nlog(double x) { return log(x); }
-__device__ __noinline__ double nexp(double x) { return exp(x); }
+// Below log(DBL_MIN) libdevice's exp returns 0 for x < -745.0 or so, where glibc rounds to the denormal grid down to x = -745.133
+// (the smallest denormal): a QUAL of 10000 instead of 3233.07 for chi2 in [1482.25, 1482.51] (tests/test_gpu_numerics.py).  There
+// exp(x + 40) * exp(-40) is exact to a few ulp of a normal value, far below the one step of the denormal grid it is rounded to.
+__device__ __noinline__ double nexp(double x) {
+    return x < -708.39641853226410622 ? exp(x + 40.0) * 4.248354255291589e-18 : exp(x);
+}
 __device__ __noinline__ double nlog10(double x) { return log10(x); }
 
 // ---- kf_lgamma (AS245), kfunc.c:39-52 ------------------------------------------------------------
@@ -154,7 +159,8 @@ __device__ __noinline__ double fisher_two_sided(const double* __restrict__ lf, i
     if (side != kFisherLeft) {
         // The right walk starts from the observed table again, not from where the left walk stopped (the reference carries its
         // state over, which matters only when the left walk ends next to hi: an incremental step from there instead of a direct
-        // evaluation, 1e-15 relative).  So the two tails share nothing and a lane pair forms the same value as one thread.
+        // evaluation, i.e. the rounding of exp() of lgamma differences, up to ~12 ulp of lgamma(n + 1) relative: 1.3e-10 measured at
+        // n = 100,001).  So the two tails share nothing and a lane pair forms the same value as one thread.
         st.n11 = n11; st.p = q;
         p = hg_move(lf, st, hi);
         for (j = hi - 1; p < 0.99999999 * q && j >= 0; --j) {
