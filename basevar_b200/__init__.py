@@ -5,7 +5,7 @@ this package is its thin Python host layer (ctypes).  There is no CPU fallback a
 """
 from . import capi, synth  # noqa: F401
 from .capi import BvError, SITE_OUT_DTYPE, cli_min_af  # noqa: F401
-from .engine import (BaseTypeEngine, dense_to_sparse, sparse_encode16, synth_fill_host, synth_fill_rpr_host,  # noqa: F401
-                     synth_fill_sparse_host)
+from .engine import (BaseTypeEngine, DeviceResult, dense_to_sparse, device_to_numpy, sparse_encode16, synth_fill_host,  # noqa: F401
+                     synth_fill_rpr_host, synth_fill_sparse_host)
 
 __version__ = "0.1.0"

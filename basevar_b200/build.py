@@ -18,6 +18,7 @@ DEPS = SOURCES + [os.path.join(CSRC, f) for f in ("bv_common.cuh", "bv_count_ker
                                                   "bv_fisher_fast.h", "bv_synth.cuh")] + [
     os.path.join(HERE, "..", "include", "basevar_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+CUDA_HOME = os.path.dirname(os.path.dirname(os.path.realpath(NVCC)))
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
@@ -48,7 +49,10 @@ CLI = os.path.join(HERE, "bin", "basevar")   # `basevar basetype ...` over BAM f
 ROOT = os.path.dirname(HERE)
 CPP_TESTS = {"test_host_cpu": [], "test_host_gpu": ["-ldl"], "test_fisher_fast": ["-ldl", "-lm"], "test_caller_cpu": [],
              "test_caller_gpu": ["-lz"], "pileup_dump": ["-lz"], "test_lists_gpu": ["-ldl", "-lm"],
-             "test_ranksum_gpu": ["-ldl", "-lm"], "test_vcf_row_gpu": ["-ldl", "-lm"]}
+             "test_ranksum_gpu": ["-ldl", "-lm"], "test_vcf_row_gpu": ["-ldl", "-lm"],
+             # (allocates the device buffers of Context::run_device with the CUDA runtime; the host layer itself has no CUDA)
+             "test_device_gpu": ["-I" + os.path.join(CUDA_HOME, "include"), "-L" + os.path.join(CUDA_HOME, "lib64"), "-lcudart",
+                                 "-Wl,-rpath," + os.path.join(CUDA_HOME, "lib64")]}
 
 
 # What the programs linked against the host layer compile in: they are linked again when their source or one of these changes.

@@ -105,6 +105,26 @@ class BvSparseTile(C.Structure):
 CELLS_U32, CELLS_U16 = 0, 1
 OUT_RECORDS, OUT_COMPACT = 0, 1
 SITE_BRIEF_DTYPE = np.dtype([("w0", "<u4"), ("w1", "<u4")])   # struct bv_site_brief
+RUN_PLAIN, RUN_CALLS, RUN_LISTS = 0, 1, 2
+
+
+class BvDeviceOut(C.Structure):
+    """struct bv_device_out: the device buffers of a device-resident tile's results (bv_tile_run_device_ex / _sparse)."""
+    _fields_ = [
+        ("kind", C.c_int32),
+        ("out_mode", C.c_int32),
+        ("d_out", C.c_void_p),
+        ("d_brief", C.c_void_p),
+        ("d_full", C.c_void_p),
+        ("d_n_full", C.c_void_p),
+        ("d_calls", C.c_void_p),
+        ("d_groups", C.c_void_p),
+        ("d_n_calls", C.c_void_p),
+        ("d_lists", C.c_void_p),
+        ("d_lrt", C.c_void_p),
+        ("d_n_lrt", C.c_void_p),
+        ("d_status", C.c_void_p),
+    ]
 
 
 def cell_pack(sample, base, strand, phred):
@@ -171,6 +191,8 @@ _SIGNATURES = [
     ("bv_tile_submit_sparse_lists", C.c_int, [C.c_void_p, C.c_int, C.POINTER(BvSparseTile), C.c_void_p]),
     ("bv_tile_wait_lists_compact", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_uint32),
                                              C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
+    ("bv_tile_run_device_sparse", C.c_int, [C.c_void_p, C.POINTER(BvSparseTile), C.POINTER(BvDeviceOut), C.c_void_p]),
+    ("bv_tile_run_device_ex", C.c_int, [C.c_void_p, C.POINTER(BvTile), C.POINTER(BvTileAux), C.POINTER(BvDeviceOut), C.c_void_p]),
     ("bv_sparse_encode16_bound", C.c_uint64, [C.c_uint64, C.c_uint32, C.c_uint32]),
     ("bv_sparse_encode16", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
                                      C.POINTER(C.c_uint64)]),

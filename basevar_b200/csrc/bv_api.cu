@@ -196,6 +196,7 @@ struct bv_ctx {
     bool ev_list_valid = false;
     bool list_kernel_ready = false;   // bv_list_kernel's shared-memory attribute is set (first lists tile)
     bool list_packed_ready = false;   // the same for bv_list_packed_kernel (first sparse lists tile with compact results)
+    bool list_packed_dev_ready = false;   // ... and for bv_list_packed_dev_kernel (first device-resident one)
     // free-standing rank-sum tests (bv_ranksum_test): stream and device scratch made on first use, grown only
     cudaStream_t rs_stream = nullptr;
     uint8_t* d_rs_bases = nullptr;    // [rs_entries_cap]
@@ -212,6 +213,15 @@ struct bv_ctx {
     cudaEvent_t ev_trace0 = nullptr;  // recorded at the first traced submit: the origin of the timeline
     uint64_t tiles_traced = 0;
     double t_trace0 = 0;
+    // device-resident tiles with results of any form (bv_tile_run_device_ex / _sparse): allocated on first use, grown only
+    uint8_t* d_dev_planes = nullptr;      // base | qual | strand planes K0 writes, each max_sites * pitch_cap
+    uint8_t* d_dev_aux = nullptr;         // mapq | rpr planes K0 writes for the called-site kernels, 3 * max_sites * pitch_cap
+    bv_site_out* d_dev_rec = nullptr;     // [dev_rec_cap] records of a compact tile, before K7 packs those that travel
+    uint32_t dev_rec_cap = 0;
+    uint2* d_dev_pairs = nullptr;         // [dev_pairs_cap] packed list of a compact lists tile (bv_list_pairs_kernel)
+    unsigned long long* d_dev_chunks = nullptr;   // its per-chunk counts, tagged with pair_epoch
+    uint32_t dev_pairs_cap = 0;
+    uint32_t pair_epoch = 0;              // tag of the last call's chunk counts (0: the buffer's initial zeros)
 };
 
 static char g_err[512] = "";
@@ -360,8 +370,9 @@ static int set_call_args(bv_ctx* ctx, const bv_tile* t, const bv_tile_aux* aux, 
 //     it ran 8 us longer than it does behind a drained K1.
 // Profiled tiles launch every kernel without the attribute, with the events between them: per-kernel times of a
 // serialised chain, comparable over the history of the project.
-static cudaError_t launch_chained(bool pdl, void (*kernel)(bv::SiteKernelArgs), uint32_t grid, uint32_t block, size_t smem,
-                                  cudaStream_t stream, const bv::SiteKernelArgs& a) {
+template <typename... Args>
+static cudaError_t launch_chained(bool pdl, void (*kernel)(Args...), uint32_t grid, uint32_t block, size_t smem,
+                                  cudaStream_t stream, const Args&... a) {
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -372,7 +383,7 @@ static cudaError_t launch_chained(bool pdl, void (*kernel)(bv::SiteKernelArgs), 
     cfg.stream = stream;
     cfg.attrs = attr;
     cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, a);
+    return cudaLaunchKernelEx(&cfg, kernel, a...);
 }
 
 // The basetype core of one tile: K1 (counts, every cell), K2 (scalar finish, one thread per site), K3 / K4 (sites whose
@@ -474,9 +485,10 @@ static int launch_site_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, cudaStre
 
 // K8 after the standard kernels of the tile (it reads their records), one warp per listed site: over the n = n_sites words of
 // d_lists (bv_list_kernel), or over the n {site, list word} pairs of a compact tile's packed list, entry k for pair k
-// (bv_list_packed_kernel, d_pairs).
+// (bv_list_packed_kernel, d_pairs).  d_n_pairs: the number of pairs is in device memory and n only bounds it
+// (bv_list_packed_dev_kernel).
 static int launch_list_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const uint32_t* d_lists, const uint2* d_pairs, uint32_t n,
-                              bv_lrt_out* d_lrt, cudaStream_t stream) {
+                              bv_lrt_out* d_lrt, cudaStream_t stream, const uint32_t* d_n_pairs = nullptr) {
     BvRange range(d_pairs ? "bv: launch K8 list (packed)" : "bv: launch K8 list");
     if (n == 0) return BV_OK;
     if (a.n_samples == 0) {   // no reads anywhere: every entry is all-zero
@@ -484,17 +496,19 @@ static int launch_list_kernel(bv_ctx* ctx, const bv::SiteKernelArgs& a, const ui
         return BV_OK;
     }
     // on first use: a context that never runs K8 loads and sets up exactly what it did without it
-    bool& ready = d_pairs ? ctx->list_packed_ready : ctx->list_kernel_ready;
+    bool& ready = d_n_pairs ? ctx->list_packed_dev_ready : d_pairs ? ctx->list_packed_ready : ctx->list_kernel_ready;
     if (!ready) {
-        BV_CUDA(ctx, cudaFuncSetAttribute(d_pairs ? (const void*)bv::bv_list_packed_kernel : (const void*)bv::bv_list_kernel,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
+        const void* k = d_n_pairs ? (const void*)bv::bv_list_packed_dev_kernel
+                                  : d_pairs ? (const void*)bv::bv_list_packed_kernel : (const void*)bv::bv_list_kernel;
+        BV_CUDA(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bv::kQualSmemBytes));
         ready = true;
     }
     const bool prof = ctx->profiling;
     if (prof) BV_CUDA(ctx, cudaEventRecord(ctx->ev_list[0], stream));
     uint32_t grid = (n + bv::kQualWarps - 1) / bv::kQualWarps;
     if (grid > (uint32_t)ctx->num_sms) grid = (uint32_t)ctx->num_sms;   // (the bin spill rows are sized for this grid)
-    if (d_pairs) bv::bv_list_packed_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_pairs, n, d_lrt);
+    if (d_n_pairs) bv::bv_list_packed_dev_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_pairs, d_n_pairs, d_lrt);
+    else if (d_pairs) bv::bv_list_packed_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_pairs, n, d_lrt);
     else bv::bv_list_kernel<<<grid, bv::kQualWarps * 32, bv::kQualSmemBytes, stream>>>(a, d_lists, d_lrt);
     BV_CUDA(ctx, cudaGetLastError());
     ctx->launches += 1;
@@ -813,6 +827,7 @@ void bv_destroy(bv_ctx* ctx) {
     }
     cudaFree(ctx->d_lut); cudaFree(ctx->d_logfact); cudaFree(ctx->d_model); cudaFree(ctx->d_group);
     scratch_free(ctx->dev_scratch);
+    cudaFree(ctx->d_dev_planes); cudaFree(ctx->d_dev_aux); cudaFree(ctx->d_dev_rec); cudaFree(ctx->d_dev_pairs); cudaFree(ctx->d_dev_chunks);
     for (int i = 0; i < 7; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 3; ++i) if (ctx->ev_call[i]) cudaEventDestroy(ctx->ev_call[i]);
     for (int i = 0; i < 2; ++i) if (ctx->ev_list[i]) cudaEventDestroy(ctx->ev_list[i]);
@@ -1018,6 +1033,18 @@ static int upload_dense(bv_ctx* ctx, bv_slot& s, const bv_tile* tile, const bv_t
     return rc;
 }
 
+// K0: the cells of a sparse tile (in device memory) -> the dense planes of x.
+static int launch_expand(bv_ctx* ctx, const bv::ExpandArgs& x, bool u16, cudaStream_t stream) {
+    uint32_t grid = (x.n_sites + bv::kExpandWarps - 1) / bv::kExpandWarps;
+    const uint32_t cap = (uint32_t)ctx->num_sms * 2u;   // persistent: 2 CTAs of 16 warps per SM (96 KB of staging each)
+    if (grid > cap) grid = cap;
+    if (u16) bv::bv_expand_kernel<BV_CELLS_U16><<<grid, bv::kExpandWarps * 32, bv::kExpandSmemBytes, stream>>>(x);
+    else bv::bv_expand_kernel<BV_CELLS_U32><<<grid, bv::kExpandWarps * 32, bv::kExpandSmemBytes, stream>>>(x);
+    BV_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    return BV_OK;
+}
+
 // Sparse host tile: upload the covered cells (4 or 2 bytes each) and expand them into the slot's dense planes (K0).  The qual
 // plane -- and for the called-site kernels the mapq / rpr planes -- are device resident here (there is no host plane to read in
 // place).  Fills `a` and s.h2d_bytes; trace: records the first two events of the tile's timeline.
@@ -1085,13 +1112,7 @@ static int upload_sparse(bv_ctx* ctx, bv_slot& s, const bv_sparse_tile* t, bool 
         x.rpr = with_calls ? reinterpret_cast<uint16_t*>(s.d_aux + plane) : nullptr;
         x.counters = a->counters;
         x.pitch = dp; x.rpr_pitch = dp; x.n_cells = n_cells; x.n_sites = t->n_sites; x.n_samples = t->n_samples;
-        uint32_t grid = (t->n_sites + bv::kExpandWarps - 1) / bv::kExpandWarps;
-        const uint32_t cap = (uint32_t)ctx->num_sms * 2u;   // persistent: 2 CTAs of 16 warps per SM (96 KB of staging each)
-        if (grid > cap) grid = cap;
-        if (u16) bv::bv_expand_kernel<BV_CELLS_U16><<<grid, bv::kExpandWarps * 32, bv::kExpandSmemBytes, s.stream>>>(x);
-        else bv::bv_expand_kernel<BV_CELLS_U32><<<grid, bv::kExpandWarps * 32, bv::kExpandSmemBytes, s.stream>>>(x);
-        BV_CUDA(ctx, cudaGetLastError());
-        ctx->launches += 1;
+        return launch_expand(ctx, x, u16, s.stream);
     }
     return BV_OK;
 }
@@ -1226,6 +1247,235 @@ int bv_tile_submit_sparse_lists(bv_ctx* ctx, int slot, const bv_sparse_tile* til
     if (tile && tile->n_sites && !lists) return set_err(ctx, BV_ERR_ARG, "bv_tile_submit_sparse_lists: null lists");
     static const uint8_t no_lists[1][4] = {{BV_LIST_END, BV_LIST_END, BV_LIST_END, BV_LIST_END}};   // (an empty tile may pass NULL)
     return tile_submit_sparse(ctx, slot, tile, false, lists ? lists : no_lists);
+}
+
+// ======================================================================================================
+// Device-resident tiles with results of every form (bv_device_out): bv_tile_run_device_ex / bv_tile_run_device_sparse
+// ======================================================================================================
+// Memory of the context's device (cudaMalloc or managed), aligned to `align` bytes; else the error (BV_ERR_ARG) is set.
+static int check_device_ptr(bv_ctx* ctx, const void* p, size_t align, const char* what) {
+    if (!p) return set_err(ctx, BV_ERR_ARG, "%s: null pointer", what);
+    if ((uintptr_t)p % align) return set_err(ctx, BV_ERR_ARG, "%s: must be %zu-byte aligned", what, align);
+    cudaPointerAttributes at;
+    const cudaError_t e = cudaPointerGetAttributes(&at, p);
+    cudaGetLastError();
+    if (e != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != ctx->device)
+        return set_err(ctx, BV_ERR_ARG, "%s: not memory of device %d (host memory is refused here)", what, ctx->device);
+    return BV_OK;
+}
+
+// The buffers `o` must name for a tile of n_sites sites.
+static int check_device_out(bv_ctx* ctx, const bv_device_out* o, uint32_t n_sites) {
+    if (!o) return set_err(ctx, BV_ERR_ARG, "null bv_device_out");
+    if (o->kind != BV_RUN_PLAIN && o->kind != BV_RUN_CALLS && o->kind != BV_RUN_LISTS)
+        return set_err(ctx, BV_ERR_ARG, "bv_device_out: unknown kind %d", o->kind);
+    if (o->out_mode != BV_OUT_RECORDS && o->out_mode != BV_OUT_COMPACT)
+        return set_err(ctx, BV_ERR_ARG, "bv_device_out: unknown out_mode %d", o->out_mode);
+    const bool compact = o->out_mode == BV_OUT_COMPACT;
+    int rc = BV_OK;
+    if (o->d_status) rc = check_device_ptr(ctx, o->d_status, 4, "bv_device_out::d_status");
+    if (rc == BV_OK && compact) rc = check_device_ptr(ctx, o->d_n_full, 4, "bv_device_out::d_n_full");
+    if (rc == BV_OK && o->kind == BV_RUN_CALLS) rc = check_device_ptr(ctx, o->d_n_calls, 4, "bv_device_out::d_n_calls");
+    if (rc == BV_OK && o->kind == BV_RUN_LISTS && compact) rc = check_device_ptr(ctx, o->d_n_lrt, 4, "bv_device_out::d_n_lrt");
+    if (rc != BV_OK || n_sites == 0) return rc;
+    if (compact) {
+        rc = check_device_ptr(ctx, o->d_brief, 8, "bv_device_out::d_brief");
+        if (rc == BV_OK) rc = check_device_ptr(ctx, o->d_full, 16, "bv_device_out::d_full");
+    } else {
+        rc = check_device_ptr(ctx, o->d_out, 16, "bv_device_out::d_out");
+    }
+    if (rc == BV_OK && o->kind == BV_RUN_CALLS) {
+        rc = check_device_ptr(ctx, o->d_calls, 16, "bv_device_out::d_calls");
+        if (rc == BV_OK && ctx->n_groups) rc = check_device_ptr(ctx, o->d_groups, 8, "bv_device_out::d_groups");
+    }
+    if (rc == BV_OK && o->kind == BV_RUN_LISTS) {
+        rc = check_device_ptr(ctx, o->d_lists, 4, "bv_device_out::d_lists");
+        if (rc == BV_OK) rc = check_device_ptr(ctx, o->d_lrt, 16, "bv_device_out::d_lrt");
+    }
+    return rc;
+}
+
+// The counts of an empty tile: every one 0.
+static int zero_device_counts(bv_ctx* ctx, const bv_device_out* o, cudaStream_t st) {
+    uint32_t* const words[4] = {o->d_status, o->out_mode == BV_OUT_COMPACT ? o->d_n_full : nullptr,
+                                o->kind == BV_RUN_CALLS ? o->d_n_calls : nullptr,
+                                o->kind == BV_RUN_LISTS && o->out_mode == BV_OUT_COMPACT ? o->d_n_lrt : nullptr};
+    for (uint32_t* w : words)
+        if (w) BV_CUDA(ctx, cudaMemsetAsync(w, 0, sizeof(uint32_t), st));
+    return BV_OK;
+}
+
+// Where K1..KF write the tile's records: the caller's d_out, or for compact results the context's record buffer, from which K7
+// copies the records that travel into d_full.  Called once the tile has been checked (n_sites <= 2^22).
+static int device_records(bv_ctx* ctx, const bv_device_out* o, uint32_t n_sites, bv_site_out** rec) {
+    if (o->out_mode != BV_OUT_COMPACT) { *rec = o->d_out; return BV_OK; }
+    if (n_sites > ctx->dev_rec_cap) {
+        cudaFree(ctx->d_dev_rec);
+        ctx->d_dev_rec = nullptr; ctx->dev_rec_cap = 0;
+        BV_CUDA(ctx, cudaMalloc(&ctx->d_dev_rec, (size_t)n_sites * sizeof(bv_site_out)));
+        ctx->dev_rec_cap = n_sites;
+    }
+    *rec = ctx->d_dev_rec;
+    return BV_OK;
+}
+
+// Everything after K0 of a device-resident tile of n_sites > 0 sites, on `st`, the scratch counters already zeroed: K1..KF (+ K5 /
+// K6), for lists K8 (per site, or over the packed list bv_list_pairs_kernel builds), for compact results K7 into d_full, and the
+// counts the caller reads from device memory.
+static int run_device_tail(bv_ctx* ctx, bv::SiteKernelArgs& a, const bv_device_out* o, cudaStream_t st) {
+    const bool compact = o->out_mode == BV_OUT_COMPACT;
+    if (compact) { a.brief = reinterpret_cast<uint2*>(o->d_brief); a.full_out = o->d_full; }
+    int rc = launch_site_kernel(ctx, a, st, true);
+    if (rc != BV_OK) return rc;
+    const uint32_t n_sites = a.n_sites;
+    if (o->kind == BV_RUN_LISTS) {
+        const uint32_t* lists = reinterpret_cast<const uint32_t*>(o->d_lists);
+        if (!compact) {
+            rc = launch_list_kernel(ctx, a, lists, nullptr, n_sites, o->d_lrt, st);
+        } else {
+            if (n_sites > ctx->dev_pairs_cap) {
+                cudaFree(ctx->d_dev_pairs); cudaFree(ctx->d_dev_chunks);
+                ctx->d_dev_pairs = nullptr; ctx->d_dev_chunks = nullptr; ctx->dev_pairs_cap = 0;
+                const size_t chunks = (n_sites + bv::kListPairSites - 1) / bv::kListPairSites;
+                BV_CUDA(ctx, cudaMalloc(&ctx->d_dev_pairs, (size_t)n_sites * sizeof(uint2)));
+                BV_CUDA(ctx, cudaMalloc(&ctx->d_dev_chunks, chunks * sizeof(unsigned long long)));
+                BV_CUDA(ctx, cudaMemsetAsync(ctx->d_dev_chunks, 0, chunks * sizeof(unsigned long long), st));
+                ctx->dev_pairs_cap = n_sites;
+                ctx->pair_epoch = 0;
+            }
+            if (++ctx->pair_epoch == 0) {   // (after 2^32 - 1 calls: the tags start again from a clean buffer)
+                const size_t chunks = (ctx->dev_pairs_cap + bv::kListPairSites - 1) / bv::kListPairSites;
+                BV_CUDA(ctx, cudaMemsetAsync(ctx->d_dev_chunks, 0, chunks * sizeof(unsigned long long), st));
+                ctx->pair_epoch = 1;
+            }
+            // chained behind KF like the step's kernels (a profiled tile keeps the launches serialised)
+            const uint32_t grid = (n_sites + bv::kListPairSites - 1) / bv::kListPairSites;
+            uint32_t* counters = a.counters;
+            uint2* pairs = ctx->d_dev_pairs;
+            unsigned long long* chunk_count = ctx->d_dev_chunks;
+            uint32_t* n_pairs = o->d_n_lrt;
+            const uint32_t epoch = ctx->pair_epoch;
+            BV_CUDA(ctx, launch_chained(!ctx->profiling, bv::bv_list_pairs_kernel, grid, (uint32_t)bv::kListPairThreads, (size_t)0, st,
+                                        lists, n_sites, pairs, chunk_count, epoch, counters, n_pairs));
+            ctx->launches += 1;
+            rc = launch_list_kernel(ctx, a, nullptr, ctx->d_dev_pairs, n_sites, o->d_lrt, st, o->d_n_lrt);
+        }
+        if (rc != BV_OK) return rc;
+    }
+    if (compact) {
+        if (a.n_samples) {
+            uint32_t grid = (n_sites + 255) / 256;
+            if (grid > (uint32_t)ctx->num_sms * 8u) grid = (uint32_t)ctx->num_sms * 8u;
+            bv::bv_pack_kernel<<<grid, 256, 0, st>>>(a);
+            BV_CUDA(ctx, cudaGetLastError());
+            ctx->launches += 1;
+        }
+        BV_CUDA(ctx, cudaMemcpyAsync(o->d_n_full, a.counters + bv::kCntFull, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+    }
+    if (o->kind == BV_RUN_CALLS)
+        BV_CUDA(ctx, cudaMemcpyAsync(o->d_n_calls, a.counters + bv::kCntCalled, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+    if (o->d_status)
+        BV_CUDA(ctx, cudaMemcpyAsync(o->d_status, a.counters + bv::kCntBadCell, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+    return BV_OK;
+}
+
+int bv_tile_run_device_ex(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux* aux, const bv_device_out* o, void* stream) {
+    BvRange range("bv_tile_run_device_ex");
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (!tile) return set_err(ctx, BV_ERR_ARG, "null tile");
+    if (tile->location != BV_LOC_DEVICE) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_ex: tile must be device resident");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = check_device_out(ctx, o, tile->n_sites);
+    if (rc != BV_OK) return rc;
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (tile->n_sites) {
+        const void* planes[4] = {tile->base, tile->qual, tile->strand, tile->ref_base};
+        for (int k = 0; k < 4 && rc == BV_OK; ++k) rc = check_device_ptr(ctx, planes[k], k < 3 ? 16 : 1, "bv_tile plane");
+        if (rc == BV_OK && o->kind == BV_RUN_CALLS) {
+            if (!aux) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_ex: null aux");
+            rc = check_device_ptr(ctx, aux->mapq, 16, "bv_tile_aux::mapq");
+            if (rc == BV_OK) rc = check_device_ptr(ctx, aux->rpr, 16, "bv_tile_aux::rpr");
+        }
+        if (rc != BV_OK) return rc;
+    }
+    // the tile's shape, before anything is allocated or queued (fill_kernel_args / set_call_args check the same again)
+    if (tile->pitch % 16 != 0 || tile->pitch < tile->n_samples || tile->n_samples > ctx->prm.max_samples)
+        return set_err(ctx, BV_ERR_ARG, "bv_tile: pitch %llu must be a multiple of 16 and >= n_samples %u <= max_samples %u",
+                       (unsigned long long)tile->pitch, tile->n_samples, ctx->prm.max_samples);
+    if (tile->n_sites > kMaxTileSites) return set_err(ctx, BV_ERR_ARG, "bv_tile: more than 2^22 sites in one tile");
+    if (tile->n_sites && o->kind == BV_RUN_CALLS && (aux->rpr_pitch % 8 != 0 || aux->rpr_pitch < tile->n_samples))
+        return set_err(ctx, BV_ERR_ARG, "bv_tile_aux: rpr_pitch %llu must be a multiple of 8 and >= n_samples %u",
+                       (unsigned long long)aux->rpr_pitch, tile->n_samples);
+    if (tile->n_sites == 0) return zero_device_counts(ctx, o, st);
+    bv_site_out* rec = nullptr;
+    rc = device_records(ctx, o, tile->n_sites, &rec);
+    if (rc != BV_OK) return rc;
+    bv::SiteKernelArgs a;
+    rc = fill_kernel_args(ctx, tile, rec, ctx->dev_scratch, &a);
+    if (rc == BV_OK && o->kind == BV_RUN_CALLS) rc = set_call_args(ctx, tile, aux, ctx->dev_scratch, o->d_calls, o->d_groups, &a);
+    if (rc != BV_OK) return rc;
+    BV_CUDA(ctx, cudaMemsetAsync(a.counters, 0, bv::kNumCounters * sizeof(uint32_t), st));
+    return run_device_tail(ctx, a, o, st);
+}
+
+int bv_tile_run_device_sparse(bv_ctx* ctx, const bv_sparse_tile* t, const bv_device_out* o, void* stream) {
+    BvRange range("bv_tile_run_device_sparse (K0 expand from device memory, kernels)");
+    if (!ctx) return set_err(nullptr, BV_ERR_ARG, "null context");
+    if (!t) return set_err(ctx, BV_ERR_ARG, "null tile");
+    if (t->n_sites > ctx->prm.max_sites) return set_err(ctx, BV_ERR_ARG, "tile has %u sites > max_sites %u", t->n_sites, ctx->prm.max_sites);
+    if (t->n_samples > ctx->prm.max_samples || t->n_samples > BV_CELL_MAX_SAMPLES)
+        return set_err(ctx, BV_ERR_ARG, "sparse tile: n_samples %u > max_samples %u or > %u", t->n_samples, ctx->prm.max_samples, BV_CELL_MAX_SAMPLES);
+    if (t->n_sites > kMaxTileSites) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: more than 2^22 sites in one tile");
+    if (t->format != BV_CELLS_U32 && t->format != BV_CELLS_U16) return set_err(ctx, BV_ERR_ARG, "bv_sparse_tile: unknown format %u", t->format);
+    if (t->out) return set_err(ctx, BV_ERR_ARG, "bv_tile_run_device_sparse: `out` must be NULL (bv_device_out names the results)");
+    BV_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = check_device_out(ctx, o, t->n_sites);
+    if (rc != BV_OK) return rc;
+    const bool u16 = t->format == BV_CELLS_U16;
+    const bool with_calls = o->kind == BV_RUN_CALLS;
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (t->n_sites == 0) return zero_device_counts(ctx, o, st);
+    rc = check_device_ptr(ctx, t->site_start, 4, "bv_sparse_tile::site_start");
+    if (rc == BV_OK) rc = check_device_ptr(ctx, t->ref_base, 1, "bv_sparse_tile::ref_base");
+    if (rc == BV_OK && t->n_samples) rc = check_device_ptr(ctx, t->cells, u16 ? 2 : 4, "bv_sparse_tile::cells");
+    if (rc == BV_OK && t->n_samples && with_calls) rc = check_device_ptr(ctx, t->cells_aux, 4, "bv_sparse_tile::cells_aux");
+    if (rc != BV_OK) return rc;
+    // the planes K0 writes: on the first call, sized like a slot's
+    const size_t plane = (size_t)ctx->prm.max_sites * ctx->pitch_cap;
+    if (!ctx->d_dev_planes) BV_CUDA(ctx, cudaMalloc(&ctx->d_dev_planes, 3 * plane));
+    if (with_calls && !ctx->d_dev_aux) BV_CUDA(ctx, cudaMalloc(&ctx->d_dev_aux, 3 * plane));
+    bv_site_out* rec = nullptr;
+    rc = device_records(ctx, o, t->n_sites, &rec);
+    if (rc != BV_OK) return rc;
+    const uint64_t dp = ((uint64_t)t->n_samples + 15) / 16 * 16;
+    bv_tile dev;
+    dev.base = ctx->d_dev_planes; dev.qual = ctx->d_dev_planes + plane; dev.strand = ctx->d_dev_planes + 2 * plane; dev.ref_base = t->ref_base;
+    dev.pitch = dp; dev.n_sites = t->n_sites; dev.n_samples = t->n_samples; dev.location = BV_LOC_DEVICE; dev.out_mode = BV_OUT_RECORDS;
+    bv::SiteKernelArgs a;
+    rc = fill_kernel_args(ctx, &dev, rec, ctx->dev_scratch, &a);
+    if (rc == BV_OK && with_calls) {
+        bv_tile_aux dev_aux;
+        dev_aux.mapq = ctx->d_dev_aux; dev_aux.rpr = reinterpret_cast<const uint16_t*>(ctx->d_dev_aux + plane); dev_aux.rpr_pitch = dp;
+        rc = set_call_args(ctx, &dev, &dev_aux, ctx->dev_scratch, o->d_calls, o->d_groups, &a);
+    }
+    if (rc != BV_OK) return rc;
+    BV_CUDA(ctx, cudaMemsetAsync(a.counters, 0, bv::kNumCounters * sizeof(uint32_t), st));
+    if (t->n_samples) {
+        // K0 straight from the caller's cells.  Their count, site_start[n_sites], is in device memory: K0 is given the most
+        // cells a well-formed tile of this shape can have, and checks every site's offsets against each other and that bound.
+        bv::ExpandArgs x;
+        x.cells = t->cells; x.cells_aux = with_calls ? t->cells_aux : nullptr; x.site_start = t->site_start;
+        x.base = ctx->d_dev_planes; x.qual = ctx->d_dev_planes + plane; x.strand = ctx->d_dev_planes + 2 * plane;
+        x.mapq = with_calls ? ctx->d_dev_aux : nullptr;
+        x.rpr = with_calls ? reinterpret_cast<uint16_t*>(ctx->d_dev_aux + plane) : nullptr;
+        x.counters = a.counters;
+        x.pitch = dp; x.rpr_pitch = dp;
+        x.n_cells = (uint64_t)t->n_sites * ((uint64_t)t->n_samples + (u16 ? t->n_samples / BV_CELL16_GAP_SKIP + 2u : 0u));
+        x.n_sites = t->n_sites; x.n_samples = t->n_samples;
+        rc = launch_expand(ctx, x, u16, st);
+        if (rc != BV_OK) return rc;
+    }
+    return run_device_tail(ctx, a, o, st);
 }
 
 uint64_t bv_sparse_encode16_bound(uint64_t n_cells, uint32_t n_sites, uint32_t n_samples) {

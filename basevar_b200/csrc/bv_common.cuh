@@ -4,7 +4,8 @@
 // every kernel is small and all of its warps execute the same code (one fused kernel was measured instruction-cache bound:
 // 59 % of its stall samples were "no instruction" with 24 warps per SM spread over 76 KB of code):
 //
-//   K0  bv_expand_kernel  (bv_expand_kernel.cuh)   sparse host tiles only: the covered cells -> the dense planes in HBM.
+//   K0  bv_expand_kernel  (bv_expand_kernel.cuh)   sparse tiles only (host or device resident): the covered cells -> the dense
+//        planes in HBM.
 //   K1  bv_count_kernel   (bv_count_kernel.cuh)    every site, every cell: streams the base + strand planes through
 //        per-warp TMA rings and counts -- per-base depths and the 2x4 strand table.  Sites whose reads all equal REF get
 //        their final record here; the others get their counts and the state BV_STATE_SCALAR.
@@ -54,7 +55,8 @@ constexpr uint32_t kStateScalar = 1;         // counts are final, K2 has to fini
 constexpr uint32_t kStateBound = 2;          // result depends on base qualities; K3 tries the likelihood-ratio bound
 constexpr uint32_t kStateEM = 3;             // result depends on base qualities; K4 runs EM + LRT
 
-constexpr int kCntSlow = 0, kCntBound = 1, kCntEm = 2;                    // SiteKernelArgs::counters (3 and 10 are unused)
+constexpr int kCntSlow = 0, kCntBound = 1, kCntEm = 2;                    // SiteKernelArgs::counters (10 is unused)
+constexpr int kCntListPairs = 3;                                          // chunk ticket of bv_list_pairs_kernel (bv_list_kernel.cuh)
 constexpr int kCntCalled = 4, kCntGroupNext = 5;                          // called sites (K4 -> K5, K6)
 constexpr int kCntBadCell = 6;                                            // malformed sparse input (K0, bv_expand_kernel.cuh)
 constexpr int kCntEmHdr = 7, kCntEmPool = 8;                              // K4a -> K4b: EM sites and the pool of their bins
@@ -117,7 +119,8 @@ struct SiteKernelArgs {
     uint32_t em_resume;      // bv_em_task_kernel: the EM iterations were run by bv_em_iter_kernel, start from its frequencies
     uint32_t em_task_split;  // tiles with more EM tasks than this run bv_em_task_kernel<kTaskHiCtas>, the others <kTaskLoCtas>
     uint2* brief;            // [n_sites] device copy of the briefs: K1 writes them, bv_pack_kernel completes them
-    bv_site_out* full_out;   // pinned host memory (mapped): the full records, written by bv_pack_kernel
+    bv_site_out* full_out;   // the full records, written by bv_pack_kernel: pinned host memory (mapped) of a slot, or the device
+                             // buffer of a device-resident tile (bv_device_out::d_full)
     // called sites (n_alt > 0): rank sums (K5) and population-group frequencies (K6); all null / 0 when not asked for
     uint32_t* list_called;   // K4 -> K5, K6: site indices, room for n_sites entries
     const uint8_t* mapq;     // [n_sites][aux_pitch]

@@ -268,8 +268,9 @@ __global__ void __launch_bounds__(128) bv_fs_kernel(const int4* __restrict__ tab
 
 // =====================================================================================================================
 // K7 bv_pack_kernel (BV_OUT_COMPACT tiles, after everything else): the sites K1 could not finish from their counts get their
-// full record copied into the pinned host list -- the kernel writes across PCIe itself, 8 lanes per 128-byte record, the
-// records of a warp's sites next to each other -- and their brief becomes the record's index in that list.
+// full record copied into the list at a.full_out -- for a host tile the slot's mapped pinned staging, which the kernel writes across
+// PCIe itself; for a device-resident tile the caller's device buffer -- 8 lanes per 128-byte record, the records of a warp's sites
+// next to each other, and their brief becomes the record's index in that list.
 // =====================================================================================================================
 __global__ void __launch_bounds__(256) bv_pack_kernel(const __grid_constant__ SiteKernelArgs a) {
     const int lane = threadIdx.x & 31;

@@ -169,4 +169,88 @@ __global__ void __launch_bounds__(kQualWarps * 32, 1) bv_list_packed_kernel(cons
     }
 }
 
+// The same over the packed list of a device-resident tile (bv_list_pairs_kernel built it): the number of pairs is in device memory
+// and the host never sees it; the grid is sized for one pair per site.  A kernel of its own, so that the host path's stays as it is.
+__global__ void __launch_bounds__(kQualWarps * 32, 1) bv_list_packed_dev_kernel(const __grid_constant__ SiteKernelArgs a,
+                                                                                const uint2* __restrict__ pairs,
+                                                                                const uint32_t* __restrict__ n_pairs,
+                                                                                bv_lrt_out* __restrict__ lrt_out) {
+    list_cta_setup(a);
+    const uint32_t n = *n_pairs;
+    const uint32_t total_warps = gridDim.x * (blockDim.x >> 5);
+    for (uint32_t k = (threadIdx.x >> 5) * gridDim.x + blockIdx.x; k < n; k += total_warps) {
+        const uint2 p = __ldg(pairs + k);
+        list_site<true>(p.x, p.y, lrt_out + k);
+    }
+}
+
+// The packed list of a device-resident lists tile with compact results: {site, list word} of every site whose list is valid and
+// non-empty, in site order, and their number -- what stage_lists (bv_api.cu) builds on the host from a host tile's lists.  A list
+// that list_decode refuses counts as empty here (the host entry points refuse the tile instead; a device tile's lists are not
+// seen before this kernel runs).
+// One CTA per kListPairSites consecutive sites.  A CTA's place in the output is the sum of the counts of the chunks in front of
+// it: every CTA first publishes its own count -- tagged with the call's epoch, so that the words need no reset between calls --
+// then adds up those of its predecessors.  Chunks are handed out in the order CTAs start (a ticket, counters[kCntListPairs]),
+// so every CTA one waits for has started, and has published or is about to: no CTA waits for one that cannot run.
+// Launched chained behind KF (launch_chained): it reads nothing the step writes, so it runs while KF's last CTAs finish, and
+// waits for KF's completion at its end only so that it never completes before KF.
+constexpr int kListPairThreads = 256;
+constexpr int kListPairPerThread = 16;           // consecutive sites per thread
+constexpr uint32_t kListPairSites = (uint32_t)kListPairThreads * kListPairPerThread;
+
+__global__ void __launch_bounds__(kListPairThreads) bv_list_pairs_kernel(const uint32_t* __restrict__ lists, uint32_t n_sites,
+                                                                         uint2* __restrict__ pairs,
+                                                                         unsigned long long* __restrict__ chunk_count,
+                                                                         uint32_t epoch, uint32_t* __restrict__ counters,
+                                                                         uint32_t* __restrict__ n_pairs) {
+    __shared__ uint32_t s_chunk, s_warp[kListPairThreads / 32], s_pred[kListPairThreads / 32];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (threadIdx.x == 0) s_chunk = atomicAdd(counters + kCntListPairs, 1u);
+    __syncthreads();
+    const uint32_t chunk = s_chunk;
+    const uint32_t s0 = chunk * kListPairSites + (uint32_t)threadIdx.x * kListPairPerThread;
+    uint32_t w[kListPairPerThread], keep = 0;
+#pragma unroll
+    for (int k = 0; k < kListPairPerThread; ++k) {
+        uint32_t order;
+        w[k] = s0 + k < n_sites ? __ldg(lists + s0 + k) : 0xffffffffu;
+        if (list_decode(w[k], order) > 0) keep |= 1u << k;
+    }
+    // exclusive scan of the per-thread counts over the CTA
+    const uint32_t cnt = (uint32_t)__popc(keep);
+    uint32_t x = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t y = __shfl_up_sync(kFull, x, o);
+        if (lane >= o) x += y;
+    }
+    if (lane == 31) s_warp[wid] = x;
+    __syncthreads();
+    uint32_t before = x - cnt, total = 0;
+    for (int j = 0; j < kListPairThreads / 32; ++j) {
+        const uint32_t v = s_warp[j];
+        if (j < wid) before += v;
+        total += v;
+    }
+    if (threadIdx.x == 0) atomicExch(chunk_count + chunk, ((unsigned long long)epoch << 32) | total);   // publish
+    // the counts of the chunks in front of this one (each thread adds up a strided share, spinning until it is published)
+    uint32_t pred = 0;
+    for (uint32_t j = threadIdx.x; j < chunk; j += kListPairThreads) {
+        unsigned long long v;
+        do { v = atomicAdd(chunk_count + j, 0ull); } while ((uint32_t)(v >> 32) != epoch);   // (an atomic read: from L2)
+        pred += (uint32_t)v;
+    }
+    pred = __reduce_add_sync(kFull, pred);
+    if (lane == 0) s_pred[wid] = pred;
+    __syncthreads();
+    uint32_t base = 0;
+    for (int j = 0; j < kListPairThreads / 32; ++j) base += s_pred[j];
+    uint32_t pos = base + before;
+#pragma unroll
+    for (int k = 0; k < kListPairPerThread; ++k)
+        if (keep >> k & 1u) pairs[pos++] = make_uint2(s0 + k, w[k]);
+    if (chunk == gridDim.x - 1 && threadIdx.x == 0) *n_pairs = base + total;
+    grid_dep_wait();
+}
+
 }  // namespace bv

@@ -420,6 +420,102 @@ class BaseTypeEngine:
         self._check(self.lib.bv_tile_run_device(self._ctx, C.byref(t), C.c_void_p(int(d_out)),
                                                 C.c_void_p(int(stream))), "bv_tile_run_device")
 
+    # -- pileups held in device memory: every result form, into torch CUDA tensors -------------------------
+    def call_device_sparse(self, cells, site_start, ref_base, n_samples, cells_aux=None, lists=None, calls=False, compact=False,
+                           out=None):
+        """One sparse tile whose cells are torch CUDA tensors (bv_tile_run_device_sparse): cells int32/uint32 BV_CELL_PACK words
+        or int16/uint16 BV_CELLS_U16 words (the element size picks the format), site_start int32 [S + 1], ref_base uint8 [S],
+        cells_aux int32 [like cells] with calls=True, lists uint8 [S][4] for lrt(list) per site.  K0 expands the cells where they
+        are; nothing crosses PCIe.  Runs on torch.cuda.current_stream() and returns at once: a DeviceResult of tensors, newly
+        allocated, or `out` (a DeviceResult of device_result() of the same shape and form) filled again."""
+        import torch
+        S = int(ref_base.shape[0])
+        assert site_start.shape[0] == S + 1 and cells.element_size() in (2, 4)
+        fmt = capi.CELLS_U16 if cells.element_size() == 2 else capi.CELLS_U32
+        if cells.numel() == 0:   # (a tile without cells still names a cell array)
+            cells = torch.zeros(1, dtype=cells.dtype, device=ref_base.device)
+        if calls and cells_aux is not None and cells_aux.numel() == 0:
+            cells_aux = torch.zeros(1, dtype=torch.int32, device=ref_base.device)
+        t = BvSparseTile(cells.data_ptr(), cells_aux.data_ptr() if cells_aux is not None else None, site_start.data_ptr(),
+                         ref_base.data_ptr(), None, S, n_samples, fmt, 0)
+        res, o = self._device_out(S, ref_base.device, lists, calls, compact, out)
+        self._check(self.lib.bv_tile_run_device_sparse(self._ctx, C.byref(t), C.byref(o), C.c_void_p(self._torch_stream())),
+                    "bv_tile_run_device_sparse")
+        return res._issued((cells, cells_aux, site_start, ref_base, lists))
+
+    def call_device_dense(self, base, qual, strand, ref_base, n_samples, mapq=None, rpr=None, lists=None, calls=False, compact=False,
+                          out=None):
+        """The dense twin of call_device_sparse (bv_tile_run_device_ex): planes uint8 CUDA tensors [S][pitch] (pitch a multiple of
+        16), with calls=True mapq uint8 [S][pitch] and rpr int16/uint16 [S][rpr_pitch] (a multiple of 8)."""
+        S, pitch = base.shape
+        t = BvTile(base.data_ptr(), qual.data_ptr(), strand.data_ptr(), ref_base.data_ptr(), pitch, S, n_samples, capi.BV_LOC_DEVICE, 0)
+        aux = BvTileAux(mapq.data_ptr(), rpr.data_ptr(), rpr.shape[1]) if calls else None
+        res, o = self._device_out(S, base.device, lists, calls, compact, out)
+        self._check(self.lib.bv_tile_run_device_ex(self._ctx, C.byref(t), C.byref(aux) if aux is not None else None, C.byref(o),
+                                                   C.c_void_p(self._torch_stream())), "bv_tile_run_device_ex")
+        return res._issued((base, qual, strand, ref_base, mapq, rpr, lists))
+
+    @staticmethod
+    def _torch_stream():
+        import torch
+        return int(torch.cuda.current_stream().cuda_stream)
+
+    def device_result(self, n_sites, calls=False, lists=False, compact=False, device="cuda"):
+        """The result tensors of a device-resident tile of n_sites sites in the given form, allocated once: pass it as `out` to
+        call_device_sparse / call_device_dense to run tiles without allocating (the counts start at 0, the rest uninitialised)."""
+        import torch
+        if calls and lists:
+            raise ValueError("lists and the called-site kernels do not run in one call")
+        S = int(n_sites)
+
+        def buf(n, itemsize):
+            return torch.empty((n, itemsize), dtype=torch.uint8, device=device)
+
+        def word():
+            return torch.zeros(1, dtype=torch.int32, device=device)
+
+        r = DeviceResult(n_sites=S, compact=compact, calls=calls, lists=lists, n_groups=getattr(self, "n_groups", 0))
+        r.status = word()
+        if compact:
+            r.brief, r.full, r.n_full = buf(S, 8), buf(S, 128), word()
+        else:
+            r.records = buf(S, 128)
+        if calls:
+            r.call_out, r.n_calls = buf(S, 16), word()
+            r.groups = buf(S * r.n_groups, 40) if r.n_groups else None
+        if lists:
+            r.lrt = buf(S, 64)
+            r.n_lrt = word() if compact else None
+        return r
+
+    def _device_out(self, S, device, lists, calls, compact, out):
+        """The result tensors of a device-resident tile (`out`, or new ones) and the bv_device_out that names them."""
+        import torch
+        if calls and lists is not None:
+            raise ValueError("lists and the called-site kernels do not run in one call")
+        r = out if out is not None else self.device_result(S, calls, lists is not None, compact, device)
+        if (r.n_sites, r.calls, r.lists, r.compact) != (S, bool(calls), lists is not None, bool(compact)):
+            raise ValueError("`out` was made for another shape or form of tile")
+        if calls and r.n_groups != getattr(self, "n_groups", 0):
+            raise ValueError("`out` was made for another number of population groups")
+        o = capi.BvDeviceOut()
+        o.kind = capi.RUN_CALLS if calls else capi.RUN_LISTS if lists is not None else capi.RUN_PLAIN
+        o.out_mode = capi.OUT_COMPACT if compact else capi.OUT_RECORDS
+        o.d_status = r.status.data_ptr()
+        if compact:
+            o.d_brief, o.d_full, o.d_n_full = r.brief.data_ptr(), r.full.data_ptr(), r.n_full.data_ptr()
+        else:
+            o.d_out = r.records.data_ptr()
+        if calls:
+            o.d_calls, o.d_n_calls = r.call_out.data_ptr(), r.n_calls.data_ptr()
+            o.d_groups = r.groups.data_ptr() if r.groups is not None else None
+        if lists is not None:
+            assert lists.dtype == torch.uint8 and tuple(lists.shape) == (S, 4) and lists.is_contiguous()
+            o.d_lists, o.d_lrt = lists.data_ptr(), r.lrt.data_ptr()
+            if compact:
+                o.d_n_lrt = r.n_lrt.data_ptr()
+        return r, o
+
     # -- synthetic pileups -------------------------------------------------------------------------
     def synth_set_model(self, model):
         self._model = model
@@ -429,6 +525,58 @@ class BaseTypeEngine:
         self._check(self.lib.bv_synth_fill_device(self._ctx, site0, n_sites, n_samples, pitch, int(d_base), int(d_qual),
                                                   int(d_strand), int(d_mapq) if d_mapq else None, int(d_ref),
                                                   C.c_void_p(int(stream))), "bv_synth_fill_device")
+
+
+class DeviceResult:
+    """The results of one device-resident tile (call_device_sparse / call_device_dense): torch CUDA tensors of bytes, written on
+    the stream the call ran on.  records [S][128] (records mode) or brief [S][8], full [S][128] and n_full (compact mode);
+    call_out [S][16], groups [S * n_groups][40] and n_calls (calls); lrt [S][64] and, compact, n_lrt (lists); status: non-zero
+    when the cells were malformed.  to_numpy() copies them to the host, cut to their counts, as the numpy dtypes of capi."""
+
+    def __init__(self, **kw):
+        self.records = self.brief = self.full = self.n_full = None
+        self.call_out = self.groups = self.n_calls = self.lrt = self.n_lrt = None
+        self.done = None
+        self.__dict__.update(kw)
+
+    def _issued(self, inputs):
+        """The call was queued on the current stream: remember where it ends, and keep its inputs alive with the results."""
+        import torch
+        self.done = torch.cuda.Event()
+        self.done.record(torch.cuda.current_stream())
+        self._keep = inputs
+        return self
+
+    def to_numpy(self):
+        """dict of numpy arrays: records (SITE_OUT_DTYPE) or brief (SITE_BRIEF_DTYPE) + full, calls (CALL_OUT_DTYPE) + groups
+        (GROUP_OUT_DTYPE), lrt (LRT_OUT_DTYPE), status (int).  The copies run on the current stream, after the call's end on the
+        stream it ran on (an event), and wait for it."""
+        import torch
+        if self.done is not None:
+            torch.cuda.current_stream().wait_event(self.done)
+        status = device_to_numpy(self.status, np.uint32)[0]
+        r = {"status": int(status)}
+        if self.compact:
+            r["brief"] = device_to_numpy(self.brief, capi.SITE_BRIEF_DTYPE)
+            r["full"] = device_to_numpy(self.full, SITE_OUT_DTYPE, int(device_to_numpy(self.n_full, np.uint32)[0]))
+        else:
+            r["records"] = device_to_numpy(self.records, SITE_OUT_DTYPE)
+        if self.calls:
+            nc = int(device_to_numpy(self.n_calls, np.uint32)[0])
+            r["calls"] = device_to_numpy(self.call_out, CALL_OUT_DTYPE, nc)
+            r["groups"] = device_to_numpy(self.groups, GROUP_OUT_DTYPE, nc * self.n_groups) if self.n_groups else None
+        if self.lists:
+            n = int(device_to_numpy(self.n_lrt, np.uint32)[0]) if self.compact else self.n_sites
+            r["lrt"] = device_to_numpy(self.lrt, LRT_OUT_DTYPE, n)
+        return r
+
+
+def device_to_numpy(t, dtype, n=None):
+    """A host copy of the bytes of torch tensor `t` viewed as numpy `dtype` (SITE_OUT_DTYPE, CALL_OUT_DTYPE, ...), its first n
+    entries.  The copy runs on the current stream and waits for it."""
+    import torch
+    a = t.detach().contiguous().reshape(-1).view(torch.uint8).cpu().numpy().view(dtype)
+    return a[:n] if n is not None else a
 
 
 def synth_fill_rpr_host(model, site0, n_sites, n_samples):

@@ -329,6 +329,12 @@ const bv_group_out* TileResult::group(uint32_t site, uint32_t g) const {
     return &groups[(size_t)(c - calls.data()) * n_groups + g];
 }
 
+void Context::run_device(const bv_sparse_tile& tile, const DeviceResult& out, void* stream) {
+    check(bv_tile_run_device_sparse(ctx_, &tile, &out, stream), ctx_, "bv_tile_run_device_sparse");
+}
+void Context::run_device(const bv_tile& tile, const DeviceResult& out, void* stream, const bv_tile_aux* aux) {
+    check(bv_tile_run_device_ex(ctx_, &tile, aux, &out, stream), ctx_, "bv_tile_run_device_ex");
+}
 uint64_t Context::launch_count() const { return bv_launch_count(ctx_); }
 double Context::fisher_fs(int ref_fwd, int ref_rev, int alt_fwd, int alt_rev) {
     const int32_t t[4] = {ref_fwd, ref_rev, alt_fwd, alt_rev};

@@ -173,6 +173,17 @@ struct TileResult {
     const bv_group_out* group(uint32_t site, uint32_t g) const;   // null when the site is not called
 };
 
+// ---- results of a device-resident tile ---------------------------------------------------------------------------------
+// The device buffers of one tile whose pileup is already in GPU memory (Context::run_device): the fields of bv_device_out
+// (include/basevar_b200.h), all null but kind / out_mode until set.  The caller owns the buffers (cudaMalloc or any device
+// allocator); the mirror never touches device memory itself.
+struct DeviceResult : bv_device_out {
+    explicit DeviceResult(int kind_ = BV_RUN_PLAIN, int out_mode_ = BV_OUT_RECORDS) : bv_device_out() {
+        kind = kind_;
+        out_mode = out_mode_;
+    }
+};
+
 // ---- a context bound to one GPU ---------------------------------------------------------------------------------------
 class Context {
 public:
@@ -203,6 +214,11 @@ public:
     void submit_calls(int slot, const bv_tile& tile, const bv_tile_aux& aux);
     void submit_calls(int slot, const bv_sparse_tile& tile);
     TileResult wait_calls(int slot);   // records or compact view, `calls` and `groups`
+    // A pileup already in GPU memory: sparse cells (bv_tile_run_device_sparse) or dense planes (bv_tile_run_device_ex, with the
+    // mapq / rpr planes in `aux` for BV_RUN_CALLS), every result into the device buffers `out` names.  `stream` is a
+    // cudaStream_t; stream ordered, returns at once.  Throws std::runtime_error when the call is refused (nothing is queued then).
+    void run_device(const bv_sparse_tile& tile, const DeviceResult& out, void* stream = nullptr);
+    void run_device(const bv_tile& tile, const DeviceResult& out, void* stream = nullptr, const bv_tile_aux* aux = nullptr);
     uint32_t n_slots() const { return n_slots_; }
     uint64_t launch_count() const;
     bv_ctx* raw() { return ctx_; }

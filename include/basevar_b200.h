@@ -33,6 +33,9 @@
  *   lrt([REF, ALT...]) at called sites  src/basetype_caller.cpp:747-760   bv_tile_submit_sparse_lists (K8 on the expanded planes);
  *     of a sparse tile                                                    with BV_OUT_COMPACT one packed entry per listed site,
  *                                                                         bv_tile_wait_lists_compact
+ *   any of the above for a pileup that                                    bv_tile_run_device_sparse (cells in device memory) /
+ *     is already in device memory                                         bv_tile_run_device_ex (dense planes), results of every
+ *                                                                         form into device buffers named by bv_device_out
  *
  * Everything is `extern "C"`, plain pointers and sizes, POD structs; no exception crosses the
  * boundary.  Every entry point returns BV_OK (0) or a negative status; bv_last_error() gives text.
@@ -128,9 +131,10 @@ typedef struct bv_tile {
     int32_t  location;       /* BV_LOC_HOST (pinned or pageable) or BV_LOC_DEVICE                         */
     int32_t  out_mode;       /* BV_OUT_RECORDS, or BV_OUT_COMPACT (host tiles; collect with bv_tile_wait_compact) */
 } bv_tile;
-/* Device-resident tiles have no compact form.  bv_tile_submit_calls (device tile), bv_tile_run_device_calls and
- * bv_tile_run_device_lists refuse out_mode BV_OUT_COMPACT with BV_ERR_ARG; bv_tile_run_device, and bv_tile_submit of a device
- * tile, do not read out_mode and return records. */
+/* bv_tile_submit_calls (device tile), bv_tile_run_device_calls and bv_tile_run_device_lists refuse out_mode BV_OUT_COMPACT with
+ * BV_ERR_ARG; bv_tile_run_device, and bv_tile_submit of a device tile, do not read out_mode and return records.  The compact
+ * form of a device-resident tile is asked for through bv_device_out (bv_tile_run_device_ex, bv_tile_run_device_sparse), which
+ * ignores bv_tile::out_mode. */
 
 /* ---- per-site result record: fixed 128 bytes --------------------------------------------------- */
 typedef struct bv_site_out {
@@ -372,7 +376,7 @@ int bv_set_groups(bv_ctx* ctx, const uint8_t* sample_group, uint32_t n_samples, 
 /* bv_tile_submit + the kernels of the called sites.  `aux` planes live where the tile lives (host or device);
  * pageable host planes are uploaded whole, pinned ones are read in place for the called rows only.  Host tiles may ask for
  * BV_OUT_COMPACT (collect with bv_tile_wait_calls_compact); a device-resident tile that asks for it is refused (BV_ERR_ARG):
- * there is no device-resident compact form. */
+ * the compact form of a device-resident tile goes through bv_device_out (bv_tile_run_device_ex). */
 int bv_tile_submit_calls(bv_ctx* ctx, int slot, const bv_tile* tile, const bv_tile_aux* aux);
 /* Blocks; `out` receives n_sites records, `calls` up to max_calls entries, `groups` (may be NULL when no groups are
  * set) n_groups entries per call, groups[k * n_groups + g] belonging to calls[k].  *n_calls = number of called sites
@@ -401,9 +405,59 @@ int bv_tile_submit_lists(bv_ctx* ctx, int slot, const bv_tile* tile, const uint8
 int bv_tile_wait_lists(bv_ctx* ctx, int slot, bv_site_out* out, bv_lrt_out* lrt_out);
 /* Device-resident variant: tile planes, d_lists [n_sites][4] (4-byte aligned), d_out and d_lrt_out are device pointers.
  * Stream ordered, so the lists are not seen before the kernel runs: a list the host entry points would refuse is treated
- * as an empty one here (all-zero entry).  out_mode must be BV_OUT_RECORDS (there is no device-resident compact form). */
+ * as an empty one here (all-zero entry).  out_mode must be BV_OUT_RECORDS (compact lists of a device-resident tile: bv_device_out). */
 int bv_tile_run_device_lists(bv_ctx* ctx, const bv_tile* tile, const uint8_t (*d_lists)[4], bv_site_out* d_out,
                              bv_lrt_out* d_lrt_out, void* stream);
+
+/* ---- pileups on the device: every form of a host tile, nothing crosses PCIe ------------------------------------------------ */
+/* A pileup built on the GPU (a generator, a torch pipeline, a pileup builder on the device) runs through the same kernels as a
+ * host tile, and its results of every form land in device buffers: bv_device_out names them.  Every pointer in it is a device
+ * pointer; which of them must be set follows from `kind` and `out_mode`, the others are not read:
+ *   BV_OUT_RECORDS  d_out [n_sites] records (bytes bv_tile_wait gives);
+ *   BV_OUT_COMPACT  d_brief [n_sites] briefs, d_full with room for n_sites records, *d_n_full = the records it received: the
+ *                   bytes bv_tile_wait_compact gives (a brief's index points into d_full; bv_site_expand rebuilds the others);
+ *   BV_RUN_CALLS    d_calls [n_sites], d_groups [n_sites * n_groups] (when groups are set), *d_n_calls: as bv_tile_wait_calls
+ *                   gives them (in no particular order; bv_call_out::site names the row);
+ *   BV_RUN_LISTS    d_lists [n_sites][4] (4-byte aligned) and d_lrt [n_sites]: one entry per site in records mode; in compact mode
+ *                   one entry per site whose list is non-empty, packed in site order, *d_n_lrt = their number (d_n_lrt is not
+ *                   written in records mode).  A list the host entry points would refuse (a repeated base, a code that is neither
+ *                   BV_BASE_A..T nor BV_LIST_END) is treated as an empty one: the kernels see the lists, the host does not.
+ *   d_status        (optional) one word: 0, or non-zero when the cells of a sparse tile are malformed (a sample >= n_samples,
+ *                   offsets that descend) -- what makes bv_tile_wait fail with BV_ERR_ARG for a host tile.  Nothing waits here,
+ *                   so the caller reads this word; the results of such a tile are undefined, the context stays usable.
+ * Lists and the called-site kernels do not run in one call, as on the host (there is no kind for both). */
+#define BV_RUN_PLAIN 0
+#define BV_RUN_CALLS 1
+#define BV_RUN_LISTS 2
+typedef struct bv_device_out {
+    int32_t        kind;       /* BV_RUN_PLAIN, BV_RUN_CALLS or BV_RUN_LISTS (the three host submits)                   */
+    int32_t        out_mode;   /* BV_OUT_RECORDS or BV_OUT_COMPACT                                                       */
+    bv_site_out*   d_out;      /* records mode                                                                           */
+    bv_site_brief* d_brief;    /* compact mode                                                                           */
+    bv_site_out*   d_full;
+    uint32_t*      d_n_full;
+    bv_call_out*   d_calls;    /* BV_RUN_CALLS                                                                           */
+    bv_group_out*  d_groups;
+    uint32_t*      d_n_calls;
+    const uint8_t (*d_lists)[4];   /* BV_RUN_LISTS                                                                       */
+    bv_lrt_out*    d_lrt;
+    uint32_t*      d_n_lrt;
+    uint32_t*      d_status;
+} bv_device_out;
+
+/* A sparse tile whose cells, cells_aux (BV_RUN_CALLS), site_start and ref_base are device pointers: K0 expands the cells straight
+ * from them into planes of the context (max_sites x round16(max_samples) x 3 bytes, allocated by the first such call), then the
+ * kernels of bv_tile_submit_sparse / _calls / _lists run.  Either cell format; tile->out must be NULL.  `stream` is a
+ * cudaStream_t (NULL = the legacy default stream); stream ordered, returns at once.  BV_ERR_ARG, before anything is queued:
+ * n_sites > max_sites, n_samples > max_samples, a null or misaligned pointer, a host pointer where a device one is due.  The
+ * offsets in site_start cannot be read before K0 runs: every one of them must lie within the words `cells` holds (those that
+ * descend within it are reported through d_status). */
+int bv_tile_run_device_sparse(bv_ctx* ctx, const bv_sparse_tile* t, const bv_device_out* out, void* stream);
+/* The same for a dense device-resident tile (bv_tile::location BV_LOC_DEVICE; bv_tile::out_mode is not read, `out` decides).
+ * aux: the mapq / rpr device planes for BV_RUN_CALLS, else NULL. */
+int bv_tile_run_device_ex(bv_ctx* ctx, const bv_tile* tile, const bv_tile_aux* aux, const bv_device_out* out, void* stream);
+/* All device-resident entry points of a context (bv_tile_run_device*) share its device scratch: calls of one context on different
+ * streams must not overlap (order them with an event, or use one context per stream). */
 
 /* ---- synthetic pileups --------------------------------------------------------------------------- */
 int bv_synth_set_model(bv_ctx* ctx, const bv_synth_model* model);
